@@ -30,6 +30,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from untouched (it may be read-only)
 
 TAU = 0.05
 KNN_CAP = 0.25  # radius cap of the k-NN mode (gm_set_knn_max_radius): isolated outliers do not drag the search across the grid
@@ -54,6 +55,8 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-points", type=int, default=0, help="points of the CPU baseline sample (0 = full scan)")
     ap.add_argument("--knn", type=int, default=0, help="k-nearest-neighbour normals with this k instead of the radius search (0 = radius)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline leg computed to DIR/<name>.npy (rank 0)")
     return ap.parse_args()
 
 
@@ -271,6 +274,55 @@ def load_peaks():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def scan_outputs(cx):
+    """What a caller of process_scan receives for one scan, as float32 / float64 arrays (integers are exact in float64)."""
+    from geometric_mapping_b200 import capi
+
+    c = cx.counts()
+    fr = cx.frame()
+    out = {"counts": np.array([getattr(c, f) for f, _ in c._fields_], np.float64),
+           "frame_vals": fr["vals"], "frame_vecs": fr["vecs"]}
+    for kind, name in ((capi.GM_MODEL_PLANE, "plane"), (capi.GM_MODEL_CYLINDER, "cylinder")):
+        m = cx.model(kind)
+        out[f"{name}_coef"] = m["coef"]
+        out[f"{name}_fit"] = np.array([m["best_id"], m["best_count"], m["refit_count"], m["rms"]], np.float64)
+    out["cloud"] = cx.download_cloud(1)
+    out["normals"] = cx.download_normals(1)
+    out["labels"] = cx.download_labels().astype(np.float32)
+    v = cx.download_voxels(with_nn=True)
+    # a 1-NN index outside the compacted cloud (nn_index_mode 0, counted in nn_out_of_range) has no normal: the library
+    # returns NaN there, the dump zeros; voxel_nn_index tells those rows apart
+    has_normal = (v["nn_index"] >= 0) & (v["nn_index"] < c.n_valid)
+    out["voxel_centroids"] = v["centroids"]
+    out["voxel_nn_index"] = v["nn_index"].astype(np.float64)
+    out["voxel_nn_normals"] = np.where(has_normal[:, None], v["nn_normal"], np.float32(0))
+    pl = cx.download_polyline()
+    out["polyline"] = np.concatenate([pl["center"], pl["dir"]] + [pl[k][:, None] for k in ("radius", "rms", "t_mid", "count")],
+                                     axis=1).astype(np.float64)
+    return out
+
+
+def dump_outputs(outs: dict, path: str):
+    """DIR/<name>.npy for every array, DUMP_LIMIT bytes in all: when the arrays are larger, every array of more than 4096
+    rows keeps the same share of its rows, a fixed seeded sample in row order, so two runs keep the same rows."""
+    bad = [name for name, a in outs.items() if not np.isfinite(a).all()]
+    if bad:
+        raise SystemExit(f"bench.py: non-finite values in the outputs {bad}")
+    limit = DUMP_LIMIT - 256 * len(outs)   # room for the .npy headers
+    total = sum(a.nbytes for a in outs.values())
+    big = sum(a.nbytes for a in outs.values() if len(a) > 4096)
+    keep = 1.0 if total <= limit else max(0.0, (limit - (total - big)) / big)
+    os.makedirs(path, exist_ok=True)
+    for name, a in outs.items():
+        if keep < 1.0 and len(a) > 4096:
+            rows = np.random.default_rng(0).choice(len(a), int(len(a) * keep), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 _REAL_STDOUT = None
 
 
@@ -425,6 +477,8 @@ def main():
     for cx in tctx:
         if cx.counts().device_error:
             raise SystemExit("device-side error flag set")
+    if a.dump_outputs and rank == 0:
+        dump_outputs(scan_outputs(tctx[(a.steps - 1) % NFLIGHT]), a.dump_outputs)   # the legs below reuse these contexts
     c = ctx.counts()
     value = world * n * a.steps / (ms * 1e-3)
     # the same throughput measurement at the north-star's hypothesis count (2048 plane + 2048 cylinder)

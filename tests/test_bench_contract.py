@@ -46,6 +46,33 @@ def test_reference_arm_other_ranks_print_nothing():
     assert res.returncode == 0 and res.stdout.strip() == ""
 
 
+@pytest.mark.gpu
+def test_dump_outputs_are_reproducible_and_bounded(tmp_path):
+    """--dump-outputs: two runs with the same arguments write the same finite arrays (float32 / float64, at most 64 MB in all;
+    2M points per scan is over that, so the per-point arrays are sampled)."""
+    import numpy as np
+
+    dumps = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        res = _run(["--steps", "3", "--warmup", "1", "--points", "2000000", "--map-points", "0", "--shard-hyp-large", "0",
+                    "--no-cpu-baseline", "--dump-outputs", str(d)])
+        assert res.returncode == 0, res.stderr[-3000:]
+        assert json.loads(res.stdout.strip())["steps"] == 3
+        files = sorted(os.listdir(d))
+        assert {"cloud.npy", "normals.npy", "labels.npy", "plane_coef.npy", "cylinder_coef.npy", "frame_vecs.npy"} <= set(files)
+        assert sum(os.path.getsize(d / f) for f in files) <= 64 << 20
+        dumps.append({f: np.load(d / f) for f in files})
+    a, b = dumps
+    assert a.keys() == b.keys()
+    for f in a:
+        assert a[f].dtype in (np.float32, np.float64) and np.isfinite(a[f]).all(), f
+        assert a[f].tobytes() == b[f].tobytes(), f
+    assert len(a["voxel_nn_index.npy"]) == len(a["voxel_nn_normals.npy"])
+    n_valid = int(a["counts.npy"][2])
+    assert 0 < len(a["cloud.npy"]) < n_valid and len(a["normals.npy"]) == len(a["cloud.npy"])
+
+
 def test_cuda_arm_fails_loudly_without_a_device():
     import torch
 

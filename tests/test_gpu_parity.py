@@ -627,7 +627,7 @@ def test_strided_upload_and_results_are_reproducible():
     assert a[4].tobytes() == b[4].tobytes() and np.array_equal(a[5], b[5])
 
 
-def test_cpp_host_shim_node_harness_runs_cloud_cb():
+def test_cpp_host_shim_node_harness_runs_cloud_cb(tmp_path):
     """The compiled C++ mirror of the node (geometric_mapping_b200/host) through the C-ABI."""
     import subprocess
 
@@ -635,7 +635,7 @@ def test_cpp_host_shim_node_harness_runs_cloud_cb():
 
     exe = gm_build.build_host()
     pts = synth.straight_cylinder(50_000, seed=1, noise=0.01)
-    path = "/tmp/gm_scan_test.f32x4"
+    path = str(tmp_path / "scan.f32x4")
     pts.tofile(path)
     res = subprocess.run([exe, "--set", "neighborRadius=0.2", "--set", "voxelGridLeafSize=0.5", "--set", "displayNormals=true",
                           "--scan", path], capture_output=True, text=True, timeout=120)
@@ -1357,7 +1357,7 @@ def test_sharded_round_and_map_collectives_with_a_single_rank():
         comm.close()
 
 
-def test_cpp_host_shim_keeps_the_quirk_switches_of_the_parameters():
+def test_cpp_host_shim_keeps_the_quirk_switches_of_the_parameters(tmp_path):
     """The per-call parameters of the seam (bound, radius, leaf, wf) are written into the context read-modify-write: the
     quirk switches installed with useParameters() survive them (a thread-local all-defaults cache used to reset them)."""
     import subprocess
@@ -1366,7 +1366,7 @@ def test_cpp_host_shim_keeps_the_quirk_switches_of_the_parameters():
 
     exe = gm_build.build_host()
     pts = synth.straight_cylinder(40_000, seed=3, noise=0.01)
-    path = "/tmp/gm_scan_quirk.f32x4"
+    path = str(tmp_path / "scan.f32x4")
     pts.tofile(path)
     args = [exe, "--set", "neighborRadius=0.2", "--set", "voxelGridLeafSize=0.5", "--set", "weightingFactor=0.25", "--scan", path]
     vals = {}
