@@ -47,7 +47,7 @@ struct SummaryDev {  // same layout as gm_scan_summary
 static_assert(sizeof(SummaryDev) == sizeof(gm_scan_summary), "summary layout");
 
 __global__ void k_pack_summary(const DevState* st, const FrameOut* fr, const ModelState* ms, const PolyState* ps,
-                               int have_mask, SummaryDev* out) {
+                               int held_mask, SummaryDev* out) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   out->counts.n_input = st->n_input; out->counts.n_cropped = st->n_crop; out->counts.n_valid = st->n_valid;
   out->counts.n_voxels = st->vox.n_voxels; out->counts.n_cells = st->n_cells; out->counts.voxel_overflow = st->vox.overflow;
@@ -57,15 +57,41 @@ __global__ void k_pack_summary(const DevState* st, const FrameOut* fr, const Mod
   for (int m = 0; m < 2; ++m) {
     gm_model* o = m == 0 ? &out->plane : &out->cylinder;
     const ModelState* i = ms + m;
-    const bool have = (have_mask >> m) & 1;
+    const bool have = (held_mask >> m) & 1;
     o->kind = m; o->best_id = have ? i->best_id : -1; o->best_count = have ? i->best_count : -1;
     o->refit_count = have ? i->refit_count : 0;
     for (int k = 0; k < 8; ++k) { o->hyp[k] = have ? i->hyp[k] : 0.f; o->coef[k] = have ? i->coef[k] : 0.f; }
     o->rms = have ? i->rms : 0.f; o->pad_ = 0.f;
   }
-  out->n_slices = ((have_mask >> 2) & 1) ? ps->S : 0;
+  out->n_slices = ((held_mask >> 2) & 1) ? ps->S : 0;
   out->pad_ = 0;
 }
+
+// One cudaMalloc'd array of `count` elements (at least one is allocated), freed with its owner.  Captured CUDA graphs
+// hold the raw address: alloc() may only run where a new graph generation starts or before the first capture.
+template <class T>
+struct DevBuf {
+  T* p = nullptr;
+  size_t count = 0;
+  DevBuf() = default;
+  DevBuf(DevBuf&& o) noexcept : p(o.p), count(o.count) { o.p = nullptr; o.count = 0; }
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { reset(); }
+  void reset() {
+    if (p) cudaFree(p);
+    p = nullptr;
+    count = 0;
+  }
+  cudaError_t alloc(size_t n) {
+    reset();
+    cudaError_t e = cudaMalloc((void**)&p, std::max<size_t>(n, 1) * sizeof(T));
+    if (e == cudaSuccess) count = n;
+    return e;
+  }
+  operator T*() const { return p; }
+  T* operator->() const { return p; }
+};
 }  // namespace
 
 struct gm_ctx {
@@ -83,84 +109,78 @@ struct gm_ctx {
   std::string err;
   int64_t launches = 0;
 
-  // scan + stage flags
+  // scan + valid stages
   size_t n_input = 0;
   const float4* d_scan = nullptr;  // points to d_in or to the caller's device buffer
-  bool have_scan = false, have_crop = false, have_normals = false, have_compacted = false, injected = false;
-  bool have_voxel = false, have_frame = false, have_labels = false, have_poly = false;
-  bool have_ransac[2] = {false, false}, have_model[2] = {false, false};
+  unsigned stages = 0;             // bit set over Stage
+  bool injected = false;           // the compacted cloud came from gm_inject_compacted, not from this scan's normals
   int ransac_H[2] = {0, 0};
   GridSpec grid{};
-  bool have_grid_box = false;
+  bool grid_box_set = false;
   double grid_box_min[3] = {0, 0, 0}, grid_box_max[3] = {0, 0, 0};
   OwnedRange own{-1, 0.f, 0.f};
-  bool have_vox_bbox = false;
+  bool vox_bbox_set = false;
   bool vox_bbox_is_hint = false;  // the box only bounds the lattice (dense-table sizing); the real box is computed / all-reduced on the device
   float vox_bbox[6] = {0, 0, 0, 0, 0, 0};
 
   // device buffers
-  unsigned char* d_raw = nullptr;  // PointCloud2 staging (grown on demand)
-  size_t raw_cap = 0;
-  float4 *d_in = nullptr, *d_crop = nullptr, *d_sorted = nullptr, *d_cloud_c = nullptr;
-  float4 *d_sorted_valid = nullptr, *d_leaf_bounds = nullptr;  // inputs of the tile-culled counting (written by k_normals)
+  DevBuf<unsigned char> d_raw;  // PointCloud2 staging (grown on demand)
+  DevBuf<float4> d_in, d_crop, d_sorted, d_cloud_c;
+  DevBuf<float4> d_sorted_valid, d_leaf_bounds;  // inputs of the tile-culled counting (written by k_normals)
   int count_mode = 0;  // 0 = tile-culled when the cell-sorted cloud exists, 1 = always brute force
-  float4 *d_normals = nullptr, *d_normals_c = nullptr, *d_centroid = nullptr, *d_nn_normal = nullptr;
-  unsigned *d_keys[2] = {nullptr, nullptr}, *d_vals[2] = {nullptr, nullptr};
-  unsigned* d_ucell_key = nullptr;
-  int *d_cell_id = nullptr, *d_ucell_start = nullptr, *d_nbr = nullptr, *d_valid_map = nullptr;
-  int2* d_runs = nullptr;
-  int2* d_cell_nruns = nullptr;  // per occupied cell: {number of runs, number of candidates}
-  // dense VoxelGrid tables (sort-free path): count, voxel id and 3 fixed-point sums per key
-  int *d_dense_cnt = nullptr, *d_dense_id = nullptr;
-  long long* d_dense_sum = nullptr;
-  unsigned long long* d_dense_state = nullptr;  // look-back tile states of the scan over the tables
-  size_t dense_cap = 0;
+  DevBuf<float4> d_normals, d_normals_c, d_centroid, d_nn_normal;
+  DevBuf<unsigned> d_keys[2], d_vals[2];
+  DevBuf<unsigned> d_ucell_key;
+  DevBuf<int> d_cell_id, d_ucell_start, d_nbr, d_valid_map;
+  DevBuf<int2> d_runs;
+  DevBuf<int2> d_cell_nruns;  // per occupied cell: {number of runs, number of candidates}
+  // dense VoxelGrid tables (sort-free path): count, voxel id and 3 fixed-point sums per key; the count of d_dense_cnt
+  // is the number of keys the tables hold
+  DevBuf<int> d_dense_cnt, d_dense_id;
+  DevBuf<long long> d_dense_sum;
+  DevBuf<unsigned long long> d_dense_state;  // look-back tile states of the scan over the tables
   int voxel_mode = 0;  // 0 = dense tables when the key range fits, 1 = always sort
   int normals_mode = 0;  // 0 = neighbours summed in cell-run order (fast), 1 = in FLANN's (d2, index) order (bit-identical to the oracle)
   int knn_k = 0;         // > 0: k-nearest-neighbour normals (setKSearch) instead of the radius search
   double knn_max_radius = 0.0;  // > 0: only neighbours nearer than this count (FLANN's radius + max_nn form); 0 = plain k-NN
-  int* d_knn_idx = nullptr;  // optional M x k neighbour indices of the last gm_normals (gm_set_knn(.., keep_indices = 1))
-  size_t knn_idx_cap = 0;
+  DevBuf<int> d_knn_idx;  // optional M x k neighbour indices of the last gm_normals (gm_set_knn(.., keep_indices = 1))
   bool knn_keep = false;
-  BlockEntry* d_tab = nullptr;  // dense block table of the neighbour grid (1 << (key_bits - 6) entries)
-  size_t tab_entries = 0;
-  int *d_vkey_pt = nullptr, *d_assign = nullptr, *d_vox_start = nullptr, *d_vox_key = nullptr, *d_vox_count = nullptr, *d_nn_idx = nullptr;
-  unsigned char* d_labels = nullptr;
-  unsigned long long* d_state64 = nullptr;
-  unsigned long long* d_state64_b = nullptr;  // tile states of the cylinder-refit compaction (may run concurrently with the voxel branch)
-  unsigned* d_rs_hist = nullptr;                           // segment histograms [segments][256]
-  Rs2Aux* d_rs_aux = nullptr;                              // group sums / totals / completion counter of one pass; zero between passes
-  size_t rs_hist_words = 0;
-  TileCtl* d_ctl = nullptr;      // [3] launch control of the look-back kernels: d_state64 | d_state64_b | d_dense_state
+  DevBuf<BlockEntry> d_tab;  // dense block table of the neighbour grid (1 << (key_bits - 6) entries)
+  DevBuf<int> d_vkey_pt, d_assign, d_vox_start, d_vox_key, d_vox_count, d_nn_idx;
+  DevBuf<unsigned char> d_labels;
+  DevBuf<unsigned long long> d_state64;
+  DevBuf<unsigned long long> d_state64_b;  // tile states of the cylinder-refit compaction (may run concurrently with the voxel branch)
+  DevBuf<unsigned> d_rs_hist;              // segment histograms [segments][256]
+  DevBuf<Rs2Aux> d_rs_aux;                 // group sums / totals / completion counter of one pass; zero between passes
+  DevBuf<TileCtl> d_ctl;         // [3] launch control of the look-back kernels: d_state64 | d_state64_b | d_dense_state
   size_t n_grid = 0;             // n_input rounded up to a bucket: what grids are sized by (kernels read the true n on the device)
-  DevState* d_st = nullptr;
-  double* d_partials = nullptr;
-  FrameOut* d_frame = nullptr;
+  DevBuf<DevState> d_st;
+  DevBuf<double> d_partials;
+  DevBuf<FrameOut> d_frame;
   // ransac (index = kind)
-  int* d_samples[2] = {nullptr, nullptr};
+  DevBuf<int> d_samples[2];
   int* h_samples[2] = {nullptr, nullptr};
   cudaEvent_t ev_samples[2] = {nullptr, nullptr};
-  float4* d_plane_coef = nullptr;
-  float *d_model7 = nullptr, *d_test12 = nullptr;
-  int *d_hvalid[2] = {nullptr, nullptr}, *d_counts[2] = {nullptr, nullptr};
-  unsigned long long* d_key = nullptr;  // [2]
-  ModelState* d_model = nullptr;        // [2]
+  DevBuf<float4> d_plane_coef;
+  DevBuf<float> d_model7, d_test12;
+  DevBuf<int> d_hvalid[2], d_counts[2];
+  DevBuf<unsigned long long> d_key;  // [2]
+  DevBuf<ModelState> d_model;        // [2]
   // polyline
-  PolyState* d_poly = nullptr;
-  long long* d_poly_acc = nullptr;
-  unsigned long long* d_poly_part = nullptr;  // per-block (min,max) of the polyline range pass
-  gm_slice* d_slices = nullptr;
-  SummaryDev* d_summary = nullptr;
+  DevBuf<PolyState> d_poly;
+  DevBuf<long long> d_poly_acc;
+  DevBuf<unsigned long long> d_poly_part;  // per-block (min,max) of the polyline range pass
+  DevBuf<gm_slice> d_slices;
+  DevBuf<SummaryDev> d_summary;
   // compression stage: residual (label 0) cloud and its voxel grid
-  VoxState* d_res_vs = nullptr;
-  CompStats* d_comp = nullptr;
-  float4 *d_res_pts = nullptr, *d_res_centroid = nullptr;
-  int *d_res_key_pt = nullptr, *d_res_assign = nullptr, *d_res_vox_start = nullptr, *d_res_vox_key = nullptr, *d_res_vox_count = nullptr;
-  double* d_comp_part = nullptr;
-  unsigned long long* d_comp_mm = nullptr;
-  bool have_comp = false;
-  unsigned* d_counters = nullptr;  // last-block tickets: [0] frame, [1] plane refit, [2] cylinder GN
-  float4* d_inl = nullptr;          // compacted cylinder inliers
+  DevBuf<VoxState> d_res_vs;
+  DevBuf<CompStats> d_comp;
+  DevBuf<float4> d_res_pts, d_res_centroid;
+  DevBuf<int> d_res_key_pt, d_res_assign, d_res_vox_start, d_res_vox_key, d_res_vox_count;
+  DevBuf<double> d_comp_part;
+  DevBuf<unsigned long long> d_comp_mm;
+  DevBuf<unsigned> d_counters;  // last-block tickets: [0] frame, [1] plane refit, [2] cylinder GN
+  DevBuf<float4> d_inl;         // compacted cylinder inliers
   // CUDA-graph replay of gm_process_scan: the launch sequence of one scan depends only on (bucketed size, hypothesis
   // counts, parameters / modes), never on per-scan host values (tile epochs, barrier parities and the scan pointer
   // live in device memory), so it is captured once per key and replayed with ONE cudaGraphLaunch
@@ -175,7 +195,7 @@ struct gm_ctx {
   // peer-memory collectives (gm_comm.cuh); `sharded` marks a RANSAC round whose keys travel through the mailboxes
   struct gm_comm* comm = nullptr;
   bool sharded = false;
-  double* d_frame_sums = nullptr;  // [8] the 6 scatter sums of the last gm_local_frame, kept for gm_allreduce_frame
+  DevBuf<double> d_frame_sums;  // [8] the 6 scatter sums of the last gm_local_frame, kept for gm_allreduce_frame
   // profiling
   bool profiling = false;
   std::vector<cudaEvent_t> ev_pool;
@@ -199,6 +219,26 @@ struct SegTimer {
   }
   ~SegTimer() { if (e1) cudaEventRecord(e1, ctx->stream); }
 };
+
+// The results a context holds, in pipeline order.  A stage's entry point fails with GM_ERR_STAGE_ORDER unless the
+// stages it reads are held, and marks its own stage.  Running a stage again does not drop the later ones.  A change
+// of input drops a stage and everything after it: a new scan from CROP on, a new crop box or is_dense from CROP on, a
+// new neighbour grid from NORMALS on (the compacted cloud too, even an injected one).
+enum Stage {
+  SCAN, CROP, NORMALS, COMPACTED, VOXEL, FRAME, RANSAC_PLANE, RANSAC_CYL, MODEL_PLANE, MODEL_CYL, LABELS, POLY, COMP
+};
+inline Stage ransac_stage(int kind) { return Stage(RANSAC_PLANE + kind); }
+inline Stage model_stage(int kind) { return Stage(MODEL_PLANE + kind); }
+
+inline bool has(const gm_ctx* ctx, Stage s) { return (ctx->stages >> s) & 1u; }
+template <class... S>
+gm_status require(const gm_ctx* ctx, S... s) { return (has(ctx, s) && ...) ? GM_OK : GM_ERR_STAGE_ORDER; }
+template <class... S>
+void mark(gm_ctx* ctx, S... s) { ((ctx->stages |= 1u << s), ...); }
+inline void invalidate_from(gm_ctx* ctx, Stage s) { ctx->stages &= (1u << s) - 1u; }
+
+// Every setter that changes what a scan launches calls this: captured graphs of older generations are no longer used.
+inline void new_graph_generation(gm_ctx* ctx) { ++ctx->graph_gen; }
 }  // namespace
 
 #define GM_CUDA(call)                                                                            \
@@ -236,9 +276,6 @@ inline WeightLaw weight_law(const gm_params& p) {
   else { w.scale = 1.0; w.shift = .001 / p.weightingFactor; w.sgn = 1.0; }
   return w;
 }
-
-template <class T>
-cudaError_t dmalloc(T** p, size_t count) { return cudaMalloc((void**)p, std::max<size_t>(count, 1) * sizeof(T)); }
 
 int bits_for(unsigned long long max_value) {
   int b = 0;
@@ -296,14 +333,13 @@ gm_status ensure_block_table(gm_ctx* ctx);
 // table of the old one (rare path, synchronous).
 gm_status regrid(gm_ctx* ctx) {
   const GridSpec old = ctx->grid;
-  ctx->grid = make_grid(ctx->prm, ctx->have_grid_box ? ctx->grid_box_min : nullptr, ctx->have_grid_box ? ctx->grid_box_max : nullptr);
+  ctx->grid = make_grid(ctx->prm, ctx->grid_box_set ? ctx->grid_box_min : nullptr, ctx->grid_box_set ? ctx->grid_box_max : nullptr);
   if (!same_grid(old, ctx->grid)) {
     GM_CUDA(cudaStreamSynchronize(ctx->stream));
     // everything built on the old grid (runs, block table, normals, and whatever consumed them) is stale: the next stage
     // after gm_crop must be gm_normals again (GM_ERR_STAGE_ORDER otherwise), not a search over an empty table
-    ctx->have_normals = ctx->have_compacted = ctx->have_voxel = ctx->have_frame = ctx->have_labels = ctx->have_poly = ctx->have_comp = false;
-    ctx->have_ransac[0] = ctx->have_ransac[1] = ctx->have_model[0] = ctx->have_model[1] = false;
-    ctx->tab_entries = 0;  // forces reallocation + clear
+    invalidate_from(ctx, NORMALS);
+    ctx->d_tab.reset();  // forces reallocation + clear
     return ensure_block_table(ctx);
   }
   return GM_OK;
@@ -312,12 +348,7 @@ gm_status regrid(gm_ctx* ctx) {
 // (Re)allocate and zero the dense block table for the current grid.
 gm_status ensure_block_table(gm_ctx* ctx) {
   const size_t need = (size_t)1 << (ctx->grid.key_bits - 6);
-  if (need != ctx->tab_entries) {
-    if (ctx->d_tab) cudaFree(ctx->d_tab);
-    ctx->d_tab = nullptr;
-    GM_CUDA(cudaMalloc((void**)&ctx->d_tab, need * sizeof(BlockEntry)));
-    ctx->tab_entries = need;
-  }
+  if (need != ctx->d_tab.count) GM_CUDA(ctx->d_tab.alloc(need));
   GM_CUDA(cudaMemset(ctx->d_tab, 0, need * sizeof(BlockEntry)));
   GM_CUDA(cudaMemset(&ctx->d_st->tab_cells, 0, sizeof(int)));
   // cudaMemset runs on the legacy default stream, which does NOT order with this ctx's non-blocking streams:
@@ -336,7 +367,7 @@ inline size_t grid_bucket(size_t n, size_t cap) { return n == 0 ? 0 : std::min(c
 // form (3 launches per pass) is kept as a baseline in tools/microbench/sort_v1.cuh.
 gm_status radix_sort(gm_ctx* ctx, const int* n_ptr, size_t n_cap, int key_bits, int* result_buf) {
   const Rs2Plan plan = rs2_plan(n_cap, key_bits);
-  if ((size_t)plan.segments * 256 > ctx->rs_hist_words) { ctx->err = "radix histogram capacity"; return GM_ERR_CAPACITY; }
+  if ((size_t)plan.segments * 256 > ctx->d_rs_hist.count) { ctx->err = "radix histogram capacity"; return GM_ERR_CAPACITY; }
   unsigned* const keys[2] = {ctx->d_keys[0], ctx->d_keys[1]};
   unsigned* const vals[2] = {ctx->d_vals[0], ctx->d_vals[1]};
   *result_buf = rs2_sort(ctx->stream, keys, vals, n_ptr, n_cap, key_bits, ctx->d_rs_hist, ctx->d_rs_aux, nullptr);
@@ -348,6 +379,27 @@ gm_status radix_sort(gm_ctx* ctx, const int* n_ptr, size_t n_cap, int key_bits, 
 gm_status sync_state(gm_ctx* ctx, DevState* host) {
   GM_CUDA(cudaMemcpyAsync(host, ctx->d_st, sizeof(DevState), cudaMemcpyDeviceToHost, ctx->stream));
   GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  return GM_OK;
+}
+
+int n_crop(const DevState& h) { return h.n_crop; }
+int n_valid(const DevState& h) { return h.n_valid; }
+int n_voxels(const DevState& h) { return h.vox.n_voxels; }
+
+struct Copy { void* dst; const void* src; size_t item_bytes; };
+
+// Device -> host download of per-point or per-voxel arrays: reads the device counts into *h, fails with
+// GM_ERR_CAPACITY unless count(*h) items fit `capacity`, then copies that many items to every non-null destination
+// and waits for the copies unless `wait` is false.
+gm_status download(gm_ctx* ctx, DevState* h, int (*count)(const DevState&), size_t capacity, std::initializer_list<Copy> copies,
+                   bool wait = true) {
+  gm_status s = sync_state(ctx, h);
+  if (s != GM_OK) return s;
+  const size_t n = (size_t)count(*h);
+  if (n > capacity) return GM_ERR_CAPACITY;
+  for (const Copy& c : copies)
+    if (c.dst && n * c.item_bytes > 0) GM_CUDA(cudaMemcpyAsync(c.dst, c.src, n * c.item_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  if (wait) GM_CUDA(cudaStreamSynchronize(ctx->stream));
   return GM_OK;
 }
 
@@ -431,7 +483,7 @@ gm_status gm_create(const gm_params* p, size_t max_points, int32_t max_hypothese
   ctx->num_sms = prop.multiProcessorCount;
   if ((e = cudaStreamCreateWithFlags(&ctx->own_stream, cudaStreamNonBlocking)) != cudaSuccess) return fail(e, "cudaStreamCreate");
   ctx->stream = ctx->own_stream;
-#define A(ptr, count) if ((e = dmalloc(&ctx->ptr, (count))) != cudaSuccess) return fail(e, #ptr)
+#define A(buf, count) if ((e = ctx->buf.alloc(count)) != cudaSuccess) return fail(e, #buf)
   A(d_in, N); A(d_crop, N); A(d_sorted, N + 1); A(d_cloud_c, N);  // d_walk_runs reads candidates in pairs: one element of slack
   A(d_sorted_valid, N); A(d_leaf_bounds, 2 * ((N + 31) / 32));
   A(d_normals, 2 * N); A(d_normals_c, 2 * N); A(d_centroid, N); A(d_nn_normal, 2 * N);
@@ -441,8 +493,7 @@ gm_status gm_create(const gm_params* p, size_t max_points, int32_t max_hypothese
   A(d_vkey_pt, N); A(d_assign, N); A(d_vox_start, N + 1); A(d_vox_key, N); A(d_vox_count, N); A(d_nn_idx, N);
   A(d_labels, N);
   A(d_state64, (size_t)div_up((long long)N, CP_TILE) + 2); A(d_state64_b, (size_t)div_up((long long)N, CP_TILE) + 2);
-  ctx->rs_hist_words = RS2_HIST_WORDS;
-  A(d_rs_hist, ctx->rs_hist_words); A(d_rs_aux, 1);
+  A(d_rs_hist, RS2_HIST_WORDS); A(d_rs_aux, 1);
   A(d_st, 1); A(d_ctl, 3); A(d_frame_sums, 8);
   A(d_partials, 3 * kPartialsRegion);  // 3 regions: frame | plane refit | cylinder GN (may run concurrently)
   A(d_frame, 1);
@@ -492,16 +543,6 @@ gm_status gm_create(const gm_params* p, size_t max_points, int32_t max_hypothese
 void gm_destroy(gm_ctx* ctx) {
   if (!ctx) return;
   if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-  void* ptrs[] = {ctx->d_knn_idx, ctx->d_dense_state, ctx->d_dense_cnt, ctx->d_dense_id, ctx->d_dense_sum, ctx->d_tab, ctx->d_cell_nruns, ctx->d_sorted_valid, ctx->d_leaf_bounds, ctx->d_raw, ctx->d_in, ctx->d_crop, ctx->d_sorted, ctx->d_cloud_c, ctx->d_normals, ctx->d_normals_c, ctx->d_centroid,
-                  ctx->d_nn_normal, ctx->d_keys[0], ctx->d_keys[1], ctx->d_vals[0], ctx->d_vals[1], ctx->d_ucell_key,
-                  ctx->d_cell_id, ctx->d_ucell_start, ctx->d_nbr, ctx->d_valid_map, ctx->d_runs, ctx->d_vkey_pt, ctx->d_assign,
-                  ctx->d_vox_start, ctx->d_vox_key, ctx->d_vox_count, ctx->d_nn_idx, ctx->d_labels, ctx->d_state64, ctx->d_state64_b,
-                  ctx->d_rs_hist, ctx->d_rs_aux, ctx->d_st, ctx->d_ctl, ctx->d_frame_sums, ctx->d_partials, ctx->d_frame,
-                  ctx->d_samples[0], ctx->d_samples[1], ctx->d_plane_coef, ctx->d_model7, ctx->d_test12, ctx->d_hvalid[0],
-                  ctx->d_hvalid[1], ctx->d_counts[0], ctx->d_counts[1], ctx->d_key, ctx->d_model, ctx->d_poly,
-                  ctx->d_res_vs, ctx->d_comp, ctx->d_res_pts, ctx->d_res_centroid, ctx->d_res_key_pt, ctx->d_res_assign, ctx->d_res_vox_start,
-                  ctx->d_res_vox_key, ctx->d_res_vox_count, ctx->d_comp_part, ctx->d_comp_mm, ctx->d_poly_acc, ctx->d_slices, ctx->d_summary, ctx->d_counters, ctx->d_inl, ctx->d_poly_part};
-  for (void* p : ptrs) if (p) cudaFree(p);
   for (int k = 0; k < 2; ++k) {
     if (ctx->h_samples[k]) cudaFreeHost(ctx->h_samples[k]);
     if (ctx->ev_samples[k]) cudaEventDestroy(ctx->ev_samples[k]);
@@ -512,17 +553,14 @@ void gm_destroy(gm_ctx* ctx) {
   for (int b = 0; b < 3; ++b) { if (ctx->branch[b]) cudaStreamDestroy(ctx->branch[b]); if (ctx->ev_join[b]) cudaEventDestroy(ctx->ev_join[b]); }
   if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
   if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
-  delete ctx;
+  delete ctx;  // frees the device buffers
 }
 
 gm_status gm_set_params(gm_ctx* ctx, const gm_params* p) {
   if (!ctx || validate_params(p) != GM_OK) return GM_ERR_INVALID_ARG;
-  ++ctx->graph_gen;  // what a scan launches may change: captured graphs of older generations are no longer used
+  new_graph_generation(ctx);
   if (p->maxSlices > ctx->prm.maxSlices) { ctx->err = "maxSlices cannot grow after gm_create"; return GM_ERR_CAPACITY; }
-  if (p->boxFilterBound != ctx->prm.boxFilterBound || p->is_dense != ctx->prm.is_dense) {  // the crop itself is stale
-    ctx->have_crop = ctx->have_normals = ctx->have_compacted = ctx->have_voxel = ctx->have_frame = ctx->have_labels = ctx->have_poly = ctx->have_comp = false;
-    ctx->have_ransac[0] = ctx->have_ransac[1] = ctx->have_model[0] = ctx->have_model[1] = false;
-  }
+  if (p->boxFilterBound != ctx->prm.boxFilterBound || p->is_dense != ctx->prm.is_dense) invalidate_from(ctx, CROP);  // the crop itself is stale
   ctx->prm = *p;
   return regrid(ctx);
 }
@@ -535,9 +573,9 @@ gm_status gm_get_params(const gm_ctx* ctx, gm_params* out) {
 
 gm_status gm_set_grid_box(gm_ctx* ctx, const float* min3, const float* max3) {
   if (!ctx || ((min3 == nullptr) != (max3 == nullptr))) return GM_ERR_INVALID_ARG;
-  ++ctx->graph_gen;  // what a scan launches may change: captured graphs of older generations are no longer used
+  new_graph_generation(ctx);
   if (min3 && ctx->knn_k > 0) { ctx->err = "k-NN normals need the default neighbour grid"; return GM_ERR_INVALID_ARG; }
-  ctx->have_grid_box = min3 != nullptr;
+  ctx->grid_box_set = min3 != nullptr;
   if (min3) {
     for (int a = 0; a < 3; ++a) {
       if (!(max3[a] >= min3[a])) return GM_ERR_INVALID_ARG;
@@ -549,7 +587,7 @@ gm_status gm_set_grid_box(gm_ctx* ctx, const float* min3, const float* max3) {
 
 gm_status gm_set_owned_range(gm_ctx* ctx, int32_t axis, float lo, float hi) {
   if (!ctx || axis > 2 || (axis >= 0 && !(hi >= lo))) return GM_ERR_INVALID_ARG;
-  ++ctx->graph_gen;  // what a scan launches may change: captured graphs of older generations are no longer used
+  new_graph_generation(ctx);
   ctx->own.axis = axis < 0 ? -1 : axis;
   ctx->own.lo = lo; ctx->own.hi = hi;
   return GM_OK;
@@ -557,8 +595,8 @@ gm_status gm_set_owned_range(gm_ctx* ctx, int32_t axis, float lo, float hi) {
 
 gm_status gm_set_voxel_bbox(gm_ctx* ctx, const float* min3, const float* max3) {
   if (!ctx || ((min3 == nullptr) != (max3 == nullptr))) return GM_ERR_INVALID_ARG;
-  ++ctx->graph_gen;  // what a scan launches may change: captured graphs of older generations are no longer used
-  ctx->have_vox_bbox = min3 != nullptr;
+  new_graph_generation(ctx);
+  ctx->vox_bbox_set = min3 != nullptr;
   ctx->vox_bbox_is_hint = false;
   if (min3) for (int a = 0; a < 3; ++a) { ctx->vox_bbox[a] = min3[a]; ctx->vox_bbox[3 + a] = max3[a]; }
   return GM_OK;
@@ -572,7 +610,7 @@ gm_status gm_set_voxel_bbox_hint(gm_ctx* ctx, const float* min3, const float* ma
 
 gm_status gm_get_search_stats(gm_ctx* ctx, int64_t* candidates, int64_t* neighbors) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_normals) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, NORMALS)) return s;
   DevState h;
   gm_status s = sync_state(ctx, &h);
   if (s != GM_OK) return s;
@@ -583,7 +621,7 @@ gm_status gm_get_search_stats(gm_ctx* ctx, int64_t* candidates, int64_t* neighbo
 
 gm_status gm_get_voxel_bbox(gm_ctx* ctx, float* min3, float* max3) {
   if (!ctx || !min3 || !max3) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_compacted) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, COMPACTED)) return s;
   DevState h;
   gm_status s = sync_state(ctx, &h);
   if (s != GM_OK) return s;
@@ -594,7 +632,7 @@ gm_status gm_get_voxel_bbox(gm_ctx* ctx, float* min3, float* max3) {
 
 gm_status gm_set_stream(gm_ctx* ctx, void* cuda_stream) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  ++ctx->graph_gen;  // what a scan launches may change: captured graphs of older generations are no longer used
+  new_graph_generation(ctx);
   GM_CUDA(cudaStreamSynchronize(ctx->stream));
   ctx->stream = cuda_stream ? (cudaStream_t)cuda_stream : ctx->own_stream;
   return GM_OK;
@@ -602,22 +640,22 @@ gm_status gm_set_stream(gm_ctx* ctx, void* cuda_stream) {
 
 gm_status gm_set_voxel_mode(gm_ctx* ctx, int32_t mode) {
   if (!ctx || (mode != 0 && mode != 1)) return GM_ERR_INVALID_ARG;
-  ++ctx->graph_gen;  // what a scan launches may change: captured graphs of older generations are no longer used
+  new_graph_generation(ctx);
   ctx->voxel_mode = mode;
   return GM_OK;
 }
 
 gm_status gm_set_normals_mode(gm_ctx* ctx, int32_t mode) {
   if (!ctx || (mode != 0 && mode != 1)) return GM_ERR_INVALID_ARG;
-  ++ctx->graph_gen;  // what a scan launches may change: captured graphs of older generations are no longer used
+  new_graph_generation(ctx);
   ctx->normals_mode = mode;
   return GM_OK;
 }
 
 gm_status gm_set_knn(gm_ctx* ctx, int32_t k, int32_t keep_indices) {
   if (!ctx || k < 0 || k > KNN_MAX) return GM_ERR_INVALID_ARG;
-  ++ctx->graph_gen;
-  if (k > 0 && ctx->have_grid_box) { ctx->err = "k-NN normals need the default neighbour grid (the crop cube): clear gm_set_grid_box first"; return GM_ERR_INVALID_ARG; }
+  new_graph_generation(ctx);
+  if (k > 0 && ctx->grid_box_set) { ctx->err = "k-NN normals need the default neighbour grid (the crop cube): clear gm_set_grid_box first"; return GM_ERR_INVALID_ARG; }
   ctx->knn_k = k;
   ctx->knn_keep = k > 0 && keep_indices != 0;
   return GM_OK;
@@ -625,26 +663,22 @@ gm_status gm_set_knn(gm_ctx* ctx, int32_t k, int32_t keep_indices) {
 
 gm_status gm_set_knn_max_radius(gm_ctx* ctx, double max_radius) {
   if (!ctx || !(max_radius >= 0.0)) return GM_ERR_INVALID_ARG;
-  ++ctx->graph_gen;
+  new_graph_generation(ctx);
   ctx->knn_max_radius = max_radius;
   return GM_OK;
 }
 
 gm_status gm_download_knn_indices(gm_ctx* ctx, int32_t* out, size_t capacity_points) {
   if (!ctx || !out) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_normals || ctx->knn_k <= 0 || !ctx->knn_keep || !ctx->d_knn_idx) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, NORMALS)) return s;
+  if (ctx->knn_k <= 0 || !ctx->knn_keep || !ctx->d_knn_idx) return GM_ERR_STAGE_ORDER;
   DevState h;
-  gm_status s = sync_state(ctx, &h);
-  if (s != GM_OK) return s;
-  if ((size_t)h.n_crop > capacity_points) return GM_ERR_CAPACITY;
-  GM_CUDA(cudaMemcpyAsync(out, ctx->d_knn_idx, (size_t)h.n_crop * ctx->knn_k * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  GM_CUDA(cudaStreamSynchronize(ctx->stream));
-  return GM_OK;
+  return download(ctx, &h, n_crop, capacity_points, {{out, ctx->d_knn_idx, ctx->knn_k * sizeof(int)}});
 }
 
 gm_status gm_set_count_mode(gm_ctx* ctx, int32_t mode) {
   if (!ctx || (mode != 0 && mode != 1)) return GM_ERR_INVALID_ARG;
-  ++ctx->graph_gen;  // what a scan launches may change: captured graphs of older generations are no longer used
+  new_graph_generation(ctx);
   ctx->count_mode = mode;
   return GM_OK;
 }
@@ -658,17 +692,17 @@ gm_status gm_synchronize(gm_ctx* ctx) {
   return GM_OK;
 }
 
-static void clear_stages(gm_ctx* ctx) {
-  ctx->have_crop = ctx->have_normals = ctx->have_compacted = ctx->injected = false;
-  ctx->have_voxel = ctx->have_frame = ctx->have_labels = ctx->have_poly = ctx->have_comp = false;
-  ctx->have_ransac[0] = ctx->have_ransac[1] = ctx->have_model[0] = ctx->have_model[1] = false;
+// A new input cloud: nothing computed from the previous one is valid any more.
+static void new_scan(gm_ctx* ctx, size_t n) {
+  ctx->n_input = n;
+  ctx->n_grid = grid_bucket(n, ctx->cap);
+  invalidate_from(ctx, CROP);
+  mark(ctx, SCAN);
+  ctx->injected = false;
 }
 
 static gm_status begin_scan(gm_ctx* ctx, size_t n) {
-  ctx->n_input = n;
-  ctx->n_grid = grid_bucket(n, ctx->cap);
-  ctx->have_scan = true;
-  clear_stages(ctx);
+  new_scan(ctx, n);
   GM_LAUNCH(ctx, k_begin_scan, 1, 32, ctx->d_st, (int)n, ctx->d_scan);
   GM_CHECK_LAUNCHES(ctx);
   return GM_OK;
@@ -695,12 +729,9 @@ gm_status gm_upload_pointcloud2(gm_ctx* ctx, const void* data_host, size_t n, si
   if (n > ctx->cap) { ctx->err = "scan larger than max_points"; return GM_ERR_CAPACITY; }
   if (n) {
     const size_t bytes = n * point_step;
-    if (bytes > ctx->raw_cap) {  // not on the per-scan fast path: only when a larger message arrives
+    if (bytes > ctx->d_raw.count) {  // not on the per-scan fast path: only when a larger message arrives
       GM_CUDA(cudaStreamSynchronize(ctx->stream));
-      if (ctx->d_raw) cudaFree(ctx->d_raw);
-      ctx->d_raw = nullptr; ctx->raw_cap = 0;
-      GM_CUDA(cudaMalloc((void**)&ctx->d_raw, ctx->cap * point_step));
-      ctx->raw_cap = ctx->cap * point_step;
+      GM_CUDA(ctx->d_raw.alloc(ctx->cap * point_step));
     }
     GM_CUDA(cudaMemcpyAsync(ctx->d_raw, data_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
     GM_LAUNCH(ctx, k_decode_pointcloud2, div_up((long long)n, 256), 256, ctx->d_raw, (int)n, (int)point_step, (int)ox, (int)oy, (int)oz, ctx->d_in);
@@ -719,7 +750,7 @@ gm_status gm_set_scan_device(gm_ctx* ctx, const float* xyzw_device, size_t n) {
 // ---- a1 --------------------------------------------------------------------------------------
 gm_status gm_crop(gm_ctx* ctx) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_scan) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, SCAN)) return s;
   const size_t n = ctx->n_grid;
   if (n) {
     float hi = (float)ctx->prm.boxFilterBound, lo = (float)(-ctx->prm.boxFilterBound);
@@ -728,7 +759,7 @@ gm_status gm_crop(gm_ctx* ctx) {
               ctx->d_crop, ctx->d_state64, ctx->d_ctl + 0, ctx->d_st);
     GM_CHECK_LAUNCHES(ctx);
   }
-  ctx->have_crop = true;
+  mark(ctx, CROP);
   return GM_OK;
 }
 
@@ -736,7 +767,7 @@ gm_status gm_crop(gm_ctx* ctx) {
 // ---- a2 + a3 ---------------------------------------------------------------------------------
 gm_status gm_normals(gm_ctx* ctx) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_crop) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, CROP)) return s;
   const size_t n = ctx->n_grid;  // upper bound of M (bucketed)
   if (n) {
     const int* n_ptr = &ctx->d_st->n_crop;
@@ -763,12 +794,9 @@ gm_status gm_normals(gm_ctx* ctx) {
         int* idx_out = nullptr;
         if (ctx->knn_keep) {
           const size_t need = ctx->cap * (size_t)K;
-          if (need > ctx->knn_idx_cap) {  // rare path (first use / larger k)
+          if (need > ctx->d_knn_idx.count) {  // rare path (first use / larger k)
             GM_CUDA(cudaStreamSynchronize(ctx->stream));
-            if (ctx->d_knn_idx) cudaFree(ctx->d_knn_idx);
-            ctx->d_knn_idx = nullptr; ctx->knn_idx_cap = 0;
-            GM_CUDA(cudaMalloc((void**)&ctx->d_knn_idx, need * sizeof(int)));
-            ctx->knn_idx_cap = need;
+            GM_CUDA(ctx->d_knn_idx.alloc(need));
           }
           idx_out = ctx->d_knn_idx;
         }
@@ -789,8 +817,7 @@ gm_status gm_normals(gm_ctx* ctx) {
                 ctx->d_normals_c, ctx->d_valid_map, ctx->d_state64, ctx->d_ctl + 0, ctx->d_st, ctx->own); }
     GM_CHECK_LAUNCHES(ctx);
   }
-  ctx->have_normals = true;
-  ctx->have_compacted = true;
+  mark(ctx, NORMALS, COMPACTED);
   ctx->injected = false;
   return GM_OK;
 }
@@ -803,22 +830,20 @@ constexpr size_t kDenseMaxKeys = (size_t)1 << 23;  // 8M keys x 32 B = 256 MB of
 
 // Make the dense tables hold `range` keys (zero-initialised; they clean themselves afterwards).  Rare path.
 gm_status ensure_dense(gm_ctx* ctx, size_t range) {
-  if (range <= ctx->dense_cap) return GM_OK;
+  if (range <= ctx->d_dense_cnt.count) return GM_OK;
   GM_CUDA(cudaStreamSynchronize(ctx->stream));
   for (int b = 0; b < 3; ++b) if (ctx->branch[b]) GM_CUDA(cudaStreamSynchronize(ctx->branch[b]));
-  cudaFree(ctx->d_dense_cnt); cudaFree(ctx->d_dense_id); cudaFree(ctx->d_dense_sum); cudaFree(ctx->d_dense_state);
-  ctx->d_dense_cnt = ctx->d_dense_id = nullptr; ctx->d_dense_sum = nullptr; ctx->d_dense_state = nullptr; ctx->dense_cap = 0;
+  ctx->d_dense_cnt.reset();  // holds the capacity: allocated last, so that a failure below leaves it 0
   const size_t ntiles = (size_t)div_up((long long)range, CPL_TILE) + 2;
-  GM_CUDA(dmalloc(&ctx->d_dense_state, ntiles));
+  GM_CUDA(ctx->d_dense_state.alloc(ntiles));
   GM_CUDA(cudaMemset(ctx->d_dense_state, 0, ntiles * sizeof(unsigned long long)));
-  GM_CUDA(dmalloc(&ctx->d_dense_cnt, range));
-  GM_CUDA(dmalloc(&ctx->d_dense_id, range));
-  GM_CUDA(dmalloc(&ctx->d_dense_sum, 3 * range));
+  GM_CUDA(ctx->d_dense_id.alloc(range));
+  GM_CUDA(ctx->d_dense_sum.alloc(3 * range));
+  GM_CUDA(ctx->d_dense_cnt.alloc(range));
   GM_CUDA(cudaMemset(ctx->d_dense_cnt, 0, range * sizeof(int)));
   GM_CUDA(cudaMemset(ctx->d_dense_id, 0, range * sizeof(int)));
   GM_CUDA(cudaMemset(ctx->d_dense_sum, 0, 3 * range * sizeof(long long)));
   GM_CUDA(cudaDeviceSynchronize());  // legacy-stream memsets do not order with the ctx's non-blocking streams (this raced: zero centroids)
-  ctx->dense_cap = range;
   return GM_OK;
 }
 
@@ -834,12 +859,12 @@ gm_status voxel_downsample(gm_ctx* ctx, const float4* pts, VoxState* vs, size_t 
   if (ctx->voxel_mode == 0 && key_range > 0 && key_range <= kDenseMaxKeys) {
     if ((s = ensure_dense(ctx, key_range)) != GM_OK) return s;
     { SegTimer seg_(ctx, SEG_VOX_KEYS);
-      if (pts == ctx->d_cloud_c && ctx->have_normals && !ctx->injected) {
+      if (pts == ctx->d_cloud_c && has(ctx, NORMALS) && !ctx->injected) {
         // the scan's own compacted cloud: accumulate over its cell-sorted copy with warp-combined atomics
         GM_LAUNCH(ctx, k_voxel_accumulate_sorted, blocks, 256, ctx->d_sorted_valid, &ctx->d_st->n_crop, vs, inv,
-                  ctx->d_dense_cnt, (unsigned long long*)ctx->d_dense_sum, (int)key_range, &ctx->d_st->error);
+                  ctx->d_dense_cnt, (unsigned long long*)ctx->d_dense_sum.p, (int)key_range, &ctx->d_st->error);
       } else {
-        GM_LAUNCH(ctx, k_voxel_accumulate, blocks, 256, pts, vs, inv, ctx->d_dense_cnt, (unsigned long long*)ctx->d_dense_sum,
+        GM_LAUNCH(ctx, k_voxel_accumulate, blocks, 256, pts, vs, inv, ctx->d_dense_cnt, (unsigned long long*)ctx->d_dense_sum.p,
                   (int)key_range, &ctx->d_st->error);
       } }
     { SegTimer seg_(ctx, SEG_VOX_REDUCE);
@@ -876,7 +901,7 @@ int voxel_key_bits(const gm_ctx* ctx, size_t n, size_t* key_range) {
   double total = div * div * div;
   int bits = 32;
   if (total < 2147483647.0 && (double)n < 2147483647.0) { *key_range = (size_t)total; bits = bits_for((unsigned long long)total); }
-  if (ctx->have_vox_bbox) {
+  if (ctx->vox_bbox_set) {
     // a caller-supplied box (gm_set_voxel_bbox) holds the whole cloud, hence every sub-cloud: its lattice bounds the key range
     // (same float expressions as k_voxel_keys)
     const float* b = ctx->vox_bbox;
@@ -890,20 +915,20 @@ int voxel_key_bits(const gm_ctx* ctx, size_t n, size_t* key_range) {
 
 gm_status gm_voxel(gm_ctx* ctx) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_compacted) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, COMPACTED)) return s;
   const size_t n = ctx->n_grid;
   if (n) {
     VoxBuffers o{ctx->d_vkey_pt, ctx->d_assign, ctx->d_vox_start, ctx->d_vox_key, ctx->d_vox_count, ctx->d_centroid};
     int buf = 0;
     size_t key_range = 0;
     int key_bits = voxel_key_bits(ctx, n, &key_range);
-    if (ctx->have_vox_bbox && !ctx->vox_bbox_is_hint) {
+    if (ctx->vox_bbox_set && !ctx->vox_bbox_is_hint) {
       const float* b = ctx->vox_bbox;
       GM_LAUNCH(ctx, k_set_bbox, 1, 32, &ctx->d_st->vox, b[0], b[1], b[2], b[3], b[4], b[5]);
     }
     gm_status s = voxel_downsample(ctx, ctx->d_cloud_c, &ctx->d_st->vox, n, key_bits, key_range, o, &buf);
     if (s != GM_OK) return s;
-    if (ctx->have_normals) {
+    if (has(ctx, NORMALS)) {
       SegTimer seg_(ctx, SEG_VOX_NN);
       GM_LAUNCH(ctx, k_voxel_nn, std::min(div_up((long long)n * 32, NN_BLOCK), ctx->num_sms * 16), NN_BLOCK, ctx->d_centroid, ctx->d_sorted,
                 ctx->d_tab, ctx->d_ucell_start, ctx->d_runs, ctx->d_cell_nruns, ctx->d_valid_map, ctx->d_normals_c, ctx->grid, ctx->prm.nn_index_mode,
@@ -911,20 +936,20 @@ gm_status gm_voxel(gm_ctx* ctx) {
     }
     GM_CHECK_LAUNCHES(ctx);
   }
-  ctx->have_voxel = true;
+  mark(ctx, VOXEL);
   return GM_OK;
 }
 
 // ---- a5 --------------------------------------------------------------------------------------
 gm_status gm_local_frame(gm_ctx* ctx) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_compacted) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, COMPACTED)) return s;
   const WeightLaw law = weight_law(ctx->prm);
   SegTimer seg_(ctx, SEG_FRAME);
   GM_LAUNCH(ctx, k_frame, FRAME_BLOCKS, FR_BLOCK, ctx->d_normals_c, &ctx->d_st->n_valid, law, ctx->d_partials + 0 * kPartialsRegion, ctx->d_counters + 0,
             ctx->d_frame, ctx->d_frame_sums);
   GM_CHECK_LAUNCHES(ctx);
-  ctx->have_frame = true;
+  mark(ctx, FRAME);
   return GM_OK;
 }
 
@@ -943,7 +968,7 @@ static gm_status stage_samples(gm_ctx* ctx, int kind, const int32_t* samples_hos
 
 gm_status gm_ransac(gm_ctx* ctx, int32_t kind, const int32_t* samples_host, int32_t H, int32_t h_begin, int32_t h_end) {
   if (!ctx || (kind != 0 && kind != 1) || H < 0 || (H > 0 && !samples_host)) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_compacted) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, COMPACTED)) return s;
   if (H > ctx->hcap) { ctx->err = "H larger than max_hypotheses"; return GM_ERR_CAPACITY; }
   h_begin = std::max(h_begin, 0);
   h_end = std::min(h_end, H);
@@ -967,7 +992,7 @@ gm_status gm_ransac(gm_ctx* ctx, int32_t kind, const int32_t* samples_host, int3
     } }
     const int hloc = h_end - h_begin;
     bool argmax_done = false;
-    if (hloc > 0 && ctx->n_input > 0 && ctx->count_mode == 0 && ctx->have_normals && !ctx->injected) {
+    if (hloc > 0 && ctx->n_input > 0 && ctx->count_mode == 0 && has(ctx, NORMALS) && !ctx->injected) {
       // tile-culled counting over the cell-sorted cloud of this scan (same counts, see gm_ransac.cuh)
       argmax_done = true;
       SegTimer seg_(ctx, kind == 0 ? SEG_PLANE_COUNT : SEG_CYL_COUNT);
@@ -1006,9 +1031,9 @@ gm_status gm_ransac(gm_ctx* ctx, int32_t kind, const int32_t* samples_host, int3
     GM_CUDA(cudaMemsetAsync(ctx->d_key + kind, 0, sizeof(unsigned long long), ctx->stream));
   }
   GM_CHECK_LAUNCHES(ctx);
-  ctx->have_ransac[kind] = true;
+  mark(ctx, ransac_stage(kind));
   ctx->ransac_H[kind] = H;
-  ctx->have_model[kind] = false;
+  ctx->stages &= ~(1u << model_stage(kind));  // the model of the previous round is stale until gm_ransac_select
   return GM_OK;
 }
 
@@ -1020,21 +1045,21 @@ gm_status gm_ransac_key_device_ptr(gm_ctx* ctx, int32_t kind, void** key_dev) {
 
 gm_status gm_ransac_export_key(gm_ctx* ctx, int32_t kind, void* dst_device) {
   if (!ctx || !dst_device || (kind != 0 && kind != 1)) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_ransac[kind]) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, ransac_stage(kind))) return s;
   GM_CUDA(cudaMemcpyAsync(dst_device, ctx->d_key + kind, sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
   return GM_OK;
 }
 
 gm_status gm_ransac_import_key(gm_ctx* ctx, int32_t kind, const void* src_device) {
   if (!ctx || !src_device || (kind != 0 && kind != 1)) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_ransac[kind]) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, ransac_stage(kind))) return s;
   GM_CUDA(cudaMemcpyAsync(ctx->d_key + kind, src_device, sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
   return GM_OK;
 }
 
 gm_status gm_ransac_select(gm_ctx* ctx, int32_t kind) {
   if (!ctx || (kind != 0 && kind != 1)) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_ransac[kind]) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, ransac_stage(kind))) return s;
   const int* n_ptr = &ctx->d_st->n_valid;
   ModelState* ms = ctx->d_model + kind;
   SegTimer seg_(ctx, kind == 0 ? SEG_PLANE_REFIT : SEG_CYL_REFIT);
@@ -1059,27 +1084,27 @@ gm_status gm_ransac_select(gm_ctx* ctx, int32_t kind) {
     }
   }
   GM_CHECK_LAUNCHES(ctx);
-  ctx->have_model[kind] = true;
+  mark(ctx, model_stage(kind));
   return GM_OK;
 }
 
 gm_status gm_label(gm_ctx* ctx) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_compacted) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, COMPACTED)) return s;
   if (ctx->n_input) {
     int blocks = std::min(div_up((long long)ctx->n_grid, 256), ctx->num_sms * 16);
     SegTimer seg_(ctx, SEG_LABEL);
     GM_LAUNCH(ctx, k_label, blocks, 256, ctx->d_cloud_c, &ctx->d_st->n_valid, ctx->d_model + 0, ctx->d_model + 1,
-              ctx->have_model[0] ? 1 : 0, ctx->have_model[1] ? 1 : 0, (float)ctx->prm.ransacThreshold, ctx->d_labels);
+              has(ctx, MODEL_PLANE) ? 1 : 0, has(ctx, MODEL_CYL) ? 1 : 0, (float)ctx->prm.ransacThreshold, ctx->d_labels);
     GM_CHECK_LAUNCHES(ctx);
   }
-  ctx->have_labels = true;
+  mark(ctx, LABELS);
   return GM_OK;
 }
 
 gm_status gm_axis_polyline(gm_ctx* ctx) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_frame || !ctx->have_labels) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, FRAME, LABELS)) return s;
   const int S = ctx->prm.maxSlices;
   const int* n_ptr = &ctx->d_st->n_valid;
   const WeightLaw shift = weight_law(ctx->prm);
@@ -1090,26 +1115,26 @@ gm_status gm_axis_polyline(gm_ctx* ctx) {
     int blocks = std::max(1, std::min(div_up((long long)std::max<size_t>(ctx->n_grid, 1), POLY_BLOCK), ctx->num_sms * 4));
     GM_LAUNCH(ctx, k_poly_range, blocks, POLY_BLOCK, ctx->d_cloud_c, ctx->d_labels, n_ptr, ctx->d_frame, ctx->d_poly, ctx->d_poly_acc,
               POLY_NACC * S, ctx->d_poly_part, ctx->d_counters + 8, ctx->prm.sliceLength, S);
-    const ModelState* cylm = ctx->have_model[1] ? ctx->d_model + 1 : nullptr;
+    const ModelState* cylm = has(ctx, MODEL_CYL) ? ctx->d_model + 1 : nullptr;
     GM_LAUNCH(ctx, k_poly_pass<0>, blocks, POLY_BLOCK, ctx->d_cloud_c, ctx->d_normals_c, ctx->d_labels, n_ptr, ctx->d_poly, shift,
               ctx->d_poly_acc, ctx->d_slices, ctx->d_counters + 9, cylm);
     GM_LAUNCH(ctx, k_poly_pass<2>, blocks, POLY_BLOCK, ctx->d_cloud_c, ctx->d_normals_c, ctx->d_labels, n_ptr, ctx->d_poly, shift,
               ctx->d_poly_acc, ctx->d_slices, ctx->d_counters + 11, cylm);
   }
   GM_CHECK_LAUNCHES(ctx);
-  ctx->have_poly = true;
+  mark(ctx, POLY);
   return GM_OK;
 }
 
 gm_status gm_compress(gm_ctx* ctx) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_labels || !ctx->have_poly) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, LABELS, POLY)) return s;
   const size_t n = std::max<size_t>(ctx->n_grid, 1);
   gm_status s;
   GM_LAUNCH(ctx, k_vox_reset, 1, 32, ctx->d_res_vs);
   const int tiles = div_up((long long)n, CP_TILE);
   GM_LAUNCH(ctx, k_comp_split, tiles, CP_BLOCK, ctx->d_cloud_c, ctx->d_labels, &ctx->d_st->n_valid, ctx->d_model + 0, ctx->d_model + 1,
-            ctx->have_model[0] ? 1 : 0, ctx->have_model[1] ? 1 : 0, ctx->d_res_pts, ctx->d_res_vs, ctx->d_state64, ctx->d_ctl + 0, &ctx->d_st->error,
+            has(ctx, MODEL_PLANE) ? 1 : 0, has(ctx, MODEL_CYL) ? 1 : 0, ctx->d_res_pts, ctx->d_res_vs, ctx->d_state64, ctx->d_ctl + 0, &ctx->d_st->error,
             ctx->d_comp_part, ctx->d_comp_mm, ctx->d_counters + 12, ctx->d_comp);
   VoxBuffers o{ctx->d_res_key_pt, ctx->d_res_assign, ctx->d_res_vox_start, ctx->d_res_vox_key, ctx->d_res_vox_count, ctx->d_res_centroid};
   int buf = 0;
@@ -1119,7 +1144,7 @@ gm_status gm_compress(gm_ctx* ctx) {
   GM_LAUNCH(ctx, k_comp_residual_error, ctx->num_sms * 2, CR_BLOCK, ctx->d_res_pts, ctx->d_res_assign, ctx->d_res_centroid, ctx->d_res_vs,
             ctx->d_comp_part, ctx->d_counters + 13, ctx->d_comp);
   GM_CHECK_LAUNCHES(ctx);
-  ctx->have_comp = true;
+  mark(ctx, COMP);
   return GM_OK;
 }
 
@@ -1152,14 +1177,14 @@ gm_status fetch_compression(gm_ctx* ctx, gm_compression* out, VoxState* vs_host)
 
 gm_status gm_get_compression(gm_ctx* ctx, gm_compression* out) {
   if (!ctx || !out) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_comp) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, COMP)) return s;
   VoxState vs;
   return fetch_compression(ctx, out, &vs);
 }
 
 gm_status gm_download_compressed(gm_ctx* ctx, void* buf, size_t capacity, size_t* bytes) {
   if (!ctx || !bytes) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_comp) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, COMP)) return s;
   gm_compression h;
   VoxState vs;
   gm_status s = fetch_compression(ctx, &h, &vs);
@@ -1231,14 +1256,13 @@ static gm_status process_scan_body(gm_ctx* ctx, const int32_t* plane_samples_hos
   return GM_OK;
 }
 
-// host-side stage flags after a whole scan (what process_scan_body leaves behind)
+// the stages a whole scan holds afterwards (what process_scan_body marks when it runs as plain launches)
 static void mark_processed(gm_ctx* ctx, int Hp, int Hc) {
-  ctx->have_crop = ctx->have_normals = ctx->have_compacted = true;
+  mark(ctx, CROP, NORMALS, COMPACTED, VOXEL, FRAME, LABELS, POLY);
   ctx->injected = false;
-  ctx->have_voxel = ctx->have_frame = ctx->have_labels = ctx->have_poly = true;
   const int H[2] = {Hp, Hc};
   for (int k = 0; k < 2; ++k)
-    if (H[k] > 0) { ctx->have_ransac[k] = true; ctx->have_model[k] = true; ctx->ransac_H[k] = H[k]; }
+    if (H[k] > 0) { mark(ctx, ransac_stage(k), model_stage(k)); ctx->ransac_H[k] = H[k]; }
 }
 
 static void drop_graph(gm_ctx::ScanGraph& g) {
@@ -1315,7 +1339,7 @@ extern "C" {
 
 gm_status gm_process_scan(gm_ctx* ctx, const int32_t* plane_samples_host, int32_t Hp, const int32_t* cyl_samples_host, int32_t Hc) {
   if (!ctx || Hp < 0 || Hc < 0 || (Hp > 0 && !plane_samples_host) || (Hc > 0 && !cyl_samples_host)) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_scan) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, SCAN)) return s;
   if (Hp > ctx->hcap || Hc > ctx->hcap) { ctx->err = "H larger than max_hypotheses"; return GM_ERR_CAPACITY; }
   auto body = [&] { return process_scan_body(ctx, plane_samples_host, Hp, cyl_samples_host, Hc); };
   const bool graphable = use_graph(ctx) && ctx->concurrent && !ctx->profiling && ctx->n_grid > 0;
@@ -1350,7 +1374,7 @@ gm_status gm_get_graph_stats(const gm_ctx* ctx, int64_t* captures, int64_t* repl
 gm_status gm_ransac_pair(gm_ctx* ctx, const int32_t* plane_samples_host, int32_t Hp, int32_t p_begin, int32_t p_end,
                          const int32_t* cyl_samples_host, int32_t Hc, int32_t c_begin, int32_t c_end) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_compacted) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, COMPACTED)) return s;
   gm_status s;
   if (ctx->concurrent && !ctx->profiling) {
     GM_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
@@ -1365,7 +1389,7 @@ gm_status gm_ransac_pair(gm_ctx* ctx, const int32_t* plane_samples_host, int32_t
 
 gm_status gm_ransac_select_pair(gm_ctx* ctx) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_ransac[0] || !ctx->have_ransac[1]) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, RANSAC_PLANE, RANSAC_CYL)) return s;
   gm_status s;
   if (ctx->concurrent && !ctx->profiling) {
     GM_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
@@ -1381,13 +1405,13 @@ gm_status gm_ransac_select_pair(gm_ctx* ctx) {
 /* both keys (plane, cylinder) as 16 contiguous bytes */
 gm_status gm_ransac_export_keys(gm_ctx* ctx, void* dst_device) {
   if (!ctx || !dst_device) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_ransac[0] || !ctx->have_ransac[1]) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, RANSAC_PLANE, RANSAC_CYL)) return s;
   GM_CUDA(cudaMemcpyAsync(dst_device, ctx->d_key, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
   return GM_OK;
 }
 gm_status gm_ransac_import_keys(gm_ctx* ctx, const void* src_device) {
   if (!ctx || !src_device) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_ransac[0] || !ctx->have_ransac[1]) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, RANSAC_PLANE, RANSAC_CYL)) return s;
   GM_CUDA(cudaMemcpyAsync(ctx->d_key, src_device, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
   return GM_OK;
 }
@@ -1398,11 +1422,11 @@ gm_status gm_get_counts(gm_ctx* ctx, gm_counts* out) {
   DevState h;
   gm_status s = sync_state(ctx, &h);
   if (s != GM_OK) return s;
-  out->n_input = ctx->have_scan ? h.n_input : -1;
-  out->n_cropped = ctx->have_crop ? h.n_crop : -1;
-  out->n_valid = ctx->have_compacted ? h.n_valid : -1;
-  out->n_voxels = ctx->have_voxel ? h.vox.n_voxels : -1;
-  out->n_cells = ctx->have_normals ? h.n_cells : -1;
+  out->n_input = has(ctx, SCAN) ? h.n_input : -1;
+  out->n_cropped = has(ctx, CROP) ? h.n_crop : -1;
+  out->n_valid = has(ctx, COMPACTED) ? h.n_valid : -1;
+  out->n_voxels = has(ctx, VOXEL) ? h.vox.n_voxels : -1;
+  out->n_cells = has(ctx, NORMALS) ? h.n_cells : -1;
   out->voxel_overflow = h.vox.overflow;
   out->nn_out_of_range = h.nn_oor;
   out->device_error = h.error;
@@ -1417,91 +1441,64 @@ gm_status gm_get_counts(gm_ctx* ctx, gm_counts* out) {
 
 gm_status gm_download_cloud(gm_ctx* ctx, int32_t which, float* out, size_t capacity_points) {
   if (!ctx || !out) return GM_ERR_INVALID_ARG;
-  if ((which == 0 && !ctx->have_crop) || (which == 1 && !ctx->have_compacted) || which < 0 || which > 1) return GM_ERR_STAGE_ORDER;
+  if (which < 0 || which > 1) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, which == 0 ? CROP : COMPACTED)) return s;
   DevState h;
-  gm_status s = sync_state(ctx, &h);
-  if (s != GM_OK) return s;
-  size_t n = (size_t)(which == 0 ? h.n_crop : h.n_valid);
-  if (n > capacity_points) return GM_ERR_CAPACITY;
-  GM_D2H(out, which == 0 ? ctx->d_crop : ctx->d_cloud_c, n * 16);
-  GM_CUDA(cudaStreamSynchronize(ctx->stream));
-  return GM_OK;
+  return download(ctx, &h, which == 0 ? n_crop : n_valid, capacity_points, {{out, which == 0 ? ctx->d_crop : ctx->d_cloud_c, 16}});
 }
 
 gm_status gm_download_normals(gm_ctx* ctx, int32_t which, float* out8, size_t capacity_points) {
   if (!ctx || !out8) return GM_ERR_INVALID_ARG;
-  if ((which == 0 && !ctx->have_normals) || (which == 1 && !ctx->have_compacted) || which < 0 || which > 1) return GM_ERR_STAGE_ORDER;
+  if (which < 0 || which > 1) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, which == 0 ? NORMALS : COMPACTED)) return s;
   DevState h;
-  gm_status s = sync_state(ctx, &h);
-  if (s != GM_OK) return s;
-  size_t n = (size_t)(which == 0 ? h.n_crop : h.n_valid);
-  if (n > capacity_points) return GM_ERR_CAPACITY;
-  GM_D2H(out8, which == 0 ? ctx->d_normals : ctx->d_normals_c, n * 32);
-  GM_CUDA(cudaStreamSynchronize(ctx->stream));
-  return GM_OK;
+  return download(ctx, &h, which == 0 ? n_crop : n_valid, capacity_points, {{out8, which == 0 ? ctx->d_normals : ctx->d_normals_c, 32}});
 }
 
 gm_status gm_download_neighbor_counts(gm_ctx* ctx, int32_t* out, size_t capacity_points) {
   if (!ctx || !out) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_normals) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, NORMALS)) return s;
   DevState h;
-  gm_status s = sync_state(ctx, &h);
-  if (s != GM_OK) return s;
-  if ((size_t)h.n_crop > capacity_points) return GM_ERR_CAPACITY;
-  GM_D2H(out, ctx->d_nbr, (size_t)h.n_crop * 4);
-  GM_CUDA(cudaStreamSynchronize(ctx->stream));
-  return GM_OK;
+  return download(ctx, &h, n_crop, capacity_points, {{out, ctx->d_nbr, 4}});
 }
 
 gm_status gm_download_valid_map(gm_ctx* ctx, int32_t* out, size_t capacity_points) {
   if (!ctx || !out) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_normals) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, NORMALS)) return s;
   DevState h;
-  gm_status s = sync_state(ctx, &h);
-  if (s != GM_OK) return s;
-  if ((size_t)h.n_crop > capacity_points) return GM_ERR_CAPACITY;
-  GM_D2H(out, ctx->d_valid_map, (size_t)h.n_crop * 4);
-  GM_CUDA(cudaStreamSynchronize(ctx->stream));
-  return GM_OK;
+  return download(ctx, &h, n_crop, capacity_points, {{out, ctx->d_valid_map, 4}});
 }
 
 gm_status gm_download_voxel_assignment(gm_ctx* ctx, int32_t* keys, int32_t* assign, size_t capacity_points) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_voxel) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, VOXEL)) return s;
   DevState h;
-  gm_status s = sync_state(ctx, &h);
+  gm_status s = download(ctx, &h, n_valid, capacity_points, {{keys, ctx->d_vkey_pt, 4}, {assign, ctx->d_assign, 4}});
   if (s != GM_OK) return s;
-  if ((size_t)h.n_valid > capacity_points) return GM_ERR_CAPACITY;
-  if (keys) GM_D2H(keys, ctx->d_vkey_pt, (size_t)h.n_valid * 4);
-  if (assign) GM_D2H(assign, ctx->d_assign, (size_t)h.n_valid * 4);
-  GM_CUDA(cudaStreamSynchronize(ctx->stream));
   return h.vox.overflow ? GM_WARN_VOXEL_OVERFLOW : GM_OK;
 }
 
 gm_status gm_download_voxels(gm_ctx* ctx, float* centroids, int32_t* keys, int32_t* counts, int32_t* nn_index, float* nn_normal8,
                              size_t capacity_voxels) {
   if (!ctx) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_voxel) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, VOXEL)) return s;
+  // asking for the 1-NN outputs without normals fails after the other copies are queued, without waiting for them
+  const bool nn_missing = (nn_index || nn_normal8) && !has(ctx, NORMALS);
   DevState h;
-  gm_status s = sync_state(ctx, &h);
+  gm_status s = download(ctx, &h, n_voxels, capacity_voxels,
+                         {{centroids, ctx->d_centroid, 16}, {keys, ctx->d_vox_key, 4}, {counts, ctx->d_vox_count, 4},
+                          {nn_missing ? nullptr : nn_index, ctx->d_nn_idx, 4}, {nn_missing ? nullptr : nn_normal8, ctx->d_nn_normal, 32}},
+                         !nn_missing);
   if (s != GM_OK) return s;
-  size_t V = (size_t)h.vox.n_voxels;
-  if (V > capacity_voxels) return GM_ERR_CAPACITY;
-  if (centroids) GM_D2H(centroids, ctx->d_centroid, V * 16);
-  if (keys) GM_D2H(keys, ctx->d_vox_key, V * 4);
-  if (counts) GM_D2H(counts, ctx->d_vox_count, V * 4);
-  if ((nn_index || nn_normal8) && !ctx->have_normals) return GM_ERR_STAGE_ORDER;
-  if (nn_index) GM_D2H(nn_index, ctx->d_nn_idx, V * 4);
-  if (nn_normal8) GM_D2H(nn_normal8, ctx->d_nn_normal, V * 32);
-  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (nn_missing) return GM_ERR_STAGE_ORDER;
   if (h.vox.overflow) return GM_WARN_VOXEL_OVERFLOW;
-  if (h.nn_oor && ctx->have_normals) return GM_ERR_NN_INDEX_RANGE;
+  if (h.nn_oor && has(ctx, NORMALS)) return GM_ERR_NN_INDEX_RANGE;
   return GM_OK;
 }
 
 gm_status gm_get_voxel_grid(gm_ctx* ctx, int32_t grid6[6]) {
   if (!ctx || !grid6) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_voxel) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, VOXEL)) return s;
   DevState h;
   gm_status s = sync_state(ctx, &h);
   if (s != GM_OK) return s;
@@ -1511,7 +1508,7 @@ gm_status gm_get_voxel_grid(gm_ctx* ctx, int32_t grid6[6]) {
 
 gm_status gm_get_frame(gm_ctx* ctx, gm_frame* out) {
   if (!ctx || !out) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_frame) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, FRAME)) return s;
   static_assert(sizeof(FrameOut) == sizeof(gm_frame), "frame layout");
   GM_D2H(out, ctx->d_frame, sizeof(gm_frame));
   GM_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1520,7 +1517,7 @@ gm_status gm_get_frame(gm_ctx* ctx, gm_frame* out) {
 
 gm_status gm_download_hypotheses(gm_ctx* ctx, int32_t kind, float* coef, float* test12, int32_t* counts, int32_t capacity_h) {
   if (!ctx || (kind != 0 && kind != 1)) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_ransac[kind]) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, ransac_stage(kind))) return s;
   size_t H = (size_t)ctx->ransac_H[kind];
   if ((int)H > capacity_h) return GM_ERR_CAPACITY;
   if (coef) {
@@ -1535,7 +1532,7 @@ gm_status gm_download_hypotheses(gm_ctx* ctx, int32_t kind, float* coef, float* 
 
 gm_status gm_get_model(gm_ctx* ctx, int32_t kind, gm_model* out) {
   if (!ctx || !out || (kind != 0 && kind != 1)) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_model[kind]) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, model_stage(kind))) return s;
   ModelState h;
   GM_D2H(&h, ctx->d_model + kind, sizeof(ModelState));
   GM_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1548,19 +1545,14 @@ gm_status gm_get_model(gm_ctx* ctx, int32_t kind, gm_model* out) {
 
 gm_status gm_download_labels(gm_ctx* ctx, uint8_t* out, size_t capacity_points) {
   if (!ctx || !out) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_labels) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, LABELS)) return s;
   DevState h;
-  gm_status s = sync_state(ctx, &h);
-  if (s != GM_OK) return s;
-  if ((size_t)h.n_valid > capacity_points) return GM_ERR_CAPACITY;
-  GM_D2H(out, ctx->d_labels, (size_t)h.n_valid);
-  GM_CUDA(cudaStreamSynchronize(ctx->stream));
-  return GM_OK;
+  return download(ctx, &h, n_valid, capacity_points, {{out, ctx->d_labels, 1}});
 }
 
 gm_status gm_download_polyline(gm_ctx* ctx, gm_slice* out, int32_t capacity, int32_t* n_slices) {
   if (!ctx || !n_slices) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_poly) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, POLY)) return s;
   PolyState h;
   GM_D2H(&h, ctx->d_poly, sizeof(PolyState));
   GM_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1576,22 +1568,22 @@ gm_status gm_download_polyline(gm_ctx* ctx, gm_slice* out, int32_t capacity, int
 // ---- pipelined fetch + profiling ---------------------------------------------------------------
 gm_status gm_fetch_async(gm_ctx* ctx, const gm_host_outputs* out) {
   if (!ctx || !out) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_scan) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, SCAN)) return s;
   const size_t n = ctx->n_input;
   if (out->summary) {
-    int mask = (ctx->have_model[0] ? 1 : 0) | (ctx->have_model[1] ? 2 : 0) | (ctx->have_poly ? 4 : 0);
+    int mask = (has(ctx, MODEL_PLANE) ? 1 : 0) | (has(ctx, MODEL_CYL) ? 2 : 0) | (has(ctx, POLY) ? 4 : 0);
     GM_LAUNCH(ctx, k_pack_summary, 1, 32, ctx->d_st, ctx->d_frame, ctx->d_model, ctx->d_poly, mask, ctx->d_summary);
     GM_CHECK_LAUNCHES(ctx);
     GM_CUDA(cudaMemcpyAsync(out->summary, ctx->d_summary, sizeof(SummaryDev), cudaMemcpyDeviceToHost, ctx->stream));
   }
-  if (out->cloud_xyzw && ctx->have_compacted) GM_D2H(out->cloud_xyzw, ctx->d_cloud_c, std::min(n, out->cloud_capacity) * 16);
-  if (out->normals8 && ctx->have_compacted) GM_D2H(out->normals8, ctx->d_normals_c, std::min(n, out->normals_capacity) * 32);
-  if (out->labels && ctx->have_labels) GM_D2H(out->labels, ctx->d_labels, std::min(n, out->labels_capacity));
-  if (out->slices && ctx->have_poly)
+  if (out->cloud_xyzw && has(ctx, COMPACTED)) GM_D2H(out->cloud_xyzw, ctx->d_cloud_c, std::min(n, out->cloud_capacity) * 16);
+  if (out->normals8 && has(ctx, COMPACTED)) GM_D2H(out->normals8, ctx->d_normals_c, std::min(n, out->normals_capacity) * 32);
+  if (out->labels && has(ctx, LABELS)) GM_D2H(out->labels, ctx->d_labels, std::min(n, out->labels_capacity));
+  if (out->slices && has(ctx, POLY))
     GM_D2H(out->slices, ctx->d_slices, (size_t)std::min(ctx->prm.maxSlices, out->slices_capacity) * sizeof(gm_slice));
-  if (ctx->have_voxel) {
+  if (has(ctx, VOXEL)) {
     if (out->centroids_xyzw) GM_D2H(out->centroids_xyzw, ctx->d_centroid, std::min(n, out->voxel_capacity) * 16);
-    if (out->nn_normal8 && ctx->have_normals) GM_D2H(out->nn_normal8, ctx->d_nn_normal, std::min(n, out->voxel_capacity) * 32);
+    if (out->nn_normal8 && has(ctx, NORMALS)) GM_D2H(out->nn_normal8, ctx->d_nn_normal, std::min(n, out->voxel_capacity) * 32);
   }
   return GM_OK;
 }
@@ -1624,10 +1616,7 @@ gm_status gm_profile_read(gm_ctx* ctx, float* ms_sum, int32_t* calls) {
 gm_status gm_inject_compacted(gm_ctx* ctx, const float* xyzw_host, const float* normals8_host, size_t n) {
   if (!ctx || (n && !xyzw_host)) return GM_ERR_INVALID_ARG;
   if (n > ctx->cap) return GM_ERR_CAPACITY;
-  ctx->n_input = n;
-  ctx->n_grid = grid_bucket(n, ctx->cap);
-  ctx->have_scan = true;
-  clear_stages(ctx);
+  new_scan(ctx, n);
   GM_LAUNCH(ctx, k_begin_scan, 1, 32, ctx->d_st, (int)n, (const float4*)nullptr);
   if (n) {
     GM_CUDA(cudaMemcpyAsync(ctx->d_cloud_c, xyzw_host, n * 16, cudaMemcpyHostToDevice, ctx->stream));
@@ -1641,7 +1630,7 @@ gm_status gm_inject_compacted(gm_ctx* ctx, const float* xyzw_host, const float* 
   GM_CUDA(cudaStreamSynchronize(ctx->stream));  // nn is a stack variable
   if (n) GM_LAUNCH(ctx, k_bbox, std::min(div_up((long long)n, 256), ctx->num_sms * 8), 256, ctx->d_cloud_c, &ctx->d_st->vox);
   GM_CHECK_LAUNCHES(ctx);
-  ctx->have_compacted = true;
+  mark(ctx, COMPACTED);
   ctx->injected = true;
   return GM_OK;
 }
@@ -1919,15 +1908,15 @@ gm_status gm_encode_marker_array(const gm_arrow* arrows, int32_t n, const char* 
 // ---- peer-memory collectives (gm_comm.cuh) -----------------------------------------------------------------------
 struct gm_comm {
   int rank = 0, world = 1, device = 0;
-  CommBox* d_box = nullptr;        // this rank's mailbox
-  CommDev* d_dev = nullptr;        // device copy of the peer table
+  DevBuf<CommBox> d_box;  // this rank's mailbox
+  DevBuf<CommDev> d_dev;  // device copy of the peer table
   CommDev h_dev{};
   bool connected = false;
   void* opened[COMM_MAX_RANKS] = {};
   std::string err;
 };
 
-static const CommDev* comm_dev(const gm_ctx* ctx) { return ctx->comm ? ctx->comm->d_dev : nullptr; }
+static const CommDev* comm_dev(const gm_ctx* ctx) { return ctx->comm ? ctx->comm->d_dev.p : nullptr; }
 
 extern "C" {
 
@@ -1941,7 +1930,7 @@ gm_status gm_comm_create(int32_t rank, int32_t world, gm_comm** out) {
   if (!c) return GM_ERR_INTERNAL;
   c->rank = rank; c->world = world;
   cudaGetDevice(&c->device);
-  if (cudaMalloc((void**)&c->d_box, sizeof(CommBox)) != cudaSuccess || cudaMalloc((void**)&c->d_dev, sizeof(CommDev)) != cudaSuccess ||
+  if (c->d_box.alloc(1) != cudaSuccess || c->d_dev.alloc(1) != cudaSuccess ||
       cudaMemset(c->d_box, 0, sizeof(CommBox)) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess) {
     cudaGetLastError();
     gm_comm_destroy(c);
@@ -2006,10 +1995,8 @@ void gm_comm_destroy(gm_comm* c) {
   if (!c) return;
   cudaDeviceSynchronize();
   for (int r = 0; r < COMM_MAX_RANKS; ++r) if (c->opened[r]) cudaIpcCloseMemHandle(c->opened[r]);
-  if (c->d_box) cudaFree(c->d_box);
-  if (c->d_dev) cudaFree(c->d_dev);
-  cudaGetLastError();
   delete c;
+  cudaGetLastError();
 }
 
 int32_t gm_comm_rank(const gm_comm* c) { return c ? c->rank : -1; }
@@ -2019,7 +2006,7 @@ const char* gm_comm_last_error(const gm_comm* c) { return c ? c->err.c_str() : "
 gm_status gm_set_comm(gm_ctx* ctx, gm_comm* comm) {
   if (!ctx) return GM_ERR_INVALID_ARG;
   if (comm && !comm->connected) { ctx->err = "gm_comm is not connected"; return GM_ERR_STAGE_ORDER; }
-  ++ctx->graph_gen;
+  new_graph_generation(ctx);
   ctx->comm = comm;
   return GM_OK;
 }
@@ -2032,7 +2019,7 @@ gm_status gm_set_comm(gm_ctx* ctx, gm_comm* comm) {
 gm_status gm_ransac_sharded(gm_ctx* ctx, const int32_t* plane_samples_host, int32_t Hp, const int32_t* cyl_samples_host, int32_t Hc) {
   if (!ctx || Hp <= 0 || Hc <= 0 || !plane_samples_host || !cyl_samples_host) return GM_ERR_INVALID_ARG;
   if (!ctx->comm) { ctx->err = "gm_ransac_sharded needs gm_set_comm"; return GM_ERR_STAGE_ORDER; }
-  if (!ctx->have_compacted) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, COMPACTED)) return s;
   const int W = ctx->comm->world, R = ctx->comm->rank;
   auto range = [&](int H, int& b, int& e) { const int per = (H + W - 1) / W; b = std::min(R * per, H); e = std::min((R + 1) * per, H); };
   int pb, pe, cb, ce;
@@ -2077,7 +2064,10 @@ gm_status gm_ransac_sharded(gm_ctx* ctx, const int32_t* plane_samples_host, int3
   };
   // (world, rank) are part of what is launched: the comm is attached with gm_set_comm, which starts a new graph generation
   gm_status s = run_graphed(ctx, 1, Hp, Hc, stage, body);
-  if (s == GM_OK) for (int k = 0; k < 2; ++k) { ctx->have_ransac[k] = true; ctx->have_model[k] = true; ctx->ransac_H[k] = k == 0 ? Hp : Hc; }
+  if (s == GM_OK) {
+    mark(ctx, RANSAC_PLANE, RANSAC_CYL, MODEL_PLANE, MODEL_CYL);
+    ctx->ransac_H[0] = Hp; ctx->ransac_H[1] = Hc;
+  }
   return s;
 }
 
@@ -2086,7 +2076,7 @@ gm_status gm_ransac_sharded(gm_ctx* ctx, const int32_t* plane_samples_host, int3
 gm_status gm_allreduce_voxel_bbox(gm_ctx* ctx) {
   if (!ctx) return GM_ERR_INVALID_ARG;
   if (!ctx->comm) { ctx->err = "needs gm_set_comm"; return GM_ERR_STAGE_ORDER; }
-  if (!ctx->have_compacted) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, COMPACTED)) return s;
   GM_LAUNCH(ctx, k_comm_bbox, 1, 32, ctx->comm->h_dev, ctx->d_st->vox.bbox_min, ctx->d_st->vox.bbox_max, &ctx->d_st->error);
   GM_CHECK_LAUNCHES(ctx);
   return GM_OK;
@@ -2097,7 +2087,7 @@ gm_status gm_allreduce_voxel_bbox(gm_ctx* ctx) {
 gm_status gm_allreduce_frame(gm_ctx* ctx) {
   if (!ctx) return GM_ERR_INVALID_ARG;
   if (!ctx->comm) { ctx->err = "needs gm_set_comm"; return GM_ERR_STAGE_ORDER; }
-  if (!ctx->have_frame) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, FRAME)) return s;
   GM_LAUNCH(ctx, k_comm_sum, 1, 32, ctx->comm->h_dev, ctx->d_frame_sums, 6, &ctx->d_st->error);
   GM_LAUNCH(ctx, k_frame_solve, 1, 32, ctx->d_frame_sums, ctx->d_frame);
   GM_CHECK_LAUNCHES(ctx);
@@ -2111,11 +2101,11 @@ struct gm_map {
   double leaf = 0.1;
   float inv_leaf = 10.f;
   unsigned long long n_slots = 0;
-  unsigned long long* d_keys = nullptr;
-  int* d_cnt = nullptr;
-  long long* d_sums = nullptr;
-  MapState* d_st = nullptr;
-  int* d_cursor = nullptr;
+  DevBuf<unsigned long long> d_keys;
+  DevBuf<int> d_cnt;
+  DevBuf<long long> d_sums;
+  DevBuf<MapState> d_st;
+  DevBuf<int> d_cursor;
   int num_sms = 148;
   std::string err;
 };
@@ -2138,10 +2128,8 @@ gm_status map_dump(gm_map* m, MapDump* out, MapState* st_out) {
   if (cudaMemcpy(&st, m->d_st, sizeof(st), cudaMemcpyDeviceToHost) != cudaSuccess) { m->err = "memcpy"; return GM_ERR_CUDA; }
   if (st_out) *st_out = st;
   const size_t V = (size_t)std::max(st.n_voxels, 0);
-  unsigned long long* dk = nullptr; int* dc = nullptr; long long* ds = nullptr;
-  if (dmalloc(&dk, V) != cudaSuccess || dmalloc(&dc, V) != cudaSuccess || dmalloc(&ds, 3 * V) != cudaSuccess) {
-    cudaFree(dk); cudaFree(dc); cudaFree(ds); m->err = "cudaMalloc"; return GM_ERR_CUDA;
-  }
+  DevBuf<unsigned long long> dk; DevBuf<int> dc; DevBuf<long long> ds;
+  if (dk.alloc(V) != cudaSuccess || dc.alloc(V) != cudaSuccess || ds.alloc(3 * V) != cudaSuccess) { m->err = "cudaMalloc"; return GM_ERR_CUDA; }
   cudaMemset(m->d_cursor, 0, sizeof(int));
   cudaDeviceSynchronize();
   if (V) k_map_export<<<std::min<unsigned long long>((m->n_slots + 255) / 256, (unsigned long long)m->num_sms * 16), 256>>>(
@@ -2150,7 +2138,6 @@ gm_status map_dump(gm_map* m, MapDump* out, MapState* st_out) {
   cudaError_t e = cudaMemcpy(k.data(), dk, V * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
   if (e == cudaSuccess) e = cudaMemcpy(c.data(), dc, V * sizeof(int), cudaMemcpyDeviceToHost);
   if (e == cudaSuccess) e = cudaMemcpy(su.data(), ds, 3 * V * sizeof(long long), cudaMemcpyDeviceToHost);
-  cudaFree(dk); cudaFree(dc); cudaFree(ds);
   if (e != cudaSuccess) { m->err = cudaGetErrorString(e); return GM_ERR_CUDA; }
   std::vector<size_t> order(V);
   for (size_t i = 0; i < V; ++i) order[i] = i;
@@ -2182,8 +2169,8 @@ gm_status gm_map_create(double leaf, size_t capacity_voxels, gm_map** out) {
   int dev = 0; cudaGetDevice(&dev);
   cudaDeviceProp prop;
   if (cudaGetDeviceProperties(&prop, dev) == cudaSuccess) m->num_sms = prop.multiProcessorCount;
-  if (dmalloc(&m->d_keys, slots) != cudaSuccess || dmalloc(&m->d_cnt, slots) != cudaSuccess || dmalloc(&m->d_sums, 3 * slots) != cudaSuccess ||
-      dmalloc(&m->d_st, 1) != cudaSuccess || dmalloc(&m->d_cursor, 1) != cudaSuccess || map_clear_device(m) != GM_OK) {
+  if (m->d_keys.alloc(slots) != cudaSuccess || m->d_cnt.alloc(slots) != cudaSuccess || m->d_sums.alloc(3 * slots) != cudaSuccess ||
+      m->d_st.alloc(1) != cudaSuccess || m->d_cursor.alloc(1) != cudaSuccess || map_clear_device(m) != GM_OK) {
     gm_map_destroy(m);
     return GM_ERR_CUDA;
   }
@@ -2194,7 +2181,6 @@ gm_status gm_map_create(double leaf, size_t capacity_voxels, gm_map** out) {
 void gm_map_destroy(gm_map* m) {
   if (!m) return;
   cudaDeviceSynchronize();
-  cudaFree(m->d_keys); cudaFree(m->d_cnt); cudaFree(m->d_sums); cudaFree(m->d_st); cudaFree(m->d_cursor);
   delete m;
 }
 
@@ -2206,7 +2192,8 @@ gm_status gm_map_clear(gm_map* m) {
 
 gm_status gm_map_insert(gm_map* m, gm_ctx* ctx, const float* pose34, int32_t label_filter) {
   if (!m || !ctx || label_filter > 255) return GM_ERR_INVALID_ARG;
-  if (!ctx->have_compacted || (label_filter >= 0 && !ctx->have_labels)) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(ctx, COMPACTED)) return s;
+  if (label_filter >= 0 && !has(ctx, LABELS)) return GM_ERR_STAGE_ORDER;
   if (ctx->n_input == 0) return GM_OK;
   Pose34 T{};
   if (pose34) std::memcpy(T.r, pose34, sizeof(T.r));
@@ -2292,10 +2279,10 @@ gm_status gm_map_load(const char* path, size_t min_capacity_voxels, gm_map** out
   gm_status s = gm_map_create(leaf, std::max<size_t>(std::max<size_t>(min_capacity_voxels, (size_t)V), 1), &m);
   if (s != GM_OK) return s;
   if (V) {
-    unsigned long long* dk = nullptr; int* dc = nullptr; long long* ds = nullptr;
-    cudaError_t e = dmalloc(&dk, (size_t)V);
-    if (e == cudaSuccess) e = dmalloc(&dc, (size_t)V);
-    if (e == cudaSuccess) e = dmalloc(&ds, 3 * (size_t)V);
+    DevBuf<unsigned long long> dk; DevBuf<int> dc; DevBuf<long long> ds;
+    cudaError_t e = dk.alloc((size_t)V);
+    if (e == cudaSuccess) e = dc.alloc((size_t)V);
+    if (e == cudaSuccess) e = ds.alloc(3 * (size_t)V);
     if (e == cudaSuccess) e = cudaMemcpy(dk, k.data(), V * 8, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaMemcpy(dc, c.data(), V * 4, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaMemcpy(ds, su.data(), 3 * V * 8, cudaMemcpyHostToDevice);
@@ -2304,7 +2291,6 @@ gm_status gm_map_load(const char* path, size_t min_capacity_voxels, gm_map** out
                                                                                                      m->n_slots - 1ull, m->d_st);
       e = cudaDeviceSynchronize();
     }
-    cudaFree(dk); cudaFree(dc); cudaFree(ds);
     if (e != cudaSuccess) { gm_map_destroy(m); return GM_ERR_CUDA; }
   }
   *out = m;
