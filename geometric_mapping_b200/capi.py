@@ -84,6 +84,20 @@ class gm_compression(C.Structure):
                 ("bytes_out", C.c_uint64)]
 
 
+class gm_primitive(C.Structure):
+    _fields_ = [("model", gm_model), ("n_remaining", C.c_int32), ("pad_", C.c_int32)]
+
+
+class gm_primitive_compression(C.Structure):
+    _fields_ = [("n_points", C.c_int32), ("n_primitives", C.c_int32), ("n_residual", C.c_int32), ("n_residual_voxels", C.c_int32),
+                ("leaf", C.c_float), ("residual_rms", C.c_float), ("total_rms", C.c_float), ("ratio", C.c_float),
+                ("bytes_in", C.c_uint64), ("bytes_out", C.c_uint64)]
+
+
+GM_MAX_PRIMITIVES = 64
+PRIMITIVE_RECORD_DTYPE = np.dtype([("kind", "<i4"), ("count", "<i4"), ("coef", "<f4", 7), ("extents", "<f4", 4), ("rms", "<f4")])
+
+
 class gm_scan_summary(C.Structure):
     _fields_ = [("counts", gm_counts), ("frame", gm_frame), ("plane", gm_model), ("cylinder", gm_model),
                 ("n_slices", C.c_int32), ("pad_", C.c_int32)]
@@ -129,6 +143,8 @@ SYMBOLS = [
     "gm_ransac_import_keys", "gm_map_create", "gm_map_destroy", "gm_map_clear", "gm_map_insert", "gm_map_stats", "gm_map_download", "gm_map_save",
     "gm_map_load", "gm_map_leaf", "gm_set_normals_mode", "gm_set_graph_mode", "gm_get_graph_stats",
     "gm_comm_create", "gm_comm_handle", "gm_comm_connect", "gm_comm_mailbox", "gm_comm_connect_local", "gm_comm_destroy", "gm_comm_rank", "gm_comm_world", "gm_comm_last_error", "gm_set_comm", "gm_ransac_sharded", "gm_allreduce_voxel_bbox", "gm_allreduce_frame", "gm_set_voxel_bbox_hint", "gm_set_knn", "gm_download_knn_indices", "gm_set_knn_max_radius", "gm_pointcloud2_size", "gm_encode_pointcloud2", "gm_marker_array_size",
+    "gm_extract_primitives", "gm_get_primitives", "gm_download_primitive_ids", "gm_compress_primitives",
+    "gm_download_compressed_primitives",
     "gm_encode_marker_array", "gm_store_open", "gm_store_close", "gm_store_append", "gm_store_append_blob", "gm_store_count", "gm_store_info", "gm_store_read",
 ]
 
@@ -250,6 +266,11 @@ def _lib():
         "gm_map_save": (i32, [vp, C.c_char_p]),
         "gm_map_load": (i32, [C.c_char_p, sz, C.POINTER(vp)]),
         "gm_map_leaf": (C.c_double, [vp]),
+        "gm_extract_primitives": (i32, [vp, i32, i32, vp, i32, vp, i32]),
+        "gm_get_primitives": (i32, [vp, vp, i32, C.POINTER(i32)]),
+        "gm_download_primitive_ids": (i32, [vp, vp, sz]),
+        "gm_compress_primitives": (i32, [vp]),
+        "gm_download_compressed_primitives": (i32, [vp, vp, sz, C.POINTER(sz)]),
     }
     assert set(sig) == set(SYMBOLS)
     for name, (res, args) in sig.items():
@@ -648,6 +669,79 @@ def _ctx_download_compressed(self) -> bytes:
     return buf.tobytes()
 
 
+def _ctx_extract_primitives(self, plane_draws: np.ndarray | None, cyl_draws: np.ndarray | None, max_primitives: int,
+                            min_inliers: int):
+    """Sequential multi-primitive extraction (gm_extract_primitives).  plane_draws: max_primitives x Hp x 3 uint32,
+    cyl_draws: max_primitives x Hc x 2 uint32 (None = no hypotheses of that kind)."""
+    draws = []
+    for d, per in ((plane_draws, 3), (cyl_draws, 2)):
+        if d is None:
+            draws.append((None, 0))
+            continue
+        a = np.ascontiguousarray(d, dtype=np.uint32)
+        if a.ndim != 3 or a.shape[0] != max_primitives or a.shape[2] != per:
+            raise ValueError(f"draws must be max_primitives x H x {per}")
+        draws.append((a, a.shape[1]))
+    (pd, hp), (cd, hc) = draws
+    self._ck(_lib().gm_extract_primitives(self._h, int(max_primitives), int(min_inliers), _ptr(pd), hp, _ptr(cd), hc),
+             "gm_extract_primitives")
+
+
+def _ctx_primitives(self) -> list:
+    """The extracted primitives in extraction order: dicts of gm_primitive (hyp / coef trimmed to 4 or 7 values)."""
+    n = C.c_int32(0)
+    self._ck(_lib().gm_get_primitives(self._h, None, 0, C.byref(n)), "gm_get_primitives")
+    out = (gm_primitive * max(n.value, 1))()
+    self._ck(_lib().gm_get_primitives(self._h, out, n.value, C.byref(n)), "gm_get_primitives")
+    res = []
+    for p in out[: n.value]:
+        m = p.model
+        k = 4 if m.kind == GM_MODEL_PLANE else 7
+        res.append({"kind": m.kind, "best_id": m.best_id, "best_count": m.best_count, "refit_count": m.refit_count,
+                    "hyp": np.array(m.hyp[:k], np.float32), "coef": np.array(m.coef[:k], np.float32), "rms": float(m.rms),
+                    "n_remaining": p.n_remaining})
+    return res
+
+
+def _ctx_download_primitive_ids(self) -> np.ndarray:
+    out = np.empty(max(self.counts().n_valid, 0), np.uint8)
+    self._ck(_lib().gm_download_primitive_ids(self._h, _ptr(out), out.shape[0]), "gm_download_primitive_ids")
+    return out
+
+
+def _ctx_compress_primitives(self):
+    self._ck(_lib().gm_compress_primitives(self._h), "gm_compress_primitives")
+
+
+def _ctx_download_compressed_primitives(self) -> bytes:
+    n = C.c_size_t(0)
+    self._ck(_lib().gm_download_compressed_primitives(self._h, None, 0, C.byref(n)), "gm_download_compressed_primitives")
+    buf = np.empty(n.value, np.uint8)
+    self._ck(_lib().gm_download_compressed_primitives(self._h, _ptr(buf), buf.shape[0], C.byref(n)), "gm_download_compressed_primitives")
+    return buf.tobytes()
+
+
+def parse_compressed_primitives(blob: bytes) -> dict:
+    """GMP1 blob -> {"header": gm_primitive_compression, "records": PRIMITIVE_RECORD_DTYPE array, "residual": V x 3 float32}."""
+    magic, version = np.frombuffer(blob, "<u4", 2)
+    if magic != 0x31504D47 or version != 1:
+        raise ValueError("not a GMP1 blob")
+    hs = C.sizeof(gm_primitive_compression)
+    h = gm_primitive_compression.from_buffer_copy(blob[8:8 + hs])
+    off = 8 + hs
+    rec = np.frombuffer(blob, PRIMITIVE_RECORD_DTYPE, h.n_primitives, off).copy()
+    off += h.n_primitives * PRIMITIVE_RECORD_DTYPE.itemsize
+    res = np.frombuffer(blob, "<f4", 3 * h.n_residual_voxels, off).reshape(-1, 3).copy()
+    if off + res.nbytes != len(blob):
+        raise ValueError("GMP1 blob size does not match its header")
+    return {"header": h, "records": rec, "residual": res}
+
+
+Context.extract_primitives = _ctx_extract_primitives
+Context.primitives = _ctx_primitives
+Context.download_primitive_ids = _ctx_download_primitive_ids
+Context.compress_primitives = _ctx_compress_primitives
+Context.download_compressed_primitives = _ctx_download_compressed_primitives
 Context.compress = _ctx_compress
 Context.compression = _ctx_compression
 Context.download_compressed = _ctx_download_compressed

@@ -6,6 +6,7 @@
 #include "gm_ransac.cuh"
 #include "gm_polyline.cuh"
 #include "gm_compress.cuh"
+#include "gm_primitives.cuh"
 #include "gm_map.cuh"
 #include "gm_comm.cuh"
 #include <new>
@@ -181,6 +182,24 @@ struct gm_ctx {
   DevBuf<unsigned long long> d_comp_mm;
   DevBuf<unsigned> d_counters;  // last-block tickets: [0] frame, [1] plane refit, [2] cylinder GN
   DevBuf<float4> d_inl;         // compacted cylinder inliers
+  // sequential multi-primitive extraction (gm_primitives.cuh), allocated by the first gm_extract_primitives.  Its
+  // tickets, partials, look-back states and d_inl are the scratch gm_ransac uses (same stream order, never concurrent).
+  DevBuf<float4> d_pr_sv, d_pr_cc, d_pr_lb;  // working copies with the claimed points blanked: cell-sorted cloud, compacted cloud, leaf bounds
+  DevBuf<int> d_pr_rem;                      // R_r
+  DevBuf<unsigned char> d_pr_ids;            // primitive id per compacted point
+  DevBuf<unsigned> d_pr_draws[2];
+  DevBuf<int> d_pr_samples[2];
+  DevBuf<float4> d_pr_plane_coef;
+  DevBuf<float> d_pr_model7, d_pr_test12;
+  DevBuf<int> d_pr_hvalid[2], d_pr_counts[2];
+  DevBuf<unsigned long long> d_pr_key;  // [2]
+  DevBuf<ModelState> d_pr_model;        // [2]
+  DevBuf<PrimState> d_pr_state;
+  // compression of the extracted primitives: the residual cloud goes to d_pr_sv, its centroids to d_pr_cc
+  DevBuf<int> d_pr_assign, d_pr_vox_start, d_pr_vox_key, d_pr_vox_count;
+  DevBuf<VoxState> d_pr_vs;
+  DevBuf<PrimComp> d_pr_comp;
+  DevBuf<CompStats> d_pr_stats;
   // CUDA-graph replay of gm_process_scan: the launch sequence of one scan depends only on (bucketed size, hypothesis
   // counts, parameters / modes), never on per-scan host values (tile epochs, barrier parities and the scan pointer
   // live in device memory), so it is captured once per key and replayed with ONE cudaGraphLaunch
@@ -223,9 +242,11 @@ struct SegTimer {
 // The results a context holds, in pipeline order.  A stage's entry point fails with GM_ERR_STAGE_ORDER unless the
 // stages it reads are held, and marks its own stage.  Running a stage again does not drop the later ones.  A change
 // of input drops a stage and everything after it: a new scan from CROP on, a new crop box or is_dense from CROP on, a
-// new neighbour grid from NORMALS on (the compacted cloud too, even an injected one).
+// new neighbour grid from NORMALS on (the compacted cloud too, even an injected one).  A new extraction drops the
+// compression of the previous one (PRIMS_COMP), whose buffers it reuses.
 enum Stage {
-  SCAN, CROP, NORMALS, COMPACTED, VOXEL, FRAME, RANSAC_PLANE, RANSAC_CYL, MODEL_PLANE, MODEL_CYL, LABELS, POLY, COMP
+  SCAN, CROP, NORMALS, COMPACTED, VOXEL, FRAME, RANSAC_PLANE, RANSAC_CYL, MODEL_PLANE, MODEL_CYL, LABELS, POLY, COMP,
+  PRIMS, PRIMS_COMP
 };
 inline Stage ransac_stage(int kind) { return Stage(RANSAC_PLANE + kind); }
 inline Stage model_stage(int kind) { return Stage(MODEL_PLANE + kind); }
@@ -1413,6 +1434,259 @@ gm_status gm_ransac_import_keys(gm_ctx* ctx, const void* src_device) {
   if (!ctx || !src_device) return GM_ERR_INVALID_ARG;
   if (gm_status s = require(ctx, RANSAC_PLANE, RANSAC_CYL)) return s;
   GM_CUDA(cudaMemcpyAsync(ctx->d_key, src_device, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
+  return GM_OK;
+}
+
+}  // extern "C"
+
+// ---- sequential multi-primitive extraction (gm_primitives.cuh) -------------------------------------------------------
+namespace {
+static_assert(sizeof(PrimRec) == sizeof(gm_primitive), "primitive layout");
+static_assert(sizeof(PrimCompRec) == sizeof(gm_primitive_record), "primitive record layout");
+
+// The first call allocates the working copies and hypothesis tables; the draw buffers grow to the largest call.  Rare
+// path (synchronous): a context that never extracts keeps its footprint.
+gm_status ensure_prim_buffers(gm_ctx* ctx, size_t plane_draws, size_t cyl_draws) {
+  const bool first = ctx->d_pr_state.count == 0;
+  if (!first && plane_draws <= ctx->d_pr_draws[0].count && cyl_draws <= ctx->d_pr_draws[1].count) return GM_OK;
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (first || plane_draws > ctx->d_pr_draws[0].count) GM_CUDA(ctx->d_pr_draws[0].alloc(plane_draws));
+  if (first || cyl_draws > ctx->d_pr_draws[1].count) GM_CUDA(ctx->d_pr_draws[1].alloc(cyl_draws));
+  if (!first) return GM_OK;
+  const size_t N = ctx->cap, H = (size_t)ctx->hcap;
+  GM_CUDA(ctx->d_pr_sv.alloc(N)); GM_CUDA(ctx->d_pr_cc.alloc(N)); GM_CUDA(ctx->d_pr_lb.alloc(2 * ((N + 31) / 32)));
+  GM_CUDA(ctx->d_pr_rem.alloc(N)); GM_CUDA(ctx->d_pr_ids.alloc(N));
+  GM_CUDA(ctx->d_pr_samples[0].alloc(3 * H)); GM_CUDA(ctx->d_pr_samples[1].alloc(2 * H));
+  GM_CUDA(ctx->d_pr_plane_coef.alloc(H)); GM_CUDA(ctx->d_pr_model7.alloc(7 * H)); GM_CUDA(ctx->d_pr_test12.alloc(12 * H));
+  for (int k = 0; k < 2; ++k) { GM_CUDA(ctx->d_pr_hvalid[k].alloc(H)); GM_CUDA(ctx->d_pr_counts[k].alloc(H)); }
+  GM_CUDA(ctx->d_pr_key.alloc(2)); GM_CUDA(ctx->d_pr_model.alloc(2));
+  GM_CUDA(ctx->d_pr_state.alloc(1));  // last: a failure above leaves the set unallocated
+  return GM_OK;
+}
+
+// Hypotheses, inlier counts and argmax of one kind in one round: the launches of gm_ransac on the extraction's tables.
+// Hypotheses read the original compacted cloud (R_r indices are never blanked); counts read the blanked working copies
+// through the live sizes, which are 0 once extraction stopped.
+gm_status prim_count(gm_ctx* ctx, int kind, int H, bool tiles) {
+  PrimState* ps = ctx->d_pr_state;
+  const int* n_valid = &ctx->d_st->n_valid;
+  const float tau = (float)ctx->prm.ransacThreshold;
+  const int hb = div_up(H, 128);
+  if (kind == 0) {
+    GM_LAUNCH(ctx, k_plane_hypotheses, hb, 128, ctx->d_cloud_c, n_valid, ctx->d_pr_samples[0], H, ctx->d_pr_plane_coef, ctx->d_pr_hvalid[0],
+              ctx->d_pr_counts[0], 0, H, 1);
+  } else {
+    GM_LAUNCH(ctx, k_cyl_hypotheses, hb, 128, ctx->d_cloud_c, ctx->d_normals_c, n_valid, ctx->d_pr_samples[1], H,
+              (float)ctx->prm.cylinderRadiusMin, (float)ctx->prm.cylinderRadiusMax, tau, ctx->d_pr_model7, ctx->d_pr_test12,
+              ctx->d_pr_hvalid[1], ctx->d_pr_counts[1], 0, H, 1);
+  }
+  if (tiles) {
+    const int blocks = std::max(1, div_up((long long)ctx->n_grid, TC_SUPER));
+    if (kind == 0) {
+      GM_LAUNCH(ctx, k_count_tiles<0>, blocks, TC_BLOCK, ctx->d_pr_sv, ctx->d_pr_lb, &ps->n_crop_live, ctx->d_pr_plane_coef, ctx->d_pr_test12,
+                ctx->d_pr_hvalid[0], 0, H, tau, ctx->d_pr_counts[0], H, ctx->d_pr_key + 0, ctx->d_counters + 3, nullptr, ctx->d_pr_model7);
+    } else {
+      GM_LAUNCH(ctx, k_count_tiles<1>, blocks, TC_BLOCK, ctx->d_pr_sv, ctx->d_pr_lb, &ps->n_crop_live, ctx->d_pr_plane_coef, ctx->d_pr_test12,
+                ctx->d_pr_hvalid[1], 0, H, tau, ctx->d_pr_counts[1], H, ctx->d_pr_key + 1, ctx->d_counters + 4, nullptr, ctx->d_pr_model7);
+    }
+  } else {
+    const int K = kind == 0 ? RC_KP : RC_KC;
+    const int groups = div_up(H, RC_BLOCK * K);
+    const int slices = std::max(1, std::min(div_up((long long)ctx->n_grid, RC_TILE / 2), div_up(ctx->num_sms * 8, groups)));
+    const dim3 grid(slices, groups);
+    if (kind == 0) {
+      GM_LAUNCH(ctx, k_count_plane<RC_KP>, grid, RC_BLOCK, ctx->d_pr_cc, &ps->n_valid_live, ctx->d_pr_plane_coef, ctx->d_pr_hvalid[0], 0, H, tau,
+                ctx->d_pr_counts[0], H, ctx->d_pr_key + 0, ctx->d_counters + 3, nullptr);
+    } else {
+      GM_LAUNCH(ctx, k_count_cyl<RC_KC>, grid, RC_BLOCK, ctx->d_pr_cc, &ps->n_valid_live, ctx->d_pr_test12, 0, H, ctx->d_pr_counts[1], H,
+                ctx->d_pr_key + 1, ctx->d_counters + 4, nullptr, ctx->d_pr_model7);
+    }
+  }
+  GM_CHECK_LAUNCHES(ctx);
+  return GM_OK;
+}
+
+// Refit of one kind on the blanked compacted copy: the launches of gm_ransac_select on the extraction's key and model.
+// The key of a kind that did not win the round is 0, so its refit finds no model.
+gm_status prim_refit(gm_ctx* ctx, int kind, int H) {
+  PrimState* ps = ctx->d_pr_state;
+  ModelState* ms = ctx->d_pr_model + kind;
+  const float tau = (float)ctx->prm.ransacThreshold;
+  if (kind == 0) {
+    GM_LAUNCH(ctx, k_plane_refit, REFIT_BLOCKS, RF_BLOCK, ctx->d_pr_cc, &ps->n_valid_live, ctx->d_pr_key + 0, H, ctx->d_pr_plane_coef, ms, tau,
+              ctx->d_partials + 1 * kPartialsRegion, ctx->d_counters + 1);
+  } else {
+    GM_LAUNCH(ctx, k_cyl_inlier_compact, std::max(1, div_up((long long)ctx->n_grid, CPL_TILE)), CP_BLOCK, ctx->d_pr_cc, &ps->n_valid_live,
+              ctx->d_pr_key + 1, H, ctx->d_pr_model7, ctx->d_pr_test12, ms, ctx->d_inl, ctx->d_state64_b, ctx->d_ctl + 1, &ctx->d_st->error);
+    const float4* inl = ctx->d_inl;
+    int iters = ctx->prm.refitIterations;
+    double* partials = ctx->d_partials + 2 * kPartialsRegion;
+    unsigned* bars = ctx->d_counters + 5;
+    int* err = &ctx->d_st->error;
+    void* args[] = {(void*)&inl, (void*)&ms, (void*)&iters, (void*)&tau, (void*)&partials, (void*)&bars, (void*)&err};
+    GM_CUDA(cudaLaunchCooperativeKernel((const void*)k_cyl_gn_all, dim3(ctx->gn_blocks), dim3(RF_BLOCK), args, 0, ctx->stream));
+    ++ctx->launches;
+  }
+  GM_CHECK_LAUNCHES(ctx);
+  return GM_OK;
+}
+
+gm_status extract_rounds(gm_ctx* ctx, int K, int min_inliers, int Hp, int Hc) {
+  const size_t n = ctx->n_grid;
+  // the scan's cell-sorted copy exists: claims walk it and keep its leaf bounds current; counting uses it unless count_mode = 1
+  const bool sorted = has(ctx, NORMALS) && !ctx->injected;
+  const bool tiles = sorted && ctx->count_mode == 0;
+  GM_CUDA(cudaMemsetAsync(ctx->d_pr_ids, 0, n, ctx->stream));
+  GM_CUDA(cudaMemcpyAsync(ctx->d_pr_cc, ctx->d_cloud_c, n * sizeof(float4), cudaMemcpyDeviceToDevice, ctx->stream));
+  if (sorted) {
+    GM_CUDA(cudaMemcpyAsync(ctx->d_pr_sv, ctx->d_sorted_valid, n * sizeof(float4), cudaMemcpyDeviceToDevice, ctx->stream));
+    GM_CUDA(cudaMemcpyAsync(ctx->d_pr_lb, ctx->d_leaf_bounds, 2 * ((n + 31) / 32) * sizeof(float4), cudaMemcpyDeviceToDevice, ctx->stream));
+  }
+  const int H[2] = {Hp, Hc};
+  gm_status s;
+  // the plane step on branch stream 1 and the cylinder step on the main stream, side by side as in gm_ransac_pair
+  auto both = [&](auto&& step) -> gm_status {
+    if (ctx->concurrent && !ctx->profiling && Hp > 0 && Hc > 0) {
+      GM_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
+      if ((s = run_branch(ctx, 1, [&] { return step(0); })) != GM_OK) return s;
+      if ((s = step(1)) != GM_OK) return s;
+      GM_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join[1], 0));
+      return GM_OK;
+    }
+    for (int k = 0; k < 2; ++k)
+      if (H[k] > 0 && (s = step(k)) != GM_OK) return s;
+    return GM_OK;
+  };
+  const int draws = Hp * 3 + Hc * 2;
+  const int point_blocks = std::min(div_up((long long)n, 256), ctx->num_sms * 8);
+  for (int r = 0; r < K; ++r) {
+    GM_LAUNCH(ctx, k_prim_remaining, std::max(1, div_up((long long)n, CPL_TILE)), CP_BLOCK, ctx->d_pr_ids, ctx->d_pr_state, ctx->d_pr_rem,
+              ctx->d_state64, ctx->d_ctl + 0, &ctx->d_st->error);
+    GM_LAUNCH(ctx, k_prim_draws, std::max(1, std::min(div_up(draws, 256), ctx->num_sms * 4)), 256, ctx->d_pr_draws[0] + (size_t)r * Hp * 3, Hp * 3,
+              ctx->d_pr_draws[1] + (size_t)r * Hc * 2, Hc * 2, ctx->d_pr_rem, ctx->d_pr_state, ctx->d_pr_samples[0], ctx->d_pr_samples[1]);
+    if ((s = both([&](int k) { return prim_count(ctx, k, H[k], tiles); })) != GM_OK) return s;
+    GM_LAUNCH(ctx, k_prim_decide, 1, 32, ctx->d_pr_key, Hp > 0 ? 1 : 0, Hc > 0 ? 1 : 0, min_inliers, Hp, Hc, ctx->d_pr_plane_coef, ctx->d_pr_test12,
+              ctx->d_pr_state);
+    if ((s = both([&](int k) { return prim_refit(ctx, k, H[k]); })) != GM_OK) return s;
+    const float tau = (float)ctx->prm.ransacThreshold;
+    if (sorted) {
+      GM_LAUNCH(ctx, k_prim_claim_sorted, point_blocks, 256, ctx->d_pr_sv, ctx->d_pr_lb, ctx->d_valid_map, ctx->d_pr_cc, ctx->d_pr_ids,
+                ctx->d_pr_state, ctx->d_pr_model, tau, r);
+    } else {
+      GM_LAUNCH(ctx, k_prim_claim_compact, point_blocks, 256, ctx->d_pr_cc, ctx->d_pr_ids, ctx->d_pr_state, ctx->d_pr_model, tau, r);
+    }
+    GM_CHECK_LAUNCHES(ctx);
+  }
+  return GM_OK;
+}
+
+// Compression buffers of the extracted primitives (first gm_compress_primitives; rare path, synchronous)
+gm_status ensure_prim_comp_buffers(gm_ctx* ctx) {
+  if (ctx->d_pr_stats.count) return GM_OK;
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  const size_t N = ctx->cap;
+  GM_CUDA(ctx->d_pr_assign.alloc(N)); GM_CUDA(ctx->d_pr_vox_start.alloc(N + 1)); GM_CUDA(ctx->d_pr_vox_key.alloc(N));
+  GM_CUDA(ctx->d_pr_vox_count.alloc(N)); GM_CUDA(ctx->d_pr_vs.alloc(1)); GM_CUDA(ctx->d_pr_comp.alloc(1));
+  GM_CUDA(ctx->d_pr_stats.alloc(1));  // last: a failure above leaves the set unallocated
+  return GM_OK;
+}
+}  // namespace
+
+extern "C" {
+
+gm_status gm_extract_primitives(gm_ctx* ctx, int32_t max_primitives, int32_t min_inliers, const uint32_t* plane_draws_host, int32_t Hp,
+                                const uint32_t* cyl_draws_host, int32_t Hc) {
+  if (!ctx || max_primitives < 0 || max_primitives > GM_MAX_PRIMITIVES || Hp < 0 || Hc < 0 || (Hp > 0 && !plane_draws_host) ||
+      (Hc > 0 && !cyl_draws_host))
+    return GM_ERR_INVALID_ARG;
+  if (gm_status s = require(ctx, COMPACTED)) return s;
+  if (Hp > ctx->hcap || Hc > ctx->hcap) { ctx->err = "H larger than max_hypotheses"; return GM_ERR_CAPACITY; }
+  const size_t np = (size_t)max_primitives * Hp * 3, nc = (size_t)max_primitives * Hc * 2;
+  gm_status s = ensure_prim_buffers(ctx, np, nc);
+  if (s != GM_OK) return s;
+  ctx->stages &= ~((1u << PRIMS) | (1u << PRIMS_COMP));
+  if (np) GM_CUDA(cudaMemcpyAsync(ctx->d_pr_draws[0], plane_draws_host, np * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+  if (nc) GM_CUDA(cudaMemcpyAsync(ctx->d_pr_draws[1], cyl_draws_host, nc * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+  GM_LAUNCH(ctx, k_prim_begin, 1, 32, ctx->d_pr_state, ctx->d_st);
+  GM_CHECK_LAUNCHES(ctx);
+  if (ctx->n_grid && (s = extract_rounds(ctx, max_primitives, min_inliers, Hp, Hc)) != GM_OK) return s;
+  mark(ctx, PRIMS);
+  return GM_OK;
+}
+
+gm_status gm_get_primitives(gm_ctx* ctx, gm_primitive* out, int32_t capacity, int32_t* n) {
+  if (!ctx || !n) return GM_ERR_INVALID_ARG;
+  if (gm_status s = require(ctx, PRIMS)) return s;
+  int np = 0;
+  GM_CUDA(cudaMemcpyAsync(&np, &ctx->d_pr_state->n_prims, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  *n = np;
+  if (!out) return GM_OK;
+  if (np > capacity) return GM_ERR_CAPACITY;
+  GM_CUDA(cudaMemcpyAsync(out, ctx->d_pr_state->prim, (size_t)np * sizeof(gm_primitive), cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  return GM_OK;
+}
+
+gm_status gm_download_primitive_ids(gm_ctx* ctx, uint8_t* out, size_t capacity_points) {
+  if (!ctx || !out) return GM_ERR_INVALID_ARG;
+  if (gm_status s = require(ctx, PRIMS)) return s;
+  DevState h;
+  return download(ctx, &h, n_valid, capacity_points, {{out, ctx->d_pr_ids, 1}});
+}
+
+gm_status gm_compress_primitives(gm_ctx* ctx) {
+  if (!ctx) return GM_ERR_INVALID_ARG;
+  if (gm_status s = require(ctx, PRIMS)) return s;
+  gm_status s = ensure_prim_comp_buffers(ctx);
+  if (s != GM_OK) return s;
+  const size_t n = std::max<size_t>(ctx->n_grid, 1);
+  GM_LAUNCH(ctx, k_prim_comp_reset, 1, 64, ctx->d_pr_comp, ctx->d_pr_vs);
+  GM_LAUNCH(ctx, k_prim_comp_split, div_up((long long)n, CP_TILE), CP_BLOCK, ctx->d_cloud_c, ctx->d_pr_ids, &ctx->d_st->n_valid, ctx->d_pr_state,
+            ctx->d_pr_sv, ctx->d_pr_vs, ctx->d_state64, ctx->d_ctl + 0, &ctx->d_st->error, ctx->d_counters + 12, ctx->d_pr_comp, ctx->d_pr_stats);
+  // the residual cloud is in d_pr_sv, its voxel centroids go to d_pr_cc (extraction scratch until the next extraction)
+  VoxBuffers o{ctx->d_pr_rem, ctx->d_pr_assign, ctx->d_pr_vox_start, ctx->d_pr_vox_key, ctx->d_pr_vox_count, ctx->d_pr_cc};
+  int buf = 0;
+  size_t res_range = 0;
+  const int res_bits = voxel_key_bits(ctx, n, &res_range);
+  if ((s = voxel_downsample(ctx, ctx->d_pr_sv, ctx->d_pr_vs, n, res_bits, res_range, o, &buf)) != GM_OK) return s;
+  GM_LAUNCH(ctx, k_comp_residual_error, ctx->num_sms * 2, CR_BLOCK, ctx->d_pr_sv, ctx->d_pr_assign, ctx->d_pr_cc, ctx->d_pr_vs, ctx->d_comp_part,
+            ctx->d_counters + 13, ctx->d_pr_stats);
+  GM_CHECK_LAUNCHES(ctx);
+  mark(ctx, PRIMS_COMP);
+  return GM_OK;
+}
+
+gm_status gm_download_compressed_primitives(gm_ctx* ctx, void* buf, size_t capacity, size_t* bytes) {
+  if (!ctx || !bytes) return GM_ERR_INVALID_ARG;
+  if (gm_status s = require(ctx, PRIMS_COMP)) return s;
+  std::vector<PrimComp> pc(1);  // ~7 KB
+  CompStats cs;
+  VoxState vs;
+  GM_CUDA(cudaMemcpyAsync(pc.data(), ctx->d_pr_comp, sizeof(PrimComp), cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaMemcpyAsync(&cs, ctx->d_pr_stats, sizeof(CompStats), cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaMemcpyAsync(&vs, ctx->d_pr_vs, sizeof(VoxState), cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  const PrimComp& c = pc[0];
+  gm_primitive_compression h;
+  std::memset(&h, 0, sizeof(h));
+  h.n_points = c.n_points; h.n_primitives = c.n_prims; h.n_residual = c.n_residual; h.n_residual_voxels = vs.n_voxels;
+  h.leaf = (float)ctx->prm.voxelGridLeafSize;
+  h.residual_rms = cs.residual_rms; h.total_rms = cs.total_rms;
+  h.bytes_in = 16ull * (uint64_t)std::max(c.n_points, 0);
+  h.bytes_out = 8 + sizeof(h) + (uint64_t)std::max(c.n_prims, 0) * sizeof(gm_primitive_record) + 12ull * (uint64_t)std::max(vs.n_voxels, 0);
+  h.ratio = (float)((double)h.bytes_in / (double)h.bytes_out);
+  *bytes = (size_t)h.bytes_out;
+  if (!buf) return GM_OK;
+  if (capacity < h.bytes_out) return GM_ERR_CAPACITY;
+  unsigned char* p = (unsigned char*)buf;
+  const uint32_t magic = 0x31504D47u /* 'GMP1' */, version = 1;
+  std::memcpy(p, &magic, 4); std::memcpy(p + 4, &version, 4); p += 8;
+  std::memcpy(p, &h, sizeof(h)); p += sizeof(h);
+  std::memcpy(p, c.rec, (size_t)h.n_primitives * sizeof(gm_primitive_record)); p += (size_t)h.n_primitives * sizeof(gm_primitive_record);
+  if (h.n_residual_voxels > 0)  // strided copy: float4 centroids -> packed xyz
+    GM_CUDA(cudaMemcpy2DAsync(p, 12, ctx->d_pr_cc, 16, 12, (size_t)h.n_residual_voxels, cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
   return GM_OK;
 }
 

@@ -83,3 +83,29 @@ def sample_indices(n_points: int, H: int, per: int, seed: int = 3) -> np.ndarray
     """H x per int32 sample indices, Philox(seed); injected identically into oracle and GPU."""
     g = _rng(seed)
     return g.integers(0, max(n_points, 1), size=(H, per), dtype=np.int64).astype(np.int32)
+
+
+def rectangular_drift(n: int = 100_000, seed: int = 6, width: float = 4.0, height: float = 3.0, length: float = 8.0,
+                      noise: float = 0.005, outlier_frac: float = 0.01) -> np.ndarray:
+    """Multi-surface scene: a rectangular drift along x (floor z = -height/2, walls y = +-width/2, roof z = +height/2),
+    each surface sampled in proportion to its area, Gaussian noise along its normal, `outlier_frac` of the points uniform
+    inside the section.  One plane per surface: the scene needs four primitives."""
+    g = _rng(seed)
+    x = g.uniform(-0.5 * length, 0.5 * length, n)
+    side = g.choice(4, size=n, p=np.array([width, height, width, height]) / (2.0 * (width + height)))
+    a = g.uniform(-0.5, 0.5, n)
+    e = g.normal(0.0, noise, n) if noise > 0 else np.zeros(n)
+    hw, hh = 0.5 * width, 0.5 * height
+    y = np.select([side == 0, side == 1, side == 2], [a * width, hw + e, a * width], -hw + e)
+    z = np.select([side == 0, side == 1, side == 2], [-hh + e, a * height, hh + e], a * height)
+    k = int(round(outlier_frac * n))
+    if k > 0:
+        idx = g.choice(n, size=k, replace=False)
+        y[idx], z[idx] = g.uniform(-0.8 * hw, 0.8 * hw, k), g.uniform(-0.8 * hh, 0.8 * hh, k)
+    return _xyzw(x, y, z)
+
+
+def sample_draws(K: int, H: int, per: int, seed: int = 7) -> np.ndarray:
+    """K x H x per uint32 draws for gm_extract_primitives, Philox(seed): round r maps draw u to the sample index
+    R_r[(u * n_r) >> 32] of the points still unclaimed."""
+    return _rng(seed).integers(0, 1 << 32, size=(K, H, per), dtype=np.uint64).astype(np.uint32)

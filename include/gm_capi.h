@@ -276,6 +276,60 @@ GM_API gm_status gm_get_compression(gm_ctx* ctx, gm_compression* out);
  * x {x,y,z} float.  Pass buf = NULL to query the size. */
 GM_API gm_status gm_download_compressed(gm_ctx* ctx, void* buf, size_t capacity, size_t* bytes);
 
+/* ---- sequential multi-primitive extraction (builder-defined, SURVEY A.9: "repeat after removing inliers") --------
+ * Up to max_primitives rounds over the compacted cloud (M' points).  Round r (0-based):
+ *   1. R_r = the ascending compacted indices no earlier round claimed, n_r = |R_r|.
+ *   2. Sampling: the caller's uint32 draws (max_primitives x Hp x 3 for planes, max_primitives x Hc x 2 for cylinders, one
+ *      block per round) map to sample indices R_r[(uint64(u) * n_r) >> 32], or -1 when n_r = 0.
+ *   3. Plane / cylinder hypotheses are generated from those indices exactly as gm_ransac generates them (same
+ *      coefficients for the same indices); inliers are counted over R_r only; the best of each kind is the packed-key
+ *      argmax of gm_ransac (ties -> lowest id).
+ *   4. The kind with the larger best count wins (tie -> plane).  The round is accepted iff
+ *      best_count >= max(min_inliers, 1); otherwise extraction stops and this and every later round add nothing.
+ *   5. The winner is refitted on its inliers within R_r as gm_ransac_select does (plane PCA; cylinder Gauss-Newton).
+ *   6. Exactly the points of R_r the WINNING HYPOTHESIS counted as inliers get primitive id r + 1 (so the number claimed
+ *      equals best_count).  The refined coefficients are reported and used by gm_compress_primitives only.
+ * Every compacted point gets one uint8 id: 0 = residual, k = the k-th extracted primitive.  The rounds run without host
+ * synchronisation: the launch sequence depends only on (max_primitives, Hp > 0, Hc > 0).  Needs the compacted cloud
+ * (cylinders read its normals, as gm_ransac does).  Extraction has buffers of its own (allocated by the first call):
+ * gm_ransac's hypotheses, models, labels and compression are untouched. */
+#define GM_MAX_PRIMITIVES 64
+typedef struct gm_primitive {
+  gm_model model;       /* kind, best_id (within its round), best_count (= points claimed), refit_count, hyp, coef, rms */
+  int32_t n_remaining;  /* unclaimed points at the start of its round */
+  int32_t pad_;
+} gm_primitive;
+GM_API gm_status gm_extract_primitives(gm_ctx* ctx, int32_t max_primitives, int32_t min_inliers,
+                                       const uint32_t* plane_draws_host, int32_t Hp,
+                                       const uint32_t* cyl_draws_host, int32_t Hc);
+/* *n = number of primitives extracted; GM_ERR_CAPACITY if it exceeds capacity (out may be NULL to query it). */
+GM_API gm_status gm_get_primitives(gm_ctx* ctx, gm_primitive* out, int32_t capacity, int32_t* n);
+/* M' primitive ids, in compacted order. */
+GM_API gm_status gm_download_primitive_ids(gm_ctx* ctx, uint8_t* out, size_t capacity_points);
+
+/* Compression of the extracted primitives, the counterpart of gm_compress: every primitive as its refined surface and
+ * extents, the residual (id 0) points voxel-downsampled at voxelGridLeafSize.  Needs gm_extract_primitives. */
+typedef struct gm_primitive_compression {
+  int32_t n_points, n_primitives, n_residual, n_residual_voxels;
+  float leaf;          /* residual voxel size                                                   */
+  float residual_rms;  /* RMS distance of a residual point to its voxel centroid                */
+  float total_rms;     /* reconstruction RMS over all n_points (claimed points: to their surface) */
+  float ratio;         /* bytes_in / bytes_out                                                  */
+  uint64_t bytes_in;   /* 16 * n_points                                                         */
+  uint64_t bytes_out;  /* size of the blob gm_download_compressed_primitives writes             */
+} gm_primitive_compression;
+typedef struct gm_primitive_record {
+  int32_t kind;        /* gm_model_kind */
+  int32_t count;       /* points claimed */
+  float coef[7];       /* refined plane {a,b,c,d} or cylinder {q, dir, r} */
+  float extents[4];    /* plane: umin, umax, vmin, vmax in gm_compress's canonical in-plane basis; cylinder: tmin, tmax along dir from q, 0, 0 */
+  float rms;           /* RMS distance of its claimed points to the refined surface */
+} gm_primitive_record;
+GM_API gm_status gm_compress_primitives(gm_ctx* ctx);
+/* Packed little-endian blob: 'GMP1' | version u32 | gm_primitive_compression | n_primitives x gm_primitive_record |
+ * n_residual_voxels x {x,y,z} float.  Pass buf = NULL to query the size. */
+GM_API gm_status gm_download_compressed_primitives(gm_ctx* ctx, void* buf, size_t capacity, size_t* bytes);
+
 /* Fused per-scan path = the body of cloud_cb (src/geometric_mapping.cpp:48-125) plus the
  * builder-defined segmentation: crop -> normals -> voxel -> local frame -> RANSAC plane(Hp)
  * + cylinder(Hc) -> select/refit -> labels -> polyline.  samples may be NULL when H == 0. */
