@@ -25,8 +25,11 @@ def map_draws(draws, rem):
     return np.asarray(rem, np.int32)[draw_positions(draws, n)]
 
 
-def extract(cloud, normals8, plane_draws, cyl_draws, max_primitives, min_inliers, tau=0.05, rmin=0.5, rmax=10.0, refit_iters=5):
-    """-> (list of primitive dicts, uint8 ids).  plane_draws: K x Hp x 3, cyl_draws: K x Hc x 2 (None = no such kind)."""
+def extract(cloud, normals8, plane_draws, cyl_draws, max_primitives, min_inliers, tau=0.05, rmin=0.5, rmax=10.0, refit_iters=5,
+            trace=None):
+    """-> (list of primitive dicts, uint8 ids).  plane_draws: K x Hp x 3, cyl_draws: K x Hc x 2 (None = no such kind).
+    trace: a list that receives (n_r, best plane count, best cylinder count) of every round run, the stopping one
+    included (-1 = no valid hypothesis of that kind)."""
     cloud = np.ascontiguousarray(cloud, np.float32)
     ids = np.zeros(len(cloud), np.uint8)
     work = cloud.copy()
@@ -46,6 +49,8 @@ def extract(cloud, normals8, plane_draws, cyl_draws, max_primitives, min_inliers
             b = O.argmax(counts)
             if b >= 0:
                 best[1] = (int(counts[b]), b, (m7, t12))
+        if trace is not None:
+            trace.append((len(rem), best[0][0], best[1][0]))
         kind = 0 if best[0][0] >= best[1][0] else 1
         count, b, tab = best[kind]
         if count < max(min_inliers, 1):
@@ -108,3 +113,59 @@ def compress(cloud, ids, prims, leaf):
     return {"records": recs, "n_points": n, "n_residual": len(res), "n_residual_voxels": V, "residual_centroids": vox["centroids_fx"],
             "residual_rms": float(np.sqrt(rsq / len(res))) if len(res) else 0.0,
             "total_rms": float(np.sqrt((sq + rsq) / n)) if n else 0.0}
+
+
+# ---- float64 refit references, independent of the oracle's refit code ---------------------------------------------
+def plane_fit_d(pts):
+    """Total-least-squares plane of `pts` in float64: the normal is the eigenvector of the smallest eigenvalue of the
+    (population) covariance, d = -n . mean and rms = sqrt(lambda_min).  -> (n, d, rms)."""
+    p = np.asarray(pts, np.float64)[:, :3]
+    m = p.mean(0)
+    q = p - m
+    vals, vecs = np.linalg.eigh(q.T @ q / len(p))
+    n = vecs[:, 0]
+    return n, float(-n @ m), float(np.sqrt(max(vals[0], 0.0)))
+
+
+def cylinder_residuals_d(pts, q, axis, r):
+    """Orthogonal distances |p - axis line| - r in float64 (axis need not be unit)."""
+    p = np.asarray(pts, np.float64)[:, :3]
+    a = np.asarray(axis, np.float64)
+    a = a / np.linalg.norm(a)
+    v = p - np.asarray(q, np.float64)
+    return np.linalg.norm(v - np.outer(v @ a, a), axis=1) - float(r)
+
+
+def cylinder_rms_d(pts, coef7):
+    """RMS of the orthogonal residuals of `pts` at the cylinder coef7 = (q, axis, r), evaluated directly in float64."""
+    c = np.asarray(coef7, np.float64)
+    e = cylinder_residuals_d(pts, c[:3], c[3:6], c[6])
+    return float(np.sqrt((e * e).mean()))
+
+
+def cylinder_fit_d(pts, coef7, tol=1e-15, passes=4):
+    """Least-squares cylinder of `pts` in float64 (scipy.optimize.least_squares) from the start coef7 = (q, axis, r).
+    The five free parameters are a chart around the current model: q moves in the plane perpendicular to the axis and
+    the axis tilts along the same basis; the chart is recentred after every pass.  -> (q, unit axis, r, rms)."""
+    from scipy.optimize import least_squares
+
+    p = np.asarray(pts, np.float64)[:, :3]
+    c = np.asarray(coef7, np.float64)
+    q, a, r = c[:3].copy(), c[3:6] / np.linalg.norm(c[3:6]), float(c[6])
+    for _ in range(passes):
+        u, w = perp_basis_d(a)
+
+        def model(x, q=q, a=a, u=u, w=w):
+            d = a + x[2] * u + x[3] * w
+            return q + x[0] * u + x[1] * w, d / np.linalg.norm(d)
+
+        def fun(x):
+            qq, dd = model(x)
+            return cylinder_residuals_d(p, qq, dd, r + x[4])
+
+        x = least_squares(fun, np.zeros(5), method="lm", xtol=tol, ftol=tol, gtol=tol, x_scale=1.0).x
+        q, a = model(x)
+        r += x[4]
+        if np.abs(x).max() < 1e-13:
+            break
+    return q, a, r, cylinder_rms_d(p, np.concatenate([q, a, [r]]))

@@ -81,3 +81,54 @@ def test_draw_mapping_stays_in_range():
     n = (1 << 31) - 1
     pos = P.draw_positions(draws, n)
     assert pos.min() == 0 and pos.max() == n - 1 and np.all(pos < n)
+
+
+def test_trace_records_every_round_and_the_stop():
+    cloud, normals8, _ = _known_scene()
+    K = 8
+    trace = []
+    prims, ids = P.extract(cloud, normals8, synth.sample_draws(K, 256, 3, seed=1), synth.sample_draws(K, 256, 2, seed=2), K,
+                           min_inliers=500, rmin=0.5, rmax=3.0, trace=trace)
+    assert len(trace) == len(prims) + 1
+    assert [t[0] for t in trace[:-1]] == [p["n_remaining"] for p in prims]
+    assert [max(t[1:]) for t in trace[:-1]] == [p["best_count"] for p in prims]
+    assert trace[-1][0] == int((ids == 0).sum()) and max(trace[-1][1:]) < 500
+
+
+def test_plane_reference_recovers_a_known_plane():
+    n = np.array([1.0, 2.0, -2.0]) / 3.0
+    p = synth.plane_patch(20_000, seed=31, normal=n, offset=1.25, half=1.5, noise=0.01)
+    nr, d, rms = P.plane_fit_d(p)
+    s = np.sign(nr @ n)
+    assert np.linalg.norm(np.cross(nr, n)) < 1e-3 and abs(s * d + 1.25) < 1e-3 and abs(rms - 0.01) < 5e-4
+    # exact points: the eigen-decomposition of the float64 covariance is exact to rounding
+    u, v = P.perp_basis_d(n)
+    g = np.random.Generator(np.random.Philox(32)).uniform(-1.0, 1.0, (500, 2))
+    q = g[:, :1] * u + g[:, 1:] * v - 0.5 * n
+    nr, d, rms = P.plane_fit_d(q)
+    assert np.linalg.norm(np.cross(nr, n)) < 1e-12 and abs(np.sign(nr @ n) * d - 0.5) < 1e-12 and rms < 1e-7
+
+
+def test_cylinder_reference_recovers_a_known_cylinder():
+    """Points exactly on a tilted cylinder: from a start 0.05 rad and 3 cm off, the fit lands on it to rounding; with
+    radial noise, its RMS is the lowest of nearby models."""
+    axis = np.array([0.3, -0.2, 1.0]) / np.linalg.norm([0.3, -0.2, 1.0])
+    q0, r0 = np.array([0.5, -1.0, 0.2]), 1.7
+    u, w = P.perp_basis_d(axis)
+    g = np.random.Generator(np.random.Philox(33))
+    th, t = g.uniform(0.0, 2.0 * np.pi, 4000), g.uniform(-2.0, 2.0, 4000)
+    pts = q0 + t[:, None] * axis + r0 * (np.cos(th)[:, None] * u + np.sin(th)[:, None] * w)
+    assert np.abs(P.cylinder_residuals_d(pts, q0, axis, r0)).max() < 1e-12
+    start = np.concatenate([q0 + 0.03 * u, axis + 0.05 * w, [r0 + 0.02]])
+    assert P.cylinder_rms_d(pts, start) > 1e-3
+    q, a, r, rms = P.cylinder_fit_d(pts, start)
+    dq = q - q0
+    assert np.linalg.norm(np.cross(a, axis)) < 1e-10 and abs(r - r0) < 1e-10 and np.linalg.norm(dq - axis * (dq @ axis)) < 1e-10
+    assert rms < 1e-10
+    noisy = pts + (g.normal(0.0, 0.01, 4000)[:, None] * (pts - q0 - ((pts - q0) @ axis)[:, None] * axis) / r0)
+    q, a, r, rms = P.cylinder_fit_d(noisy, start)
+    assert abs(rms - 0.01) < 1e-3 and abs(r - r0) < 1e-3
+    best = np.concatenate([q, a, [r]])
+    for k in range(7):
+        for h in (-1e-4, 1e-4):
+            assert P.cylinder_rms_d(noisy, best + h * np.eye(7)[k]) >= rms - 1e-15
