@@ -171,6 +171,7 @@ struct gm_ctx {
   DevBuf<PolyState> d_poly;
   DevBuf<long long> d_poly_acc;
   DevBuf<unsigned long long> d_poly_part;  // per-block (min,max) of the polyline range pass
+  DevBuf<float4> d_poly_list;  // the cylinder points the polyline passes walk (k_poly_range), count in d_counters[10]
   DevBuf<gm_slice> d_slices;
   DevBuf<SummaryDev> d_summary;
   // compression stage: residual (label 0) cloud and its voxel grid
@@ -523,7 +524,7 @@ gm_status gm_create(const gm_params* p, size_t max_points, int32_t max_hypothese
   A(d_hvalid[0], H); A(d_hvalid[1], H); A(d_counts[0], H); A(d_counts[1], H);
   A(d_key, 2); A(d_model, 2);
   A(d_poly, 1); A(d_summary, 1); A(d_res_vs, 1); A(d_comp, 1); A(d_res_pts, N); A(d_res_centroid, N); A(d_res_key_pt, N); A(d_res_assign, N);
-  A(d_res_vox_start, N + 1); A(d_res_vox_key, N); A(d_res_vox_count, N); A(d_comp_part, (size_t)CS_NV * (div_up((long long)N, CP_TILE) + 1) + 1024); A(d_comp_mm, (size_t)6 * (div_up((long long)N, CP_TILE) + 1)); A(d_counters, 16); A(d_poly_part, 2 * 4096); A(d_inl, N); A(d_poly_acc, (size_t)POLY_NACC * (size_t)std::max(p->maxSlices, 1)); A(d_slices, (size_t)std::max(p->maxSlices, 1));
+  A(d_res_vox_start, N + 1); A(d_res_vox_key, N); A(d_res_vox_count, N); A(d_comp_part, (size_t)CS_NV * (div_up((long long)N, CP_TILE) + 1) + 1024); A(d_comp_mm, (size_t)6 * (div_up((long long)N, CP_TILE) + 1)); A(d_counters, 16); A(d_poly_part, 2 * 4096); A(d_poly_list, 2 * N); A(d_inl, N); A(d_poly_acc, (size_t)POLY_NACC * (size_t)std::max(p->maxSlices, 1)); A(d_slices, (size_t)std::max(p->maxSlices, 1));
 #undef A
   if ((e = cudaMallocHost((void**)&ctx->h_samples[0], 3 * H * sizeof(int))) != cudaSuccess) return fail(e, "h_samples0");
   if ((e = cudaMallocHost((void**)&ctx->h_samples[1], 2 * H * sizeof(int))) != cudaSuccess) return fail(e, "h_samples1");
@@ -1131,16 +1132,19 @@ gm_status gm_axis_polyline(gm_ctx* ctx) {
   const WeightLaw shift = weight_law(ctx->prm);
   SegTimer seg_(ctx, SEG_POLYLINE);
   {
-    // 3 launches: range (+basis, +zeroing, +slice layout) and two accumulation passes (moments -> means + circle fit;
-    // residuals -> output), each with the per-slice step that consumes it folded into its last block
+    // 3 launches: range (+basis, +zeroing, +slice layout, +the list of cylinder points) and two accumulation passes over
+    // that list (moments -> means + circle fit; residuals -> output), each with the per-slice step that consumes it
+    // folded into its last block
     int blocks = std::max(1, std::min(div_up((long long)std::max<size_t>(ctx->n_grid, 1), POLY_BLOCK), ctx->num_sms * 4));
-    GM_LAUNCH(ctx, k_poly_range, blocks, POLY_BLOCK, ctx->d_cloud_c, ctx->d_labels, n_ptr, ctx->d_frame, ctx->d_poly, ctx->d_poly_acc,
-              POLY_NACC * S, ctx->d_poly_part, ctx->d_counters + 8, ctx->prm.sliceLength, S);
+    const int cap = (int)ctx->cap;
+    unsigned* n_list = ctx->d_counters + 10;
+    GM_LAUNCH(ctx, k_poly_range, blocks, POLY_BLOCK, ctx->d_cloud_c, ctx->d_normals_c, ctx->d_labels, n_ptr, ctx->d_frame, shift, ctx->d_poly,
+              ctx->d_poly_acc, POLY_NACC * S, ctx->d_poly_part, ctx->d_counters + 8, ctx->d_poly_list, cap, n_list, ctx->prm.sliceLength, S);
     const ModelState* cylm = has(ctx, MODEL_CYL) ? ctx->d_model + 1 : nullptr;
-    GM_LAUNCH(ctx, k_poly_pass<0>, blocks, POLY_BLOCK, ctx->d_cloud_c, ctx->d_normals_c, ctx->d_labels, n_ptr, ctx->d_poly, shift,
-              ctx->d_poly_acc, ctx->d_slices, ctx->d_counters + 9, cylm);
-    GM_LAUNCH(ctx, k_poly_pass<2>, blocks, POLY_BLOCK, ctx->d_cloud_c, ctx->d_normals_c, ctx->d_labels, n_ptr, ctx->d_poly, shift,
-              ctx->d_poly_acc, ctx->d_slices, ctx->d_counters + 11, cylm);
+    GM_LAUNCH(ctx, k_poly_pass<0>, blocks, POLY_BLOCK, ctx->d_poly_list, cap, n_list, ctx->d_poly, ctx->d_poly_acc, ctx->d_slices,
+              ctx->d_counters + 9, cylm);
+    GM_LAUNCH(ctx, k_poly_pass<2>, blocks, POLY_BLOCK, ctx->d_poly_list, cap, n_list, ctx->d_poly, ctx->d_poly_acc, ctx->d_slices,
+              ctx->d_counters + 11, cylm);
   }
   GM_CHECK_LAUNCHES(ctx);
   mark(ctx, POLY);
