@@ -79,6 +79,21 @@ def plane_patch(n: int = 10_000, seed: int = 5, normal=(0.0, 0.0, 1.0), offset: 
     return _xyzw(p[:, 0], p[:, 1], p[:, 2])
 
 
+def dyadic(pts: np.ndarray, e: int) -> np.ndarray:
+    """A copy of `pts` with x, y, z rounded to the nearest multiple of q = 2^-e (ties to even) and -0.0 turned into
+    +0.0.  NaN and inf stay as they are, and so does every coordinate that already is a multiple of q (the crop
+    faces +-bound for dyadic bounds).  On such a cloud every float product and partial sum of coordinates is a
+    multiple of q^2 (or q), hence exact while it stays below 2^24 of those units: sums of them do not depend on
+    the order of the additions."""
+    out = np.array(pts, np.float32, copy=True)
+    xyz = out[:, :3].astype(np.float64)
+    fin = np.isfinite(xyz)
+    s = 2.0 ** e
+    xyz[fin] = np.round(xyz[fin] * s) / s + 0.0   # exact in float64; the result is a float32 (|x| < 2^(24-e) or already dyadic)
+    out[:, :3] = xyz.astype(np.float32)
+    return out
+
+
 def sample_indices(n_points: int, H: int, per: int, seed: int = 3) -> np.ndarray:
     """H x per int32 sample indices, Philox(seed); injected identically into oracle and GPU."""
     g = _rng(seed)

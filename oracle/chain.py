@@ -74,33 +74,44 @@ def _bits(a):
 
 def gpu_chain(pts, ps, cs, canonical, radius, leaf, bound=5.0, tau=0.05, slice_len=1.0, refit_iters=5, knn=0, knn_max_radius=0.0):
     """The same path on the CUDA library through the C-ABI: everything compare() looks at, downloaded."""
-    from geometric_mapping_b200 import capi
-
-    n = len(pts)
-    H = max(len(ps) if ps is not None else 0, len(cs) if cs is not None else 0, 1)
-    prm = capi.default_params(boxFilterBound=bound, neighborRadius=radius, voxelGridLeafSize=leaf, ransacThreshold=tau,
-                              sliceLength=slice_len, refitIterations=refit_iters)
-    with capi.Context(prm, max_points=max(n, 1), max_hypotheses=H) as ctx:
+    with gpu_context(len(pts), ps, cs, radius, leaf, bound, tau, slice_len, refit_iters) as ctx:
         ctx.set_normals_mode(1 if canonical else 0)
         if knn:
             ctx.set_knn(knn, max_radius=knn_max_radius)
         ctx.upload_scan(pts)
         ctx.process_scan(ps, cs)
-        c = ctx.counts()
-        assert c.device_error == 0
-        keys, assign, _ = ctx.download_voxel_assignment()
-        vox = ctx.download_voxels()
-        g = {"n_cropped": c.n_cropped, "n_valid": c.n_valid, "n_voxels": c.n_voxels, "cropped": ctx.download_cloud(0),
-             "normals": ctx.download_normals(0), "nbr_count": ctx.download_neighbor_counts(), "valid_map": ctx.download_valid_map(),
-             "cloud": ctx.download_cloud(1), "normals_c": ctx.download_normals(1), "grid6": ctx.voxel_grid(), "vox_key_pt": keys,
-             "vox_assign": assign, "vox_keys": vox["keys"], "vox_counts": vox["counts"], "centroids": vox["centroids"],
-             "nn_index": vox["nn_index"], "frame": ctx.frame(), "labels": ctx.download_labels(), "polyline": ctx.download_polyline()}
-        if ps is not None and len(ps):
-            g["plane_coef"], _, g["plane_counts"] = ctx.download_hypotheses(capi.GM_MODEL_PLANE, len(ps))
-            g["plane"] = ctx.model(capi.GM_MODEL_PLANE)
-        if cs is not None and len(cs):
-            g["cyl_model"], g["cyl_test"], g["cyl_counts"] = ctx.download_hypotheses(capi.GM_MODEL_CYLINDER, len(cs))
-            g["cyl"] = ctx.model(capi.GM_MODEL_CYLINDER)
+        return gpu_outputs(ctx, ps, cs)
+
+
+def gpu_context(n, ps, cs, radius, leaf, bound=5.0, tau=0.05, slice_len=1.0, refit_iters=5):
+    """A context with the parameters gpu_chain uses, sized for n points and the hypotheses ps / cs."""
+    from geometric_mapping_b200 import capi
+
+    H = max(len(ps) if ps is not None else 0, len(cs) if cs is not None else 0, 1)
+    prm = capi.default_params(boxFilterBound=bound, neighborRadius=radius, voxelGridLeafSize=leaf, ransacThreshold=tau,
+                              sliceLength=slice_len, refitIterations=refit_iters)
+    return capi.Context(prm, max_points=max(n, 1), max_hypotheses=H)
+
+
+def gpu_outputs(ctx, ps, cs):
+    """Everything compare() looks at, downloaded from a context after process_scan(ps, cs)."""
+    from geometric_mapping_b200 import capi
+
+    c = ctx.counts()
+    assert c.device_error == 0
+    keys, assign, _ = ctx.download_voxel_assignment()
+    vox = ctx.download_voxels()
+    g = {"n_cropped": c.n_cropped, "n_valid": c.n_valid, "n_voxels": c.n_voxels, "cropped": ctx.download_cloud(0),
+         "normals": ctx.download_normals(0), "nbr_count": ctx.download_neighbor_counts(), "valid_map": ctx.download_valid_map(),
+         "cloud": ctx.download_cloud(1), "normals_c": ctx.download_normals(1), "grid6": ctx.voxel_grid(), "vox_key_pt": keys,
+         "vox_assign": assign, "vox_keys": vox["keys"], "vox_counts": vox["counts"], "centroids": vox["centroids"],
+         "nn_index": vox["nn_index"], "frame": ctx.frame(), "labels": ctx.download_labels(), "polyline": ctx.download_polyline()}
+    if ps is not None and len(ps):
+        g["plane_coef"], _, g["plane_counts"] = ctx.download_hypotheses(capi.GM_MODEL_PLANE, len(ps))
+        g["plane"] = ctx.model(capi.GM_MODEL_PLANE)
+    if cs is not None and len(cs):
+        g["cyl_model"], g["cyl_test"], g["cyl_counts"] = ctx.download_hypotheses(capi.GM_MODEL_CYLINDER, len(cs))
+        g["cyl"] = ctx.model(capi.GM_MODEL_CYLINDER)
     return g
 
 
