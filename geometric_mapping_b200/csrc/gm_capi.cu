@@ -93,6 +93,24 @@ struct DevBuf {
   operator T*() const { return p; }
   T* operator->() const { return p; }
 };
+
+// The RANSAC tables of one set of H hypotheses per kind (index = kind): sample indices, hypotheses, counts, the
+// winner's key and its refitted model.
+struct HypSet {
+  DevBuf<int> samples[2];  // [3H] plane, [2H] cylinder
+  DevBuf<float4> plane_coef;
+  DevBuf<float> model7, test12;
+  DevBuf<int> hvalid[2], counts[2];
+  DevBuf<unsigned long long> key;  // [2]
+  DevBuf<ModelState> model;        // [2]
+  cudaError_t alloc(size_t H) {  // stops at the first failure and returns it
+    cudaError_t e;
+    (void)((e = samples[0].alloc(3 * H)) || (e = samples[1].alloc(2 * H)) || (e = plane_coef.alloc(H)) || (e = model7.alloc(7 * H)) ||
+           (e = test12.alloc(12 * H)) || (e = hvalid[0].alloc(H)) || (e = hvalid[1].alloc(H)) || (e = counts[0].alloc(H)) ||
+           (e = counts[1].alloc(H)) || (e = key.alloc(2)) || (e = model.alloc(2)));
+    return e;
+  }
+};
 }  // namespace
 
 struct gm_ctx {
@@ -158,15 +176,10 @@ struct gm_ctx {
   DevBuf<DevState> d_st;
   DevBuf<double> d_partials;
   DevBuf<FrameOut> d_frame;
-  // ransac (index = kind)
-  DevBuf<int> d_samples[2];
+  // ransac (index = kind): the scan's hypothesis set, its samples staged from the host through h_samples
+  HypSet hyp;
   int* h_samples[2] = {nullptr, nullptr};
   cudaEvent_t ev_samples[2] = {nullptr, nullptr};
-  DevBuf<float4> d_plane_coef;
-  DevBuf<float> d_model7, d_test12;
-  DevBuf<int> d_hvalid[2], d_counts[2];
-  DevBuf<unsigned long long> d_key;  // [2]
-  DevBuf<ModelState> d_model;        // [2]
   // polyline
   DevBuf<PolyState> d_poly;
   DevBuf<long long> d_poly_acc;
@@ -189,12 +202,7 @@ struct gm_ctx {
   DevBuf<int> d_pr_rem;                      // R_r
   DevBuf<unsigned char> d_pr_ids;            // primitive id per compacted point
   DevBuf<unsigned> d_pr_draws[2];
-  DevBuf<int> d_pr_samples[2];
-  DevBuf<float4> d_pr_plane_coef;
-  DevBuf<float> d_pr_model7, d_pr_test12;
-  DevBuf<int> d_pr_hvalid[2], d_pr_counts[2];
-  DevBuf<unsigned long long> d_pr_key;  // [2]
-  DevBuf<ModelState> d_pr_model;        // [2]
+  HypSet pr_hyp;                             // the hypothesis set of one extraction round
   DevBuf<PrimState> d_pr_state;
   // compression of the extracted primitives: the residual cloud goes to d_pr_sv, its centroids to d_pr_cc
   DevBuf<int> d_pr_assign, d_pr_vox_start, d_pr_vox_key, d_pr_vox_count;
@@ -231,8 +239,8 @@ struct SegTimer {
     if (!c->ev_pool.empty()) { cudaEvent_t e = c->ev_pool.back(); c->ev_pool.pop_back(); return e; }
     cudaEvent_t e = nullptr; cudaEventCreate(&e); return e;
   }
-  SegTimer(gm_ctx* c, int s) : ctx(c), seg(s) {
-    if (!c->profiling) return;
+  SegTimer(gm_ctx* c, int s) : ctx(c), seg(s) {  // s < 0: not timed
+    if (!c->profiling || s < 0) return;
     cudaEvent_t e0 = get(c); e1 = get(c);
     cudaEventRecord(e0, c->stream);
     c->seg_events[s].push_back({e0, e1});
@@ -518,11 +526,7 @@ gm_status gm_create(const gm_params* p, size_t max_points, int32_t max_hypothese
   A(d_rs_hist, RS2_HIST_WORDS); A(d_rs_aux, 1);
   A(d_st, 1); A(d_ctl, 3); A(d_frame_sums, 8);
   A(d_partials, 3 * kPartialsRegion);  // 3 regions: frame | plane refit | cylinder GN (may run concurrently)
-  A(d_frame, 1);
-  A(d_samples[0], 3 * H); A(d_samples[1], 2 * H);
-  A(d_plane_coef, H); A(d_model7, 7 * H); A(d_test12, 12 * H);
-  A(d_hvalid[0], H); A(d_hvalid[1], H); A(d_counts[0], H); A(d_counts[1], H);
-  A(d_key, 2); A(d_model, 2);
+  A(d_frame, 1); A(hyp, H);
   A(d_poly, 1); A(d_summary, 1); A(d_res_vs, 1); A(d_comp, 1); A(d_res_pts, N); A(d_res_centroid, N); A(d_res_key_pt, N); A(d_res_assign, N);
   A(d_res_vox_start, N + 1); A(d_res_vox_key, N); A(d_res_vox_count, N); A(d_comp_part, (size_t)CS_NV * (div_up((long long)N, CP_TILE) + 1) + 1024); A(d_comp_mm, (size_t)6 * (div_up((long long)N, CP_TILE) + 1)); A(d_counters, 16); A(d_poly_part, 2 * 4096); A(d_poly_list, 2 * N); A(d_inl, N); A(d_poly_acc, (size_t)POLY_NACC * (size_t)std::max(p->maxSlices, 1)); A(d_slices, (size_t)std::max(p->maxSlices, 1));
 #undef A
@@ -546,9 +550,9 @@ gm_status gm_create(const gm_params* p, size_t max_points, int32_t max_hypothese
   { const char* env = std::getenv("GM_GRAPH"); ctx->graph_mode = env ? std::max(0, std::min(2, std::atoi(env))) : 2; }
   { const char* env = std::getenv("GM_NORMALS_MODE"); ctx->normals_mode = (env && env[0] == '1') ? 1 : 0; }
 
-  if ((e = cudaMemset(ctx->d_key, 0, 2 * sizeof(unsigned long long))) != cudaSuccess) return fail(e, "memset");
+  if ((e = cudaMemset(ctx->hyp.key, 0, 2 * sizeof(unsigned long long))) != cudaSuccess) return fail(e, "memset");
   if ((e = cudaMemset(ctx->d_counters, 0, 16 * sizeof(unsigned))) != cudaSuccess) return fail(e, "memset");
-  if ((e = cudaMemset(ctx->d_model, 0, 2 * sizeof(ModelState))) != cudaSuccess) return fail(e, "memset");
+  if ((e = cudaMemset(ctx->hyp.model, 0, 2 * sizeof(ModelState))) != cudaSuccess) return fail(e, "memset");
   {
     int per_sm = 0;
     if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_cyl_gn_all, RF_BLOCK, 0)) != cudaSuccess) return fail(e, "occupancy");
@@ -983,8 +987,88 @@ static gm_status stage_samples(gm_ctx* ctx, int kind, const int32_t* samples_hos
   const size_t off = (size_t)h_begin * per, cnt = (size_t)(h_end - h_begin) * per;
   GM_CUDA(cudaEventSynchronize(ctx->ev_samples[kind]));
   std::memcpy(ctx->h_samples[kind] + off, samples_host + off, cnt * sizeof(int));
-  GM_CUDA(cudaMemcpyAsync(ctx->d_samples[kind] + off, ctx->h_samples[kind] + off, cnt * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+  GM_CUDA(cudaMemcpyAsync(ctx->hyp.samples[kind] + off, ctx->h_samples[kind] + off, cnt * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
   GM_CUDA(cudaEventRecord(ctx->ev_samples[kind], ctx->stream));
+  return GM_OK;
+}
+
+// The cloud an inlier count reads: the compacted points and their device count, and optionally the cell-sorted copy
+// with its leaf bounds and device count, which selects tile-culled counting (same counts, see gm_ransac.cuh).
+struct CountView {
+  const float4* pts;
+  const int* n;
+  const float4* sorted = nullptr;
+  const float4* leaf_bounds = nullptr;
+  const int* n_sorted = nullptr;
+};
+
+// co-resident 64-thread blocks per SM (register limited to 14) of the brute-force count
+constexpr int kCountBlocksPerSm = 8;
+
+// Hypotheses [h_begin, h_end) of `kind` into `hs` (all H when gen_all) from the scan's compacted cloud, then, unless
+// `cloud` is null, their inlier counts over `cloud` with the argmax folded into the counting kernel's last block.
+// `comm` is the peer table of a sharded round (or null); `timed` records the *_hyp and *_count profile segments.
+static gm_status launch_hyp_count(gm_ctx* ctx, HypSet& hs, int kind, int H, int h_begin, int h_end, int gen_all, const CommDev* comm,
+                                  const CountView* cloud, bool timed) {
+  const int* n_valid = &ctx->d_st->n_valid;
+  const float tau = (float)ctx->prm.ransacThreshold;
+  const int hb = div_up(H, 128);
+  { SegTimer seg_(ctx, !timed ? -1 : kind == 0 ? SEG_PLANE_HYP : SEG_CYL_HYP);
+  if (kind == 0) {
+    GM_LAUNCH(ctx, k_plane_hypotheses, hb, 128, ctx->d_cloud_c, n_valid, hs.samples[0], H, hs.plane_coef, hs.hvalid[0], hs.counts[0],
+              h_begin, h_end, gen_all);
+  } else {
+    GM_LAUNCH(ctx, k_cyl_hypotheses, hb, 128, ctx->d_cloud_c, ctx->d_normals_c, n_valid, hs.samples[1], H, (float)ctx->prm.cylinderRadiusMin,
+              (float)ctx->prm.cylinderRadiusMax, tau, hs.model7, hs.test12, hs.hvalid[1], hs.counts[1], h_begin, h_end, gen_all);
+  } }
+  if (cloud) {
+    SegTimer seg_(ctx, !timed ? -1 : kind == 0 ? SEG_PLANE_COUNT : SEG_CYL_COUNT);
+    unsigned* ticket = ctx->d_counters + 3 + kind;
+    if (cloud->sorted) {
+      const int blocks = std::max(1, div_up((long long)ctx->n_grid, TC_SUPER));
+      const auto count_tiles = kind == 0 ? k_count_tiles<0> : k_count_tiles<1>;
+      GM_LAUNCH(ctx, count_tiles, blocks, TC_BLOCK, cloud->sorted, cloud->leaf_bounds, cloud->n_sorted, hs.plane_coef, hs.test12,
+                hs.hvalid[kind], h_begin, h_end, tau, hs.counts[kind], H, hs.key + kind, ticket, comm, hs.model7);
+    } else {
+      const int K = kind == 0 ? RC_KP : RC_KC;
+      const int groups = div_up(h_end - h_begin, RC_BLOCK * K);
+      // every slice at least half a tile
+      const int slices = std::max(1, std::min(div_up((long long)ctx->n_grid, RC_TILE / 2), div_up(ctx->num_sms * kCountBlocksPerSm, groups)));
+      const dim3 grid(slices, groups);
+      if (kind == 0) {
+        GM_LAUNCH(ctx, k_count_plane<RC_KP>, grid, RC_BLOCK, cloud->pts, cloud->n, hs.plane_coef, hs.hvalid[0], h_begin, h_end, tau,
+                  hs.counts[0], H, hs.key + 0, ticket, comm);
+      } else {
+        GM_LAUNCH(ctx, k_count_cyl<RC_KC>, grid, RC_BLOCK, cloud->pts, cloud->n, hs.test12, h_begin, h_end, hs.counts[1], H, hs.key + 1,
+                  ticket, comm, hs.model7);
+      }
+    }
+  }
+  GM_CHECK_LAUNCHES(ctx);
+  return GM_OK;
+}
+
+// Refit of the winner of `kind` in `hs` over `pts` and its device count `n`: the plane refit, or the cylinder's inlier
+// compaction and all its Gauss-Newton passes in one cooperative launch (grid barrier between passes).
+static gm_status launch_refit(gm_ctx* ctx, HypSet& hs, int kind, int H, const float4* pts, const int* n) {
+  ModelState* ms = hs.model + kind;
+  const float tau = (float)ctx->prm.ransacThreshold;
+  if (kind == 0) {
+    GM_LAUNCH(ctx, k_plane_refit, REFIT_BLOCKS, RF_BLOCK, pts, n, hs.key + 0, H, hs.plane_coef, ms, tau, ctx->d_partials + 1 * kPartialsRegion,
+              ctx->d_counters + 1);
+  } else {
+    GM_LAUNCH(ctx, k_cyl_inlier_compact, std::max(1, div_up((long long)ctx->n_grid, CPL_TILE)), CP_BLOCK, pts, n, hs.key + 1, H, hs.model7,
+              hs.test12, ms, ctx->d_inl, ctx->d_state64_b, ctx->d_ctl + 1, &ctx->d_st->error);
+    const float4* inl = ctx->d_inl;
+    int iters = ctx->prm.refitIterations;
+    double* partials = ctx->d_partials + 2 * kPartialsRegion;
+    unsigned* bars = ctx->d_counters + 5;  // counters [5],[6]: the two barrier counters, [7]: which one the next launch uses
+    int* err = &ctx->d_st->error;
+    void* args[] = {(void*)&inl, (void*)&ms, (void*)&iters, (void*)&tau, (void*)&partials, (void*)&bars, (void*)&err};
+    GM_CUDA(cudaLaunchCooperativeKernel((const void*)k_cyl_gn_all, dim3(ctx->gn_blocks), dim3(RF_BLOCK), args, 0, ctx->stream));
+    ++ctx->launches;
+  }
+  GM_CHECK_LAUNCHES(ctx);
   return GM_OK;
 }
 
@@ -995,62 +1079,25 @@ gm_status gm_ransac(gm_ctx* ctx, int32_t kind, const int32_t* samples_host, int3
   h_begin = std::max(h_begin, 0);
   h_end = std::min(h_end, H);
   const int per = kind == 0 ? 3 : 2;
-  const int* n_ptr = &ctx->d_st->n_valid;
   if (H > 0) {
     // a peer-memory sharded round ships the winner's coefficients with its key, so only this rank's share is uploaded and
     // generated; otherwise (single GPU, or keys all-reduced by the caller) every rank generates all H to be able to refit any winner
     const int gen_all = ctx->sharded ? 0 : 1;
     if (!ctx->samples_staged) { gm_status st_ = stage_samples(ctx, kind, samples_host, gen_all ? 0 : h_begin, gen_all ? H : h_end, per); if (st_ != GM_OK) return st_; }
     const CommDev* commdev = ctx->sharded ? comm_dev(ctx) : nullptr;
-    int hb = div_up(H, 128);
-    { SegTimer seg_(ctx, kind == 0 ? SEG_PLANE_HYP : SEG_CYL_HYP);
-    if (kind == 0) {
-      GM_LAUNCH(ctx, k_plane_hypotheses, hb, 128, ctx->d_cloud_c, n_ptr, ctx->d_samples[0], H, ctx->d_plane_coef, ctx->d_hvalid[0],
-                ctx->d_counts[0], h_begin, h_end, gen_all);
-    } else {
-      GM_LAUNCH(ctx, k_cyl_hypotheses, hb, 128, ctx->d_cloud_c, ctx->d_normals_c, n_ptr, ctx->d_samples[1], H,
-                (float)ctx->prm.cylinderRadiusMin, (float)ctx->prm.cylinderRadiusMax, (float)ctx->prm.ransacThreshold,
-                ctx->d_model7, ctx->d_test12, ctx->d_hvalid[1], ctx->d_counts[1], h_begin, h_end, gen_all);
-    } }
-    const int hloc = h_end - h_begin;
-    bool argmax_done = false;
-    if (hloc > 0 && ctx->n_input > 0 && ctx->count_mode == 0 && has(ctx, NORMALS) && !ctx->injected) {
-      // tile-culled counting over the cell-sorted cloud of this scan (same counts, see gm_ransac.cuh)
-      argmax_done = true;
-      SegTimer seg_(ctx, kind == 0 ? SEG_PLANE_COUNT : SEG_CYL_COUNT);
-      const int blocks = std::max(1, div_up((long long)ctx->n_grid, TC_SUPER));
-      if (kind == 0) {
-        GM_LAUNCH(ctx, k_count_tiles<0>, blocks, TC_BLOCK, ctx->d_sorted_valid, ctx->d_leaf_bounds, &ctx->d_st->n_crop, ctx->d_plane_coef,
-                  ctx->d_test12, ctx->d_hvalid[0], h_begin, h_end, (float)ctx->prm.ransacThreshold, ctx->d_counts[0], H, ctx->d_key + 0,
-                  ctx->d_counters + 3, commdev, ctx->d_model7);
-      } else {
-        GM_LAUNCH(ctx, k_count_tiles<1>, blocks, TC_BLOCK, ctx->d_sorted_valid, ctx->d_leaf_bounds, &ctx->d_st->n_crop, ctx->d_plane_coef,
-                  ctx->d_test12, ctx->d_hvalid[1], h_begin, h_end, (float)ctx->prm.ransacThreshold, ctx->d_counts[1], H, ctx->d_key + 1,
-                  ctx->d_counters + 4, commdev, ctx->d_model7);
-      }
-    } else if (hloc > 0 && ctx->n_input > 0) {
-      argmax_done = true;  // folded into the count kernel's last block
-      SegTimer seg_(ctx, kind == 0 ? SEG_PLANE_COUNT : SEG_CYL_COUNT);
-      const int K = kind == 0 ? RC_KP : RC_KC;
-      int groups = div_up(hloc, RC_BLOCK * K);
-      // co-resident 64-thread blocks per SM (register limited to 14), every slice at least half a tile
-      static const int kBlocksPerSm = [] { const char* e = std::getenv("GM_COUNT_BLOCKS_PER_SM"); int v = e ? std::atoi(e) : 0; return v > 0 ? v : 8; }();
-      int slices = std::max(1, std::min(div_up((long long)ctx->n_grid, RC_TILE / 2), div_up(ctx->num_sms * kBlocksPerSm, groups)));
-      dim3 grid(slices, groups);
-      if (kind == 0) {
-        GM_LAUNCH(ctx, k_count_plane<RC_KP>, grid, RC_BLOCK, ctx->d_cloud_c, n_ptr, ctx->d_plane_coef, ctx->d_hvalid[0], h_begin, h_end,
-                  (float)ctx->prm.ransacThreshold, ctx->d_counts[0], H, ctx->d_key + 0, ctx->d_counters + 3, commdev);
-      } else {
-        GM_LAUNCH(ctx, k_count_cyl<RC_KC>, grid, RC_BLOCK, ctx->d_cloud_c, n_ptr, ctx->d_test12, h_begin, h_end, ctx->d_counts[1], H,
-                  ctx->d_key + 1, ctx->d_counters + 4, commdev, ctx->d_model7);
-      }
+    CountView cloud{ctx->d_cloud_c, &ctx->d_st->n_valid};
+    if (ctx->count_mode == 0 && has(ctx, NORMALS) && !ctx->injected) {  // the cell-sorted cloud of this scan
+      cloud.sorted = ctx->d_sorted_valid; cloud.leaf_bounds = ctx->d_leaf_bounds; cloud.n_sorted = &ctx->d_st->n_crop;
     }
-    if (!argmax_done) {
+    const bool count = h_end > h_begin && ctx->n_input > 0;
+    if (gm_status s = launch_hyp_count(ctx, ctx->hyp, kind, H, h_begin, h_end, gen_all, commdev, count ? &cloud : nullptr, true)) return s;
+    if (!count) {
       SegTimer seg_(ctx, kind == 0 ? SEG_PLANE_ARGMAX : SEG_CYL_ARGMAX);
-      GM_LAUNCH(ctx, k_argmax, 1, AM_BLOCK, ctx->d_counts[kind], H, ctx->d_key + kind, commdev, kind, ctx->d_plane_coef, ctx->d_model7, ctx->d_test12);
+      GM_LAUNCH(ctx, k_argmax, 1, AM_BLOCK, ctx->hyp.counts[kind], H, ctx->hyp.key + kind, commdev, kind, ctx->hyp.plane_coef, ctx->hyp.model7,
+                ctx->hyp.test12);
     }
   } else {
-    GM_CUDA(cudaMemsetAsync(ctx->d_key + kind, 0, sizeof(unsigned long long), ctx->stream));
+    GM_CUDA(cudaMemsetAsync(ctx->hyp.key + kind, 0, sizeof(unsigned long long), ctx->stream));
   }
   GM_CHECK_LAUNCHES(ctx);
   mark(ctx, ransac_stage(kind));
@@ -1061,51 +1108,29 @@ gm_status gm_ransac(gm_ctx* ctx, int32_t kind, const int32_t* samples_host, int3
 
 gm_status gm_ransac_key_device_ptr(gm_ctx* ctx, int32_t kind, void** key_dev) {
   if (!ctx || !key_dev || (kind != 0 && kind != 1)) return GM_ERR_INVALID_ARG;
-  *key_dev = (void*)(ctx->d_key + kind);
+  *key_dev = (void*)(ctx->hyp.key + kind);
   return GM_OK;
 }
 
 gm_status gm_ransac_export_key(gm_ctx* ctx, int32_t kind, void* dst_device) {
   if (!ctx || !dst_device || (kind != 0 && kind != 1)) return GM_ERR_INVALID_ARG;
   if (gm_status s = require(ctx, ransac_stage(kind))) return s;
-  GM_CUDA(cudaMemcpyAsync(dst_device, ctx->d_key + kind, sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
+  GM_CUDA(cudaMemcpyAsync(dst_device, ctx->hyp.key + kind, sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
   return GM_OK;
 }
 
 gm_status gm_ransac_import_key(gm_ctx* ctx, int32_t kind, const void* src_device) {
   if (!ctx || !src_device || (kind != 0 && kind != 1)) return GM_ERR_INVALID_ARG;
   if (gm_status s = require(ctx, ransac_stage(kind))) return s;
-  GM_CUDA(cudaMemcpyAsync(ctx->d_key + kind, src_device, sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
+  GM_CUDA(cudaMemcpyAsync(ctx->hyp.key + kind, src_device, sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
   return GM_OK;
 }
 
 gm_status gm_ransac_select(gm_ctx* ctx, int32_t kind) {
   if (!ctx || (kind != 0 && kind != 1)) return GM_ERR_INVALID_ARG;
   if (gm_status s = require(ctx, ransac_stage(kind))) return s;
-  const int* n_ptr = &ctx->d_st->n_valid;
-  ModelState* ms = ctx->d_model + kind;
   SegTimer seg_(ctx, kind == 0 ? SEG_PLANE_REFIT : SEG_CYL_REFIT);
-  const int H = ctx->ransac_H[kind];
-  const float tau = (float)ctx->prm.ransacThreshold;
-  if (kind == 0) {
-    GM_LAUNCH(ctx, k_plane_refit, REFIT_BLOCKS, RF_BLOCK, ctx->d_cloud_c, n_ptr, ctx->d_key + 0, H, ctx->d_plane_coef, ms, tau,
-              ctx->d_partials + 1 * kPartialsRegion, ctx->d_counters + 1);
-  } else {
-    GM_LAUNCH(ctx, k_cyl_inlier_compact, std::max(1, div_up((long long)ctx->n_grid, CPL_TILE)), CP_BLOCK, ctx->d_cloud_c, n_ptr,
-              ctx->d_key + 1, H, ctx->d_model7, ctx->d_test12, ms, ctx->d_inl, ctx->d_state64_b, ctx->d_ctl + 1, &ctx->d_st->error);
-    // all Gauss-Newton passes in one cooperative launch (grid barrier between passes)
-    {
-      const float4* inl = ctx->d_inl;
-      int iters = ctx->prm.refitIterations;
-      double* partials = ctx->d_partials + 2 * kPartialsRegion;
-      unsigned* bars = ctx->d_counters + 5;  // counters [5],[6]: the two barrier counters, [7]: which one the next launch uses
-      int* err = &ctx->d_st->error;
-      void* args[] = {(void*)&inl, (void*)&ms, (void*)&iters, (void*)&tau, (void*)&partials, (void*)&bars, (void*)&err};
-      GM_CUDA(cudaLaunchCooperativeKernel((const void*)k_cyl_gn_all, dim3(ctx->gn_blocks), dim3(RF_BLOCK), args, 0, ctx->stream));
-      ++ctx->launches;
-    }
-  }
-  GM_CHECK_LAUNCHES(ctx);
+  if (gm_status s = launch_refit(ctx, ctx->hyp, kind, ctx->ransac_H[kind], ctx->d_cloud_c, &ctx->d_st->n_valid)) return s;
   mark(ctx, model_stage(kind));
   return GM_OK;
 }
@@ -1116,7 +1141,7 @@ gm_status gm_label(gm_ctx* ctx) {
   if (ctx->n_input) {
     int blocks = std::min(div_up((long long)ctx->n_grid, 256), ctx->num_sms * 16);
     SegTimer seg_(ctx, SEG_LABEL);
-    GM_LAUNCH(ctx, k_label, blocks, 256, ctx->d_cloud_c, &ctx->d_st->n_valid, ctx->d_model + 0, ctx->d_model + 1,
+    GM_LAUNCH(ctx, k_label, blocks, 256, ctx->d_cloud_c, &ctx->d_st->n_valid, ctx->hyp.model + 0, ctx->hyp.model + 1,
               has(ctx, MODEL_PLANE) ? 1 : 0, has(ctx, MODEL_CYL) ? 1 : 0, (float)ctx->prm.ransacThreshold, ctx->d_labels);
     GM_CHECK_LAUNCHES(ctx);
   }
@@ -1140,7 +1165,7 @@ gm_status gm_axis_polyline(gm_ctx* ctx) {
     unsigned* n_list = ctx->d_counters + 10;
     GM_LAUNCH(ctx, k_poly_range, blocks, POLY_BLOCK, ctx->d_cloud_c, ctx->d_normals_c, ctx->d_labels, n_ptr, ctx->d_frame, shift, ctx->d_poly,
               ctx->d_poly_acc, POLY_NACC * S, ctx->d_poly_part, ctx->d_counters + 8, ctx->d_poly_list, cap, n_list, ctx->prm.sliceLength, S);
-    const ModelState* cylm = has(ctx, MODEL_CYL) ? ctx->d_model + 1 : nullptr;
+    const ModelState* cylm = has(ctx, MODEL_CYL) ? ctx->hyp.model + 1 : nullptr;
     GM_LAUNCH(ctx, k_poly_pass<0>, blocks, POLY_BLOCK, ctx->d_poly_list, cap, n_list, ctx->d_poly, ctx->d_poly_acc, ctx->d_slices,
               ctx->d_counters + 9, cylm);
     GM_LAUNCH(ctx, k_poly_pass<2>, blocks, POLY_BLOCK, ctx->d_poly_list, cap, n_list, ctx->d_poly, ctx->d_poly_acc, ctx->d_slices,
@@ -1158,7 +1183,7 @@ gm_status gm_compress(gm_ctx* ctx) {
   gm_status s;
   GM_LAUNCH(ctx, k_vox_reset, 1, 32, ctx->d_res_vs);
   const int tiles = div_up((long long)n, CP_TILE);
-  GM_LAUNCH(ctx, k_comp_split, tiles, CP_BLOCK, ctx->d_cloud_c, ctx->d_labels, &ctx->d_st->n_valid, ctx->d_model + 0, ctx->d_model + 1,
+  GM_LAUNCH(ctx, k_comp_split, tiles, CP_BLOCK, ctx->d_cloud_c, ctx->d_labels, &ctx->d_st->n_valid, ctx->hyp.model + 0, ctx->hyp.model + 1,
             has(ctx, MODEL_PLANE) ? 1 : 0, has(ctx, MODEL_CYL) ? 1 : 0, ctx->d_res_pts, ctx->d_res_vs, ctx->d_state64, ctx->d_ctl + 0, &ctx->d_st->error,
             ctx->d_comp_part, ctx->d_comp_mm, ctx->d_counters + 12, ctx->d_comp);
   VoxBuffers o{ctx->d_res_key_pt, ctx->d_res_assign, ctx->d_res_vox_start, ctx->d_res_vox_key, ctx->d_res_vox_count, ctx->d_res_centroid};
@@ -1174,6 +1199,24 @@ gm_status gm_compress(gm_ctx* ctx) {
 }
 
 namespace {
+// A compressed blob (GMC1, GMP1) starts with its 4-byte magic, a 4-byte version 1 and its header; returns where the
+// body starts.
+unsigned char* put_blob_header(void* buf, uint32_t magic, const void* header, size_t header_bytes) {
+  unsigned char* p = (unsigned char*)buf;
+  const uint32_t version = 1;
+  std::memcpy(p, &magic, 4); std::memcpy(p + 4, &version, 4);
+  std::memcpy(p + 8, header, header_bytes);
+  return p + 8 + header_bytes;
+}
+
+// ... and ends with the `n` residual voxel centroids as packed xyz; waits for every copy of the blob.
+gm_status put_blob_centroids(gm_ctx* ctx, unsigned char* p, const float4* centroids, int n) {
+  if (n > 0)  // strided copy: float4 centroids -> packed xyz
+    GM_CUDA(cudaMemcpy2DAsync(p, 12, centroids, 16, 12, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  return GM_OK;
+}
+
 gm_status fetch_compression(gm_ctx* ctx, gm_compression* out, VoxState* vs_host) {
   CompStats c;
   PolyState ps;
@@ -1217,15 +1260,9 @@ gm_status gm_download_compressed(gm_ctx* ctx, void* buf, size_t capacity, size_t
   *bytes = (size_t)h.bytes_out;
   if (!buf) return GM_OK;
   if (capacity < h.bytes_out) return GM_ERR_CAPACITY;
-  unsigned char* p = (unsigned char*)buf;
-  const uint32_t magic = 0x31434D47u /* 'GMC1' */, version = 1;
-  std::memcpy(p, &magic, 4); std::memcpy(p + 4, &version, 4); p += 8;
-  std::memcpy(p, &h, sizeof(h)); p += sizeof(h);
+  unsigned char* p = put_blob_header(buf, 0x31434D47u /* 'GMC1' */, &h, sizeof(h));
   if (h.n_slices > 0) { GM_CUDA(cudaMemcpyAsync(p, ctx->d_slices, (size_t)h.n_slices * sizeof(gm_slice), cudaMemcpyDeviceToHost, ctx->stream)); p += (size_t)h.n_slices * sizeof(gm_slice); }
-  if (h.n_residual_voxels > 0)  // strided copy: float4 centroids -> packed xyz
-    GM_CUDA(cudaMemcpy2DAsync(p, 12, ctx->d_res_centroid, 16, 12, (size_t)h.n_residual_voxels, cudaMemcpyDeviceToHost, ctx->stream));
-  GM_CUDA(cudaStreamSynchronize(ctx->stream));
-  return GM_OK;
+  return put_blob_centroids(ctx, p, ctx->d_res_centroid, h.n_residual_voxels);
 }
 
 }  // extern "C" (templates need C++ linkage)
@@ -1244,6 +1281,22 @@ static gm_status run_branch(gm_ctx* ctx, int b, F&& body) {
   e = cudaEventRecord(ctx->ev_join[b], ctx->branch[b]);
   if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return GM_ERR_CUDA; }
   return GM_OK;
+}
+
+// The plane step on branch stream 1 and the cylinder step on the main stream, side by side, then the main stream waits
+// for the branch.  They run one after the other unless the context is concurrent, not profiling, and `may_fork`.
+template <class P, class C>
+static gm_status plane_and_cylinder(gm_ctx* ctx, P&& plane, C&& cylinder, bool may_fork = true) {
+  gm_status s;
+  if (ctx->concurrent && !ctx->profiling && may_fork) {
+    GM_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
+    if ((s = run_branch(ctx, 1, plane)) != GM_OK) return s;
+    if ((s = cylinder()) != GM_OK) return s;
+    GM_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join[1], 0));
+    return GM_OK;
+  }
+  if ((s = plane()) != GM_OK) return s;
+  return cylinder();
 }
 
 static gm_status process_scan_body(gm_ctx* ctx, const int32_t* plane_samples_host, int32_t Hp, const int32_t* cyl_samples_host, int32_t Hc) {
@@ -1400,44 +1453,27 @@ gm_status gm_ransac_pair(gm_ctx* ctx, const int32_t* plane_samples_host, int32_t
                          const int32_t* cyl_samples_host, int32_t Hc, int32_t c_begin, int32_t c_end) {
   if (!ctx) return GM_ERR_INVALID_ARG;
   if (gm_status s = require(ctx, COMPACTED)) return s;
-  gm_status s;
-  if (ctx->concurrent && !ctx->profiling) {
-    GM_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
-    if ((s = run_branch(ctx, 1, [&] { return gm_ransac(ctx, GM_MODEL_PLANE, plane_samples_host, Hp, p_begin, p_end); })) != GM_OK) return s;
-    if ((s = gm_ransac(ctx, GM_MODEL_CYLINDER, cyl_samples_host, Hc, c_begin, c_end)) != GM_OK) return s;
-    GM_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join[1], 0));
-    return GM_OK;
-  }
-  if ((s = gm_ransac(ctx, GM_MODEL_PLANE, plane_samples_host, Hp, p_begin, p_end)) != GM_OK) return s;
-  return gm_ransac(ctx, GM_MODEL_CYLINDER, cyl_samples_host, Hc, c_begin, c_end);
+  return plane_and_cylinder(ctx, [&] { return gm_ransac(ctx, GM_MODEL_PLANE, plane_samples_host, Hp, p_begin, p_end); },
+                            [&] { return gm_ransac(ctx, GM_MODEL_CYLINDER, cyl_samples_host, Hc, c_begin, c_end); });
 }
 
 gm_status gm_ransac_select_pair(gm_ctx* ctx) {
   if (!ctx) return GM_ERR_INVALID_ARG;
   if (gm_status s = require(ctx, RANSAC_PLANE, RANSAC_CYL)) return s;
-  gm_status s;
-  if (ctx->concurrent && !ctx->profiling) {
-    GM_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
-    if ((s = run_branch(ctx, 1, [&] { return gm_ransac_select(ctx, GM_MODEL_PLANE); })) != GM_OK) return s;
-    if ((s = gm_ransac_select(ctx, GM_MODEL_CYLINDER)) != GM_OK) return s;
-    GM_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join[1], 0));
-    return GM_OK;
-  }
-  if ((s = gm_ransac_select(ctx, GM_MODEL_PLANE)) != GM_OK) return s;
-  return gm_ransac_select(ctx, GM_MODEL_CYLINDER);
+  return plane_and_cylinder(ctx, [&] { return gm_ransac_select(ctx, GM_MODEL_PLANE); }, [&] { return gm_ransac_select(ctx, GM_MODEL_CYLINDER); });
 }
 
 /* both keys (plane, cylinder) as 16 contiguous bytes */
 gm_status gm_ransac_export_keys(gm_ctx* ctx, void* dst_device) {
   if (!ctx || !dst_device) return GM_ERR_INVALID_ARG;
   if (gm_status s = require(ctx, RANSAC_PLANE, RANSAC_CYL)) return s;
-  GM_CUDA(cudaMemcpyAsync(dst_device, ctx->d_key, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
+  GM_CUDA(cudaMemcpyAsync(dst_device, ctx->hyp.key, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
   return GM_OK;
 }
 gm_status gm_ransac_import_keys(gm_ctx* ctx, const void* src_device) {
   if (!ctx || !src_device) return GM_ERR_INVALID_ARG;
   if (gm_status s = require(ctx, RANSAC_PLANE, RANSAC_CYL)) return s;
-  GM_CUDA(cudaMemcpyAsync(ctx->d_key, src_device, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
+  GM_CUDA(cudaMemcpyAsync(ctx->hyp.key, src_device, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, ctx->stream));
   return GM_OK;
 }
 
@@ -1460,86 +1496,21 @@ gm_status ensure_prim_buffers(gm_ctx* ctx, size_t plane_draws, size_t cyl_draws)
   const size_t N = ctx->cap, H = (size_t)ctx->hcap;
   GM_CUDA(ctx->d_pr_sv.alloc(N)); GM_CUDA(ctx->d_pr_cc.alloc(N)); GM_CUDA(ctx->d_pr_lb.alloc(2 * ((N + 31) / 32)));
   GM_CUDA(ctx->d_pr_rem.alloc(N)); GM_CUDA(ctx->d_pr_ids.alloc(N));
-  GM_CUDA(ctx->d_pr_samples[0].alloc(3 * H)); GM_CUDA(ctx->d_pr_samples[1].alloc(2 * H));
-  GM_CUDA(ctx->d_pr_plane_coef.alloc(H)); GM_CUDA(ctx->d_pr_model7.alloc(7 * H)); GM_CUDA(ctx->d_pr_test12.alloc(12 * H));
-  for (int k = 0; k < 2; ++k) { GM_CUDA(ctx->d_pr_hvalid[k].alloc(H)); GM_CUDA(ctx->d_pr_counts[k].alloc(H)); }
-  GM_CUDA(ctx->d_pr_key.alloc(2)); GM_CUDA(ctx->d_pr_model.alloc(2));
+  GM_CUDA(ctx->pr_hyp.alloc(H));
   GM_CUDA(ctx->d_pr_state.alloc(1));  // last: a failure above leaves the set unallocated
-  return GM_OK;
-}
-
-// Hypotheses, inlier counts and argmax of one kind in one round: the launches of gm_ransac on the extraction's tables.
-// Hypotheses read the original compacted cloud (R_r indices are never blanked); counts read the blanked working copies
-// through the live sizes, which are 0 once extraction stopped.
-gm_status prim_count(gm_ctx* ctx, int kind, int H, bool tiles) {
-  PrimState* ps = ctx->d_pr_state;
-  const int* n_valid = &ctx->d_st->n_valid;
-  const float tau = (float)ctx->prm.ransacThreshold;
-  const int hb = div_up(H, 128);
-  if (kind == 0) {
-    GM_LAUNCH(ctx, k_plane_hypotheses, hb, 128, ctx->d_cloud_c, n_valid, ctx->d_pr_samples[0], H, ctx->d_pr_plane_coef, ctx->d_pr_hvalid[0],
-              ctx->d_pr_counts[0], 0, H, 1);
-  } else {
-    GM_LAUNCH(ctx, k_cyl_hypotheses, hb, 128, ctx->d_cloud_c, ctx->d_normals_c, n_valid, ctx->d_pr_samples[1], H,
-              (float)ctx->prm.cylinderRadiusMin, (float)ctx->prm.cylinderRadiusMax, tau, ctx->d_pr_model7, ctx->d_pr_test12,
-              ctx->d_pr_hvalid[1], ctx->d_pr_counts[1], 0, H, 1);
-  }
-  if (tiles) {
-    const int blocks = std::max(1, div_up((long long)ctx->n_grid, TC_SUPER));
-    if (kind == 0) {
-      GM_LAUNCH(ctx, k_count_tiles<0>, blocks, TC_BLOCK, ctx->d_pr_sv, ctx->d_pr_lb, &ps->n_crop_live, ctx->d_pr_plane_coef, ctx->d_pr_test12,
-                ctx->d_pr_hvalid[0], 0, H, tau, ctx->d_pr_counts[0], H, ctx->d_pr_key + 0, ctx->d_counters + 3, nullptr, ctx->d_pr_model7);
-    } else {
-      GM_LAUNCH(ctx, k_count_tiles<1>, blocks, TC_BLOCK, ctx->d_pr_sv, ctx->d_pr_lb, &ps->n_crop_live, ctx->d_pr_plane_coef, ctx->d_pr_test12,
-                ctx->d_pr_hvalid[1], 0, H, tau, ctx->d_pr_counts[1], H, ctx->d_pr_key + 1, ctx->d_counters + 4, nullptr, ctx->d_pr_model7);
-    }
-  } else {
-    const int K = kind == 0 ? RC_KP : RC_KC;
-    const int groups = div_up(H, RC_BLOCK * K);
-    const int slices = std::max(1, std::min(div_up((long long)ctx->n_grid, RC_TILE / 2), div_up(ctx->num_sms * 8, groups)));
-    const dim3 grid(slices, groups);
-    if (kind == 0) {
-      GM_LAUNCH(ctx, k_count_plane<RC_KP>, grid, RC_BLOCK, ctx->d_pr_cc, &ps->n_valid_live, ctx->d_pr_plane_coef, ctx->d_pr_hvalid[0], 0, H, tau,
-                ctx->d_pr_counts[0], H, ctx->d_pr_key + 0, ctx->d_counters + 3, nullptr);
-    } else {
-      GM_LAUNCH(ctx, k_count_cyl<RC_KC>, grid, RC_BLOCK, ctx->d_pr_cc, &ps->n_valid_live, ctx->d_pr_test12, 0, H, ctx->d_pr_counts[1], H,
-                ctx->d_pr_key + 1, ctx->d_counters + 4, nullptr, ctx->d_pr_model7);
-    }
-  }
-  GM_CHECK_LAUNCHES(ctx);
-  return GM_OK;
-}
-
-// Refit of one kind on the blanked compacted copy: the launches of gm_ransac_select on the extraction's key and model.
-// The key of a kind that did not win the round is 0, so its refit finds no model.
-gm_status prim_refit(gm_ctx* ctx, int kind, int H) {
-  PrimState* ps = ctx->d_pr_state;
-  ModelState* ms = ctx->d_pr_model + kind;
-  const float tau = (float)ctx->prm.ransacThreshold;
-  if (kind == 0) {
-    GM_LAUNCH(ctx, k_plane_refit, REFIT_BLOCKS, RF_BLOCK, ctx->d_pr_cc, &ps->n_valid_live, ctx->d_pr_key + 0, H, ctx->d_pr_plane_coef, ms, tau,
-              ctx->d_partials + 1 * kPartialsRegion, ctx->d_counters + 1);
-  } else {
-    GM_LAUNCH(ctx, k_cyl_inlier_compact, std::max(1, div_up((long long)ctx->n_grid, CPL_TILE)), CP_BLOCK, ctx->d_pr_cc, &ps->n_valid_live,
-              ctx->d_pr_key + 1, H, ctx->d_pr_model7, ctx->d_pr_test12, ms, ctx->d_inl, ctx->d_state64_b, ctx->d_ctl + 1, &ctx->d_st->error);
-    const float4* inl = ctx->d_inl;
-    int iters = ctx->prm.refitIterations;
-    double* partials = ctx->d_partials + 2 * kPartialsRegion;
-    unsigned* bars = ctx->d_counters + 5;
-    int* err = &ctx->d_st->error;
-    void* args[] = {(void*)&inl, (void*)&ms, (void*)&iters, (void*)&tau, (void*)&partials, (void*)&bars, (void*)&err};
-    GM_CUDA(cudaLaunchCooperativeKernel((const void*)k_cyl_gn_all, dim3(ctx->gn_blocks), dim3(RF_BLOCK), args, 0, ctx->stream));
-    ++ctx->launches;
-  }
-  GM_CHECK_LAUNCHES(ctx);
   return GM_OK;
 }
 
 gm_status extract_rounds(gm_ctx* ctx, int K, int min_inliers, int Hp, int Hc) {
   const size_t n = ctx->n_grid;
+  PrimState* ps = ctx->d_pr_state;
+  HypSet& hs = ctx->pr_hyp;
   // the scan's cell-sorted copy exists: claims walk it and keep its leaf bounds current; counting uses it unless count_mode = 1
   const bool sorted = has(ctx, NORMALS) && !ctx->injected;
-  const bool tiles = sorted && ctx->count_mode == 0;
+  // Hypotheses read the original compacted cloud (R_r indices are never blanked); counts and refits read the blanked
+  // working copies through the live sizes, which are 0 once extraction stopped.
+  CountView cloud{ctx->d_pr_cc, &ps->n_valid_live};
+  if (sorted && ctx->count_mode == 0) { cloud.sorted = ctx->d_pr_sv; cloud.leaf_bounds = ctx->d_pr_lb; cloud.n_sorted = &ps->n_crop_live; }
   GM_CUDA(cudaMemsetAsync(ctx->d_pr_ids, 0, n, ctx->stream));
   GM_CUDA(cudaMemcpyAsync(ctx->d_pr_cc, ctx->d_cloud_c, n * sizeof(float4), cudaMemcpyDeviceToDevice, ctx->stream));
   if (sorted) {
@@ -1548,18 +1519,10 @@ gm_status extract_rounds(gm_ctx* ctx, int K, int min_inliers, int Hp, int Hc) {
   }
   const int H[2] = {Hp, Hc};
   gm_status s;
-  // the plane step on branch stream 1 and the cylinder step on the main stream, side by side as in gm_ransac_pair
+  // the step of each kind that has hypotheses; side by side as in gm_ransac_pair when both have
   auto both = [&](auto&& step) -> gm_status {
-    if (ctx->concurrent && !ctx->profiling && Hp > 0 && Hc > 0) {
-      GM_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
-      if ((s = run_branch(ctx, 1, [&] { return step(0); })) != GM_OK) return s;
-      if ((s = step(1)) != GM_OK) return s;
-      GM_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join[1], 0));
-      return GM_OK;
-    }
-    for (int k = 0; k < 2; ++k)
-      if (H[k] > 0 && (s = step(k)) != GM_OK) return s;
-    return GM_OK;
+    return plane_and_cylinder(ctx, [&]() -> gm_status { return Hp > 0 ? step(0) : GM_OK; },
+                              [&]() -> gm_status { return Hc > 0 ? step(1) : GM_OK; }, Hp > 0 && Hc > 0);
   };
   const int draws = Hp * 3 + Hc * 2;
   const int point_blocks = std::min(div_up((long long)n, 256), ctx->num_sms * 8);
@@ -1567,17 +1530,17 @@ gm_status extract_rounds(gm_ctx* ctx, int K, int min_inliers, int Hp, int Hc) {
     GM_LAUNCH(ctx, k_prim_remaining, std::max(1, div_up((long long)n, CPL_TILE)), CP_BLOCK, ctx->d_pr_ids, ctx->d_pr_state, ctx->d_pr_rem,
               ctx->d_state64, ctx->d_ctl + 0, &ctx->d_st->error);
     GM_LAUNCH(ctx, k_prim_draws, std::max(1, std::min(div_up(draws, 256), ctx->num_sms * 4)), 256, ctx->d_pr_draws[0] + (size_t)r * Hp * 3, Hp * 3,
-              ctx->d_pr_draws[1] + (size_t)r * Hc * 2, Hc * 2, ctx->d_pr_rem, ctx->d_pr_state, ctx->d_pr_samples[0], ctx->d_pr_samples[1]);
-    if ((s = both([&](int k) { return prim_count(ctx, k, H[k], tiles); })) != GM_OK) return s;
-    GM_LAUNCH(ctx, k_prim_decide, 1, 32, ctx->d_pr_key, Hp > 0 ? 1 : 0, Hc > 0 ? 1 : 0, min_inliers, Hp, Hc, ctx->d_pr_plane_coef, ctx->d_pr_test12,
-              ctx->d_pr_state);
-    if ((s = both([&](int k) { return prim_refit(ctx, k, H[k]); })) != GM_OK) return s;
+              ctx->d_pr_draws[1] + (size_t)r * Hc * 2, Hc * 2, ctx->d_pr_rem, ctx->d_pr_state, hs.samples[0], hs.samples[1]);
+    if ((s = both([&](int k) { return launch_hyp_count(ctx, hs, k, H[k], 0, H[k], 1, nullptr, &cloud, false); })) != GM_OK) return s;
+    GM_LAUNCH(ctx, k_prim_decide, 1, 32, hs.key, Hp > 0 ? 1 : 0, Hc > 0 ? 1 : 0, min_inliers, Hp, Hc, hs.plane_coef, hs.test12, ctx->d_pr_state);
+    // the key of a kind that did not win the round is 0, so its refit finds no model
+    if ((s = both([&](int k) { return launch_refit(ctx, hs, k, H[k], ctx->d_pr_cc, &ps->n_valid_live); })) != GM_OK) return s;
     const float tau = (float)ctx->prm.ransacThreshold;
     if (sorted) {
       GM_LAUNCH(ctx, k_prim_claim_sorted, point_blocks, 256, ctx->d_pr_sv, ctx->d_pr_lb, ctx->d_valid_map, ctx->d_pr_cc, ctx->d_pr_ids,
-                ctx->d_pr_state, ctx->d_pr_model, tau, r);
+                ctx->d_pr_state, hs.model, tau, r);
     } else {
-      GM_LAUNCH(ctx, k_prim_claim_compact, point_blocks, 256, ctx->d_pr_cc, ctx->d_pr_ids, ctx->d_pr_state, ctx->d_pr_model, tau, r);
+      GM_LAUNCH(ctx, k_prim_claim_compact, point_blocks, 256, ctx->d_pr_cc, ctx->d_pr_ids, ctx->d_pr_state, hs.model, tau, r);
     }
     GM_CHECK_LAUNCHES(ctx);
   }
@@ -1683,15 +1646,9 @@ gm_status gm_download_compressed_primitives(gm_ctx* ctx, void* buf, size_t capac
   *bytes = (size_t)h.bytes_out;
   if (!buf) return GM_OK;
   if (capacity < h.bytes_out) return GM_ERR_CAPACITY;
-  unsigned char* p = (unsigned char*)buf;
-  const uint32_t magic = 0x31504D47u /* 'GMP1' */, version = 1;
-  std::memcpy(p, &magic, 4); std::memcpy(p + 4, &version, 4); p += 8;
-  std::memcpy(p, &h, sizeof(h)); p += sizeof(h);
+  unsigned char* p = put_blob_header(buf, 0x31504D47u /* 'GMP1' */, &h, sizeof(h));
   std::memcpy(p, c.rec, (size_t)h.n_primitives * sizeof(gm_primitive_record)); p += (size_t)h.n_primitives * sizeof(gm_primitive_record);
-  if (h.n_residual_voxels > 0)  // strided copy: float4 centroids -> packed xyz
-    GM_CUDA(cudaMemcpy2DAsync(p, 12, ctx->d_pr_cc, 16, 12, (size_t)h.n_residual_voxels, cudaMemcpyDeviceToHost, ctx->stream));
-  GM_CUDA(cudaStreamSynchronize(ctx->stream));
-  return GM_OK;
+  return put_blob_centroids(ctx, p, ctx->d_pr_cc, h.n_residual_voxels);
 }
 
 // ---- results ---------------------------------------------------------------------------------
@@ -1799,11 +1756,11 @@ gm_status gm_download_hypotheses(gm_ctx* ctx, int32_t kind, float* coef, float* 
   size_t H = (size_t)ctx->ransac_H[kind];
   if ((int)H > capacity_h) return GM_ERR_CAPACITY;
   if (coef) {
-    if (kind == 0) GM_D2H(coef, ctx->d_plane_coef, H * 16);
-    else GM_D2H(coef, ctx->d_model7, H * 28);
+    if (kind == 0) GM_D2H(coef, ctx->hyp.plane_coef, H * 16);
+    else GM_D2H(coef, ctx->hyp.model7, H * 28);
   }
-  if (test12 && kind == 1) GM_D2H(test12, ctx->d_test12, H * 48);
-  if (counts) GM_D2H(counts, ctx->d_counts[kind], H * 4);
+  if (test12 && kind == 1) GM_D2H(test12, ctx->hyp.test12, H * 48);
+  if (counts) GM_D2H(counts, ctx->hyp.counts[kind], H * 4);
   GM_CUDA(cudaStreamSynchronize(ctx->stream));
   return GM_OK;
 }
@@ -1812,7 +1769,7 @@ gm_status gm_get_model(gm_ctx* ctx, int32_t kind, gm_model* out) {
   if (!ctx || !out || (kind != 0 && kind != 1)) return GM_ERR_INVALID_ARG;
   if (gm_status s = require(ctx, model_stage(kind))) return s;
   ModelState h;
-  GM_D2H(&h, ctx->d_model + kind, sizeof(ModelState));
+  GM_D2H(&h, ctx->hyp.model + kind, sizeof(ModelState));
   GM_CUDA(cudaStreamSynchronize(ctx->stream));
   out->kind = h.kind; out->best_id = h.best_id; out->best_count = h.best_count; out->refit_count = h.refit_count;
   std::memcpy(out->hyp, h.hyp, sizeof(out->hyp));
@@ -1850,7 +1807,7 @@ gm_status gm_fetch_async(gm_ctx* ctx, const gm_host_outputs* out) {
   const size_t n = ctx->n_input;
   if (out->summary) {
     int mask = (has(ctx, MODEL_PLANE) ? 1 : 0) | (has(ctx, MODEL_CYL) ? 2 : 0) | (has(ctx, POLY) ? 4 : 0);
-    GM_LAUNCH(ctx, k_pack_summary, 1, 32, ctx->d_st, ctx->d_frame, ctx->d_model, ctx->d_poly, mask, ctx->d_summary);
+    GM_LAUNCH(ctx, k_pack_summary, 1, 32, ctx->d_st, ctx->d_frame, ctx->hyp.model, ctx->d_poly, mask, ctx->d_summary);
     GM_CHECK_LAUNCHES(ctx);
     GM_CUDA(cudaMemcpyAsync(out->summary, ctx->d_summary, sizeof(SummaryDev), cudaMemcpyDeviceToHost, ctx->stream));
   }
@@ -2303,8 +2260,8 @@ gm_status gm_ransac_sharded(gm_ctx* ctx, const int32_t* plane_samples_host, int3
   int pb, pe, cb, ce;
   range(Hp, pb, pe); range(Hc, cb, ce);
   auto recv = [&](int kind, int H) -> gm_status {
-    GM_LAUNCH(ctx, k_comm_recv_model, 1, 32, ctx->comm->h_dev, kind, H, ctx->d_key + kind, ctx->d_plane_coef, ctx->d_model7, ctx->d_test12,
-              ctx->d_counts[kind], &ctx->d_st->error);
+    GM_LAUNCH(ctx, k_comm_recv_model, 1, 32, ctx->comm->h_dev, kind, H, ctx->hyp.key + kind, ctx->hyp.plane_coef, ctx->hyp.model7, ctx->hyp.test12,
+              ctx->hyp.counts[kind], &ctx->d_st->error);
     GM_CHECK_LAUNCHES(ctx);
     return GM_OK;
   };
@@ -2319,18 +2276,8 @@ gm_status gm_ransac_sharded(gm_ctx* ctx, const int32_t* plane_samples_host, int3
     return r != GM_OK ? r : gm_ransac_select(ctx, GM_MODEL_CYLINDER);
   };
   auto body = [&]() -> gm_status {
-    gm_status s;
     ctx->sharded = true;
-    if (ctx->concurrent && !ctx->profiling) {
-      cudaError_t e = cudaEventRecord(ctx->ev_fork, ctx->stream);
-      if (e != cudaSuccess) { ctx->sharded = false; ctx->err = cudaGetErrorString(e); return GM_ERR_CUDA; }
-      s = run_branch(ctx, 1, plane);
-      if (s == GM_OK) s = cylinder();
-      if (s == GM_OK && cudaStreamWaitEvent(ctx->stream, ctx->ev_join[1], 0) != cudaSuccess) s = GM_ERR_CUDA;
-    } else {
-      s = plane();
-      if (s == GM_OK) s = cylinder();
-    }
+    const gm_status s = plane_and_cylinder(ctx, plane, cylinder);
     ctx->sharded = false;
     return s;
   };
