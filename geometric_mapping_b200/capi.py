@@ -94,6 +94,19 @@ class gm_primitive_compression(C.Structure):
                 ("bytes_in", C.c_uint64), ("bytes_out", C.c_uint64)]
 
 
+class gm_icp_params(C.Structure):
+    _fields_ = [("init_pose34", C.c_float * 12), ("max_correspondence_distance", C.c_double), ("max_iterations", C.c_int32),
+                ("pad_", C.c_int32), ("min_rotation_step", C.c_double), ("min_translation_step", C.c_double),
+                ("degeneracy_ratio", C.c_double)]
+
+
+class gm_registration(C.Structure):
+    _fields_ = [("pose34", C.c_float * 12), ("iterations", C.c_int32), ("converged", C.c_int32), ("n_source", C.c_int32),
+                ("n_correspondences", C.c_int32), ("rmse", C.c_float), ("fitness", C.c_float), ("n_degenerate", C.c_int32),
+                ("pad_", C.c_int32), ("eigenvalues", C.c_double * 6), ("eigenvectors", C.c_double * 36)]
+
+
+GM_MAX_ICP_ITERATIONS = 64
 GM_MAX_PRIMITIVES = 64
 PRIMITIVE_RECORD_DTYPE = np.dtype([("kind", "<i4"), ("count", "<i4"), ("coef", "<f4", 7), ("extents", "<f4", 4), ("rms", "<f4")])
 
@@ -144,7 +157,8 @@ SYMBOLS = [
     "gm_map_load", "gm_map_leaf", "gm_set_normals_mode", "gm_set_graph_mode", "gm_get_graph_stats",
     "gm_comm_create", "gm_comm_handle", "gm_comm_connect", "gm_comm_mailbox", "gm_comm_connect_local", "gm_comm_destroy", "gm_comm_rank", "gm_comm_world", "gm_comm_last_error", "gm_set_comm", "gm_ransac_sharded", "gm_allreduce_voxel_bbox", "gm_allreduce_frame", "gm_set_voxel_bbox_hint", "gm_set_knn", "gm_download_knn_indices", "gm_set_knn_max_radius", "gm_pointcloud2_size", "gm_encode_pointcloud2", "gm_marker_array_size",
     "gm_extract_primitives", "gm_get_primitives", "gm_download_primitive_ids", "gm_compress_primitives",
-    "gm_download_compressed_primitives",
+    "gm_download_compressed_primitives", "gm_icp_params_default", "gm_register", "gm_get_registration",
+    "gm_download_correspondences",
     "gm_encode_marker_array", "gm_store_open", "gm_store_close", "gm_store_append", "gm_store_append_blob", "gm_store_count", "gm_store_info", "gm_store_read",
 ]
 
@@ -271,6 +285,10 @@ def _lib():
         "gm_download_primitive_ids": (i32, [vp, vp, sz]),
         "gm_compress_primitives": (i32, [vp]),
         "gm_download_compressed_primitives": (i32, [vp, vp, sz, C.POINTER(sz)]),
+        "gm_icp_params_default": (None, [C.POINTER(gm_icp_params)]),
+        "gm_register": (i32, [vp, vp, C.POINTER(gm_icp_params)]),
+        "gm_get_registration": (i32, [vp, C.POINTER(gm_registration)]),
+        "gm_download_correspondences": (i32, [vp, vp, vp, sz]),
     }
     assert set(sig) == set(SYMBOLS)
     for name, (res, args) in sig.items():
@@ -737,6 +755,61 @@ def parse_compressed_primitives(blob: bytes) -> dict:
     return {"header": h, "records": rec, "residual": res}
 
 
+def icp_params(init_pose34=None, **overrides) -> gm_icp_params:
+    """gm_icp_params with the library defaults, the initial guess (3x4 or 4x4 row-major [R|t], None = identity) and
+    any field overridden by keyword."""
+    p = gm_icp_params()
+    _lib().gm_icp_params_default(C.byref(p))
+    if init_pose34 is not None:
+        p.init_pose34[:] = [float(v) for v in np.asarray(init_pose34, np.float32)[:3, :4].reshape(12)]
+    for k, v in overrides.items():
+        if not hasattr(p, k) or k == "pad_":
+            raise AttributeError(f"gm_icp_params has no field {k}")
+        setattr(p, k, v)
+    return p
+
+
+def _registration_dict(r: gm_registration) -> dict:
+    return {"pose": np.array(r.pose34, np.float32).reshape(3, 4), "iterations": r.iterations, "converged": r.converged,
+            "n_source": r.n_source, "n_correspondences": r.n_correspondences, "rmse": float(r.rmse), "fitness": float(r.fitness),
+            "n_degenerate": r.n_degenerate, "eigenvalues": np.array(r.eigenvalues, np.float64),
+            "eigenvectors": np.array(r.eigenvectors, np.float64).reshape(6, 6), "_struct": r}
+
+
+def _ctx_register_async(self, target: "Context", init_pose34=None, **params):
+    """Enqueue gm_register(self = source, target) without waiting; read the result with registration()."""
+    p = icp_params(init_pose34, **params)
+    self._ck(_lib().gm_register(self._h, target._h, C.byref(p)), "gm_register")
+
+
+def _ctx_registration(self) -> dict:
+    r = gm_registration()
+    self._ck(_lib().gm_get_registration(self._h, C.byref(r)), "gm_get_registration")
+    return _registration_dict(r)
+
+
+def _ctx_register(self, target: "Context", init_pose34=None, **params) -> dict:
+    """Point-to-plane ICP of this context's voxel centroids (after voxel()) against `target`'s compacted cloud and normals
+    (after normals()).  Keywords: the fields of gm_icp_params.  -> {"pose": 3x4 float32 source -> target, "iterations",
+    "converged", "n_source", "n_correspondences", "rmse", "fitness", "n_degenerate", "eigenvalues" (6, ascending),
+    "eigenvectors" (6x6, column k = eigenvector k over (wx, wy, wz, vx, vy, vz))}."""
+    _ctx_register_async(self, target, init_pose34, **params)
+    return _ctx_registration(self)
+
+
+def _ctx_download_correspondences(self):
+    """-> (target_index int32 V: compacted target index or -1, residual float32 V: float(r) or NaN) of the last executed
+    iteration of the last register()."""
+    V = _ctx_registration(self)["n_source"]
+    idx, res = np.empty(max(V, 0), np.int32), np.empty(max(V, 0), np.float32)
+    self._ck(_lib().gm_download_correspondences(self._h, _ptr(idx), _ptr(res), idx.shape[0]), "gm_download_correspondences")
+    return idx, res
+
+
+Context.register = _ctx_register
+Context.register_async = _ctx_register_async
+Context.registration = _ctx_registration
+Context.download_correspondences = _ctx_download_correspondences
 Context.extract_primitives = _ctx_extract_primitives
 Context.primitives = _ctx_primitives
 Context.download_primitive_ids = _ctx_download_primitive_ids

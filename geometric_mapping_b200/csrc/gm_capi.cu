@@ -9,6 +9,7 @@
 #include "gm_primitives.cuh"
 #include "gm_map.cuh"
 #include "gm_comm.cuh"
+#include "gm_register.cuh"
 #include <new>
 
 #include <algorithm>
@@ -224,6 +225,14 @@ struct gm_ctx {
   struct gm_comm* comm = nullptr;
   bool sharded = false;
   DevBuf<double> d_frame_sums;  // [8] the 6 scatter sums of the last gm_local_frame, kept for gm_allreduce_frame
+  // registration of this context's voxel centroids (gm_register with this context as the source), allocated by the first
+  // call: block partials, last-block ticket, pose / result state, per-centroid correspondence and residual
+  DevBuf<double> d_reg_part;
+  DevBuf<unsigned> d_reg_ticket;
+  DevBuf<RegState> d_reg_state;
+  DevBuf<int> d_reg_idx;
+  DevBuf<float> d_reg_res;
+  cudaEvent_t ev_reg[2] = {nullptr, nullptr};  // target stream -> source stream, and back
   // profiling
   bool profiling = false;
   std::vector<cudaEvent_t> ev_pool;
@@ -252,10 +261,11 @@ struct SegTimer {
 // stages it reads are held, and marks its own stage.  Running a stage again does not drop the later ones.  A change
 // of input drops a stage and everything after it: a new scan from CROP on, a new crop box or is_dense from CROP on, a
 // new neighbour grid from NORMALS on (the compacted cloud too, even an injected one).  A new extraction drops the
-// compression of the previous one (PRIMS_COMP), whose buffers it reuses.
+// compression of the previous one (PRIMS_COMP), whose buffers it reuses.  REGISTRATION is the result of gm_register
+// with this context as the source; only a new scan or grid here drops it.
 enum Stage {
   SCAN, CROP, NORMALS, COMPACTED, VOXEL, FRAME, RANSAC_PLANE, RANSAC_CYL, MODEL_PLANE, MODEL_CYL, LABELS, POLY, COMP,
-  PRIMS, PRIMS_COMP
+  PRIMS, PRIMS_COMP, REGISTRATION
 };
 inline Stage ransac_stage(int kind) { return Stage(RANSAC_PLANE + kind); }
 inline Stage model_stage(int kind) { return Stage(MODEL_PLANE + kind); }
@@ -578,6 +588,7 @@ void gm_destroy(gm_ctx* ctx) {
   for (cudaEvent_t e : ctx->ev_pool) cudaEventDestroy(e);
   for (int b = 0; b < 3; ++b) { if (ctx->branch[b]) cudaStreamDestroy(ctx->branch[b]); if (ctx->ev_join[b]) cudaEventDestroy(ctx->ev_join[b]); }
   if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
+  for (cudaEvent_t e : ctx->ev_reg) if (e) cudaEventDestroy(e);
   if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
   delete ctx;  // frees the device buffers
 }
@@ -1649,6 +1660,128 @@ gm_status gm_download_compressed_primitives(gm_ctx* ctx, void* buf, size_t capac
   unsigned char* p = put_blob_header(buf, 0x31504D47u /* 'GMP1' */, &h, sizeof(h));
   std::memcpy(p, c.rec, (size_t)h.n_primitives * sizeof(gm_primitive_record)); p += (size_t)h.n_primitives * sizeof(gm_primitive_record);
   return put_blob_centroids(ctx, p, ctx->d_pr_cc, h.n_residual_voxels);
+}
+
+}  // extern "C"
+
+// ---- scan-to-scan registration (gm_register.cuh) -------------------------------------------------
+namespace {
+static_assert(sizeof(gm_icp_params) == 88 && sizeof(gm_registration) == 416, "registration layouts");
+
+int reg_blocks(const gm_ctx* ctx) { return ctx->num_sms * 8; }
+
+// First call: the source's registration buffers and events (rare path, synchronous).
+gm_status ensure_reg_buffers(gm_ctx* ctx) {
+  if (ctx->d_reg_state.count) return GM_OK;
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  for (cudaEvent_t& e : ctx->ev_reg)
+    if (!e) GM_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+  GM_CUDA(ctx->d_reg_part.alloc((size_t)reg_blocks(ctx) * REG_NV));
+  GM_CUDA(ctx->d_reg_idx.alloc(ctx->cap));
+  GM_CUDA(ctx->d_reg_res.alloc(ctx->cap));
+  GM_CUDA(ctx->d_reg_ticket.alloc(1));
+  GM_CUDA(cudaMemsetAsync(ctx->d_reg_ticket, 0, sizeof(unsigned), ctx->stream));
+  GM_CUDA(ctx->d_reg_state.alloc(1));  // last: a failure above leaves the set unallocated
+  GM_CUDA(cudaMemsetAsync(ctx->d_reg_state, 0, sizeof(RegState), ctx->stream));
+  return GM_OK;
+}
+
+bool finite_pose(const float* t) {
+  for (int k = 0; k < 12; ++k) if (!std::isfinite(t[k])) return false;
+  return true;
+}
+}  // namespace
+
+extern "C" {
+
+void gm_icp_params_default(gm_icp_params* p) {
+  if (!p) return;
+  std::memset(p, 0, sizeof(*p));
+  p->init_pose34[0] = p->init_pose34[5] = p->init_pose34[10] = 1.0f;
+  p->max_correspondence_distance = 0.5;
+  p->max_iterations = 30;
+  p->min_rotation_step = 1e-5;
+  p->min_translation_step = 1e-5;
+  p->degeneracy_ratio = 0.0;
+}
+
+gm_status gm_register(gm_ctx* source, gm_ctx* target, const gm_icp_params* p) {
+  if (!source || !target || !p) return GM_ERR_INVALID_ARG;
+  gm_ctx* ctx = source;  // GM_CUDA / GM_LAUNCH report on the source
+  if (source->device != target->device) { ctx->err = "gm_register: source and target on different devices"; return GM_ERR_INVALID_ARG; }
+  const double dmax = p->max_correspondence_distance;
+  if (!(dmax > 0.0) || !std::isfinite(dmax) || p->max_iterations < 1 || p->max_iterations > GM_MAX_ICP_ITERATIONS ||
+      !(p->min_rotation_step >= 0.0) || !(p->min_translation_step >= 0.0) || !(p->degeneracy_ratio >= 0.0) ||
+      !(p->degeneracy_ratio < 1.0) || !finite_pose(p->init_pose34))
+    return GM_ERR_INVALID_ARG;
+  if (gm_status s = require(target, NORMALS)) return s;
+  if (target->injected) return GM_ERR_STAGE_ORDER;
+  if (gm_status s = require(source, VOXEL)) return s;
+  if (gm_status s = ensure_reg_buffers(source)) return s;
+  ctx->stages &= ~(1u << REGISTRATION);
+  if (target != source) {
+    GM_CUDA(cudaEventRecord(source->ev_reg[0], target->stream));
+    GM_CUDA(cudaStreamWaitEvent(source->stream, source->ev_reg[0], 0));
+  }
+  Pose34 init;
+  std::memcpy(init.r, p->init_pose34, sizeof(init.r));
+  GM_LAUNCH(ctx, k_reg_begin, 1, 32, source->d_reg_state, init, &source->d_st->vox.n_voxels);
+  RegParams rp;
+  rp.d_max = dmax;
+  rp.r2max = (float)(dmax * dmax);
+  rp.min_rot = p->min_rotation_step;
+  rp.min_trans = p->min_translation_step;
+  rp.ratio = p->degeneracy_ratio;
+  // an empty target built no grid this scan: its block table may still describe an earlier one
+  const int search = target->n_grid > 0 ? 1 : 0;
+  const int blocks = std::max(1, std::min(div_up((long long)source->n_grid * 32, REG_BLOCK), reg_blocks(source)));
+  for (int it = 0; it < p->max_iterations; ++it)
+    GM_LAUNCH(ctx, k_reg_iter, blocks, REG_BLOCK, source->d_centroid, &source->d_st->vox.n_voxels, target->d_sorted, target->d_tab,
+              target->d_ucell_start, target->d_runs, target->d_cell_nruns, target->d_valid_map, target->d_cloud_c, target->d_normals_c,
+              target->grid, target->d_st, search, rp, source->d_reg_state, source->d_reg_part, source->d_reg_ticket, source->d_reg_idx,
+              source->d_reg_res);
+  GM_CHECK_LAUNCHES(ctx);
+  if (target != source) {
+    GM_CUDA(cudaEventRecord(source->ev_reg[1], source->stream));
+    GM_CUDA(cudaStreamWaitEvent(target->stream, source->ev_reg[1], 0));
+  }
+  mark(source, REGISTRATION);
+  return GM_OK;
+}
+
+gm_status gm_get_registration(gm_ctx* ctx, gm_registration* out) {
+  if (!ctx || !out) return GM_ERR_INVALID_ARG;
+  if (gm_status s = require(ctx, REGISTRATION)) return s;
+  RegState h;
+  GM_CUDA(cudaMemcpyAsync(&h, ctx->d_reg_state, sizeof(RegState), cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  std::memset(out, 0, sizeof(*out));
+  for (int k = 0; k < 12; ++k) out->pose34[k] = (float)h.T[k];
+  out->iterations = h.iterations;
+  out->converged = h.converged;
+  out->n_source = h.n_source;
+  out->n_correspondences = h.n_corr;
+  out->rmse = h.n_corr > 0 ? (float)std::sqrt(h.sum_r2 / (double)h.n_corr) : 0.0f;
+  out->fitness = h.n_source > 0 ? (float)((double)h.n_corr / (double)h.n_source) : 0.0f;
+  out->n_degenerate = h.n_degenerate;
+  std::memcpy(out->eigenvalues, h.eig, sizeof(h.eig));
+  std::memcpy(out->eigenvectors, h.vecs, sizeof(h.vecs));
+  return GM_OK;
+}
+
+gm_status gm_download_correspondences(gm_ctx* ctx, int32_t* target_index, float* residual, size_t capacity_points) {
+  if (!ctx || !target_index) return GM_ERR_INVALID_ARG;
+  if (gm_status s = require(ctx, REGISTRATION)) return s;
+  int V = 0;
+  GM_CUDA(cudaMemcpyAsync(&V, &ctx->d_reg_state->n_source, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  if ((size_t)V > capacity_points) return GM_ERR_CAPACITY;
+  if (V > 0) {
+    GM_CUDA(cudaMemcpyAsync(target_index, ctx->d_reg_idx, (size_t)V * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    if (residual) GM_CUDA(cudaMemcpyAsync(residual, ctx->d_reg_res, (size_t)V * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  }
+  return GM_OK;
 }
 
 // ---- results ---------------------------------------------------------------------------------

@@ -120,6 +120,60 @@ def rectangular_drift(n: int = 100_000, seed: int = 6, width: float = 4.0, heigh
     return _xyzw(x, y, z)
 
 
+def drift_end_niche(n: int = 1_000_000, seed: int = 8, width: float = 4.0, height: float = 3.0, length: float = 8.0,
+                    niche=(0.5, 1.5, -0.5, 0.5, 0.6), noise: float = 0.005) -> np.ndarray:
+    """A scene whose scans constrain all six rigid degrees of freedom, for registration: the rectangular drift of
+    `rectangular_drift` (x in [-length/2, length/2]) closed by an end face x = +length/2, with a rectangular niche
+    (x0, x1, z0, z1, depth) cut into the wall y = +width/2.  Surfaces are sampled in proportion to their area, Gaussian
+    noise along their normals.  Floor, roof and walls fix y, z, roll, pitch and yaw; the end face fixes x."""
+    g = _rng(seed)
+    L, hw, hh = float(length), 0.5 * width, 0.5 * height
+    x0, x1, z0, z1, dep = (float(v) for v in niche)
+    xe = 0.5 * L
+    # surfaces: floor, roof, wall -y, wall +y (its opening is the niche's back wall, same footprint), end face, the
+    # niche's two x-sides and its two z-sides
+    areas = np.array([L * width, L * width, L * height, L * height, width * height, 2 * dep * (z1 - z0), 2 * dep * (x1 - x0)])
+    side = g.choice(len(areas), size=n, p=areas / areas.sum())
+    a, b, c = g.uniform(0.0, 1.0, n), g.uniform(0.0, 1.0, n), g.uniform(0.0, 1.0, n)
+    e = g.normal(0.0, noise, n) if noise > 0 else np.zeros(n)
+    # every surface takes its two in-surface coordinates from two different uniforms (a and b, or b and c)
+    x, y, z = -0.5 * L + a * L, -hw + b * width, -hh + b * height
+    wall_y = np.where((x >= x0) & (x < x1) & (z >= z0) & (z < z1), hw + dep, hw)
+    ny = hw + a * dep
+    cand = [np.stack([x, y, -hh + e], 1), np.stack([x, y, hh + e], 1), np.stack([x, -hw + e, z], 1),
+            np.stack([x, wall_y + e, z], 1), np.stack([xe + e, -hw + a * width, z], 1),
+            np.stack([np.where(c < 0.5, x0, x1) + e, ny, z0 + b * (z1 - z0)], 1),
+            np.stack([x0 + b * (x1 - x0), ny, np.where(c < 0.5, z0, z1) + e], 1)]
+    out = np.empty((n, 3))
+    for k, v in enumerate(cand):
+        out[side == k] = v[side == k]
+    return _xyzw(out[:, 0], out[:, 1], out[:, 2])
+
+
+def pose34(rotvec=(0.0, 0.0, 0.0), t=(0.0, 0.0, 0.0)) -> np.ndarray:
+    """3x4 float64 [R|t] with R = exp([rotvec]x) (Rodrigues)."""
+    w = np.asarray(rotvec, np.float64)
+    th = float(np.linalg.norm(w))
+    K = np.array([[0.0, -w[2], w[1]], [w[2], 0.0, -w[0]], [-w[1], w[0], 0.0]])
+    R = np.eye(3) if th == 0.0 else np.eye(3) + np.sin(th) / th * K + (1.0 - np.cos(th)) / th ** 2 * (K @ K)
+    return np.concatenate([R, np.asarray(t, np.float64).reshape(3, 1)], axis=1)
+
+
+def view_from(points: np.ndarray, sensor_pose34) -> np.ndarray:
+    """The scene points `points` (world frame) as a sensor placed at `sensor_pose34` (sensor -> world, 3x4) sees them:
+    p_sensor = R^T (p - t).  Registering such a scan (source) against one taken at the origin (target) recovers
+    sensor_pose34."""
+    T = np.asarray(sensor_pose34, np.float64)
+    p = np.asarray(points, np.float64)[:, :3]
+    q = (p - T[:, 3]) @ T[:, :3]
+    return _xyzw(q[:, 0], q[:, 1], q[:, 2])
+
+
+def second_scan(generator, sensor_pose34, seed: int, n: int, **kw) -> np.ndarray:
+    """Another scan of the scene of `generator` (new sample draw: `seed`) seen from the sensor pose `sensor_pose34`."""
+    return view_from(generator(n, seed=seed, **kw), sensor_pose34)
+
+
 def sample_draws(K: int, H: int, per: int, seed: int = 7) -> np.ndarray:
     """K x H x per uint32 draws for gm_extract_primitives, Philox(seed): round r maps draw u to the sample index
     R_r[(u * n_r) >> 32] of the points still unclaimed."""

@@ -330,6 +330,63 @@ GM_API gm_status gm_compress_primitives(gm_ctx* ctx);
  * n_residual_voxels x {x,y,z} float.  Pass buf = NULL to query the size. */
 GM_API gm_status gm_download_compressed_primitives(gm_ctx* ctx, void* buf, size_t capacity, size_t* bytes);
 
+/* ---- scan-to-scan registration (builder-defined: the reference computes no pose) -----------------------------------
+ * Point-to-plane ICP of the SOURCE context's VoxelGrid centroids (V points, after gm_voxel; under the VoxelGrid overflow
+ * rule its cloud as it is) against the TARGET context's compacted cloud and normals (after gm_normals, which builds the
+ * neighbour grid the search walks: an injected compacted cloud has none and gives GM_ERR_STAGE_ORDER).  target == source
+ * is allowed; both must be on the same device.  The pose T_i is held in double on the device, T_0 = init_pose34.
+ * Iteration i (0-based):
+ *   1. Tf = float(T_i) element-wise; every centroid c is transformed as p = Tf c with the fmaf chains of gm_map_insert.
+ *   2. Correspondence: the compacted target point q nearest to p (FLANN ((dx^2)+dy^2)+dz^2 in float, ties -> lowest
+ *      compacted index), accepted iff d^2 < float(d_max * d_max) (product in double, as the radius search takes it).
+ *      This is the exact nearest point, not an approximation.
+ *   3. With the compacted normal n of q, in double: r = n.(p - q), J = [p x n, n] (derivative with respect to a
+ *      left-applied twist (w, v)).
+ *   4. A = sum J J^T, g = sum J r, sum r^2 and the count m over the accepted points, in fixed-order double partials:
+ *      bitwise reproducible run to run.
+ *   5. A = V L V^T by cyclic Jacobi in double (eigenvalues ascending, each eigenvector's largest-|component| positive);
+ *      xi = -sum over k with lambda_k > degeneracy_ratio * lambda_max of (v_k.g / lambda_k) v_k; the other directions
+ *      are not updated (n_degenerate of them): they stay at the initial guess.  Then T_{i+1} = [R(w) | v] o T_i, i.e.
+ *      R <- R(w) R, t <- R(w) t + v, R(w) by Rodrigues in double.
+ *   6. Stop after the update with converged = 1 when |w| < min_rotation_step and |v| < min_translation_step; stop
+ *      without an update (converged = 0) when m < 6 or lambda_max <= 0.  Later iterations are no-ops.
+ * The launch sequence depends only on max_iterations: gm_launch_count(source) grows by max_iterations + 1, and there is
+ * no host synchronisation between iterations.  The reported pose is the pose after the last update; correspondences,
+ * residuals, rmse, fitness, the spectrum and n_degenerate belong to the last executed iteration, evaluated at its input
+ * pose.  V = 0 gives n_correspondences = 0, converged = 0 and the initial pose.
+ * The work runs on the source stream after the target stream's pending work, and the target stream waits for it before
+ * any later work (a new scan on the target cannot overwrite the grid under the search).  The results live in the source
+ * context until a new scan or neighbour grid there; they have buffers of their own (allocated by the first call). */
+#define GM_MAX_ICP_ITERATIONS 64
+typedef struct gm_icp_params {
+  float init_pose34[12];               /* source -> target guess, row-major [R|t] (the layout gm_map_insert takes)        */
+  double max_correspondence_distance;  /* d_max, metres, > 0                                         default 0.5          */
+  int32_t max_iterations;              /* 1 .. GM_MAX_ICP_ITERATIONS                                 default 30           */
+  int32_t pad_;
+  double min_rotation_step;            /* rad: converged when |w| < this ...                         default 1e-5         */
+  double min_translation_step;         /* m:   ... and |v| < this                                    default 1e-5         */
+  double degeneracy_ratio;             /* [0, 1): directions with lambda_k <= ratio * lambda_max are not updated; default 0
+                                          (only lambda_k <= 0 is dropped: plain Gauss-Newton)                             */
+} gm_icp_params;
+typedef struct gm_registration {
+  float pose34[12];          /* refined source -> target                                                     */
+  int32_t iterations;        /* iterations executed (including one that stopped without an update)           */
+  int32_t converged;         /* 1 = stopped on the step thresholds                                           */
+  int32_t n_source;          /* source points (the source's voxel centroids, V)                              */
+  int32_t n_correspondences; /* of the last executed iteration                                               */
+  float rmse;                /* sqrt(sum r^2 / n_correspondences) over those (0 without correspondences)     */
+  float fitness;             /* n_correspondences / n_source (0 when V = 0)                                  */
+  int32_t n_degenerate;      /* eigen-directions not updated in the last executed iteration                  */
+  int32_t pad_;
+  double eigenvalues[6];     /* of that iteration's J^T J, ascending                                         */
+  double eigenvectors[36];   /* row-major, column k = eigenvector k, parameters (wx, wy, wz, vx, vy, vz)     */
+} gm_registration;
+GM_API void gm_icp_params_default(gm_icp_params* p);  /* identity guess and the defaults above */
+GM_API gm_status gm_register(gm_ctx* source, gm_ctx* target, const gm_icp_params* p);
+GM_API gm_status gm_get_registration(gm_ctx* source, gm_registration* out);  /* synchronises the source stream */
+/* V entries of the last executed iteration: compacted target index or -1, float(r) or NaN; residual may be NULL */
+GM_API gm_status gm_download_correspondences(gm_ctx* source, int32_t* target_index, float* residual, size_t capacity_points);
+
 /* Fused per-scan path = the body of cloud_cb (src/geometric_mapping.cpp:48-125) plus the
  * builder-defined segmentation: crop -> normals -> voxel -> local frame -> RANSAC plane(Hp)
  * + cylinder(Hc) -> select/refit -> labels -> polyline.  samples may be NULL when H == 0. */
