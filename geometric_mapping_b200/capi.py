@@ -158,7 +158,7 @@ SYMBOLS = [
     "gm_comm_create", "gm_comm_handle", "gm_comm_connect", "gm_comm_mailbox", "gm_comm_connect_local", "gm_comm_destroy", "gm_comm_rank", "gm_comm_world", "gm_comm_last_error", "gm_set_comm", "gm_ransac_sharded", "gm_allreduce_voxel_bbox", "gm_allreduce_frame", "gm_set_voxel_bbox_hint", "gm_set_knn", "gm_download_knn_indices", "gm_set_knn_max_radius", "gm_pointcloud2_size", "gm_encode_pointcloud2", "gm_marker_array_size",
     "gm_extract_primitives", "gm_get_primitives", "gm_download_primitive_ids", "gm_compress_primitives",
     "gm_download_compressed_primitives", "gm_icp_params_default", "gm_register", "gm_get_registration",
-    "gm_download_correspondences",
+    "gm_download_correspondences", "gm_register_map", "gm_download_map_correspondences", "gm_map_download_planes",
     "gm_encode_marker_array", "gm_store_open", "gm_store_close", "gm_store_append", "gm_store_append_blob", "gm_store_count", "gm_store_info", "gm_store_read",
 ]
 
@@ -289,6 +289,9 @@ def _lib():
         "gm_register": (i32, [vp, vp, C.POINTER(gm_icp_params)]),
         "gm_get_registration": (i32, [vp, C.POINTER(gm_registration)]),
         "gm_download_correspondences": (i32, [vp, vp, vp, sz]),
+        "gm_register_map": (i32, [vp, vp, C.POINTER(gm_icp_params), C.c_double]),
+        "gm_download_map_correspondences": (i32, [vp, vp, vp, sz]),
+        "gm_map_download_planes": (i32, [vp, C.c_double, vp, sz, C.POINTER(sz)]),
     }
     assert set(sig) == set(SYMBOLS)
     for name, (res, args) in sig.items():
@@ -806,7 +809,33 @@ def _ctx_download_correspondences(self):
     return idx, res
 
 
+def _ctx_register_map_async(self, vmap: "VoxelMap", init_pose34=None, max_planarity: float = 0.1, **params):
+    """Enqueue gm_register_map(self = source, vmap) without waiting; read the result with registration()."""
+    p = icp_params(init_pose34, **params)
+    self._ck(_lib().gm_register_map(self._h, vmap._h, C.byref(p), C.c_double(max_planarity)), "gm_register_map")
+
+
+def _ctx_register_map(self, vmap: "VoxelMap", init_pose34=None, max_planarity: float = 0.1, **params) -> dict:
+    """Point-to-plane ICP of this context's voxel centroids (after voxel()) against the planes of the voxel map `vmap`
+    (include/gm_capi.h, gm_register_map): init_pose34 and the result's pose are source -> map frame.  Keywords: the
+    fields of gm_icp_params.  -> the dict of register()."""
+    _ctx_register_map_async(self, vmap, init_pose34, max_planarity, **params)
+    return _ctx_registration(self)
+
+
+def _ctx_download_map_correspondences(self):
+    """-> (ijk int32 V x 3: the matched map voxel's cell or INT32_MIN x 3, residual float32 V: float(r) or NaN) of the
+    last executed iteration of the last register_map()."""
+    V = _ctx_registration(self)["n_source"]
+    ijk, res = np.empty((max(V, 0), 3), np.int32), np.empty(max(V, 0), np.float32)
+    self._ck(_lib().gm_download_map_correspondences(self._h, _ptr(ijk), _ptr(res), ijk.shape[0]), "gm_download_map_correspondences")
+    return ijk, res
+
+
 Context.register = _ctx_register
+Context.register_map = _ctx_register_map
+Context.register_map_async = _ctx_register_map_async
+Context.download_map_correspondences = _ctx_download_map_correspondences
 Context.register_async = _ctx_register_async
 Context.registration = _ctx_registration
 Context.download_correspondences = _ctx_download_correspondences
@@ -885,6 +914,15 @@ class VoxelMap:
         ijk, cnt, cen = np.empty((V, 3), np.int32), np.empty(V, np.int32), np.empty((V, 4), np.float32)
         self._ck(_lib().gm_map_download(self._h, _ptr(ijk), _ptr(cnt), _ptr(cen), V, C.byref(n)), "gm_map_download", ok=(GM_OK, GM_ERR_CAPACITY))
         return {"ijk": ijk, "counts": cnt, "centroids": cen}
+
+    def planes(self, max_planarity: float = 0.1) -> np.ndarray:
+        """V x 4 float32 in download() order: {normal, 1} of each voxel with a plane, {NaN, NaN, NaN, 0} without."""
+        n = C.c_size_t(0)
+        self._ck(_lib().gm_map_download_planes(self._h, C.c_double(max_planarity), None, 0, C.byref(n)), "gm_map_download_planes")
+        out = np.empty((int(n.value), 4), np.float32)
+        self._ck(_lib().gm_map_download_planes(self._h, C.c_double(max_planarity), _ptr(out), out.shape[0], C.byref(n)),
+                 "gm_map_download_planes")
+        return out
 
     def clear(self):
         self._ck(_lib().gm_map_clear(self._h), "gm_map_clear")

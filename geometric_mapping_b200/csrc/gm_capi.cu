@@ -233,6 +233,10 @@ struct gm_ctx {
   DevBuf<int> d_reg_idx;
   DevBuf<float> d_reg_res;
   cudaEvent_t ev_reg[2] = {nullptr, nullptr};  // target stream -> source stream, and back
+  // gm_register_map: the matched map key per centroid (allocated by the first call), and which kind of target the last
+  // registration had (0 = a context, whose correspondences are in d_reg_idx; 1 = a map, in d_reg_key)
+  DevBuf<unsigned long long> d_reg_key;
+  int reg_target = 0;
   // profiling
   bool profiling = false;
   std::vector<cudaEvent_t> ev_pool;
@@ -1745,6 +1749,7 @@ gm_status gm_register(gm_ctx* source, gm_ctx* target, const gm_icp_params* p) {
     GM_CUDA(cudaEventRecord(source->ev_reg[1], source->stream));
     GM_CUDA(cudaStreamWaitEvent(target->stream, source->ev_reg[1], 0));
   }
+  source->reg_target = 0;
   mark(source, REGISTRATION);
   return GM_OK;
 }
@@ -1772,6 +1777,7 @@ gm_status gm_get_registration(gm_ctx* ctx, gm_registration* out) {
 gm_status gm_download_correspondences(gm_ctx* ctx, int32_t* target_index, float* residual, size_t capacity_points) {
   if (!ctx || !target_index) return GM_ERR_INVALID_ARG;
   if (gm_status s = require(ctx, REGISTRATION)) return s;
+  if (ctx->reg_target != 0) return GM_ERR_STAGE_ORDER;  // a map registration: gm_download_map_correspondences
   int V = 0;
   GM_CUDA(cudaMemcpyAsync(&V, &ctx->d_reg_state->n_source, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
   GM_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -2465,7 +2471,14 @@ struct gm_map {
   DevBuf<MapState> d_st;
   DevBuf<int> d_cursor;
   int num_sms = 148;
+  int device = 0;
+  // the last map operation issued on a context stream (gm_map_insert, gm_register_map): the next one waits for it
+  cudaEvent_t ev_last = nullptr;
+  // per-slot plane tables of k_map_planes (allocated by the first use): centroid + has-plane flag, normal
+  DevBuf<float4> d_plane_cent, d_plane_nrm;
+  DevBuf<int> d_plane_box;  // [8] cells of the voxels with a plane: min x, y, z, -, -max x, y, z, - (k_map_planes)
   std::string err;
+  ~gm_map() { if (ev_last) cudaEventDestroy(ev_last); }
 };
 
 namespace {
@@ -2525,9 +2538,10 @@ gm_status gm_map_create(double leaf, size_t capacity_voxels, gm_map** out) {
   while (slots < 2ull * capacity_voxels) slots <<= 1;  // load factor <= 0.5
   m->n_slots = slots;
   int dev = 0; cudaGetDevice(&dev);
+  m->device = dev;
   cudaDeviceProp prop;
   if (cudaGetDeviceProperties(&prop, dev) == cudaSuccess) m->num_sms = prop.multiProcessorCount;
-  if (m->d_keys.alloc(slots) != cudaSuccess || m->d_cnt.alloc(slots) != cudaSuccess || m->d_sums.alloc(3 * slots) != cudaSuccess ||
+  if (cudaEventCreateWithFlags(&m->ev_last, cudaEventDisableTiming) != cudaSuccess || m->d_keys.alloc(slots) != cudaSuccess || m->d_cnt.alloc(slots) != cudaSuccess || m->d_sums.alloc(3 * slots) != cudaSuccess ||
       m->d_st.alloc(1) != cudaSuccess || m->d_cursor.alloc(1) != cudaSuccess || map_clear_device(m) != GM_OK) {
     gm_map_destroy(m);
     return GM_ERR_CUDA;
@@ -2556,9 +2570,12 @@ gm_status gm_map_insert(gm_map* m, gm_ctx* ctx, const float* pose34, int32_t lab
   Pose34 T{};
   if (pose34) std::memcpy(T.r, pose34, sizeof(T.r));
   int blocks = std::min(div_up((long long)ctx->n_input, 256), ctx->num_sms * 16);
+  const bool ordered = ctx->device == m->device;  // map operations issued on streams of the map's device run in call order
+  if (ordered) GM_CUDA(cudaStreamWaitEvent(ctx->stream, m->ev_last, 0));
   GM_LAUNCH(ctx, k_map_insert, blocks, 256, ctx->d_cloud_c, ctx->d_labels, &ctx->d_st->n_valid, label_filter < 0 ? -1 : label_filter, T,
             pose34 ? 1 : 0, m->inv_leaf, m->d_keys, m->d_cnt, m->d_sums, m->n_slots - 1ull, m->d_st);
   GM_CHECK_LAUNCHES(ctx);
+  if (ordered) GM_CUDA(cudaEventRecord(m->ev_last, ctx->stream));
   return GM_OK;
 }
 
@@ -2656,6 +2673,119 @@ gm_status gm_map_load(const char* path, size_t min_capacity_voxels, gm_map** out
 }
 
 double gm_map_leaf(const gm_map* m) { return m ? m->leaf : 0.0; }
+
+}  // extern "C"
+
+// ---- scan-to-map registration (gm_register.cuh, k_map_planes in gm_map.cuh) ------------------------------------------
+namespace {
+inline bool valid_planarity(double r) { return r > 0.0 && r <= 1.0; }
+
+cudaError_t ensure_plane_tables(gm_map* m) {
+  if (m->d_plane_cent.count) return cudaSuccess;
+  cudaError_t e = m->d_plane_nrm.alloc(m->n_slots);
+  if (e == cudaSuccess) e = m->d_plane_box.alloc(8);
+  if (e == cudaSuccess) e = m->d_plane_cent.alloc(m->n_slots);  // last: a failure above leaves the pair unallocated
+  return e;
+}
+
+int map_blocks(const gm_map* m) { return (int)std::min<unsigned long long>((m->n_slots + 255) / 256, (unsigned long long)m->num_sms * 16); }
+}  // namespace
+
+extern "C" {
+
+gm_status gm_register_map(gm_ctx* source, gm_map* map, const gm_icp_params* p, double max_planarity) {
+  if (!source || !map || !p) return GM_ERR_INVALID_ARG;
+  gm_ctx* ctx = source;  // GM_CUDA / GM_LAUNCH report on the source
+  if (source->device != map->device) { ctx->err = "gm_register_map: source and map on different devices"; return GM_ERR_INVALID_ARG; }
+  const double dmax = p->max_correspondence_distance;
+  if (!(dmax > 0.0) || !std::isfinite(dmax) || p->max_iterations < 1 || p->max_iterations > GM_MAX_ICP_ITERATIONS ||
+      !(p->min_rotation_step >= 0.0) || !(p->min_translation_step >= 0.0) || !(p->degeneracy_ratio >= 0.0) ||
+      !(p->degeneracy_ratio < 1.0) || !finite_pose(p->init_pose34) || !valid_planarity(max_planarity))
+    return GM_ERR_INVALID_ARG;
+  if (gm_status s = require(source, VOXEL)) return s;
+  if (gm_status s = ensure_reg_buffers(source)) return s;
+  if (!source->d_reg_key.count) GM_CUDA(source->d_reg_key.alloc(source->cap));
+  GM_CUDA(ensure_plane_tables(map));
+  ctx->stages &= ~(1u << REGISTRATION);
+  GM_CUDA(cudaStreamWaitEvent(source->stream, map->ev_last, 0));
+  const unsigned long long mask = map->n_slots - 1ull;
+  GM_CUDA(cudaMemsetAsync(map->d_plane_box, 0x7F, 8 * sizeof(int), source->stream));
+  GM_LAUNCH(ctx, k_map_planes, map_blocks(map), 256, map->d_keys, map->d_cnt, map->d_sums, mask, max_planarity, map->d_plane_cent,
+            map->d_plane_nrm, map->d_plane_box);
+  Pose34 init;
+  std::memcpy(init.r, p->init_pose34, sizeof(init.r));
+  GM_LAUNCH(ctx, k_reg_begin, 1, 32, source->d_reg_state, init, &source->d_st->vox.n_voxels);
+  RegParams rp;
+  rp.d_max = dmax;
+  rp.r2max = (float)(dmax * dmax);
+  rp.min_rot = p->min_rotation_step;
+  rp.min_trans = p->min_translation_step;
+  rp.ratio = p->degeneracy_ratio;
+  const int blocks = std::max(1, std::min(div_up((long long)source->n_grid * 32, REG_BLOCK), reg_blocks(source)));
+  for (int it = 0; it < p->max_iterations; ++it)
+    GM_LAUNCH(ctx, k_regmap_iter, blocks, REG_BLOCK, source->d_centroid, &source->d_st->vox.n_voxels, map->d_keys, map->d_plane_cent,
+              map->d_plane_nrm, map->d_plane_box, mask, map->inv_leaf, map->leaf, rp, source->d_reg_state, source->d_reg_part, source->d_reg_ticket,
+              source->d_reg_key, source->d_reg_res);
+  GM_CHECK_LAUNCHES(ctx);
+  GM_CUDA(cudaEventRecord(map->ev_last, source->stream));
+  source->reg_target = 1;
+  mark(source, REGISTRATION);
+  return GM_OK;
+}
+
+gm_status gm_download_map_correspondences(gm_ctx* ctx, int32_t* ijk, float* residual, size_t capacity_points) {
+  if (!ctx || !ijk) return GM_ERR_INVALID_ARG;
+  if (gm_status s = require(ctx, REGISTRATION)) return s;
+  if (ctx->reg_target != 1) return GM_ERR_STAGE_ORDER;  // a context registration: gm_download_correspondences
+  int V = 0;
+  GM_CUDA(cudaMemcpyAsync(&V, &ctx->d_reg_state->n_source, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  if ((size_t)V > capacity_points) return GM_ERR_CAPACITY;
+  if (V > 0) {
+    std::vector<unsigned long long> keys((size_t)V);
+    GM_CUDA(cudaMemcpyAsync(keys.data(), ctx->d_reg_key, (size_t)V * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+    if (residual) GM_CUDA(cudaMemcpyAsync(residual, ctx->d_reg_res, (size_t)V * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    GM_CUDA(cudaStreamSynchronize(ctx->stream));
+    for (size_t i = 0; i < (size_t)V; ++i) {
+      int x = INT32_MIN, y = INT32_MIN, z = INT32_MIN;
+      if (keys[i] != MAP_EMPTY) map_unpack(keys[i], x, y, z);
+      ijk[3 * i] = x; ijk[3 * i + 1] = y; ijk[3 * i + 2] = z;
+    }
+  }
+  return GM_OK;
+}
+
+gm_status gm_map_download_planes(gm_map* m, double max_planarity, float* normals_xyzw, size_t capacity, size_t* n) {
+  if (!m || !n || !valid_planarity(max_planarity)) return GM_ERR_INVALID_ARG;
+  if (cudaDeviceSynchronize() != cudaSuccess) { m->err = "sync"; return GM_ERR_CUDA; }
+  MapState st;
+  if (cudaMemcpy(&st, m->d_st, sizeof(st), cudaMemcpyDeviceToHost) != cudaSuccess) { m->err = "memcpy"; return GM_ERR_CUDA; }
+  const size_t V = (size_t)std::max(st.n_voxels, 0);
+  *n = V;
+  if (!normals_xyzw) return st.overflow ? GM_ERR_CAPACITY : GM_OK;
+  if (capacity < V) return GM_ERR_CAPACITY;
+  if (!V) return st.overflow ? GM_ERR_CAPACITY : GM_OK;
+  DevBuf<unsigned long long> dk; DevBuf<float4> dn;
+  if (ensure_plane_tables(m) != cudaSuccess || dk.alloc(V) != cudaSuccess || dn.alloc(V) != cudaSuccess) { m->err = "cudaMalloc"; return GM_ERR_CUDA; }
+  cudaError_t e = cudaMemset(m->d_cursor, 0, sizeof(int));
+  if (e == cudaSuccess) e = cudaMemset(m->d_plane_box, 0x7F, 8 * sizeof(int));
+  if (e == cudaSuccess) {
+    k_map_planes<<<map_blocks(m), 256>>>(m->d_keys, m->d_cnt, m->d_sums, m->n_slots - 1ull, max_planarity, m->d_plane_cent, m->d_plane_nrm,
+                                         m->d_plane_box);
+    k_map_export_planes<<<map_blocks(m), 256>>>(m->d_keys, m->d_plane_nrm, m->n_slots, dk, dn, (int)V, m->d_cursor);
+    e = cudaGetLastError();
+  }
+  std::vector<unsigned long long> k(V);
+  std::vector<float4> nr(V);
+  if (e == cudaSuccess) e = cudaMemcpy(k.data(), dk, V * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
+  if (e == cudaSuccess) e = cudaMemcpy(nr.data(), dn, V * sizeof(float4), cudaMemcpyDeviceToHost);
+  if (e != cudaSuccess) { m->err = cudaGetErrorString(e); return GM_ERR_CUDA; }
+  std::vector<size_t> order(V);
+  for (size_t i = 0; i < V; ++i) order[i] = i;
+  std::sort(order.begin(), order.end(), [&](size_t a, size_t b) { return k[a] < k[b]; });  // gm_map_download's order
+  for (size_t i = 0; i < V; ++i) std::memcpy(normals_xyzw + 4 * i, &nr[order[i]], sizeof(float4));
+  return st.overflow ? GM_ERR_CAPACITY : GM_OK;  // as gm_map_download: an insert found the table full
+}
 
 }  // extern "C"
 

@@ -105,6 +105,108 @@ __global__ void k_map_restore(const unsigned long long* __restrict__ in_keys, co
   }
 }
 
+// Slot of `key`, or -1.  Keys are never removed, so the probe sequence of an absent key ends at an empty slot (or after
+// n_slots probes in a full table).
+__device__ __forceinline__ long long d_map_find(const unsigned long long* __restrict__ keys, unsigned long long key,
+                                                unsigned long long slot_mask) {
+  unsigned long long slot = map_hash(key) & slot_mask;
+  for (unsigned long long probe = 0; probe <= slot_mask; ++probe) {
+    const unsigned long long k = keys[slot];
+    if (k == key) return (long long)slot;
+    if (k == MAP_EMPTY) return -1;
+    slot = (slot + 1) & slot_mask;
+  }
+  return -1;
+}
+
+constexpr int MAP_PLANE_MIN_VOXELS = 5;  // GM_MAP_PLANE_MIN_VOXELS
+
+// centroid of an occupied slot exactly as gm_map_download reports it: float(sum / 2^20 / count) in double
+__device__ __forceinline__ void d_map_centroid(const int* __restrict__ cnt, const long long* __restrict__ sums, long long s, float c[3]) {
+  const double n = (double)cnt[s];
+#pragma unroll
+  for (int a = 0; a < 3; ++a) c[a] = (float)((double)sums[3 * s + a] / 1048576.0 / n);
+}
+
+// Plane of every occupied voxel v (include/gm_capi.h, gm_register_map): the centroids of the occupied voxels among the
+// 27 around v, v included, in ascending (dz, dy, dx) order; their sequential double mean and covariance; d_jacobi3.
+// One thread per slot.  cent[s] = {centroid, 1 if v has a plane else 0}, nrm[s] = {normal, 1} or {NaN x3, 0}; empty slots
+// are not written (the search only reads slots d_map_find returns).  box = the cells of the voxels with a plane, as
+// atomicMin of {min x, y, z, -, -max x, y, z, -}: the caller sets its 8 ints to 0x7F7F7F7F (larger than any cell) first.
+__global__ void k_map_planes(const unsigned long long* __restrict__ keys, const int* __restrict__ cnt, const long long* __restrict__ sums,
+                             unsigned long long slot_mask, double max_planarity, float4* __restrict__ cent, float4* __restrict__ nrm,
+                             int* __restrict__ box) {
+  int bmin[3] = {INT_MAX, INT_MAX, INT_MAX}, bneg[3] = {INT_MAX, INT_MAX, INT_MAX};
+  for (unsigned long long s = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; s <= slot_mask;
+       s += (unsigned long long)gridDim.x * blockDim.x) {
+    const unsigned long long key = keys[s];
+    if (key == MAP_EMPTY) continue;
+    int ix, iy, iz;
+    map_unpack(key, ix, iy, iz);
+    float nb[27][3];
+    int m = 0;
+#pragma unroll 1
+    for (int o = 0; o < 27; ++o) {
+      unsigned long long k2;
+      if (!map_pack(ix + o % 3 - 1, iy + (o / 3) % 3 - 1, iz + o / 9 - 1, k2)) continue;
+      const long long s2 = (k2 == key) ? (long long)s : d_map_find(keys, k2, slot_mask);
+      if (s2 < 0) continue;
+      d_map_centroid(cnt, sums, s2, nb[m]);
+      ++m;
+    }
+    float self[3];
+    d_map_centroid(cnt, sums, (long long)s, self);
+    float4 n4 = make_float4(CUDART_NAN_F, CUDART_NAN_F, CUDART_NAN_F, 0.f);
+    if (m >= MAP_PLANE_MIN_VOXELS) {
+      double mu[3] = {0.0, 0.0, 0.0};
+#pragma unroll 1
+      for (int i = 0; i < m; ++i)
+        for (int a = 0; a < 3; ++a) mu[a] += (double)nb[i][a];
+      for (int a = 0; a < 3; ++a) mu[a] /= (double)m;
+      double c6[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};  // xx xy xz yy yz zz
+#pragma unroll 1
+      for (int i = 0; i < m; ++i) {
+        const double dx = (double)nb[i][0] - mu[0], dy = (double)nb[i][1] - mu[1], dz = (double)nb[i][2] - mu[2];
+        c6[0] += dx * dx; c6[1] += dx * dy; c6[2] += dx * dz;
+        c6[3] += dy * dy; c6[4] += dy * dz; c6[5] += dz * dz;
+      }
+      for (int k = 0; k < 6; ++k) c6[k] /= (double)m;
+      const double C[9] = {c6[0], c6[1], c6[2], c6[1], c6[3], c6[4], c6[2], c6[4], c6[5]};
+      double vals[3], vecs[9];
+      d_jacobi3(C, vals, vecs);
+      if (vals[0] <= max_planarity * vals[1] && vals[1] > 0.0) n4 = make_float4((float)vecs[0], (float)vecs[3], (float)vecs[6], 1.f);
+    }
+    cent[s] = make_float4(self[0], self[1], self[2], n4.w);
+    nrm[s] = n4;
+    if (n4.w != 0.f) {
+      bmin[0] = min(bmin[0], ix); bmin[1] = min(bmin[1], iy); bmin[2] = min(bmin[2], iz);
+      bneg[0] = min(bneg[0], -ix); bneg[1] = min(bneg[1], -iy); bneg[2] = min(bneg[2], -iz);
+    }
+  }
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    bmin[a] = __reduce_min_sync(0xFFFFFFFFu, bmin[a]);
+    bneg[a] = __reduce_min_sync(0xFFFFFFFFu, bneg[a]);
+  }
+  if ((threadIdx.x & 31) == 0 && bmin[0] != INT_MAX) {
+#pragma unroll
+    for (int a = 0; a < 3; ++a) { atomicMin(box + a, bmin[a]); atomicMin(box + 4 + a, bneg[a]); }
+  }
+}
+
+// Gather the occupied slots' keys and plane normals (order = slot order; the host sorts by key), as k_map_export.
+__global__ void k_map_export_planes(const unsigned long long* __restrict__ keys, const float4* __restrict__ nrm, unsigned long long n_slots,
+                                    unsigned long long* __restrict__ out_keys, float4* __restrict__ out_nrm, int capacity, int* cursor) {
+  for (unsigned long long s = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; s < n_slots; s += (unsigned long long)gridDim.x * blockDim.x) {
+    const unsigned long long k = keys[s];
+    if (k == MAP_EMPTY) continue;
+    const int o = atomicAdd(cursor, 1);
+    if (o >= capacity) continue;
+    out_keys[o] = k;
+    out_nrm[o] = nrm[s];
+  }
+}
+
 // Gather the occupied slots into dense arrays (order = slot order; the host sorts by key).
 __global__ void k_map_export(const unsigned long long* __restrict__ keys, const int* __restrict__ cnt, const long long* __restrict__ sums,
                              unsigned long long n_slots, unsigned long long* __restrict__ out_keys, int* __restrict__ out_cnt,

@@ -3,7 +3,9 @@
 // VoxelGrid centroids against a target context's compacted cloud and normals, the correspondences searched over the
 // target's neighbour grid.  One launch per iteration and no host synchronisation between them: the pose lives on the
 // device in double, and the last block of every iteration reduces, solves, updates it and decides whether to stop.
-// Semantics: include/gm_capi.h (gm_register).
+// Scan-to-map registration (k_regmap_iter) shares all of it but the search: the nearest plane of the aggregated voxel map
+// (k_map_planes, gm_map.cuh) through the map's hash table.
+// Semantics: include/gm_capi.h (gm_register, gm_register_map).
 #pragma once
 #include "gm_stages.cuh"
 #include "gm_map.cuh"
@@ -215,12 +217,58 @@ __device__ __forceinline__ void d_reg_solve(const double* fin, const RegParams& 
   if (wn < prm.min_rot && vn < prm.min_trans) { st->converged = 1; st->done = 1; }
 }
 
+// p = float(T)·c as the fmaf chains of k_map_insert
+__device__ __forceinline__ float4 d_reg_transform(const float Tf[12], const float4 c) {
+  float4 p;
+  p.x = fmaf(Tf[0], c.x, fmaf(Tf[1], c.y, fmaf(Tf[2], c.z, Tf[3])));
+  p.y = fmaf(Tf[4], c.x, fmaf(Tf[5], c.y, fmaf(Tf[6], c.z, Tf[7])));
+  p.z = fmaf(Tf[8], c.x, fmaf(Tf[9], c.y, fmaf(Tf[10], c.z, Tf[11])));
+  p.w = 1.0f;
+  return p;
+}
+
+// One accepted correspondence (lane 0 of its warp): r = n·(p - q) and J = [p x n, n] in double (unfused: -fmad=false),
+// added to the warp's slot s of REG_NV sums.  -> float(r)
+__device__ __forceinline__ float d_reg_accumulate(double* s, const float4 p, const float4 q, const float4 n) {
+  const double px = p.x, py = p.y, pz = p.z, nx = n.x, ny = n.y, nz = n.z;
+  const double dx = px - (double)q.x, dy = py - (double)q.y, dz = pz - (double)q.z;
+  const double r = (nx * dx + ny * dy) + nz * dz;
+  const double J[6] = {py * nz - pz * ny, pz * nx - px * nz, px * ny - py * nx, nx, ny, nz};
+#pragma unroll
+  for (int a = 0, k = 0; a < 6; ++a)
+#pragma unroll
+    for (int b = a; b < 6; ++b, ++k) s[k] += J[a] * J[b];
+#pragma unroll
+  for (int a = 0; a < 6; ++a) s[21 + a] += J[a] * r;
+  s[27] += r * r;
+  s[28] += 1.0;
+  return (float)r;
+}
+
+// End of an iteration, every thread of the block: the block total is the warp slots in warp order, the last block
+// reduces the block partials in block order, solves and updates (the k_frame pattern): bitwise reproducible.
+template <int W>
+__device__ __forceinline__ void d_reg_finish(double (*wsum)[REG_NV], double* fin, const RegParams& prm, RegState* st,
+                                             double* __restrict__ partials, unsigned* ticket) {
+  __syncthreads();
+  if (threadIdx.x < REG_NV) {
+    double t = 0.0;
+#pragma unroll
+    for (int w = 0; w < W; ++w) t += wsum[w][threadIdx.x];
+    partials[(size_t)blockIdx.x * REG_NV + threadIdx.x] = t;
+    __threadfence();
+  }
+  if (!d_last_block(ticket, gridDim.x)) return;
+  d_reduce_partials<REG_NV>(partials, gridDim.x, fin);
+  if (threadIdx.x != 0) return;
+  d_reg_solve(fin, prm, st);
+}
+
 // One ICP iteration.  Warp per source point: p = float(T)·c as the fmaf chains of k_map_insert, exact nearest compacted
 // target point q within d_max, r = n·(p - q) and J = [p x n, n] in double (unfused: -fmad=false).  Lane 0 of each warp
 // adds its points to the warp's slot in shared memory (in registers the 29 sums would stay live across the search and
-// spill), the block total is the warp slots in warp order, and the last block reduces the block partials in block
-// order, solves and updates (the k_frame pattern): bitwise reproducible.  Launched with REG_BLOCK threads; the register
-// budget is explicit because ptxas' own choice (72) spills around the search (96: no spills, 5 blocks per SM).
+// spill), then d_reg_finish.  Launched with REG_BLOCK threads; the register budget is explicit because ptxas' own
+// choice (72) spills around the search (96: no spills, 5 blocks per SM).
 __global__ void __maxnreg__(96)
 k_reg_iter(const float4* __restrict__ src, const int* __restrict__ n_src_ptr, const float4* __restrict__ sp,
            const BlockEntry* __restrict__ tab, const int* __restrict__ ucell_start, const int2* __restrict__ runs,
@@ -242,12 +290,7 @@ k_reg_iter(const float4* __restrict__ src, const int* __restrict__ n_src_ptr, co
   for (int k = lane; k < REG_NV; k += 32) s[k] = 0.0;
   __syncwarp();
   for (int j = (blockIdx.x * REG_BLOCK + threadIdx.x) >> 5; j < V; j += warps_total) {
-    const float4 c = src[j];
-    float4 p;
-    p.x = fmaf(Tf[0], c.x, fmaf(Tf[1], c.y, fmaf(Tf[2], c.z, Tf[3])));
-    p.y = fmaf(Tf[4], c.x, fmaf(Tf[5], c.y, fmaf(Tf[6], c.z, Tf[7])));
-    p.z = fmaf(Tf[8], c.x, fmaf(Tf[9], c.y, fmaf(Tf[10], c.z, Tf[11])));
-    p.w = 1.0f;
+    const float4 p = d_reg_transform(Tf, src[j]);
     float best = CUDART_INF_F;
     int bi = 0x7FFFFFFF;
     if (search && finite3(p.x, p.y, p.z)) d_reg_nn(p, sp, tab, ucell_start, runs, cell_info, valid_map, g, U, nf, prm.d_max, best, bi);
@@ -255,38 +298,141 @@ k_reg_iter(const float4* __restrict__ src, const int* __restrict__ n_src_ptr, co
       int id = -1;
       float rf = CUDART_NAN_F;
       if (bi != 0x7FFFFFFF && best < prm.r2max) {
-        const float4 q = cloud_c[bi], n = normals_c[2 * (size_t)bi];
-        const double px = p.x, py = p.y, pz = p.z, nx = n.x, ny = n.y, nz = n.z;
-        const double dx = px - (double)q.x, dy = py - (double)q.y, dz = pz - (double)q.z;
-        const double r = (nx * dx + ny * dy) + nz * dz;
-        const double J[6] = {py * nz - pz * ny, pz * nx - px * nz, px * ny - py * nx, nx, ny, nz};
-#pragma unroll
-        for (int a = 0, k = 0; a < 6; ++a)
-#pragma unroll
-          for (int b = a; b < 6; ++b, ++k) s[k] += J[a] * J[b];
-#pragma unroll
-        for (int a = 0; a < 6; ++a) s[21 + a] += J[a] * r;
-        s[27] += r * r;
-        s[28] += 1.0;
+        rf = d_reg_accumulate(s, p, cloud_c[bi], normals_c[2 * (size_t)bi]);
         id = bi;
-        rf = (float)r;
       }
       corr[j] = id;
       resid[j] = rf;
     }
   }
-  __syncthreads();
-  if (threadIdx.x < REG_NV) {
-    double t = 0.0;
-#pragma unroll
-    for (int w = 0; w < W; ++w) t += wsum[w][threadIdx.x];
-    partials[(size_t)blockIdx.x * REG_NV + threadIdx.x] = t;
-    __threadfence();
+  d_reg_finish<W>(wsum, fin, prm, st, partials, ticket);
+}
+
+// ---- scan-to-map registration (gm_register_map) ----------------------------------------------------------------------
+// Face f of cube shell k around (cx, cy, cz), clipped to the plane box [lo, hi] (inclusive cells): f 0/1 = the z faces,
+// 2/3 the y faces without their z edges, 4/5 the x faces without their y and z edges, 6 the centre (shell 1 only).
+// The faces partition the shell.  -> number of cells (0 when the clipped face is empty).
+struct MapFace { int x0, x1, y0, y1, z0, z1; };
+__device__ __forceinline__ long long d_shell_face(int f, int k, int cx, int cy, int cz, const int* lo, const int* hi, MapFace& r) {
+  switch (f) {
+    case 0: case 1: r.x0 = cx - k; r.x1 = cx + k; r.y0 = cy - k; r.y1 = cy + k; r.z0 = r.z1 = cz + (f == 0 ? -k : k); break;
+    case 2: case 3: r.x0 = cx - k; r.x1 = cx + k; r.y0 = r.y1 = cy + (f == 2 ? -k : k); r.z0 = cz - k + 1; r.z1 = cz + k - 1; break;
+    case 4: case 5: r.x0 = r.x1 = cx + (f == 4 ? -k : k); r.y0 = cy - k + 1; r.y1 = cy + k - 1; r.z0 = cz - k + 1; r.z1 = cz + k - 1; break;
+    default: r.x0 = r.x1 = cx; r.y0 = r.y1 = cy; r.z0 = r.z1 = cz; if (k != 1) r.x1 = r.x0 - 1; break;
   }
-  if (!d_last_block(ticket, gridDim.x)) return;
-  d_reduce_partials<REG_NV>(partials, gridDim.x, fin);
-  if (threadIdx.x != 0) return;
-  d_reg_solve(fin, prm, st);
+  r.x0 = max(r.x0, lo[0]); r.x1 = min(r.x1, hi[0]);
+  r.y0 = max(r.y0, lo[1]); r.y1 = min(r.y1, hi[1]);
+  r.z0 = max(r.z0, lo[2]); r.z1 = min(r.z1, hi[2]);
+  if (r.x1 < r.x0 || r.y1 < r.y0 || r.z1 < r.z0) return 0;
+  return (long long)(r.x1 - r.x0 + 1) * (r.y1 - r.y0 + 1) * (r.z1 - r.z0 + 1);
+}
+
+// Exact nearest map voxel of p among those with a plane (cent[s].w != 0): FLANN ((dx^2)+dy^2)+dz^2 from p to the voxel
+// centroid in float, ties -> lowest map key, or none when it is not nearer than d_max.  One warp per query over cube
+// shells of voxels around p's voxel floor(p * inv_leaf) (k_map_insert's cell), the lanes sharing each shell: shell 1 is
+// the 27 voxels around it, shell k >= 2 the voxels at Chebyshev distance k, each a hash lookup.  Only the part of a shell
+// inside `box` (the cells of the voxels with a plane: box[0..2] = min, box[4..6] = -max, k_map_planes) is visited, shells
+// that miss the box are skipped, and the search ends once no cell of the box is left unexplored, so the work per query
+// is bounded by the plane voxels' extent whatever d_max is; an empty box ends it at once.
+// The stop rules are d_reg_nn's with the leaf as the cell.  A centroid is the mean of points that all fall in its voxel,
+// so it lies in that voxel up to the 2^-20 m fixed-point rounding of the sums (and the float rounding of the centroid
+// and of p * inv_leaf): after shell k every unexplored voxel is at Chebyshev distance >= k + 1 from p's voxel, so its
+// centroid is at least k * leaf from p on some axis, less those roundings, which the 0.1 % margin covers for leaves of a
+// millimetre and more at mapping coordinates.  A query beyond +-2^22 voxels on an axis is clamped there: every map voxel
+// lies within +-2^20 (map_pack), so on that axis the true gap is larger than the clamped one and the bound still holds.
+__device__ __forceinline__ void d_regmap_nn(const float4 p, const unsigned long long* __restrict__ keys, const float4* __restrict__ cent,
+                                            const int* __restrict__ box, unsigned long long slot_mask, float inv_leaf, double leaf,
+                                            double d_max, float& best, unsigned long long& bkey, long long& bslot) {
+  const int lane = threadIdx.x & 31;
+  best = CUDART_INF_F;
+  bkey = MAP_EMPTY;
+  bslot = -1;
+  const int lo[3] = {box[0], box[1], box[2]}, hi[3] = {-box[4], -box[5], -box[6]};
+  if (lo[0] > hi[0]) return;  // no voxel has a plane
+  constexpr float CL = 4194304.0f;  // 2^22
+  const int cx = (int)fminf(fmaxf(floorf(p.x * inv_leaf), -CL), CL);
+  const int cy = (int)fminf(fmaxf(floorf(p.y * inv_leaf), -CL), CL);
+  const int cz = (int)fminf(fmaxf(floorf(p.z * inv_leaf), -CL), CL);
+  // Chebyshev distance from p's voxel to the nearest (D) and the farthest (R) cell of the box
+  const int D = max(max(max(0, max(lo[0] - cx, cx - hi[0])), max(lo[1] - cy, cy - hi[1])), max(lo[2] - cz, cz - hi[2]));
+  const int R = max(max(max(cx - lo[0], hi[0] - cx), max(cy - lo[1], hi[1] - cy)), max(cz - lo[2], hi[2] - cz));
+  const int k0 = max(1, D);
+  // shells 1 .. k0-1 hold no candidate: the state after them is "nothing found", so d_max may already end the search
+  if (k0 >= 2 && (double)(k0 - 1) * leaf * 0.999 >= d_max) return;
+  for (int k = k0;; ++k) {
+    long long T = 0;
+    MapFace fc;
+#pragma unroll 1
+    for (int f = 0; f < 7; ++f) T += d_shell_face(f, k, cx, cy, cz, lo, hi, fc);
+    int f = 0;
+    long long base = 0, area = d_shell_face(0, k, cx, cy, cz, lo, hi, fc);
+    for (long long t = lane; t < T; t += 32) {
+      while (t >= base + area) { base += area; ++f; area = d_shell_face(f, k, cx, cy, cz, lo, hi, fc); }
+      const long long u = t - base;
+      const int nx = fc.x1 - fc.x0 + 1, ny = fc.y1 - fc.y0 + 1;
+      const long long r = u / nx;
+      unsigned long long key;
+      if (!map_pack(fc.x0 + (int)(u - r * nx), fc.y0 + (int)(r % ny), fc.z0 + (int)(r / ny), key)) continue;
+      const long long s = d_map_find(keys, key, slot_mask);
+      if (s < 0) continue;
+      const float4 c = cent[s];
+      if (c.w == 0.f) continue;
+      const float ex = p.x - c.x, ey = p.y - c.y, ez = p.z - c.z;
+      const float d2 = (ex * ex + ey * ey) + ez * ez;
+      if (d2 < best || (d2 == best && key < bkey)) { best = d2; bkey = key; bslot = s; }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float ob = __shfl_xor_sync(FULL, best, o);
+      const unsigned long long ok = __shfl_xor_sync(FULL, bkey, o);
+      const long long os = __shfl_xor_sync(FULL, bslot, o);
+      if (ob < best || (ob == best && ok < bkey)) { best = ob; bkey = ok; bslot = os; }
+    }
+    const double lim = (double)k * leaf * 0.999;
+    if (bkey != MAP_EMPTY && (double)best <= lim * lim) break;
+    if (lim >= d_max) break;
+    if (k >= R) break;  // every cell of the box has been visited
+  }
+}
+
+// One ICP iteration against the map: k_reg_iter with d_regmap_nn as the search and the matched voxel's centroid and
+// plane normal (k_map_planes) as q and n.  corr_key[j] = the matched map key or MAP_EMPTY.
+__global__ void __maxnreg__(96)
+k_regmap_iter(const float4* __restrict__ src, const int* __restrict__ n_src_ptr, const unsigned long long* __restrict__ keys,
+              const float4* __restrict__ cent, const float4* __restrict__ nrm, const int* __restrict__ box, unsigned long long slot_mask,
+              float inv_leaf, double leaf, RegParams prm, RegState* st, double* __restrict__ partials, unsigned* ticket, unsigned long long* __restrict__ corr_key,
+              float* __restrict__ resid) {
+  constexpr int W = REG_BLOCK / 32;
+  __shared__ double wsum[W][REG_NV];
+  __shared__ double fin[REG_NV];
+  if (*(volatile int*)&st->done) return;  // written by an earlier launch only: every block takes the same branch
+  float Tf[12];
+#pragma unroll
+  for (int k = 0; k < 12; ++k) Tf[k] = (float)st->T[k];
+  const int V = *n_src_ptr;
+  const int lane = threadIdx.x & 31;
+  const int warps_total = (gridDim.x * REG_BLOCK) >> 5;
+  double* s = wsum[threadIdx.x >> 5];
+  for (int k = lane; k < REG_NV; k += 32) s[k] = 0.0;
+  __syncwarp();
+  for (int j = (blockIdx.x * REG_BLOCK + threadIdx.x) >> 5; j < V; j += warps_total) {
+    const float4 p = d_reg_transform(Tf, src[j]);
+    float best = CUDART_INF_F;
+    unsigned long long bkey = MAP_EMPTY;
+    long long bslot = -1;
+    if (finite3(p.x, p.y, p.z)) d_regmap_nn(p, keys, cent, box, slot_mask, inv_leaf, leaf, prm.d_max, best, bkey, bslot);
+    if (lane == 0) {
+      unsigned long long key = MAP_EMPTY;
+      float rf = CUDART_NAN_F;
+      if (bkey != MAP_EMPTY && best < prm.r2max) {
+        rf = d_reg_accumulate(s, p, cent[bslot], nrm[bslot]);
+        key = bkey;
+      }
+      corr_key[j] = key;
+      resid[j] = rf;
+    }
+  }
+  d_reg_finish<W>(wsum, fin, prm, st, partials, ticket);
 }
 
 }  // namespace gm

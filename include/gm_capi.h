@@ -528,6 +528,43 @@ GM_API gm_status gm_map_save(gm_map* map, const char* path);
 GM_API gm_status gm_map_load(const char* path, size_t min_capacity_voxels, gm_map** out);
 GM_API double gm_map_leaf(const gm_map* map);
 
+/* ---- scan-to-map registration (builder-defined: the reference keeps no map) -------------------------------------------
+ * gm_register with the aggregated voxel map as the target: localises a scan in the map being built, or in one reloaded
+ * with gm_map_load, without chaining scan-to-scan poses.  Map planes, for every occupied voxel v:
+ *   - its centroid c_v is exactly what gm_map_download reports, float((double)sum / 2^20 / count);
+ *   - N(v) = the occupied voxels among the 27 at offsets (dx, dy, dz) in {-1, 0, 1}^3, v included, visited in ascending
+ *     (dz, dy, dx) order.  With |N(v)| < GM_MAP_PLANE_MIN_VOXELS, v has no plane.  Otherwise mu = the sequential double
+ *     mean of their centroids, C = the sequential double sum of (c - mu)(c - mu)^T over N(v) divided by |N(v)|, and
+ *     cyclic Jacobi (the sign rule of gm_register's spectrum) gives lambda0 <= lambda1 <= lambda2; v has a plane iff
+ *     lambda0 <= max_planarity * lambda1 and lambda1 > 0, and its normal is float(eigenvector 0).
+ *   The neighbourhood uses the voxel centroids only, so the map's state and its file format are those of any map, saved
+ *   by any version.  How flat a voxel neighbourhood looks depends on the scan noise relative to the leaf: 0.1 suits
+ *   centimetre noise at a 10 cm leaf; 0.01 keeps only the flattest surfaces.
+ * gm_register_map runs steps 1-6 of gm_register above with the source context's VoxelGrid centroids and this search:
+ *   2'. Correspondence: among the voxels that have a plane, the one whose centroid q is nearest to p (FLANN
+ *       ((dx^2)+dy^2)+dz^2 in float, ties -> lowest map key, i.e. first in gm_map_download order), accepted iff
+ *       d^2 < float(d_max * d_max).  This is the exact nearest candidate, not an approximation.  The search walks cube
+ *       shells of voxels around p's voxel, clipped to the bounding box of the voxels with a plane: its work per point is
+ *       bounded by that box (and by d_max), and a map without planes or a point far from the box costs no search.
+ *   3'. n = that voxel's normal: r = n.(p - q), J = [p x n, n] as in step 3.
+ * Arguments are checked as by gm_register, plus 0 < max_planarity <= 1 and source and map on the same device (the one
+ * current at gm_map_create / gm_map_load).  The result is the source's registration: gm_get_registration reads it,
+ * gm_download_map_correspondences gives the matched voxels (gm_download_correspondences gives GM_ERR_STAGE_ORDER after a
+ * map registration, and gm_download_map_correspondences after a context one).  The launches are the planes of the map
+ * (k_map_planes, once per call), then those of gm_register: gm_launch_count(source) grows by max_iterations + 2, with no
+ * host synchronisation.  An empty map, or one without planes, gives 0 correspondences, converged = 0 and the initial pose.
+ * Ordering: gm_map_insert and gm_register_map wait on their context's stream for the previous of these two calls on the
+ * same map, whichever context issued it, so map operations from several contexts of the map's device run in call order
+ * without a host synchronisation. */
+#define GM_MAP_PLANE_MIN_VOXELS 5
+GM_API gm_status gm_register_map(gm_ctx* source, gm_map* map, const gm_icp_params* p, double max_planarity);
+/* V entries of the last executed iteration: the matched voxel's integer cell (the ijk of gm_map_download) or INT32_MIN x 3,
+ * float(r) or NaN; residual may be NULL */
+GM_API gm_status gm_download_map_correspondences(gm_ctx* source, int32_t* ijk /* V x 3 */, float* residual, size_t capacity_points);
+/* the plane of every voxel in gm_map_download's order and count: {nx, ny, nz, 1}, or {NaN, NaN, NaN, 0} without a plane
+ * (what gm_register_map searches with the same max_planarity); synchronises the device.  normals_xyzw = NULL: *n only */
+GM_API gm_status gm_map_download_planes(gm_map* map, double max_planarity, float* normals_xyzw, size_t capacity, size_t* n);
+
 /* ---- multi-GPU data-path collectives over NVLink peer memory (SURVEY 8e; builder-defined: the reference is one process,
  * src/geometric_mapping.cpp:128-170) -------------------------------------------------------------------------------
  * One process per GPU.  Every rank creates a gm_comm (a mailbox in its own HBM), publishes its 64-byte handle
