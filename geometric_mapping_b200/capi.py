@@ -106,6 +106,17 @@ class gm_registration(C.Structure):
                 ("pad_", C.c_int32), ("eigenvalues", C.c_double * 6), ("eigenvectors", C.c_double * 36)]
 
 
+class gm_odometry_params(C.Structure):
+    _fields_ = [("icp", gm_icp_params), ("max_planarity", C.c_double), ("min_fitness", C.c_double), ("register_first", C.c_int32),
+                ("max_steps", C.c_int32)]
+
+
+class gm_odometry_record(C.Structure):
+    _fields_ = [("pose34", C.c_float * 12), ("guess34", C.c_float * 12), ("accepted", C.c_int32), ("registered", C.c_int32),
+                ("iterations", C.c_int32), ("converged", C.c_int32), ("n_source", C.c_int32), ("n_correspondences", C.c_int32),
+                ("n_degenerate", C.c_int32), ("rmse", C.c_float), ("fitness", C.c_float), ("pad_", C.c_int32)]
+
+
 GM_MAX_ICP_ITERATIONS = 64
 GM_MAX_PRIMITIVES = 64
 PRIMITIVE_RECORD_DTYPE = np.dtype([("kind", "<i4"), ("count", "<i4"), ("coef", "<f4", 7), ("extents", "<f4", 4), ("rms", "<f4")])
@@ -159,6 +170,7 @@ SYMBOLS = [
     "gm_extract_primitives", "gm_get_primitives", "gm_download_primitive_ids", "gm_compress_primitives",
     "gm_download_compressed_primitives", "gm_icp_params_default", "gm_register", "gm_get_registration",
     "gm_download_correspondences", "gm_register_map", "gm_download_map_correspondences", "gm_map_download_planes",
+    "gm_odometry_params_default", "gm_odometry_create", "gm_odometry_destroy", "gm_odometry_step", "gm_odometry_steps", "gm_odometry_get",
     "gm_encode_marker_array", "gm_store_open", "gm_store_close", "gm_store_append", "gm_store_append_blob", "gm_store_count", "gm_store_info", "gm_store_read",
 ]
 
@@ -292,6 +304,12 @@ def _lib():
         "gm_register_map": (i32, [vp, vp, C.POINTER(gm_icp_params), C.c_double]),
         "gm_download_map_correspondences": (i32, [vp, vp, vp, sz]),
         "gm_map_download_planes": (i32, [vp, C.c_double, vp, sz, C.POINTER(sz)]),
+        "gm_odometry_params_default": (None, [C.POINTER(gm_odometry_params)]),
+        "gm_odometry_create": (i32, [vp, C.POINTER(gm_odometry_params), C.POINTER(vp)]),
+        "gm_odometry_destroy": (None, [vp]),
+        "gm_odometry_step": (i32, [vp, vp, vp]),
+        "gm_odometry_steps": (i32, [vp]),
+        "gm_odometry_get": (i32, [vp, vp, i32, C.POINTER(i32)]),
     }
     assert set(sig) == set(SYMBOLS)
     for name, (res, args) in sig.items():
@@ -947,6 +965,82 @@ class VoxelMap:
         except Exception:
             pass
 
+
+def odometry_params(init_pose34=None, **overrides) -> gm_odometry_params:
+    """gm_odometry_params with the library defaults, the first scan's pose (or its guess) as init_pose34 (3x4 or 4x4, None
+    = identity) and any field overridden by keyword: those of gm_odometry_params and of its gm_icp_params."""
+    p = gm_odometry_params()
+    _lib().gm_odometry_params_default(C.byref(p))
+    icp = {k: v for k, v in overrides.items() if k not in ("max_planarity", "min_fitness", "register_first", "max_steps")}
+    p.icp = icp_params(init_pose34, **icp)
+    for k, v in overrides.items():
+        if k not in icp:
+            setattr(p, k, v)
+    return p
+
+
+class Odometry:
+    """Map odometry on the device (include/gm_capi.h, gm_odometry_*): each step() predicts the scan's pose, registers it to
+    `vmap`, gates the result and inserts the scan at the accepted pose, without a host synchronisation.  Keywords: the
+    fields of gm_odometry_params and of its gm_icp_params.  Close it before the map."""
+
+    def __init__(self, vmap: VoxelMap, init_pose34=None, **params):
+        self.params = odometry_params(init_pose34, **params)
+        h = C.c_void_p()
+        st = _lib().gm_odometry_create(vmap._h, C.byref(self.params), C.byref(h))
+        if st != GM_OK:
+            raise GmError(st, "gm_odometry_create")
+        self._h = h
+        self.map = vmap
+
+    def step(self, ctx: "Context", delta34=None):
+        """One step with ctx after voxel(); delta34 (3x4 or 4x4) = the sensor's motion since the previous scan in its
+        frame, None = constant velocity."""
+        d = None if delta34 is None else np.ascontiguousarray(np.asarray(delta34, np.float32)[:3, :4].reshape(12))
+        ctx._ck(_lib().gm_odometry_step(self._h, ctx._h, _ptr(d)), "gm_odometry_step")
+
+    @property
+    def steps(self) -> int:
+        return int(_lib().gm_odometry_steps(self._h))
+
+    def records(self):
+        """-> the gm_odometry_record array of every step issued so far (waits for them)."""
+        n = C.c_int32(0)
+        _lib().gm_odometry_get(self._h, None, 0, C.byref(n))
+        recs = (gm_odometry_record * max(n.value, 1))()
+        st = _lib().gm_odometry_get(self._h, recs, n.value, C.byref(n))
+        if st != GM_OK:
+            raise GmError(st, "gm_odometry_get")
+        return recs[:n.value]
+
+    def trajectory(self) -> dict:
+        """-> numpy arrays over the steps: poses and guesses (k x 3 x 4 float32), accepted, registered, iterations, converged,
+        n_source, n_correspondences, n_degenerate (int32), rmse, fitness (float32)."""
+        recs = self.records()
+        out = {"poses": np.array([r.pose34[:] for r in recs], np.float32).reshape(-1, 3, 4),
+               "guesses": np.array([r.guess34[:] for r in recs], np.float32).reshape(-1, 3, 4)}
+        for f in ("accepted", "registered", "iterations", "converged", "n_source", "n_correspondences", "n_degenerate"):
+            out[f] = np.array([getattr(r, f) for r in recs], np.int32)
+        for f in ("rmse", "fitness"):
+            out[f] = np.array([getattr(r, f) for r in recs], np.float32)
+        return out
+
+    def close(self):
+        if getattr(self, "_h", None):
+            _lib().gm_odometry_destroy(self._h)
+            self._h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class PeerComm:

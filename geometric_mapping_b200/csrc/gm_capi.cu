@@ -10,6 +10,7 @@
 #include "gm_map.cuh"
 #include "gm_comm.cuh"
 #include "gm_register.cuh"
+#include "gm_odometry.cuh"
 #include <new>
 
 #include <algorithm>
@@ -2689,35 +2690,39 @@ cudaError_t ensure_plane_tables(gm_map* m) {
 }
 
 int map_blocks(const gm_map* m) { return (int)std::min<unsigned long long>((m->n_slots + 255) / 256, (unsigned long long)m->num_sms * 16); }
-}  // namespace
 
-extern "C" {
-
-gm_status gm_register_map(gm_ctx* source, gm_map* map, const gm_icp_params* p, double max_planarity) {
-  if (!source || !map || !p) return GM_ERR_INVALID_ARG;
-  gm_ctx* ctx = source;  // GM_CUDA / GM_LAUNCH report on the source
-  if (source->device != map->device) { ctx->err = "gm_register_map: source and map on different devices"; return GM_ERR_INVALID_ARG; }
+// gm_register_map's argument rules (gm_odometry_create checks its icp by them too)
+bool valid_regmap_args(const gm_icp_params* p, double max_planarity) {
   const double dmax = p->max_correspondence_distance;
-  if (!(dmax > 0.0) || !std::isfinite(dmax) || p->max_iterations < 1 || p->max_iterations > GM_MAX_ICP_ITERATIONS ||
-      !(p->min_rotation_step >= 0.0) || !(p->min_translation_step >= 0.0) || !(p->degeneracy_ratio >= 0.0) ||
-      !(p->degeneracy_ratio < 1.0) || !finite_pose(p->init_pose34) || !valid_planarity(max_planarity))
-    return GM_ERR_INVALID_ARG;
-  if (gm_status s = require(source, VOXEL)) return s;
+  return dmax > 0.0 && std::isfinite(dmax) && p->max_iterations >= 1 && p->max_iterations <= GM_MAX_ICP_ITERATIONS &&
+         p->min_rotation_step >= 0.0 && p->min_translation_step >= 0.0 && p->degeneracy_ratio >= 0.0 && p->degeneracy_ratio < 1.0 &&
+         finite_pose(p->init_pose34) && valid_planarity(max_planarity);
+}
+
+// The buffers a scan-to-map registration of `source` uses (allocated by the first call).
+gm_status regmap_buffers(gm_ctx* source, gm_map* map) {
+  gm_ctx* ctx = source;
   if (gm_status s = ensure_reg_buffers(source)) return s;
   if (!source->d_reg_key.count) GM_CUDA(source->d_reg_key.alloc(source->cap));
   GM_CUDA(ensure_plane_tables(map));
+  return GM_OK;
+}
+
+// The launches of gm_register_map on the source stream, after its checks and the wait for the map's last operation:
+// the map's planes, begin() (the kernel that sets the registration's start), then max_iterations x k_regmap_iter.
+// Shared by gm_register_map and gm_odometry_step so that a step registers exactly as the call does.
+template <class Begin>
+gm_status regmap_launch(gm_ctx* source, gm_map* map, const gm_icp_params* p, double max_planarity, Begin begin) {
+  gm_ctx* ctx = source;  // GM_CUDA / GM_LAUNCH report on the source
   ctx->stages &= ~(1u << REGISTRATION);
-  GM_CUDA(cudaStreamWaitEvent(source->stream, map->ev_last, 0));
   const unsigned long long mask = map->n_slots - 1ull;
   GM_CUDA(cudaMemsetAsync(map->d_plane_box, 0x7F, 8 * sizeof(int), source->stream));
   GM_LAUNCH(ctx, k_map_planes, map_blocks(map), 256, map->d_keys, map->d_cnt, map->d_sums, mask, max_planarity, map->d_plane_cent,
             map->d_plane_nrm, map->d_plane_box);
-  Pose34 init;
-  std::memcpy(init.r, p->init_pose34, sizeof(init.r));
-  GM_LAUNCH(ctx, k_reg_begin, 1, 32, source->d_reg_state, init, &source->d_st->vox.n_voxels);
+  begin();
   RegParams rp;
-  rp.d_max = dmax;
-  rp.r2max = (float)(dmax * dmax);
+  rp.d_max = p->max_correspondence_distance;
+  rp.r2max = (float)(rp.d_max * rp.d_max);
   rp.min_rot = p->min_rotation_step;
   rp.min_trans = p->min_translation_step;
   rp.ratio = p->degeneracy_ratio;
@@ -2727,9 +2732,29 @@ gm_status gm_register_map(gm_ctx* source, gm_map* map, const gm_icp_params* p, d
               map->d_plane_nrm, map->d_plane_box, mask, map->inv_leaf, map->leaf, rp, source->d_reg_state, source->d_reg_part, source->d_reg_ticket,
               source->d_reg_key, source->d_reg_res);
   GM_CHECK_LAUNCHES(ctx);
-  GM_CUDA(cudaEventRecord(map->ev_last, source->stream));
   source->reg_target = 1;
   mark(source, REGISTRATION);
+  return GM_OK;
+}
+}  // namespace
+
+extern "C" {
+
+gm_status gm_register_map(gm_ctx* source, gm_map* map, const gm_icp_params* p, double max_planarity) {
+  if (!source || !map || !p) return GM_ERR_INVALID_ARG;
+  gm_ctx* ctx = source;  // GM_CUDA / GM_LAUNCH report on the source
+  if (source->device != map->device) { ctx->err = "gm_register_map: source and map on different devices"; return GM_ERR_INVALID_ARG; }
+  if (!valid_regmap_args(p, max_planarity)) return GM_ERR_INVALID_ARG;
+  if (gm_status s = require(source, VOXEL)) return s;
+  if (gm_status s = regmap_buffers(source, map)) return s;
+  GM_CUDA(cudaStreamWaitEvent(source->stream, map->ev_last, 0));
+  Pose34 init;
+  std::memcpy(init.r, p->init_pose34, sizeof(init.r));
+  gm_status s = regmap_launch(source, map, p, max_planarity, [&] {
+    GM_LAUNCH(ctx, k_reg_begin, 1, 32, source->d_reg_state, init, &source->d_st->vox.n_voxels);
+  });
+  if (s != GM_OK) return s;
+  GM_CUDA(cudaEventRecord(map->ev_last, source->stream));
   return GM_OK;
 }
 
@@ -2789,3 +2814,116 @@ gm_status gm_map_download_planes(gm_map* m, double max_planarity, float* normals
 
 }  // extern "C"
 
+// ---- map odometry (gm_odometry.cuh) -----------------------------------------------------------------------------------
+static_assert(sizeof(gm_odometry_params) == 112 && sizeof(gm_odometry_record) == 136 && sizeof(OdomRecord) == sizeof(gm_odometry_record) &&
+              offsetof(OdomRecord, accepted) == offsetof(gm_odometry_record, accepted) &&
+              offsetof(OdomRecord, fitness) == offsetof(gm_odometry_record, fitness), "odometry layouts");
+
+struct gm_odometry {
+  gm_map* map = nullptr;
+  gm_odometry_params p{};
+  int32_t steps = 0;                 // steps issued
+  DevBuf<OdomRecord> d_rec;          // the trajectory, max_steps records
+  DevBuf<OdomInsert> d_ins;          // pose and flag of the current step's insert
+  cudaStream_t stream = nullptr;     // the trajectory download
+  ~gm_odometry() { if (stream) cudaStreamDestroy(stream); }
+};
+
+extern "C" {
+
+void gm_odometry_params_default(gm_odometry_params* p) {
+  if (!p) return;
+  std::memset(p, 0, sizeof(*p));
+  gm_icp_params_default(&p->icp);
+  p->max_planarity = 0.1;
+  p->min_fitness = 0.5;
+  p->register_first = 0;
+  p->max_steps = 4096;
+}
+
+gm_status gm_odometry_create(gm_map* map, const gm_odometry_params* p, gm_odometry** out) {
+  if (!out) return GM_ERR_INVALID_ARG;
+  *out = nullptr;
+  if (!map || !p || !valid_regmap_args(&p->icp, p->max_planarity) || !(p->min_fitness >= 0.0 && p->min_fitness <= 1.0) ||
+      (p->register_first != 0 && p->register_first != 1) || p->max_steps < 1)
+    return GM_ERR_INVALID_ARG;
+  int prev = 0;
+  if (cudaGetDevice(&prev) != cudaSuccess || cudaSetDevice(map->device) != cudaSuccess) { cudaGetLastError(); return GM_ERR_CUDA; }
+  gm_odometry* o = new gm_odometry();
+  o->map = map;
+  o->p = *p;
+  cudaError_t e = o->d_rec.alloc((size_t)p->max_steps);
+  if (e == cudaSuccess) e = o->d_ins.alloc(1);
+  if (e == cudaSuccess) e = cudaMemset(o->d_rec, 0, (size_t)p->max_steps * sizeof(OdomRecord));
+  if (e == cudaSuccess) e = cudaMemset(o->d_ins, 0, sizeof(OdomInsert));
+  if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&o->stream, cudaStreamNonBlocking);
+  if (e == cudaSuccess) e = cudaDeviceSynchronize();
+  cudaSetDevice(prev);
+  if (e != cudaSuccess) { delete o; return GM_ERR_CUDA; }
+  *out = o;
+  return GM_OK;
+}
+
+void gm_odometry_destroy(gm_odometry* odo) {
+  if (!odo) return;
+  cudaDeviceSynchronize();  // as gm_map_destroy: the steps in flight read the trajectory
+  delete odo;
+}
+
+gm_status gm_odometry_step(gm_odometry* odo, gm_ctx* ctx, const float* delta34) {
+  if (!odo || !ctx) return GM_ERR_INVALID_ARG;
+  gm_map* map = odo->map;
+  const int k = odo->steps;
+  if (k >= odo->p.max_steps) return GM_ERR_CAPACITY;
+  if (delta34 && (k == 0 || !finite_pose(delta34))) return GM_ERR_INVALID_ARG;
+  if (ctx->device != map->device) { ctx->err = "gm_odometry_step: context and map on different devices"; return GM_ERR_INVALID_ARG; }
+  if (gm_status s = require(ctx, COMPACTED, VOXEL)) return s;
+  const bool registered = k > 0 || odo->p.register_first;
+  if (registered)
+    if (gm_status s = regmap_buffers(ctx, map)) return s;
+  GM_CUDA(cudaStreamWaitEvent(ctx->stream, map->ev_last, 0));
+  Pose34 init{}, delta{};
+  int mode = ODOM_INIT;
+  if (k == 0) {
+    std::memcpy(init.r, odo->p.icp.init_pose34, sizeof(init.r));
+  } else if (delta34 || k == 1) {  // constant velocity at k = 1: delta = identity
+    mode = ODOM_DELTA;
+    if (delta34) std::memcpy(delta.r, delta34, sizeof(delta.r));
+    else delta.r[0] = delta.r[5] = delta.r[10] = 1.0f;
+  } else {
+    mode = ODOM_VELOCITY;
+  }
+  RegState* st = registered ? (RegState*)ctx->d_reg_state : nullptr;
+  auto begin = [&] { GM_LAUNCH(ctx, k_odom_begin, 1, 32, odo->d_rec, k, mode, init, delta, st, &ctx->d_st->vox.n_voxels); };
+  if (registered) {
+    if (gm_status s = regmap_launch(ctx, map, &odo->p.icp, odo->p.max_planarity, begin)) return s;
+  } else {
+    ctx->stages &= ~(1u << REGISTRATION);
+    begin();
+  }
+  GM_LAUNCH(ctx, k_odom_gate, 1, 32, odo->d_rec, k, st, odo->p.min_fitness, odo->d_ins);
+  // gm_map_insert's grid, at least one block: the kernel reads the point count on the device
+  const int blocks = std::max(1, std::min(div_up((long long)ctx->n_input, 256), ctx->num_sms * 16));
+  GM_LAUNCH(ctx, k_map_insert_gated, blocks, 256, ctx->d_cloud_c, &ctx->d_st->n_valid, &odo->d_ins->pose, &odo->d_ins->accept, map->inv_leaf,
+            map->d_keys, map->d_cnt, map->d_sums, map->n_slots - 1ull, map->d_st);
+  GM_CHECK_LAUNCHES(ctx);
+  GM_CUDA(cudaEventRecord(map->ev_last, ctx->stream));
+  odo->steps = k + 1;
+  return GM_OK;
+}
+
+int32_t gm_odometry_steps(const gm_odometry* odo) { return odo ? odo->steps : 0; }
+
+gm_status gm_odometry_get(gm_odometry* odo, gm_odometry_record* out, int32_t capacity, int32_t* n) {
+  if (!odo || !n) return GM_ERR_INVALID_ARG;
+  *n = odo->steps;
+  if (!out) return GM_OK;
+  if (capacity < odo->steps) return GM_ERR_CAPACITY;
+  cudaError_t e = cudaStreamWaitEvent(odo->stream, odo->map->ev_last, 0);  // after every step issued so far
+  if (e == cudaSuccess && odo->steps > 0)
+    e = cudaMemcpyAsync(out, odo->d_rec, (size_t)odo->steps * sizeof(OdomRecord), cudaMemcpyDeviceToHost, odo->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(odo->stream);
+  return e == cudaSuccess ? GM_OK : GM_ERR_CUDA;
+}
+
+}  // extern "C"

@@ -41,11 +41,10 @@ struct Pose34 { float r[12]; };  // row-major [R | t]
 
 // Insert the points pts[0..n) (optionally only those with labels[i] == label_filter) after the rigid
 // transform p' = R p + t, evaluated as fmaf chains (bit-identical to the oracle's std::fmaf).
-__global__ void k_map_insert(const float4* __restrict__ pts, const unsigned char* __restrict__ labels, const int* __restrict__ n_ptr,
-                             int label_filter, Pose34 T, int use_pose, float inv_leaf, unsigned long long* __restrict__ keys,
-                             int* __restrict__ cnt, long long* __restrict__ sums /* 3 per slot */, unsigned long long slot_mask,
-                             MapState* st) {
-  const int n = *n_ptr;
+__device__ __forceinline__ void d_map_insert(const float4* __restrict__ pts, const unsigned char* __restrict__ labels, const int n,
+                                             int label_filter, const Pose34& T, int use_pose, float inv_leaf,
+                                             unsigned long long* __restrict__ keys, int* __restrict__ cnt, long long* __restrict__ sums,
+                                             unsigned long long slot_mask, MapState* st) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     if (label_filter >= 0 && labels[i] != (unsigned char)label_filter) continue;
     const float4 p = pts[i];
@@ -81,6 +80,23 @@ __global__ void k_map_insert(const float4* __restrict__ pts, const unsigned char
     atomicAdd(reinterpret_cast<unsigned long long*>(sums) + 3 * slot + 2, (unsigned long long)__float2ll_rn(z * MAP_FX));
     atomicAdd(&st->n_points, 1ull);
   }
+}
+
+__global__ void k_map_insert(const float4* __restrict__ pts, const unsigned char* __restrict__ labels, const int* __restrict__ n_ptr,
+                             int label_filter, Pose34 T, int use_pose, float inv_leaf, unsigned long long* __restrict__ keys,
+                             int* __restrict__ cnt, long long* __restrict__ sums /* 3 per slot */, unsigned long long slot_mask,
+                             MapState* st) {
+  d_map_insert(pts, labels, *n_ptr, label_filter, T, use_pose, inv_leaf, keys, cnt, sums, slot_mask, st);
+}
+
+// k_map_insert of every point at a pose the device decided (gm_odometry_step): pose and go/no-go flag are read from
+// device memory, and a flag of 0 inserts nothing.
+__global__ void k_map_insert_gated(const float4* __restrict__ pts, const int* __restrict__ n_ptr, const Pose34* __restrict__ pose,
+                                   const int* __restrict__ accept, float inv_leaf, unsigned long long* __restrict__ keys,
+                                   int* __restrict__ cnt, long long* __restrict__ sums, unsigned long long slot_mask, MapState* st) {
+  if (!*accept) return;
+  const Pose34 T = *pose;
+  d_map_insert(pts, nullptr, *n_ptr, -1, T, 1, inv_leaf, keys, cnt, sums, slot_mask, st);
 }
 
 // Raw re-insertion of saved voxels (gm_map_load): key, count and fixed-point sums as stored.

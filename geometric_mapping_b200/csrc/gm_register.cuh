@@ -30,14 +30,19 @@ struct RegParams {
   double min_rot, min_trans, ratio;
 };
 
-__global__ void k_reg_begin(RegState* st, Pose34 init, const int* __restrict__ n_source) {
-  if (threadIdx.x != 0 || blockIdx.x != 0) return;
-  for (int k = 0; k < 12; ++k) st->T[k] = (double)init.r[k];
+// T_0 = double(init) and a cleared result: the start of every registration (k_reg_begin, k_odom_begin).  One thread.
+__device__ __forceinline__ void d_reg_start(RegState* st, const float init[12], const int* __restrict__ n_source) {
+  for (int k = 0; k < 12; ++k) st->T[k] = (double)init[k];
   for (int k = 0; k < 6; ++k) st->eig[k] = 0.0;
   for (int k = 0; k < 36; ++k) st->vecs[k] = 0.0;
   st->sum_r2 = 0.0;
   st->done = 0; st->iterations = 0; st->converged = 0; st->n_corr = 0; st->n_degenerate = 0;
   st->n_source = *n_source;
+}
+
+__global__ void k_reg_begin(RegState* st, Pose34 init, const int* __restrict__ n_source) {
+  if (threadIdx.x != 0 || blockIdx.x != 0) return;
+  d_reg_start(st, init.r, n_source);
 }
 
 // Exact nearest compacted target point of c (FLANN L2_Simple, ties -> lowest compacted index), or none when it is not

@@ -565,6 +565,71 @@ GM_API gm_status gm_download_map_correspondences(gm_ctx* source, int32_t* ijk /*
  * (what gm_register_map searches with the same max_planarity); synchronises the device.  normals_xyzw = NULL: *n only */
 GM_API gm_status gm_map_download_planes(gm_map* map, double max_planarity, float* normals_xyzw, size_t capacity, size_t* n);
 
+/* ---- map odometry (builder-defined: the reference computes no pose) ---------------------------------------------------
+ * Builds a map from the scans alone without a host round trip: each gm_odometry_step predicts the scan's pose, registers
+ * the scan to the map from it (gm_register_map), accepts or rejects the result and inserts the scan at the accepted pose
+ * (gm_map_insert), all on the context's stream.  The trajectory, one gm_odometry_record per step, lives in device memory.
+ * Step k (k = gm_odometry_steps() when it is called) needs ctx after gm_voxel: its VoxelGrid centroids are the
+ * registration source and its compacted cloud is what the insert takes.  ctx must be on the map's device; any number of
+ * contexts may take turns (e.g. two, so that the next scan is processed while a step runs).
+ *   Guess G_k.  P_j = the float pose34 of step j's record.  Poses compose rigidly in double from the float inputs, unfused:
+ *     (A o B): R[i][j] = (A[i][0]*B[0][j] + A[i][1]*B[1][j]) + A[i][2]*B[2][j],
+ *              t[i]    = ((A[i][0]*B[0][3] + A[i][1]*B[1][3]) + A[i][2]*B[2][3]) + A[i][3]   (gm_register's update order);
+ *     the inverse of a float pose is [R^T | -(R^T t)], (R^T t)[i] = (R[0][i]*t[0] + R[1][i]*t[1]) + R[2][i]*t[2].
+ *     k = 0:                 G = icp.init_pose34; delta34 must be NULL (else GM_ERR_INVALID_ARG).
+ *     k >= 1, delta34 given: G = P_{k-1} o delta, delta = the sensor's motion since the previous scan in the previous
+ *                            scan's frame (wheel odometry, an IMU; the identity gives "constant pose").
+ *     k >= 1, delta34 NULL:  constant velocity, G = P_{k-1} o (P_{k-2}^-1 o P_{k-1}), the inner product kept in double;
+ *                            at k = 1 delta = the identity.
+ *     G is rounded to float element by element and the registration starts from T_0 = double(G).
+ *   Registration.  Exactly gm_register_map(ctx, map, icp with init_pose34 = G, max_planarity): the same launches and the
+ *     same results, which gm_get_registration and gm_download_map_correspondences on ctx then report.  Step 0 with
+ *     register_first = 0 does not register (a new map) and clears ctx's registration.
+ *   Gate.  A registered step is accepted iff (double)fitness >= min_fitness and n_correspondences >= 6, with fitness and
+ *     rmse the floats gm_get_registration computes.  An unregistered step 0 is always accepted.
+ *   Insert.  An accepted step inserts all of ctx's compacted points at pose34 = float(T) element by element (what
+ *     gm_get_registration returns): the map gm_map_insert(map, ctx, pose34, -1) would give.  A rejected step inserts nothing
+ *     and records the guess as its pose, so the next guesses dead-reckon across it; its ICP result stays readable through
+ *     gm_get_registration.  The map has no removal: the gate is what keeps a failed registration out of it.
+ *   Ordering.  A step is a map operation: it waits for the previous gm_map_insert / gm_register_map / gm_odometry_step on
+ *     the map, whichever context issued it, and the next one waits for its insert.  There is no host synchronisation
+ *     (the first registration of a context allocates its buffers once, as gm_register_map does).
+ *   Launches.  A registered step launches k_odom_begin (the guess and the registration's start), k_map_planes,
+ *     icp.max_iterations x k_regmap_iter, k_odom_gate and the insert: gm_launch_count(ctx) grows by max_iterations + 4.
+ *     An unregistered step 0 launches k_odom_begin, k_odom_gate and the insert: + 3.  The insert is launched even for an
+ *     empty scan (its kernel reads the point count on the device).
+ *   Errors.  gm_odometry_create checks icp by gm_register_map's rules and 0 <= min_fitness <= 1, register_first in {0, 1},
+ *     max_steps >= 1.  A step k >= max_steps gives GM_ERR_CAPACITY, a missing stage GM_ERR_STAGE_ORDER, a context on
+ *     another device GM_ERR_INVALID_ARG: then nothing is launched and gm_odometry_steps does not move.
+ * Destroy the odometry before its map. */
+typedef struct gm_odometry gm_odometry;
+typedef struct gm_odometry_params {
+  gm_icp_params icp;        /* d_max, iterations, step thresholds, degeneracy_ratio as for gm_register_map; init_pose34 = the
+                               first scan's pose in the map frame (register_first = 0) or the guess of it (1)                */
+  double max_planarity;     /* as gm_register_map                                                 default 0.1  */
+  double min_fitness;       /* the gate, see above                                                default 0.5  */
+  int32_t register_first;   /* 0: step 0 inserts at init_pose34 without registering (a new map);
+                               1: step 0 registers from init_pose34 (a map from gm_map_load, or one another odometry fills)
+                                                                                                  default 0    */
+  int32_t max_steps;        /* trajectory capacity, >= 1                                          default 4096 */
+} gm_odometry_params;
+typedef struct gm_odometry_record {
+  float pose34[12];         /* the scan's pose in the map frame: the registered pose if accepted, else the guess */
+  float guess34[12];        /* the prediction the step started from */
+  int32_t accepted;         /* 1 = the scan was inserted into the map */
+  int32_t registered;       /* 0 only for an unregistered step 0 */
+  int32_t iterations, converged, n_source, n_correspondences, n_degenerate;
+  float rmse, fitness;      /* as gm_get_registration reports them (0 for an unregistered step) */
+  int32_t pad_;
+} gm_odometry_record;
+GM_API void gm_odometry_params_default(gm_odometry_params* p);
+GM_API gm_status gm_odometry_create(gm_map* map, const gm_odometry_params* p, gm_odometry** out);
+GM_API void gm_odometry_destroy(gm_odometry* odo);
+GM_API gm_status gm_odometry_step(gm_odometry* odo, gm_ctx* ctx, const float* delta34 /* NULL = constant velocity */);
+GM_API int32_t gm_odometry_steps(const gm_odometry* odo);  /* steps issued so far (host counter, no synchronisation) */
+/* the records of every step issued so far, in step order; *n = their number.  Waits for the last of them.  out = NULL: *n only */
+GM_API gm_status gm_odometry_get(gm_odometry* odo, gm_odometry_record* out, int32_t capacity, int32_t* n);
+
 /* ---- multi-GPU data-path collectives over NVLink peer memory (SURVEY 8e; builder-defined: the reference is one process,
  * src/geometric_mapping.cpp:128-170) -------------------------------------------------------------------------------
  * One process per GPU.  Every rank creates a gm_comm (a mailbox in its own HBM), publishes its 64-byte handle
