@@ -161,6 +161,7 @@ struct gm_ctx {
   DevBuf<long long> d_dense_sum;
   DevBuf<unsigned long long> d_dense_state;  // look-back tile states of the scan over the tables
   int voxel_mode = 0;  // 0 = dense tables when the key range fits, 1 = always sort
+  bool vox_assign_on_demand = false;  // the scan's VoxelGrid took the dense path, which leaves d_vkey_pt / d_assign unwritten
   int normals_mode = 0;  // 0 = neighbours summed in cell-run order (fast), 1 = in FLANN's (d2, index) order (bit-identical to the oracle)
   int knn_k = 0;         // > 0: k-nearest-neighbour normals (setKSearch) instead of the radius search
   double knn_max_radius = 0.0;  // > 0: only neighbours nearer than this count (FLANN's radius + max_nn form); 0 = plain k-NN
@@ -889,16 +890,19 @@ gm_status ensure_dense(gm_ctx* ctx, size_t range) {
   return GM_OK;
 }
 
+bool dense_voxel_path(const gm_ctx* ctx, size_t key_range) { return ctx->voxel_mode == 0 && key_range > 0 && key_range <= kDenseMaxKeys; }
+
 // pcl::VoxelGrid of `pts` (vs->n points, bbox already in vs).  `key_range` = host-side upper bound of the number
-// of lattice cells (0 = unknown).  Small enough: dense tables, no sort (3 launches); else keys -> sort -> heads
-// -> centroids.  Both give the same voxels in the same order with the same fixed-point centroids.
+// of lattice cells (0 = unknown).  Small enough: dense tables, no sort (2 launches, a 3rd for the per-point key and
+// voxel id in o.key_pt / o.assign unless `assign` is false); else keys -> sort -> heads -> centroids, which always
+// writes them.  Both give the same voxels in the same order with the same fixed-point centroids.
 gm_status voxel_downsample(gm_ctx* ctx, const float4* pts, VoxState* vs, size_t n_cap, int key_bits, size_t key_range, const VoxBuffers& o,
-                           int* sorted_buf) {
+                           int* sorted_buf, bool assign = true) {
   const float leaf_f = (float)ctx->prm.voxelGridLeafSize;
   const float inv = 1.0f / leaf_f;
   int blocks = std::min(div_up((long long)n_cap, 256), ctx->num_sms * 16);
   gm_status s;
-  if (ctx->voxel_mode == 0 && key_range > 0 && key_range <= kDenseMaxKeys) {
+  if (dense_voxel_path(ctx, key_range)) {
     if ((s = ensure_dense(ctx, key_range)) != GM_OK) return s;
     { SegTimer seg_(ctx, SEG_VOX_KEYS);
       if (pts == ctx->d_cloud_c && has(ctx, NORMALS) && !ctx->injected) {
@@ -912,7 +916,7 @@ gm_status voxel_downsample(gm_ctx* ctx, const float4* pts, VoxState* vs, size_t 
     { SegTimer seg_(ctx, SEG_VOX_REDUCE);
       GM_LAUNCH(ctx, k_voxel_dense_scan, div_up((long long)key_range, CPL_TILE), CP_BLOCK, ctx->d_dense_cnt, ctx->d_dense_sum, ctx->d_dense_id,
                 (int)key_range, o.vox_key, o.vox_count, o.centroid, ctx->d_dense_state, ctx->d_ctl + 2, vs, &ctx->d_st->error);
-      GM_LAUNCH(ctx, k_voxel_assign, blocks, 256, pts, vs, inv, ctx->d_dense_id, (int)key_range, o.key_pt, o.assign); }
+      if (assign) GM_LAUNCH(ctx, k_voxel_assign, blocks, 256, pts, vs, inv, ctx->d_dense_id, (int)key_range, o.key_pt, o.assign); }
     *sorted_buf = 0;
     GM_CHECK_LAUNCHES(ctx);
     return GM_OK;
@@ -968,11 +972,13 @@ gm_status gm_voxel(gm_ctx* ctx) {
       const float* b = ctx->vox_bbox;
       GM_LAUNCH(ctx, k_set_bbox, 1, 32, &ctx->d_st->vox, b[0], b[1], b[2], b[3], b[4], b[5]);
     }
-    gm_status s = voxel_downsample(ctx, ctx->d_cloud_c, &ctx->d_st->vox, n, key_bits, key_range, o, &buf);
+    // nothing in a scan reads the per-point assignment: on the dense path gm_download_voxel_assignment computes it
+    gm_status s = voxel_downsample(ctx, ctx->d_cloud_c, &ctx->d_st->vox, n, key_bits, key_range, o, &buf, false);
     if (s != GM_OK) return s;
+    ctx->vox_assign_on_demand = dense_voxel_path(ctx, key_range);
     if (has(ctx, NORMALS)) {
       SegTimer seg_(ctx, SEG_VOX_NN);
-      GM_LAUNCH(ctx, k_voxel_nn, std::min(div_up((long long)n * 32, NN_BLOCK), ctx->num_sms * 16), NN_BLOCK, ctx->d_centroid, ctx->d_sorted,
+      GM_LAUNCH(ctx, k_voxel_nn, std::min(div_up((long long)n * NN_GROUP, NN_BLOCK), ctx->num_sms * 16), NN_BLOCK, ctx->d_centroid, ctx->d_sorted,
                 ctx->d_tab, ctx->d_ucell_start, ctx->d_runs, ctx->d_cell_nruns, ctx->d_valid_map, ctx->d_normals_c, ctx->grid, ctx->prm.nn_index_mode,
                 ctx->d_st, ctx->d_nn_idx, ctx->d_nn_normal);
     }
@@ -1354,6 +1360,9 @@ static gm_status process_scan_body(gm_ctx* ctx, const int32_t* plane_samples_hos
 static void mark_processed(gm_ctx* ctx, int Hp, int Hc) {
   mark(ctx, CROP, NORMALS, COMPACTED, VOXEL, FRAME, LABELS, POLY);
   ctx->injected = false;
+  size_t key_range = 0;  // the VoxelGrid path the replayed gm_voxel took
+  voxel_key_bits(ctx, ctx->n_grid, &key_range);
+  ctx->vox_assign_on_demand = dense_voxel_path(ctx, key_range);
   const int H[2] = {Hp, Hc};
   for (int k = 0; k < 2; ++k)
     if (H[k] > 0) { mark(ctx, ransac_stage(k), model_stage(k)); ctx->ransac_H[k] = H[k]; }
@@ -1847,6 +1856,11 @@ gm_status gm_download_valid_map(gm_ctx* ctx, int32_t* out, size_t capacity_point
 gm_status gm_download_voxel_assignment(gm_ctx* ctx, int32_t* keys, int32_t* assign, size_t capacity_points) {
   if (!ctx) return GM_ERR_INVALID_ARG;
   if (gm_status s = require(ctx, VOXEL)) return s;
+  if (ctx->vox_assign_on_demand && ctx->n_grid > 0) {
+    GM_LAUNCH(ctx, k_voxel_lookup, std::min(div_up((long long)ctx->n_grid, 256), ctx->num_sms * 16), 256, ctx->d_cloud_c, &ctx->d_st->vox,
+              ctx->d_vox_key, ctx->d_vkey_pt, ctx->d_assign);
+    GM_CHECK_LAUNCHES(ctx);
+  }
   DevState h;
   gm_status s = download(ctx, &h, n_valid, capacity_points, {{keys, ctx->d_vkey_pt, 4}, {assign, ctx->d_assign, 4}});
   if (s != GM_OK) return s;

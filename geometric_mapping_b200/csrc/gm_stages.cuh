@@ -1260,6 +1260,24 @@ __global__ void k_voxel_assign(const float4* __restrict__ pts, VoxState* st, flo
   }
 }
 
+// The same point -> (key, voxel id) on demand, for the dense path run without k_voxel_assign: the key from the lattice
+// block 0 of k_voxel_accumulate(_sorted) published in *st, the id by a binary search in the ascending voxel keys (not
+// from the per-key id table: a later VoxelGrid on the same context, e.g. the compression residual, reuses it).
+__global__ void k_voxel_lookup(const float4* __restrict__ pts, const VoxState* __restrict__ st, const int* __restrict__ vox_key,
+                               int* __restrict__ key_of_point, int* __restrict__ assign) {
+  const int n = st->n, V = st->n_voxels;
+  VoxLattice L;
+  for (int a = 0; a < 3; ++a) { L.minb[a] = st->min_b[a]; L.mul[a] = st->mul[a]; }
+  L.overflow = st->overflow;
+  const float inv = st->v_inv;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const int key = L.overflow ? i : d_vox_key(L, inv, pts[i]);
+    const int v = lower_bound_u32(reinterpret_cast<const unsigned*>(vox_key), V, (unsigned)key);
+    key_of_point[i] = key;
+    assign[i] = (v < V && vox_key[v] == key) ? v : -1;
+  }
+}
+
 // After the voxel sort: number the voxels (ascending key), record their first sorted position and
 // the voxel rank of every point.
 __global__ void __launch_bounds__(CP_BLOCK)
@@ -1333,8 +1351,8 @@ k_voxel_centroids(const unsigned* __restrict__ sidx, const float4* __restrict__ 
 // mode 0 (reference-faithful): index = pre-compaction index, looked up in the COMPACTED normals;
 // index >= n_valid is counted in nn_oor (the reference would throw).  mode 1 (fixed): only points
 // that survived compaction are candidates and the index is the compacted one.
-// One warp per voxel: lanes take the x-runs of the cube shells as tasks (two binary searches + a
-// short scan each), then a lexicographic (d2, index) warp minimum.
+// Ring 1 of most voxels by a group of lanes (k_voxel_nn), the rest by a warp: lanes take the x-runs of the cube
+// shells as tasks (two popcount lookups + a short scan each), then a lexicographic (d2, index) warp minimum.
 constexpr int NN_BLOCK = 128;
 
 __device__ __forceinline__ void d_nn_scan(const float4* __restrict__ sp, const int* __restrict__ valid_map, int mode,
@@ -1362,75 +1380,164 @@ __device__ __forceinline__ void d_nn_scan_row(const float4* __restrict__ sp, con
   }
 }
 
+// Rings k0.. of the expanding cube-shell search of one centroid by the whole warp (best / bi: what the rings before k0
+// gave, the same on every lane): ring 1 as the 9 rows of the 27-cell cube, ring k >= 2 as 8k perimeter rows with the
+// full x span + (2k-1)^2 inner rows with two end cells; after each ring a lexicographic (d2, index) warp minimum.
+__device__ __forceinline__ void d_nn_rings(const float4* __restrict__ sp, const int* __restrict__ valid_map, int mode, const GridSpec& g,
+                                           const BlockEntry* __restrict__ tab, const int* __restrict__ ucell_start, int U, int nf,
+                                           const float4 c, int cx, int cy, int cz, int k0, int kmax, float& best, int& bi) {
+  const int lane = threadIdx.x & 31;
+  for (int k = k0; k <= kmax; ++k) {
+    if (k == 1) {
+      if (lane < 9)
+        d_nn_scan_row(sp, valid_map, mode, g, tab, ucell_start, U, nf, cx - 1, cx + 1, cy + (lane % 3) - 1, cz + (lane / 3) - 1, c, best, bi);
+    } else {
+      const int inner = 2 * k - 1, T = 8 * k + 2 * inner * inner;
+      for (int t = lane; t < T; t += 32) {
+        int dy, dz, x0, x1;
+        if (t < 8 * k) {
+          if (t < 2 * k + 1) { dz = -k; dy = t - k; }
+          else if (t < 4 * k + 2) { dz = k; dy = t - (2 * k + 1) - k; }
+          else if (t < 6 * k + 1) { dy = -k; dz = t - (4 * k + 2) - (k - 1); }
+          else { dy = k; dz = t - (6 * k + 1) - (k - 1); }
+          x0 = cx - k; x1 = cx + k;
+        } else {
+          int u2 = t - 8 * k, cell = u2 >> 1;
+          dy = cell % inner - (k - 1); dz = cell / inner - (k - 1);
+          x0 = x1 = (u2 & 1) ? cx + k : cx - k;
+        }
+        d_nn_scan_row(sp, valid_map, mode, g, tab, ucell_start, U, nf, x0, x1, cy + dy, cz + dz, c, best, bi);
+      }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      float ob = __shfl_xor_sync(FULL, best, o);
+      int oi = __shfl_xor_sync(FULL, bi, o);
+      if (ob < best || (ob == best && oi < bi)) { best = ob; bi = oi; }
+    }
+    // every unexplored cell is at Chebyshev distance >= k+1 from the query cell, hence every
+    // point in it is at least k*cell away from the query
+    double lim = (double)k * (double)g.cell * 0.999;
+    if (bi != 0x7FFFFFFF && (double)best <= lim * lim) break;
+  }
+}
+
+// Ring 1 of a centroid whose own cell is occupied (nearly all of them) reuses that cell's runs from the normals stage.  A
+// group of NN_GROUP lanes takes one centroid (32 / NN_GROUP in flight per warp): the runs' lengths are turned into
+// offsets of one flat candidate range by a group scan, lane l takes the candidates l, l + NN_GROUP, ... of it (slices
+// cross run boundaries freely: the (d2, index) minimum does not depend on how the candidates are split), NN_BATCH of
+// them loaded together, then a group minimum.  Centroids in an empty cell, and those whose ring-1 best is not provably
+// the nearest, go on one at a time with the whole warp (d_nn_rings).
+constexpr int NN_GROUP = 8;
+constexpr int NN_BATCH = 4;
+
 __global__ void __launch_bounds__(NN_BLOCK)
 k_voxel_nn(const float4* __restrict__ centroids, const float4* __restrict__ sp,
            const BlockEntry* __restrict__ tab, const int* __restrict__ ucell_start, const int2* __restrict__ runs, const int2* __restrict__ cell_info,
            const int* __restrict__ valid_map, const float4* __restrict__ normals_c, GridSpec g,
            int mode, DevState* st, int* __restrict__ nn_idx, float4* __restrict__ nn_normal) {
+  constexpr int G = NN_GROUP, PER_WARP = 32 / G;
+  __shared__ int2 s_run[NN_BLOCK / G][GRID_RUNS];  // per group and run of the cell: {run start - flat offset, flat end}
   const int V = st->vox.n_voxels, U = st->n_cells, nf = st->n_sorted_finite, nvalid = st->n_valid;
-  const int lane = threadIdx.x & 31;
+  const int lane = threadIdx.x & 31, gl = lane & (G - 1);
+  const unsigned gmask = ((1u << G) - 1u) << (lane & ~(G - 1));
+  int2* const sr = s_run[threadIdx.x / G];
+  const int kmax = max(g.dim[0], max(g.dim[1], g.dim[2]));
+  const double lim1 = (double)g.cell * 0.999;  // the ring-1 stop of d_nn_rings
   const int warps_total = (gridDim.x * NN_BLOCK) >> 5;
-  for (int j = (blockIdx.x * NN_BLOCK + threadIdx.x) >> 5; j < V; j += warps_total) {
-    const float4 c = centroids[j];
-    int cx, cy, cz;
-    gm_cell_of(g, c.x, c.y, c.z, cx, cy, cz);
+  for (int j0 = ((blockIdx.x * NN_BLOCK + threadIdx.x) >> 5) * PER_WARP; j0 < V; j0 += warps_total * PER_WARP) {  // warp-uniform
+    const int j = j0 + lane / G;
+    const bool live = j < V;
+    float4 c = make_float4(0.f, 0.f, 0.f, 0.f);
+    int cx = 0, cy = 0, cz = 0, k0 = kmax + 1;  // k0: the first ring the warp still has to search
     float best = CUDART_INF_F;
     int bi = 0x7FFFFFFF;
-    const int kmax = max(g.dim[0], max(g.dim[1], g.dim[2]));
-    for (int k = 1; k <= kmax; ++k) {
-      if (k == 1) {
-        // the 27-cell cube as 9 rows of 3 cells; if the centroid's own cell is occupied (the usual
-        // case) its runs were already computed for the normals stage: one search instead of 18
-        const unsigned ckey = gm_cell_key(g, cx, cy, cz);
-        const BlockEntry e = tab[ckey >> 6];
-        if ((e.mask >> (ckey & 63u)) & 1ull) {
-          const int jc = e.first + __popcll(e.mask & ((1ull << (ckey & 63u)) - 1ull));
-          // 16 runs at a time, each split in two halves over lanes l and l+16: twice the active lanes and half
-          // the longest sequential scan (the (d2, index) minimum does not depend on how the candidates are split)
-          const int nr = cell_info[jc].x;
-          for (int r0 = 0; r0 < nr; r0 += 16) {
-            const int r = r0 + (lane & 15);
-            if (r < nr) {
-              const int2 run = runs[(size_t)jc * GRID_RUNS + r];
-              const int mid = run.x + ((run.y - run.x + 1) >> 1);
-              d_nn_scan(sp, valid_map, mode, (lane < 16) ? make_int2(run.x, mid) : make_int2(mid, run.y), c, best, bi);
+    if (live) {
+      c = centroids[j];
+      gm_cell_of(g, c.x, c.y, c.z, cx, cy, cz);
+      const unsigned ckey = gm_cell_key(g, cx, cy, cz);
+      const BlockEntry e = tab[ckey >> 6];
+      if ((e.mask >> (ckey & 63u)) & 1ull) {
+        const int jc = e.first + __popcll(e.mask & ((1ull << (ckey & 63u)) - 1ull));
+        // the cell's run slots are loaded together with its run count (slots past the count hold stale values and are
+        // masked off): one dependent load less on the way to the candidates
+        constexpr int SLOTS = (GRID_RUNS + G - 1) / G;
+        const int2* const rp = runs + (size_t)jc * GRID_RUNS;
+        int2 run[SLOTS];
+#pragma unroll
+        for (int i = 0; i < SLOTS; ++i) run[i] = (i * G + gl < GRID_RUNS) ? __ldg(rp + i * G + gl) : make_int2(0, 0);
+        const int2 info = cell_info[jc];  // number of runs, number of candidates
+        int carry = 0;
+#pragma unroll
+        for (int i = 0; i < SLOTS; ++i) {
+          const int r = i * G + gl;
+          const int len = (r < info.x) ? run[i].y - run[i].x : 0;
+          int incl = len;
+#pragma unroll
+          for (int o = 1; o < G; o <<= 1) {
+            const int t = __shfl_up_sync(gmask, incl, o, G);
+            if (gl >= o) incl += t;
+          }
+          if (r < info.x) sr[r] = make_int2(run[i].x - (carry + incl - len), carry + incl);
+          carry += __shfl_sync(gmask, incl, G - 1, G);
+        }
+        __syncwarp(gmask);
+        int k = 0;
+        int2 cur = sr[0];
+        for (int f0 = 0; f0 < info.y; f0 += G * NN_BATCH) {
+          int pos[NN_BATCH];
+#pragma unroll
+          for (int u = 0; u < NN_BATCH; ++u) {
+            const int f = f0 + u * G + gl;
+            pos[u] = -1;
+            if (f < info.y) {
+              while (f >= cur.y) cur = sr[++k];
+              pos[u] = f + cur.x;
             }
           }
-        } else if (lane < 9) {
-          d_nn_scan_row(sp, valid_map, mode, g, tab, ucell_start, U, nf, cx - 1, cx + 1, cy + (lane % 3) - 1, cz + (lane / 3) - 1, c, best, bi);
-        }
-      } else {
-        // shell k: 8k perimeter rows with the full x span + (2k-1)^2 inner rows with two end cells
-        const int inner = 2 * k - 1, T = 8 * k + 2 * inner * inner;
-        for (int t = lane; t < T; t += 32) {
-          int dy, dz, x0, x1;
-          if (t < 8 * k) {
-            if (t < 2 * k + 1) { dz = -k; dy = t - k; }
-            else if (t < 4 * k + 2) { dz = k; dy = t - (2 * k + 1) - k; }
-            else if (t < 6 * k + 1) { dy = -k; dz = t - (4 * k + 2) - (k - 1); }
-            else { dy = k; dz = t - (6 * k + 1) - (k - 1); }
-            x0 = cx - k; x1 = cx + k;
-          } else {
-            int u2 = t - 8 * k, cell = u2 >> 1;
-            dy = cell % inner - (k - 1); dz = cell / inner - (k - 1);
-            x0 = x1 = (u2 & 1) ? cx + k : cx - k;
-          }
-          d_nn_scan_row(sp, valid_map, mode, g, tab, ucell_start, U, nf, x0, x1, cy + dy, cz + dz, c, best, bi);
-        }
-      }
-      // lexicographic (d2, index) minimum over the warp
+          float4 q[NN_BATCH];
+          int id[NN_BATCH];
 #pragma unroll
-      for (int o = 16; o > 0; o >>= 1) {
-        float ob = __shfl_xor_sync(FULL, best, o);
-        int oi = __shfl_xor_sync(FULL, bi, o);
-        if (ob < best || (ob == best && oi < bi)) { best = ob; bi = oi; }
+          for (int u = 0; u < NN_BATCH; ++u) {
+            q[u] = (pos[u] >= 0) ? __ldg(sp + pos[u]) : make_float4(0.f, 0.f, 0.f, 0.f);
+            id[u] = __float_as_int(q[u].w);
+          }
+          if (mode == 1) {
+#pragma unroll
+            for (int u = 0; u < NN_BATCH; ++u) id[u] = (pos[u] >= 0) ? __ldg(valid_map + id[u]) : -1;
+          }
+#pragma unroll
+          for (int u = 0; u < NN_BATCH; ++u) {
+            if (pos[u] < 0 || id[u] < 0) continue;
+            float dx = c.x - q[u].x, dy = c.y - q[u].y, dz = c.z - q[u].z;
+            float d2 = (dx * dx + dy * dy) + dz * dz;
+            if (d2 < best || (d2 == best && id[u] < bi)) { best = d2; bi = id[u]; }
+          }
+        }
+#pragma unroll
+        for (int o = G / 2; o > 0; o >>= 1) {
+          float ob = __shfl_xor_sync(gmask, best, o, G);
+          int oi = __shfl_xor_sync(gmask, bi, o, G);
+          if (ob < best || (ob == best && oi < bi)) { best = ob; bi = oi; }
+        }
+        if (!(bi != 0x7FFFFFFF && (double)best <= lim1 * lim1)) k0 = 2;
+        __syncwarp(gmask);  // s_run is rewritten by the group's next centroid
+      } else {
+        k0 = 1;
       }
-      // every unexplored cell is at Chebyshev distance >= k+1 from the query cell, hence every
-      // point in it is at least k*cell away from the query
-      double lim = (double)k * (double)g.cell * 0.999;
-      if (bi != 0x7FFFFFFF && (double)best <= lim * lim) break;
     }
-    if (lane == 0) {
+    unsigned todo = __ballot_sync(FULL, gl == 0 && k0 <= kmax);
+    while (todo) {
+      const int src = __ffs(todo) - 1;
+      todo &= todo - 1;
+      const float4 cc = make_float4(__shfl_sync(FULL, c.x, src), __shfl_sync(FULL, c.y, src), __shfl_sync(FULL, c.z, src), 0.f);
+      float b = __shfl_sync(FULL, best, src);
+      int bb = __shfl_sync(FULL, bi, src);
+      d_nn_rings(sp, valid_map, mode, g, tab, ucell_start, U, nf, cc, __shfl_sync(FULL, cx, src), __shfl_sync(FULL, cy, src),
+                 __shfl_sync(FULL, cz, src), __shfl_sync(FULL, k0, src), kmax, b, bb);
+      if (lane == src) { best = b; bi = bb; }
+    }
+    if (live && gl == 0) {
       if (bi == 0x7FFFFFFF) bi = -1;
       nn_idx[j] = bi;
       const float qnan = CUDART_NAN_F;
