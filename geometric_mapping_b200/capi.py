@@ -171,6 +171,7 @@ SYMBOLS = [
     "gm_download_compressed_primitives", "gm_icp_params_default", "gm_register", "gm_get_registration",
     "gm_download_correspondences", "gm_register_map", "gm_download_map_correspondences", "gm_map_download_planes",
     "gm_odometry_params_default", "gm_odometry_create", "gm_odometry_destroy", "gm_odometry_step", "gm_odometry_steps", "gm_odometry_get",
+    "gm_map_evict", "gm_map_merge", "gm_odometry_set_window",
     "gm_encode_marker_array", "gm_store_open", "gm_store_close", "gm_store_append", "gm_store_append_blob", "gm_store_count", "gm_store_info", "gm_store_read",
 ]
 
@@ -310,6 +311,9 @@ def _lib():
         "gm_odometry_step": (i32, [vp, vp, vp]),
         "gm_odometry_steps": (i32, [vp]),
         "gm_odometry_get": (i32, [vp, vp, i32, C.POINTER(i32)]),
+        "gm_map_evict": (i32, [vp, vp, vp, vp, i32]),
+        "gm_map_merge": (i32, [vp, vp]),
+        "gm_odometry_set_window": (i32, [vp, i32, vp]),
     }
     assert set(sig) == set(SYMBOLS)
     for name, (res, args) in sig.items():
@@ -942,6 +946,18 @@ class VoxelMap:
                  "gm_map_download_planes")
         return out
 
+    def evict(self, ctx: "Context", center, half_cells: int, archive: "VoxelMap | None" = None):
+        """Keep the voxels whose cell is within half_cells (Chebyshev, in cells) of center's cell; move the others into
+        `archive` (None = drop them).  Asynchronous on ctx's stream (include/gm_capi.h, gm_map_evict)."""
+        c = np.ascontiguousarray(np.asarray(center, np.float32).reshape(3))
+        ctx._ck(_lib().gm_map_evict(self._h, ctx._h, archive._h if archive is not None else None, _ptr(c), int(half_cells)),
+                "gm_map_evict")
+
+    def merge(self, src: "VoxelMap") -> bool:
+        """self += src (gm_map_merge; synchronises the device).  -> full: this map found its table full and dropped voxels."""
+        st = self._ck(_lib().gm_map_merge(self._h, src._h), "gm_map_merge", ok=(GM_OK, GM_ERR_CAPACITY))
+        return st == GM_ERR_CAPACITY
+
     def clear(self):
         self._ck(_lib().gm_map_clear(self._h), "gm_map_clear")
 
@@ -998,6 +1014,14 @@ class Odometry:
         frame, None = constant velocity."""
         d = None if delta34 is None else np.ascontiguousarray(np.asarray(delta34, np.float32)[:3, :4].reshape(12))
         ctx._ck(_lib().gm_odometry_step(self._h, ctx._h, _ptr(d)), "gm_odometry_step")
+
+    def set_window(self, half_cells: int, archive: VoxelMap | None = None):
+        """From the next step on, end each step by evicting the map's voxels outside half_cells cells of the step's pose
+        into `archive` (None = drop them); 0 = no window (include/gm_capi.h, gm_odometry_set_window)."""
+        st = _lib().gm_odometry_set_window(self._h, int(half_cells), archive._h if archive is not None else None)
+        if st != GM_OK:
+            raise GmError(st, "gm_odometry_set_window")
+        self.archive = archive                                   # the archive must outlive the odometry
 
     @property
     def steps(self) -> int:

@@ -2492,6 +2492,11 @@ struct gm_map {
   // per-slot plane tables of k_map_planes (allocated by the first use): centroid + has-plane flag, normal
   DevBuf<float4> d_plane_cent, d_plane_nrm;
   DevBuf<int> d_plane_box;  // [8] cells of the voxels with a plane: min x, y, z, -, -max x, y, z, - (k_map_planes)
+  // gm_map_evict's scratch (allocated by the first eviction): the kept voxels, n_slots entries, and the split's counters
+  DevBuf<unsigned long long> d_kept_keys;
+  DevBuf<int> d_kept_cnt;
+  DevBuf<long long> d_kept_sums;
+  DevBuf<MapEvictState> d_evict_st;
   std::string err;
   ~gm_map() { if (ev_last) cudaEventDestroy(ev_last); }
 };
@@ -2534,6 +2539,39 @@ gm_status map_dump(gm_map* m, MapDump* out, MapState* st_out) {
     out->keys[i] = k[j]; out->cnt[i] = c[j];
     for (int a = 0; a < 3; ++a) out->sums[3 * i + a] = su[3 * j + a];
   }
+  return GM_OK;
+}
+
+int map_blocks(const gm_map* m) { return (int)std::min<unsigned long long>((m->n_slots + 255) / 256, (unsigned long long)m->num_sms * 16); }
+
+// the leaf and device rules of gm_map_evict / gm_map_merge / gm_odometry_set_window: the same lattice, the same device
+bool same_lattice(const gm_map* a, const gm_map* b) {
+  return a->device == b->device && std::memcmp(&a->leaf, &b->leaf, sizeof(double)) == 0;
+}
+
+cudaError_t ensure_evict_buffers(gm_map* m) {
+  if (m->d_evict_st.count) return cudaSuccess;
+  cudaError_t e = m->d_kept_keys.alloc(m->n_slots);
+  if (e == cudaSuccess) e = m->d_kept_cnt.alloc(m->n_slots);
+  if (e == cudaSuccess) e = m->d_kept_sums.alloc(3 * m->n_slots);
+  if (e == cudaSuccess) e = m->d_evict_st.alloc(1);  // last: a failure above leaves the set unallocated
+  return e;
+}
+
+// The launches of gm_map_evict on ctx's stream, after its checks and waits (buffers allocated): the counters' reset, then
+// k_map_evict_split, k_map_evict_clear and k_map_evict_restore.  Centre = c3 (host), or the translation of the device pose
+// pose34_dev.  Shared by gm_map_evict and gm_odometry_step.
+gm_status map_evict_launch(gm_map* m, gm_ctx* ctx, gm_map* archive, const float* c3, const float* pose34_dev, int half_cells) {
+  GM_CUDA(cudaMemsetAsync(m->d_evict_st, 0, sizeof(MapEvictState), ctx->stream));
+  const float cx = c3 ? c3[0] : 0.f, cy = c3 ? c3[1] : 0.f, cz = c3 ? c3[2] : 0.f;
+  GM_LAUNCH(ctx, k_map_evict_split, map_blocks(m), 256, m->d_keys, m->d_cnt, m->d_sums, m->n_slots - 1ull, m->inv_leaf, cx, cy, cz, pose34_dev,
+            half_cells, archive ? (unsigned long long*)archive->d_keys : nullptr, archive ? (int*)archive->d_cnt : nullptr,
+            archive ? (long long*)archive->d_sums : nullptr, archive ? archive->n_slots - 1ull : 0ull, archive ? (MapState*)archive->d_st : nullptr,
+            m->d_kept_keys, m->d_kept_cnt, m->d_kept_sums, m->d_evict_st);
+  GM_LAUNCH(ctx, k_map_evict_clear, map_blocks(m), 256, m->d_keys, m->d_cnt, m->d_sums, m->n_slots, m->d_evict_st, m->d_st);
+  GM_LAUNCH(ctx, k_map_evict_restore, map_blocks(m), 256, m->d_kept_keys, m->d_kept_cnt, m->d_kept_sums, m->d_evict_st, m->d_keys, m->d_cnt,
+            m->d_sums, m->n_slots - 1ull, m->d_st);
+  GM_CHECK_LAUNCHES(ctx);
   return GM_OK;
 }
 }  // namespace
@@ -2689,6 +2727,39 @@ gm_status gm_map_load(const char* path, size_t min_capacity_voxels, gm_map** out
 
 double gm_map_leaf(const gm_map* m) { return m ? m->leaf : 0.0; }
 
+gm_status gm_map_evict(gm_map* m, gm_ctx* ctx, gm_map* archive, const float* center3, int32_t half_cells) {
+  if (!m || !ctx || !center3 || half_cells < 0 || archive == m) return GM_ERR_INVALID_ARG;
+  if (ctx->device != m->device) { ctx->err = "gm_map_evict: context and map on different devices"; return GM_ERR_INVALID_ARG; }
+  if (archive && !same_lattice(m, archive)) { ctx->err = "gm_map_evict: archive on another device or with another leaf"; return GM_ERR_INVALID_ARG; }
+  long long cell[3];
+  if (!map_center_cell(center3, m->inv_leaf, cell)) { ctx->err = "gm_map_evict: centre not finite or outside the key range"; return GM_ERR_INVALID_ARG; }
+  GM_CUDA(ensure_evict_buffers(m));
+  GM_CUDA(cudaStreamWaitEvent(ctx->stream, m->ev_last, 0));
+  if (archive) GM_CUDA(cudaStreamWaitEvent(ctx->stream, archive->ev_last, 0));
+  if (gm_status s = map_evict_launch(m, ctx, archive, center3, nullptr, half_cells)) return s;
+  GM_CUDA(cudaEventRecord(m->ev_last, ctx->stream));
+  if (archive) GM_CUDA(cudaEventRecord(archive->ev_last, ctx->stream));
+  return GM_OK;
+}
+
+gm_status gm_map_merge(gm_map* dst, const gm_map* src) {
+  if (!dst || !src || dst == src || !same_lattice(dst, src)) return GM_ERR_INVALID_ARG;
+  int prev = 0;
+  if (cudaGetDevice(&prev) != cudaSuccess || cudaSetDevice(dst->device) != cudaSuccess) { cudaGetLastError(); return GM_ERR_CUDA; }
+  cudaError_t e = cudaDeviceSynchronize();
+  if (e == cudaSuccess) {
+    k_map_merge<<<map_blocks(src), 256>>>(src->d_keys, src->d_cnt, src->d_sums, src->n_slots, dst->d_keys, dst->d_cnt, dst->d_sums,
+                                          dst->n_slots - 1ull, dst->d_st);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaDeviceSynchronize();
+  MapState st{};
+  if (e == cudaSuccess) e = cudaMemcpy(&st, dst->d_st, sizeof(st), cudaMemcpyDeviceToHost);
+  cudaSetDevice(prev);
+  if (e != cudaSuccess) { dst->err = cudaGetErrorString(e); return GM_ERR_CUDA; }
+  return st.overflow ? GM_ERR_CAPACITY : GM_OK;
+}
+
 }  // extern "C"
 
 // ---- scan-to-map registration (gm_register.cuh, k_map_planes in gm_map.cuh) ------------------------------------------
@@ -2702,8 +2773,6 @@ cudaError_t ensure_plane_tables(gm_map* m) {
   if (e == cudaSuccess) e = m->d_plane_cent.alloc(m->n_slots);  // last: a failure above leaves the pair unallocated
   return e;
 }
-
-int map_blocks(const gm_map* m) { return (int)std::min<unsigned long long>((m->n_slots + 255) / 256, (unsigned long long)m->num_sms * 16); }
 
 // gm_register_map's argument rules (gm_odometry_create checks its icp by them too)
 bool valid_regmap_args(const gm_icp_params* p, double max_planarity) {
@@ -2840,6 +2909,8 @@ struct gm_odometry {
   DevBuf<OdomRecord> d_rec;          // the trajectory, max_steps records
   DevBuf<OdomInsert> d_ins;          // pose and flag of the current step's insert
   cudaStream_t stream = nullptr;     // the trajectory download
+  int32_t window = 0;                // gm_odometry_set_window: half_cells of the local map's window, 0 = off
+  gm_map* archive = nullptr;         // where the window evicts to (null: dropped)
   ~gm_odometry() { if (stream) cudaStreamDestroy(stream); }
 };
 
@@ -2895,7 +2966,10 @@ gm_status gm_odometry_step(gm_odometry* odo, gm_ctx* ctx, const float* delta34) 
   const bool registered = k > 0 || odo->p.register_first;
   if (registered)
     if (gm_status s = regmap_buffers(ctx, map)) return s;
+  gm_map* archive = odo->window > 0 ? odo->archive : nullptr;
+  if (odo->window > 0) GM_CUDA(ensure_evict_buffers(map));
   GM_CUDA(cudaStreamWaitEvent(ctx->stream, map->ev_last, 0));
+  if (archive) GM_CUDA(cudaStreamWaitEvent(ctx->stream, archive->ev_last, 0));
   Pose34 init{}, delta{};
   int mode = ODOM_INIT;
   if (k == 0) {
@@ -2921,8 +2995,20 @@ gm_status gm_odometry_step(gm_odometry* odo, gm_ctx* ctx, const float* delta34) 
   GM_LAUNCH(ctx, k_map_insert_gated, blocks, 256, ctx->d_cloud_c, &ctx->d_st->n_valid, &odo->d_ins->pose, &odo->d_ins->accept, map->inv_leaf,
             map->d_keys, map->d_cnt, map->d_sums, map->n_slots - 1ull, map->d_st);
   GM_CHECK_LAUNCHES(ctx);
+  // the window: gm_map_evict's launches, centred on the translation of the pose record k holds
+  if (odo->window > 0)
+    if (gm_status s = map_evict_launch(map, ctx, archive, nullptr, odo->d_rec[k].pose34, odo->window)) return s;
   GM_CUDA(cudaEventRecord(map->ev_last, ctx->stream));
+  if (archive) GM_CUDA(cudaEventRecord(archive->ev_last, ctx->stream));
   odo->steps = k + 1;
+  return GM_OK;
+}
+
+gm_status gm_odometry_set_window(gm_odometry* odo, int32_t half_cells, gm_map* archive) {
+  if (!odo || half_cells < 0) return GM_ERR_INVALID_ARG;
+  if (archive && (archive == odo->map || !same_lattice(odo->map, archive))) return GM_ERR_INVALID_ARG;
+  odo->window = half_cells;
+  odo->archive = archive;
   return GM_OK;
 }
 

@@ -99,25 +99,128 @@ __global__ void k_map_insert_gated(const float4* __restrict__ pts, const int* __
   d_map_insert(pts, nullptr, *n_ptr, -1, T, 1, inv_leaf, keys, cnt, sums, slot_mask, st);
 }
 
+// Add one voxel (key, count, fixed-point sums s3[0..3)) to the table: the entry of `key`, created if absent, gets the
+// count and the sums added as integers.  A full table drops the voxel and raises overflow.  Shared by gm_map_load,
+// gm_map_evict (the archive, and the kept voxels' re-insertion) and gm_map_merge, so all of them add alike.
+__device__ __forceinline__ void d_map_add(unsigned long long key, int c, const long long* __restrict__ s3, unsigned long long* __restrict__ keys,
+                                          int* __restrict__ cnt, long long* __restrict__ sums, unsigned long long slot_mask, MapState* st) {
+  unsigned long long slot = map_hash(key) & slot_mask;
+  bool placed = false;
+  for (unsigned long long probe = 0; probe <= slot_mask; ++probe) {
+    unsigned long long prev = atomicCAS(&keys[slot], MAP_EMPTY, key);
+    if (prev == MAP_EMPTY) { atomicAdd(&st->n_voxels, 1); prev = key; }
+    if (prev == key) { placed = true; break; }
+    slot = (slot + 1) & slot_mask;
+  }
+  if (!placed) { atomicExch(&st->overflow, 1); return; }
+  atomicAdd(&cnt[slot], c);
+  for (int a = 0; a < 3; ++a) atomicAdd(reinterpret_cast<unsigned long long*>(sums) + 3 * slot + a, (unsigned long long)s3[a]);
+  atomicAdd(&st->n_points, (unsigned long long)c);
+}
+
 // Raw re-insertion of saved voxels (gm_map_load): key, count and fixed-point sums as stored.
 __global__ void k_map_restore(const unsigned long long* __restrict__ in_keys, const int* __restrict__ in_cnt,
                               const long long* __restrict__ in_sums, int n, unsigned long long* __restrict__ keys,
                               int* __restrict__ cnt, long long* __restrict__ sums, unsigned long long slot_mask, MapState* st) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const unsigned long long key = in_keys[i];
-    unsigned long long slot = map_hash(key) & slot_mask;
-    bool placed = false;
-    for (unsigned long long probe = 0; probe <= slot_mask; ++probe) {
-      unsigned long long prev = atomicCAS(&keys[slot], MAP_EMPTY, key);
-      if (prev == MAP_EMPTY) { atomicAdd(&st->n_voxels, 1); prev = key; }
-      if (prev == key) { placed = true; break; }
-      slot = (slot + 1) & slot_mask;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+    d_map_add(in_keys[i], in_cnt[i], in_sums + 3 * (size_t)i, keys, cnt, sums, slot_mask, st);
+}
+
+// ---- window eviction (gm_map_evict) and merge (gm_map_merge) ----------------------------------------------------------
+// Linear probing has no parallel delete, so an eviction rebuilds the table: k_map_evict_split adds the evicted voxels to
+// the archive and compacts the kept ones into the map's scratch arrays, k_map_evict_clear empties the table and
+// k_map_evict_restore re-adds the kept voxels.  The last two return at once when nothing was evicted.
+
+struct MapEvictState { int n_kept; int evicted; };  // zeroed before every eviction
+
+// The window's centre cell, c[a] = (int)floorf(center[a] * inv_leaf) as d_map_insert computes a point's cell.  false for a
+// non-finite centre or a cell outside the key range.  Host and device evaluate the same float product and floorf.
+__host__ __device__ __forceinline__ bool map_center_cell(const float c3[3], float inv_leaf, long long cell[3]) {
+  for (int a = 0; a < 3; ++a) {
+    const float f = floorf(c3[a] * inv_leaf);
+    if (!(fabsf(f) < 2.0e6f)) return false;  // NaN and infinities too
+    cell[a] = (long long)(int)f;
+    if (cell[a] < -MAP_COORD_OFF || cell[a] >= MAP_COORD_OFF) return false;
+  }
+  return true;
+}
+
+// One thread per slot.  Centre = (cx, cy, cz), or the translation (pose34[3], pose34[7], pose34[11]) of a device pose when
+// pose34 is not null (gm_odometry_step: the step's recorded pose); a centre map_center_cell refuses evicts nothing.  A voxel
+// is kept iff max_a |cell_a - c_a| <= half_cells (64-bit integers).  Kept voxels go to out_* in any order (warp-aggregated
+// cursor es->n_kept); evicted ones are added to the archive (a_keys null: dropped) and set es->evicted.  Every lane of a warp
+// runs the same number of iterations (n_slots and the stride are multiples of 32), so the ballots see full warps.
+__global__ void k_map_evict_split(const unsigned long long* __restrict__ keys, const int* __restrict__ cnt, const long long* __restrict__ sums,
+                                  unsigned long long slot_mask, float inv_leaf, float cx, float cy, float cz, const float* __restrict__ pose34,
+                                  int half_cells, unsigned long long* __restrict__ a_keys, int* __restrict__ a_cnt, long long* __restrict__ a_sums,
+                                  unsigned long long a_mask, MapState* a_st, unsigned long long* __restrict__ out_keys, int* __restrict__ out_cnt,
+                                  long long* __restrict__ out_sums, MapEvictState* es) {
+  float c3[3] = {cx, cy, cz};
+  if (pose34) { c3[0] = pose34[3]; c3[1] = pose34[7]; c3[2] = pose34[11]; }
+  long long c[3];
+  if (!map_center_cell(c3, inv_leaf, c)) return;
+  const int lane = threadIdx.x & 31;
+  bool gone_any = false;
+  for (unsigned long long s = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; s <= slot_mask;
+       s += (unsigned long long)gridDim.x * blockDim.x) {
+    const unsigned long long key = keys[s];
+    bool kept = false, gone = false;
+    if (key != MAP_EMPTY) {
+      int ix, iy, iz;
+      map_unpack(key, ix, iy, iz);
+      const long long d = max(llabs((long long)ix - c[0]), max(llabs((long long)iy - c[1]), llabs((long long)iz - c[2])));
+      kept = d <= (long long)half_cells;
+      gone = !kept;
     }
-    if (!placed) { atomicExch(&st->overflow, 1); continue; }
-    atomicAdd(&cnt[slot], in_cnt[i]);
-    for (int a = 0; a < 3; ++a)
-      atomicAdd(reinterpret_cast<unsigned long long*>(sums) + 3 * slot + a, (unsigned long long)in_sums[3 * (size_t)i + a]);
-    atomicAdd(&st->n_points, (unsigned long long)in_cnt[i]);
+    const unsigned m = __ballot_sync(0xFFFFFFFFu, kept);
+    int base = 0;
+    if (lane == 0 && m) base = atomicAdd(&es->n_kept, __popc(m));
+    base = __shfl_sync(0xFFFFFFFFu, base, 0);
+    if (kept) {
+      const int o = base + __popc(m & ((1u << lane) - 1u));
+      out_keys[o] = key;
+      out_cnt[o] = cnt[s];
+      for (int a = 0; a < 3; ++a) out_sums[3 * (size_t)o + a] = sums[3 * s + a];
+    }
+    if (gone) {
+      gone_any = true;
+      if (a_keys) d_map_add(key, cnt[s], sums + 3 * s, a_keys, a_cnt, a_sums, a_mask, a_st);
+    }
+  }
+  if (__any_sync(0xFFFFFFFFu, gone_any) && lane == 0) es->evicted = 1;
+}
+
+// Empty every slot and zero n_voxels and n_points (overflow and out_of_range stay), if anything was evicted.
+__global__ void k_map_evict_clear(unsigned long long* __restrict__ keys, int* __restrict__ cnt, long long* __restrict__ sums,
+                                  unsigned long long n_slots, const MapEvictState* __restrict__ es, MapState* st) {
+  if (!es->evicted) return;
+  if (blockIdx.x == 0 && threadIdx.x == 0) { st->n_voxels = 0; st->n_points = 0ull; }
+  for (unsigned long long s = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; s < n_slots; s += (unsigned long long)gridDim.x * blockDim.x) {
+    keys[s] = MAP_EMPTY;
+    cnt[s] = 0;
+  }
+  for (unsigned long long s = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; s < 3 * n_slots; s += (unsigned long long)gridDim.x * blockDim.x)
+    sums[s] = 0;
+}
+
+// Re-add the kept voxels to the emptied table (and so recount n_voxels and n_points), if anything was evicted.  They are
+// at most the voxels the table held, so they all fit.
+__global__ void k_map_evict_restore(const unsigned long long* __restrict__ in_keys, const int* __restrict__ in_cnt,
+                                    const long long* __restrict__ in_sums, const MapEvictState* __restrict__ es, unsigned long long* __restrict__ keys,
+                                    int* __restrict__ cnt, long long* __restrict__ sums, unsigned long long slot_mask, MapState* st) {
+  if (!es->evicted) return;
+  const int n = es->n_kept;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+    d_map_add(in_keys[i], in_cnt[i], in_sums + 3 * (size_t)i, keys, cnt, sums, slot_mask, st);
+}
+
+// dst += src: every occupied slot of src added to dst (gm_map_merge).
+__global__ void k_map_merge(const unsigned long long* __restrict__ s_keys, const int* __restrict__ s_cnt, const long long* __restrict__ s_sums,
+                            unsigned long long s_slots, unsigned long long* __restrict__ keys, int* __restrict__ cnt, long long* __restrict__ sums,
+                            unsigned long long slot_mask, MapState* st) {
+  for (unsigned long long s = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; s < s_slots; s += (unsigned long long)gridDim.x * blockDim.x) {
+    const unsigned long long key = s_keys[s];
+    if (key != MAP_EMPTY) d_map_add(key, s_cnt[s], s_sums + 3 * s, keys, cnt, sums, slot_mask, st);
   }
 }
 

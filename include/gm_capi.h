@@ -527,6 +527,37 @@ GM_API gm_status gm_map_download(gm_map* map, int32_t* ijk, int32_t* counts, flo
 GM_API gm_status gm_map_save(gm_map* map, const char* path);
 GM_API gm_status gm_map_load(const char* path, size_t min_capacity_voxels, gm_map** out);
 GM_API double gm_map_leaf(const gm_map* map);
+/* ---- a window on a map: eviction into an archive, and the exact way back ---------------------------------------------
+ * gm_map_evict keeps the voxels of `map` inside a cube of cells around center3 and moves the others into `archive`
+ * (NULL = drops them), so that a long run can work in a local map sized to what the sensor sees.
+ *   Centre cell.  c[a] = (int)floorf(center3[a] * inv_leaf), the float product of gm_map_insert's cell (inv_leaf = 1 / (float)leaf).
+ *   Kept.  A voxel of cell (i, j, k) is kept iff max(|i - c0|, |j - c1|, |k - c2|) <= half_cells, in 64-bit integers: a
+ *     Chebyshev cube of 2 half_cells + 1 cells a side, with no float test.
+ *   After the call the map holds exactly the kept voxels with their counts and sums unchanged (no tombstones); n_voxels and
+ *     n_points of gm_map_stats describe them, and overflow and out_of_range (records of earlier inserts) stay as they were
+ *     until gm_map_clear.  Each evicted voxel's count and sums are added as integers to the archive's entry of the same key,
+ *     created if absent (gm_map_load's add).  An archive that is full drops the voxels that do not fit, and its gm_map_stats
+ *     then gives GM_ERR_CAPACITY.  Counts and sums are integers, so the adds are exact: gm_map_merge(archive, map) after
+ *     any number of evictions gives back, bit for bit, the map that was never evicted.
+ *   Ordering.  Asynchronous on ctx's stream; ctx only supplies the stream and the launch count.  It is a map operation on
+ *     both maps: it waits for the previous gm_map_insert / gm_register_map / gm_odometry_step / gm_map_evict on the map and on
+ *     the archive, and the next operation on either waits for it.
+ *   Launches.  GM_MAP_EVICT_LAUNCHES kernels, always: the split (each voxel to the archive or to the map's scratch), then
+ *     the clear of the table and the re-insertion of the kept voxels, which return at once, reading it from device memory,
+ *     when nothing was evicted.  No host synchronisation; the first call allocates the map's scratch (36 bytes a slot).
+ *     The slot layout afterwards is not that of the original insertion, which changes no output: every read of a map is in
+ *     key order.
+ *   Errors.  GM_ERR_INVALID_ARG, with nothing launched, for half_cells < 0, a non-finite centre or a centre cell outside
+ *     the key range [-2^20, 2^20), archive == map, an archive whose leaf is not bitwise the map's, and a context or archive
+ *     on another device than the map.
+ * gm_map_merge adds every voxel of src into dst (dst += src by the same integer add; src is unchanged), in one kernel on
+ * the device, and synchronises the device as gm_map_clear and gm_map_load do.  The leaf and device rules are those of
+ * gm_map_evict, and dst != src.  GM_ERR_CAPACITY if dst overflowed (a voxel found it full and was dropped).  The whole map
+ * of a windowed run is gm_map_merge(archive, local) then gm_map_save(archive); an archive saved and cleared every so often
+ * gives GMM1 segment files whose key-wise sum is the same map. */
+#define GM_MAP_EVICT_LAUNCHES 3
+GM_API gm_status gm_map_evict(gm_map* map, gm_ctx* ctx, gm_map* archive, const float* center3, int32_t half_cells);
+GM_API gm_status gm_map_merge(gm_map* dst, const gm_map* src);  /* dst += src, src unchanged */
 
 /* ---- scan-to-map registration (builder-defined: the reference keeps no map) -------------------------------------------
  * gm_register with the aggregated voxel map as the target: localises a scan in the map being built, or in one reloaded
@@ -590,14 +621,30 @@ GM_API gm_status gm_map_download_planes(gm_map* map, double max_planarity, float
  *   Insert.  An accepted step inserts all of ctx's compacted points at pose34 = float(T) element by element (what
  *     gm_get_registration returns): the map gm_map_insert(map, ctx, pose34, -1) would give.  A rejected step inserts nothing
  *     and records the guess as its pose, so the next guesses dead-reckon across it; its ICP result stays readable through
- *     gm_get_registration.  The map has no removal: the gate is what keeps a failed registration out of it.
+ *     gm_get_registration.  The gate is what keeps a failed registration out of the map: nothing removes what was inserted
+ *     (a window, below, moves voxels to the archive but never drops a point unless its archive is NULL or full).
  *   Ordering.  A step is a map operation: it waits for the previous gm_map_insert / gm_register_map / gm_odometry_step on
  *     the map, whichever context issued it, and the next one waits for its insert.  There is no host synchronisation
  *     (the first registration of a context allocates its buffers once, as gm_register_map does).
  *   Launches.  A registered step launches k_odom_begin (the guess and the registration's start), k_map_planes,
  *     icp.max_iterations x k_regmap_iter, k_odom_gate and the insert: gm_launch_count(ctx) grows by max_iterations + 4.
  *     An unregistered step 0 launches k_odom_begin, k_odom_gate and the insert: + 3.  The insert is launched even for an
- *     empty scan (its kernel reads the point count on the device).
+ *     empty scan (its kernel reads the point count on the device).  With a window, add GM_MAP_EVICT_LAUNCHES to each:
+ *     max_iterations + 4 + GM_MAP_EVICT_LAUNCHES and 3 + GM_MAP_EVICT_LAUNCHES.
+ *   Window (gm_odometry_set_window; off by default).  With half_cells > 0, each step ends, after its insert, with exactly the
+ *     launches of gm_map_evict(map, ctx, archive, t, half_cells), t = (pose34[3], pose34[7], pose34[11]) of the step's own
+ *     record, read from device memory: still no host round trip.  A rejected step evicts around its guess (its recorded
+ *     pose); a centre gm_map_evict would refuse evicts nothing.  The step then also waits for and orders the archive as
+ *     gm_map_evict does.  The window may be set or changed between steps; half_cells = 0 turns it off.  Rules: half_cells
+ *     >= 0, and an archive (NULL = evicted voxels are dropped) must be another map of the same leaf on the map's device, or
+ *     GM_ERR_INVALID_ARG.  The archive must outlive the odometry.
+ *     Sizing.  With crop bound B (boxFilterBound), d_max = icp.max_correspondence_distance, and every ICP iterate of step
+ *     k + 1 within s metres of step k's pose,
+ *         half_cells >= floor((sqrt(3) * B + s + d_max) / leaf) + 2
+ *     keeps every voxel the next registration can match (a scan point lies within sqrt(3) B of its sensor, one cell for
+ *     the centre's rounding) and every neighbour its plane reads (one more cell), so the trajectory is the one without a
+ *     window.  The local map then needs capacity for the voxels of a cube of 2 half_cells + 1 cells around the sensor,
+ *     not for the run.
  *   Errors.  gm_odometry_create checks icp by gm_register_map's rules and 0 <= min_fitness <= 1, register_first in {0, 1},
  *     max_steps >= 1.  A step k >= max_steps gives GM_ERR_CAPACITY, a missing stage GM_ERR_STAGE_ORDER, a context on
  *     another device GM_ERR_INVALID_ARG: then nothing is launched and gm_odometry_steps does not move.
@@ -626,6 +673,7 @@ GM_API void gm_odometry_params_default(gm_odometry_params* p);
 GM_API gm_status gm_odometry_create(gm_map* map, const gm_odometry_params* p, gm_odometry** out);
 GM_API void gm_odometry_destroy(gm_odometry* odo);
 GM_API gm_status gm_odometry_step(gm_odometry* odo, gm_ctx* ctx, const float* delta34 /* NULL = constant velocity */);
+GM_API gm_status gm_odometry_set_window(gm_odometry* odo, int32_t half_cells /* 0 = off, the default */, gm_map* archive /* may be NULL */);
 GM_API int32_t gm_odometry_steps(const gm_odometry* odo);  /* steps issued so far (host counter, no synchronisation) */
 /* the records of every step issued so far, in step order; *n = their number.  Waits for the last of them.  out = NULL: *n only */
 GM_API gm_status gm_odometry_get(gm_odometry* odo, gm_odometry_record* out, int32_t capacity, int32_t* n);
