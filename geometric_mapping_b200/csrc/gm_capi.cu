@@ -18,6 +18,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <numeric>
 #include <string>
 
 using namespace gm;
@@ -1704,6 +1705,40 @@ bool finite_pose(const float* t) {
   for (int k = 0; k < 12; ++k) if (!std::isfinite(t[k])) return false;
   return true;
 }
+
+// gm_register's argument rules (gm_register_map adds its max_planarity's)
+bool valid_icp_args(const gm_icp_params* p) {
+  const double dmax = p->max_correspondence_distance;
+  return dmax > 0.0 && std::isfinite(dmax) && p->max_iterations >= 1 && p->max_iterations <= GM_MAX_ICP_ITERATIONS &&
+         p->min_rotation_step >= 0.0 && p->min_translation_step >= 0.0 && p->degeneracy_ratio >= 0.0 && p->degeneracy_ratio < 1.0 &&
+         finite_pose(p->init_pose34);
+}
+
+// The kernel parameters of an ICP of `source`, and the grid of its iterations: a warp per source voxel, at most
+// reg_blocks, at least one block (the kernels read the voxel count on the device).
+RegParams icp_setup(const gm_ctx* source, const gm_icp_params* p, int* blocks) {
+  *blocks = std::max(1, std::min(div_up((long long)source->n_grid * 32, REG_BLOCK), reg_blocks(source)));
+  const double dmax = p->max_correspondence_distance;
+  return RegParams{dmax, (float)(dmax * dmax), p->min_rotation_step, p->min_translation_step, p->degeneracy_ratio};
+}
+
+// The per-point outputs of ctx's last registration, whose target was a context (target 0) or a map (1): n_source of them,
+// GM_ERR_CAPACITY above capacity_points, else d_idx copied into *idx and, if not null, the residuals into residual.
+template <class T>
+gm_status download_reg_points(gm_ctx* ctx, int target, const T* d_idx, std::vector<T>* idx, float* residual, size_t capacity_points) {
+  if (gm_status s = require(ctx, REGISTRATION)) return s;
+  if (ctx->reg_target != target) return GM_ERR_STAGE_ORDER;  // the other of gm_download_correspondences / _map_correspondences
+  int V = 0;
+  GM_CUDA(cudaMemcpyAsync(&V, &ctx->d_reg_state->n_source, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  if ((size_t)V > capacity_points) return GM_ERR_CAPACITY;
+  if (V <= 0) return GM_OK;
+  idx->resize((size_t)V);
+  GM_CUDA(cudaMemcpyAsync(idx->data(), d_idx, (size_t)V * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream));
+  if (residual) GM_CUDA(cudaMemcpyAsync(residual, ctx->d_reg_res, (size_t)V * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  return GM_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -1723,11 +1758,7 @@ gm_status gm_register(gm_ctx* source, gm_ctx* target, const gm_icp_params* p) {
   if (!source || !target || !p) return GM_ERR_INVALID_ARG;
   gm_ctx* ctx = source;  // GM_CUDA / GM_LAUNCH report on the source
   if (source->device != target->device) { ctx->err = "gm_register: source and target on different devices"; return GM_ERR_INVALID_ARG; }
-  const double dmax = p->max_correspondence_distance;
-  if (!(dmax > 0.0) || !std::isfinite(dmax) || p->max_iterations < 1 || p->max_iterations > GM_MAX_ICP_ITERATIONS ||
-      !(p->min_rotation_step >= 0.0) || !(p->min_translation_step >= 0.0) || !(p->degeneracy_ratio >= 0.0) ||
-      !(p->degeneracy_ratio < 1.0) || !finite_pose(p->init_pose34))
-    return GM_ERR_INVALID_ARG;
+  if (!valid_icp_args(p)) return GM_ERR_INVALID_ARG;
   if (gm_status s = require(target, NORMALS)) return s;
   if (target->injected) return GM_ERR_STAGE_ORDER;
   if (gm_status s = require(source, VOXEL)) return s;
@@ -1740,15 +1771,10 @@ gm_status gm_register(gm_ctx* source, gm_ctx* target, const gm_icp_params* p) {
   Pose34 init;
   std::memcpy(init.r, p->init_pose34, sizeof(init.r));
   GM_LAUNCH(ctx, k_reg_begin, 1, 32, source->d_reg_state, init, &source->d_st->vox.n_voxels);
-  RegParams rp;
-  rp.d_max = dmax;
-  rp.r2max = (float)(dmax * dmax);
-  rp.min_rot = p->min_rotation_step;
-  rp.min_trans = p->min_translation_step;
-  rp.ratio = p->degeneracy_ratio;
+  int blocks;
+  const RegParams rp = icp_setup(source, p, &blocks);
   // an empty target built no grid this scan: its block table may still describe an earlier one
   const int search = target->n_grid > 0 ? 1 : 0;
-  const int blocks = std::max(1, std::min(div_up((long long)source->n_grid * 32, REG_BLOCK), reg_blocks(source)));
   for (int it = 0; it < p->max_iterations; ++it)
     GM_LAUNCH(ctx, k_reg_iter, blocks, REG_BLOCK, source->d_centroid, &source->d_st->vox.n_voxels, target->d_sorted, target->d_tab,
               target->d_ucell_start, target->d_runs, target->d_cell_nruns, target->d_valid_map, target->d_cloud_c, target->d_normals_c,
@@ -1786,17 +1812,9 @@ gm_status gm_get_registration(gm_ctx* ctx, gm_registration* out) {
 
 gm_status gm_download_correspondences(gm_ctx* ctx, int32_t* target_index, float* residual, size_t capacity_points) {
   if (!ctx || !target_index) return GM_ERR_INVALID_ARG;
-  if (gm_status s = require(ctx, REGISTRATION)) return s;
-  if (ctx->reg_target != 0) return GM_ERR_STAGE_ORDER;  // a map registration: gm_download_map_correspondences
-  int V = 0;
-  GM_CUDA(cudaMemcpyAsync(&V, &ctx->d_reg_state->n_source, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  GM_CUDA(cudaStreamSynchronize(ctx->stream));
-  if ((size_t)V > capacity_points) return GM_ERR_CAPACITY;
-  if (V > 0) {
-    GM_CUDA(cudaMemcpyAsync(target_index, ctx->d_reg_idx, (size_t)V * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    if (residual) GM_CUDA(cudaMemcpyAsync(residual, ctx->d_reg_res, (size_t)V * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    GM_CUDA(cudaStreamSynchronize(ctx->stream));
-  }
+  std::vector<int> idx;
+  if (gm_status s = download_reg_points(ctx, 0, ctx->d_reg_idx.p, &idx, residual, capacity_points)) return s;
+  std::copy(idx.begin(), idx.end(), target_index);
   return GM_OK;
 }
 
@@ -2497,52 +2515,103 @@ struct gm_map {
   DevBuf<int> d_kept_cnt;
   DevBuf<long long> d_kept_sums;
   DevBuf<MapEvictState> d_evict_st;
-  std::string err;
   ~gm_map() { if (ev_last) cudaEventDestroy(ev_last); }
 };
 
+// GM_CUDA of the map calls that take no context
+#define GM_MAP_CUDA(call) do { if ((call) != cudaSuccess) return GM_ERR_CUDA; } while (0)
+
 namespace {
-struct MapDump { std::vector<unsigned long long> keys; std::vector<int> cnt; std::vector<long long> sums; };
+// The device scope of a map call that takes no context: the map's device is current until the scope ends, then the
+// caller's again.  With sync, the caller's device is synchronised first (an insert from a context there is then complete)
+// and then, if it is another one, the map's.
+struct MapDeviceScope {
+  int caller = -1, device;
+  cudaError_t status;
+  MapDeviceScope(int map_device, bool sync) : device(map_device) {
+    status = cudaGetDevice(&caller);
+    if (status == cudaSuccess && sync) status = cudaDeviceSynchronize();
+    if (status == cudaSuccess && caller != device) status = cudaSetDevice(device);
+    if (status == cudaSuccess && sync && caller != device) status = cudaDeviceSynchronize();
+    if (status != cudaSuccess) cudaGetLastError();
+  }
+  ~MapDeviceScope() { if (caller >= 0 && caller != device) cudaSetDevice(caller); }
+};
 
 gm_status map_clear_device(gm_map* m) {
   if (cudaMemset(m->d_keys, 0xFF, m->n_slots * sizeof(unsigned long long)) != cudaSuccess ||
       cudaMemset(m->d_cnt, 0, m->n_slots * sizeof(int)) != cudaSuccess ||
       cudaMemset(m->d_sums, 0, 3 * m->n_slots * sizeof(long long)) != cudaSuccess ||
-      cudaMemset(m->d_st, 0, sizeof(MapState)) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess) { m->err = "cudaMemset"; return GM_ERR_CUDA; }
-  return GM_OK;
-}
-
-// all voxels, sorted by key (z-major, then y, then x): a deterministic order whatever the insertion history
-gm_status map_dump(gm_map* m, MapDump* out, MapState* st_out) {
-  if (cudaDeviceSynchronize() != cudaSuccess) { m->err = "sync"; return GM_ERR_CUDA; }
-  MapState st;
-  if (cudaMemcpy(&st, m->d_st, sizeof(st), cudaMemcpyDeviceToHost) != cudaSuccess) { m->err = "memcpy"; return GM_ERR_CUDA; }
-  if (st_out) *st_out = st;
-  const size_t V = (size_t)std::max(st.n_voxels, 0);
-  DevBuf<unsigned long long> dk; DevBuf<int> dc; DevBuf<long long> ds;
-  if (dk.alloc(V) != cudaSuccess || dc.alloc(V) != cudaSuccess || ds.alloc(3 * V) != cudaSuccess) { m->err = "cudaMalloc"; return GM_ERR_CUDA; }
-  cudaMemset(m->d_cursor, 0, sizeof(int));
-  cudaDeviceSynchronize();
-  if (V) k_map_export<<<std::min<unsigned long long>((m->n_slots + 255) / 256, (unsigned long long)m->num_sms * 16), 256>>>(
-      m->d_keys, m->d_cnt, m->d_sums, m->n_slots, dk, dc, ds, (int)V, m->d_cursor);
-  std::vector<unsigned long long> k(V); std::vector<int> c(V); std::vector<long long> su(3 * V);
-  cudaError_t e = cudaMemcpy(k.data(), dk, V * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess) e = cudaMemcpy(c.data(), dc, V * sizeof(int), cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess) e = cudaMemcpy(su.data(), ds, 3 * V * sizeof(long long), cudaMemcpyDeviceToHost);
-  if (e != cudaSuccess) { m->err = cudaGetErrorString(e); return GM_ERR_CUDA; }
-  std::vector<size_t> order(V);
-  for (size_t i = 0; i < V; ++i) order[i] = i;
-  std::sort(order.begin(), order.end(), [&](size_t a, size_t b) { return k[a] < k[b]; });
-  out->keys.resize(V); out->cnt.resize(V); out->sums.resize(3 * V);
-  for (size_t i = 0; i < V; ++i) {
-    const size_t j = order[i];
-    out->keys[i] = k[j]; out->cnt[i] = c[j];
-    for (int a = 0; a < 3; ++a) out->sums[3 * i + a] = su[3 * j + a];
-  }
+      cudaMemset(m->d_st, 0, sizeof(MapState)) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess) return GM_ERR_CUDA;
   return GM_OK;
 }
 
 int map_blocks(const gm_map* m) { return (int)std::min<unsigned long long>((m->n_slots + 255) / 256, (unsigned long long)m->num_sms * 16); }
+
+cudaError_t ensure_plane_tables(gm_map* m) {
+  if (m->d_plane_cent.count) return cudaSuccess;
+  cudaError_t e = m->d_plane_nrm.alloc(m->n_slots);
+  if (e == cudaSuccess) e = m->d_plane_box.alloc(8);
+  if (e == cudaSuccess) e = m->d_plane_cent.alloc(m->n_slots);  // last: a failure above leaves the pair unallocated
+  return e;
+}
+
+// What map_export gathers of every voxel besides the map's state: nothing, key + count + sums, or key + plane normal.
+enum MapExportKind { MAP_STATE, MAP_VOXELS, MAP_PLANES };
+struct MapExport {
+  MapState st{};
+  std::vector<unsigned long long> keys;
+  std::vector<int> cnt;         // MAP_VOXELS
+  std::vector<long long> sums;  // MAP_VOXELS, 3 a voxel
+  std::vector<float4> nrm;      // MAP_PLANES
+};
+
+// The gathered values d, w per voxel, copied back into *out in key order: out's voxel i = d's voxel order[i].
+template <class T>
+cudaError_t copy_in_order(const DevBuf<T>& d, size_t w, const std::vector<size_t>& order, std::vector<T>* out) {
+  std::vector<T> h(w * order.size());
+  const cudaError_t e = cudaMemcpy(h.data(), d, h.size() * sizeof(T), cudaMemcpyDeviceToHost);
+  out->resize(h.size());
+  for (size_t i = 0; i < order.size(); ++i) std::copy_n(&h[w * order[i]], w, &(*out)[w * i]);
+  return e;
+}
+
+// In the map's device scope: synchronise, read the state, then gather `what` of the occupied slots into temporary V-sized
+// buffers (MAP_PLANES: k_map_planes at max_planarity first), copy them back and sort them by key (z-major, then y, then
+// x): a deterministic order whatever the insertion history.  An empty map, or one of more than `capacity` voxels, gathers
+// nothing.
+gm_status map_export(gm_map* m, MapExportKind what, MapExport* x, double max_planarity = 0.0, size_t capacity = SIZE_MAX) {
+  MapDeviceScope scope(m->device, true);
+  GM_MAP_CUDA(scope.status);
+  GM_MAP_CUDA(cudaMemcpy(&x->st, m->d_st, sizeof(MapState), cudaMemcpyDeviceToHost));
+  const size_t V = (size_t)std::max(x->st.n_voxels, 0);
+  if (what == MAP_STATE || V == 0 || V > capacity) return GM_OK;
+  const bool planes = what == MAP_PLANES;
+  DevBuf<unsigned long long> dk; DevBuf<int> dc; DevBuf<long long> ds; DevBuf<float4> dn;
+  GM_MAP_CUDA(dk.alloc(V));
+  if (planes) {
+    GM_MAP_CUDA(ensure_plane_tables(m));
+    GM_MAP_CUDA(dn.alloc(V));
+    GM_MAP_CUDA(cudaMemset(m->d_plane_box, 0x7F, 8 * sizeof(int)));
+    k_map_planes<<<map_blocks(m), 256>>>(m->d_keys, m->d_cnt, m->d_sums, m->n_slots - 1ull, max_planarity, m->d_plane_cent, m->d_plane_nrm,
+                                         m->d_plane_box);
+  } else {
+    GM_MAP_CUDA(dc.alloc(V));
+    GM_MAP_CUDA(ds.alloc(3 * V));
+  }
+  GM_MAP_CUDA(cudaMemset(m->d_cursor, 0, sizeof(int)));
+  k_map_export<<<map_blocks(m), 256>>>(m->d_keys, m->d_cnt, m->d_sums, m->d_plane_nrm, m->n_slots, dk, dc, ds, dn, (int)V, m->d_cursor);
+  GM_MAP_CUDA(cudaGetLastError());
+  std::vector<unsigned long long> k(V);
+  GM_MAP_CUDA(cudaMemcpy(k.data(), dk, V * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+  std::vector<size_t> order(V);
+  std::iota(order.begin(), order.end(), size_t(0));
+  std::sort(order.begin(), order.end(), [&](size_t a, size_t b) { return k[a] < k[b]; });
+  for (size_t j : order) x->keys.push_back(k[j]);
+  cudaError_t e = planes ? copy_in_order(dn, 1, order, &x->nrm) : copy_in_order(dc, 1, order, &x->cnt);
+  if (e == cudaSuccess && !planes) e = copy_in_order(ds, 3, order, &x->sums);
+  return e == cudaSuccess ? GM_OK : GM_ERR_CUDA;
+}
 
 // the leaf and device rules of gm_map_evict / gm_map_merge / gm_odometry_set_window: the same lattice, the same device
 bool same_lattice(const gm_map* a, const gm_map* b) {
@@ -2559,7 +2628,7 @@ cudaError_t ensure_evict_buffers(gm_map* m) {
 }
 
 // The launches of gm_map_evict on ctx's stream, after its checks and waits (buffers allocated): the counters' reset, then
-// k_map_evict_split, k_map_evict_clear and k_map_evict_restore.  Centre = c3 (host), or the translation of the device pose
+// k_map_evict_split, k_map_evict_clear and k_map_restore.  Centre = c3 (host), or the translation of the device pose
 // pose34_dev.  Shared by gm_map_evict and gm_odometry_step.
 gm_status map_evict_launch(gm_map* m, gm_ctx* ctx, gm_map* archive, const float* c3, const float* pose34_dev, int half_cells) {
   GM_CUDA(cudaMemsetAsync(m->d_evict_st, 0, sizeof(MapEvictState), ctx->stream));
@@ -2569,7 +2638,7 @@ gm_status map_evict_launch(gm_map* m, gm_ctx* ctx, gm_map* archive, const float*
             archive ? (long long*)archive->d_sums : nullptr, archive ? archive->n_slots - 1ull : 0ull, archive ? (MapState*)archive->d_st : nullptr,
             m->d_kept_keys, m->d_kept_cnt, m->d_kept_sums, m->d_evict_st);
   GM_LAUNCH(ctx, k_map_evict_clear, map_blocks(m), 256, m->d_keys, m->d_cnt, m->d_sums, m->n_slots, m->d_evict_st, m->d_st);
-  GM_LAUNCH(ctx, k_map_evict_restore, map_blocks(m), 256, m->d_kept_keys, m->d_kept_cnt, m->d_kept_sums, m->d_evict_st, m->d_keys, m->d_cnt,
+  GM_LAUNCH(ctx, k_map_restore, map_blocks(m), 256, m->d_kept_keys, m->d_kept_cnt, m->d_kept_sums, 0, m->d_evict_st, m->d_keys, m->d_cnt,
             m->d_sums, m->n_slots - 1ull, m->d_st);
   GM_CHECK_LAUNCHES(ctx);
   return GM_OK;
@@ -2605,13 +2674,14 @@ gm_status gm_map_create(double leaf, size_t capacity_voxels, gm_map** out) {
 
 void gm_map_destroy(gm_map* m) {
   if (!m) return;
-  cudaDeviceSynchronize();
+  MapDeviceScope scope(m->device, true);
   delete m;
 }
 
 gm_status gm_map_clear(gm_map* m) {
   if (!m) return GM_ERR_INVALID_ARG;
-  if (cudaDeviceSynchronize() != cudaSuccess) return GM_ERR_CUDA;
+  MapDeviceScope scope(m->device, true);
+  GM_MAP_CUDA(scope.status);
   return map_clear_device(m);
 }
 
@@ -2634,22 +2704,20 @@ gm_status gm_map_insert(gm_map* m, gm_ctx* ctx, const float* pose34, int32_t lab
 
 gm_status gm_map_stats(gm_map* m, int64_t* n_voxels, int64_t* n_points, int64_t* n_out_of_range) {
   if (!m) return GM_ERR_INVALID_ARG;
-  if (cudaDeviceSynchronize() != cudaSuccess) return GM_ERR_CUDA;
-  MapState st;
-  if (cudaMemcpy(&st, m->d_st, sizeof(st), cudaMemcpyDeviceToHost) != cudaSuccess) return GM_ERR_CUDA;
-  if (n_voxels) *n_voxels = st.n_voxels;
-  if (n_points) *n_points = (int64_t)st.n_points;
-  if (n_out_of_range) *n_out_of_range = st.out_of_range;
-  return st.overflow ? GM_ERR_CAPACITY : GM_OK;
+  MapExport x;
+  if (gm_status s = map_export(m, MAP_STATE, &x)) return s;
+  if (n_voxels) *n_voxels = x.st.n_voxels;
+  if (n_points) *n_points = (int64_t)x.st.n_points;
+  if (n_out_of_range) *n_out_of_range = x.st.out_of_range;
+  return x.st.overflow ? GM_ERR_CAPACITY : GM_OK;
 }
 
 gm_status gm_map_download(gm_map* m, int32_t* ijk, int32_t* counts, float* centroids_xyzw, size_t capacity, size_t* n) {
   if (!m || !n) return GM_ERR_INVALID_ARG;
-  MapDump d; MapState st;
-  gm_status s = map_dump(m, &d, &st);
-  if (s != GM_OK) return s;
+  MapExport d;
+  if (gm_status s = map_export(m, MAP_VOXELS, &d)) return s;
   *n = d.keys.size();
-  if (!ijk && !counts && !centroids_xyzw) return st.overflow ? GM_ERR_CAPACITY : GM_OK;
+  if (!ijk && !counts && !centroids_xyzw) return d.st.overflow ? GM_ERR_CAPACITY : GM_OK;
   if (capacity < d.keys.size()) return GM_ERR_CAPACITY;
   for (size_t i = 0; i < d.keys.size(); ++i) {
     if (ijk) { int x, y, z; map_unpack(d.keys[i], x, y, z); ijk[3 * i] = x; ijk[3 * i + 1] = y; ijk[3 * i + 2] = z; }
@@ -2660,16 +2728,15 @@ gm_status gm_map_download(gm_map* m, int32_t* ijk, int32_t* counts, float* centr
       centroids_xyzw[4 * i + 3] = 1.0f;
     }
   }
-  return st.overflow ? GM_ERR_CAPACITY : GM_OK;
+  return d.st.overflow ? GM_ERR_CAPACITY : GM_OK;
 }
 
 gm_status gm_map_save(gm_map* m, const char* path) {
   if (!m || !path) return GM_ERR_INVALID_ARG;
-  MapDump d; MapState st;
-  gm_status s = map_dump(m, &d, &st);
-  if (s != GM_OK) return s;
+  MapExport d;
+  if (gm_status s = map_export(m, MAP_VOXELS, &d)) return s;
   FILE* f = std::fopen(path, "wb");
-  if (!f) { m->err = "cannot open file"; return GM_ERR_INVALID_ARG; }
+  if (!f) return GM_ERR_INVALID_ARG;
   const uint32_t magic = 0x314D4D47u /* 'GMM1' */, version = 1;
   const uint64_t V = d.keys.size();
   bool ok = std::fwrite(&magic, 4, 1, f) == 1 && std::fwrite(&version, 4, 1, f) == 1 && std::fwrite(&m->leaf, 8, 1, f) == 1 &&
@@ -2715,8 +2782,8 @@ gm_status gm_map_load(const char* path, size_t min_capacity_voxels, gm_map** out
     if (e == cudaSuccess) e = cudaMemcpy(dc, c.data(), V * 4, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaMemcpy(ds, su.data(), 3 * V * 8, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) {
-      k_map_restore<<<std::min<unsigned long long>((V + 255) / 256, (unsigned long long)m->num_sms * 16), 256>>>(dk, dc, ds, (int)V, m->d_keys, m->d_cnt, m->d_sums,
-                                                                                                     m->n_slots - 1ull, m->d_st);
+      k_map_restore<<<std::min<unsigned long long>((V + 255) / 256, (unsigned long long)m->num_sms * 16), 256>>>(dk, dc, ds, (int)V, nullptr, m->d_keys,
+                                                                                                     m->d_cnt, m->d_sums, m->n_slots - 1ull, m->d_st);
       e = cudaDeviceSynchronize();
     }
     if (e != cudaSuccess) { gm_map_destroy(m); return GM_ERR_CUDA; }
@@ -2744,20 +2811,14 @@ gm_status gm_map_evict(gm_map* m, gm_ctx* ctx, gm_map* archive, const float* cen
 
 gm_status gm_map_merge(gm_map* dst, const gm_map* src) {
   if (!dst || !src || dst == src || !same_lattice(dst, src)) return GM_ERR_INVALID_ARG;
-  int prev = 0;
-  if (cudaGetDevice(&prev) != cudaSuccess || cudaSetDevice(dst->device) != cudaSuccess) { cudaGetLastError(); return GM_ERR_CUDA; }
-  cudaError_t e = cudaDeviceSynchronize();
-  if (e == cudaSuccess) {
-    k_map_merge<<<map_blocks(src), 256>>>(src->d_keys, src->d_cnt, src->d_sums, src->n_slots, dst->d_keys, dst->d_cnt, dst->d_sums,
-                                          dst->n_slots - 1ull, dst->d_st);
-    e = cudaGetLastError();
-  }
-  if (e == cudaSuccess) e = cudaDeviceSynchronize();
-  MapState st{};
-  if (e == cudaSuccess) e = cudaMemcpy(&st, dst->d_st, sizeof(st), cudaMemcpyDeviceToHost);
-  cudaSetDevice(prev);
-  if (e != cudaSuccess) { dst->err = cudaGetErrorString(e); return GM_ERR_CUDA; }
-  return st.overflow ? GM_ERR_CAPACITY : GM_OK;
+  MapDeviceScope scope(dst->device, true);
+  GM_MAP_CUDA(scope.status);
+  k_map_merge<<<map_blocks(src), 256>>>(src->d_keys, src->d_cnt, src->d_sums, src->n_slots, dst->d_keys, dst->d_cnt, dst->d_sums,
+                                        dst->n_slots - 1ull, dst->d_st);
+  GM_MAP_CUDA(cudaGetLastError());
+  MapExport x;
+  if (gm_status s = map_export(dst, MAP_STATE, &x)) return s;  // synchronises: the state after the merge
+  return x.st.overflow ? GM_ERR_CAPACITY : GM_OK;
 }
 
 }  // extern "C"
@@ -2766,21 +2827,8 @@ gm_status gm_map_merge(gm_map* dst, const gm_map* src) {
 namespace {
 inline bool valid_planarity(double r) { return r > 0.0 && r <= 1.0; }
 
-cudaError_t ensure_plane_tables(gm_map* m) {
-  if (m->d_plane_cent.count) return cudaSuccess;
-  cudaError_t e = m->d_plane_nrm.alloc(m->n_slots);
-  if (e == cudaSuccess) e = m->d_plane_box.alloc(8);
-  if (e == cudaSuccess) e = m->d_plane_cent.alloc(m->n_slots);  // last: a failure above leaves the pair unallocated
-  return e;
-}
-
 // gm_register_map's argument rules (gm_odometry_create checks its icp by them too)
-bool valid_regmap_args(const gm_icp_params* p, double max_planarity) {
-  const double dmax = p->max_correspondence_distance;
-  return dmax > 0.0 && std::isfinite(dmax) && p->max_iterations >= 1 && p->max_iterations <= GM_MAX_ICP_ITERATIONS &&
-         p->min_rotation_step >= 0.0 && p->min_translation_step >= 0.0 && p->degeneracy_ratio >= 0.0 && p->degeneracy_ratio < 1.0 &&
-         finite_pose(p->init_pose34) && valid_planarity(max_planarity);
-}
+bool valid_regmap_args(const gm_icp_params* p, double max_planarity) { return valid_icp_args(p) && valid_planarity(max_planarity); }
 
 // The buffers a scan-to-map registration of `source` uses (allocated by the first call).
 gm_status regmap_buffers(gm_ctx* source, gm_map* map) {
@@ -2803,13 +2851,8 @@ gm_status regmap_launch(gm_ctx* source, gm_map* map, const gm_icp_params* p, dou
   GM_LAUNCH(ctx, k_map_planes, map_blocks(map), 256, map->d_keys, map->d_cnt, map->d_sums, mask, max_planarity, map->d_plane_cent,
             map->d_plane_nrm, map->d_plane_box);
   begin();
-  RegParams rp;
-  rp.d_max = p->max_correspondence_distance;
-  rp.r2max = (float)(rp.d_max * rp.d_max);
-  rp.min_rot = p->min_rotation_step;
-  rp.min_trans = p->min_translation_step;
-  rp.ratio = p->degeneracy_ratio;
-  const int blocks = std::max(1, std::min(div_up((long long)source->n_grid * 32, REG_BLOCK), reg_blocks(source)));
+  int blocks;
+  const RegParams rp = icp_setup(source, p, &blocks);
   for (int it = 0; it < p->max_iterations; ++it)
     GM_LAUNCH(ctx, k_regmap_iter, blocks, REG_BLOCK, source->d_centroid, &source->d_st->vox.n_voxels, map->d_keys, map->d_plane_cent,
               map->d_plane_nrm, map->d_plane_box, mask, map->inv_leaf, map->leaf, rp, source->d_reg_state, source->d_reg_part, source->d_reg_ticket,
@@ -2843,56 +2886,24 @@ gm_status gm_register_map(gm_ctx* source, gm_map* map, const gm_icp_params* p, d
 
 gm_status gm_download_map_correspondences(gm_ctx* ctx, int32_t* ijk, float* residual, size_t capacity_points) {
   if (!ctx || !ijk) return GM_ERR_INVALID_ARG;
-  if (gm_status s = require(ctx, REGISTRATION)) return s;
-  if (ctx->reg_target != 1) return GM_ERR_STAGE_ORDER;  // a context registration: gm_download_correspondences
-  int V = 0;
-  GM_CUDA(cudaMemcpyAsync(&V, &ctx->d_reg_state->n_source, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  GM_CUDA(cudaStreamSynchronize(ctx->stream));
-  if ((size_t)V > capacity_points) return GM_ERR_CAPACITY;
-  if (V > 0) {
-    std::vector<unsigned long long> keys((size_t)V);
-    GM_CUDA(cudaMemcpyAsync(keys.data(), ctx->d_reg_key, (size_t)V * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
-    if (residual) GM_CUDA(cudaMemcpyAsync(residual, ctx->d_reg_res, (size_t)V * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    GM_CUDA(cudaStreamSynchronize(ctx->stream));
-    for (size_t i = 0; i < (size_t)V; ++i) {
-      int x = INT32_MIN, y = INT32_MIN, z = INT32_MIN;
-      if (keys[i] != MAP_EMPTY) map_unpack(keys[i], x, y, z);
-      ijk[3 * i] = x; ijk[3 * i + 1] = y; ijk[3 * i + 2] = z;
-    }
+  std::vector<unsigned long long> keys;
+  if (gm_status s = download_reg_points(ctx, 1, ctx->d_reg_key.p, &keys, residual, capacity_points)) return s;
+  for (size_t i = 0; i < keys.size(); ++i) {
+    int x = INT32_MIN, y = INT32_MIN, z = INT32_MIN;
+    if (keys[i] != MAP_EMPTY) map_unpack(keys[i], x, y, z);
+    ijk[3 * i] = x; ijk[3 * i + 1] = y; ijk[3 * i + 2] = z;
   }
   return GM_OK;
 }
 
 gm_status gm_map_download_planes(gm_map* m, double max_planarity, float* normals_xyzw, size_t capacity, size_t* n) {
   if (!m || !n || !valid_planarity(max_planarity)) return GM_ERR_INVALID_ARG;
-  if (cudaDeviceSynchronize() != cudaSuccess) { m->err = "sync"; return GM_ERR_CUDA; }
-  MapState st;
-  if (cudaMemcpy(&st, m->d_st, sizeof(st), cudaMemcpyDeviceToHost) != cudaSuccess) { m->err = "memcpy"; return GM_ERR_CUDA; }
-  const size_t V = (size_t)std::max(st.n_voxels, 0);
-  *n = V;
-  if (!normals_xyzw) return st.overflow ? GM_ERR_CAPACITY : GM_OK;
-  if (capacity < V) return GM_ERR_CAPACITY;
-  if (!V) return st.overflow ? GM_ERR_CAPACITY : GM_OK;
-  DevBuf<unsigned long long> dk; DevBuf<float4> dn;
-  if (ensure_plane_tables(m) != cudaSuccess || dk.alloc(V) != cudaSuccess || dn.alloc(V) != cudaSuccess) { m->err = "cudaMalloc"; return GM_ERR_CUDA; }
-  cudaError_t e = cudaMemset(m->d_cursor, 0, sizeof(int));
-  if (e == cudaSuccess) e = cudaMemset(m->d_plane_box, 0x7F, 8 * sizeof(int));
-  if (e == cudaSuccess) {
-    k_map_planes<<<map_blocks(m), 256>>>(m->d_keys, m->d_cnt, m->d_sums, m->n_slots - 1ull, max_planarity, m->d_plane_cent, m->d_plane_nrm,
-                                         m->d_plane_box);
-    k_map_export_planes<<<map_blocks(m), 256>>>(m->d_keys, m->d_plane_nrm, m->n_slots, dk, dn, (int)V, m->d_cursor);
-    e = cudaGetLastError();
-  }
-  std::vector<unsigned long long> k(V);
-  std::vector<float4> nr(V);
-  if (e == cudaSuccess) e = cudaMemcpy(k.data(), dk, V * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess) e = cudaMemcpy(nr.data(), dn, V * sizeof(float4), cudaMemcpyDeviceToHost);
-  if (e != cudaSuccess) { m->err = cudaGetErrorString(e); return GM_ERR_CUDA; }
-  std::vector<size_t> order(V);
-  for (size_t i = 0; i < V; ++i) order[i] = i;
-  std::sort(order.begin(), order.end(), [&](size_t a, size_t b) { return k[a] < k[b]; });  // gm_map_download's order
-  for (size_t i = 0; i < V; ++i) std::memcpy(normals_xyzw + 4 * i, &nr[order[i]], sizeof(float4));
-  return st.overflow ? GM_ERR_CAPACITY : GM_OK;  // as gm_map_download: an insert found the table full
+  MapExport x;
+  if (gm_status s = map_export(m, normals_xyzw ? MAP_PLANES : MAP_STATE, &x, max_planarity, capacity)) return s;
+  *n = (size_t)std::max(x.st.n_voxels, 0);
+  if (normals_xyzw && capacity < *n) return GM_ERR_CAPACITY;
+  for (size_t i = 0; i < x.nrm.size(); ++i) std::memcpy(normals_xyzw + 4 * i, &x.nrm[i], sizeof(float4));
+  return x.st.overflow ? GM_ERR_CAPACITY : GM_OK;  // as gm_map_download: an insert found the table full
 }
 
 }  // extern "C"
@@ -2932,8 +2943,8 @@ gm_status gm_odometry_create(gm_map* map, const gm_odometry_params* p, gm_odomet
   if (!map || !p || !valid_regmap_args(&p->icp, p->max_planarity) || !(p->min_fitness >= 0.0 && p->min_fitness <= 1.0) ||
       (p->register_first != 0 && p->register_first != 1) || p->max_steps < 1)
     return GM_ERR_INVALID_ARG;
-  int prev = 0;
-  if (cudaGetDevice(&prev) != cudaSuccess || cudaSetDevice(map->device) != cudaSuccess) { cudaGetLastError(); return GM_ERR_CUDA; }
+  MapDeviceScope scope(map->device, false);
+  GM_MAP_CUDA(scope.status);
   gm_odometry* o = new gm_odometry();
   o->map = map;
   o->p = *p;
@@ -2943,7 +2954,6 @@ gm_status gm_odometry_create(gm_map* map, const gm_odometry_params* p, gm_odomet
   if (e == cudaSuccess) e = cudaMemset(o->d_ins, 0, sizeof(OdomInsert));
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&o->stream, cudaStreamNonBlocking);
   if (e == cudaSuccess) e = cudaDeviceSynchronize();
-  cudaSetDevice(prev);
   if (e != cudaSuccess) { delete o; return GM_ERR_CUDA; }
   *out = o;
   return GM_OK;
@@ -2951,7 +2961,7 @@ gm_status gm_odometry_create(gm_map* map, const gm_odometry_params* p, gm_odomet
 
 void gm_odometry_destroy(gm_odometry* odo) {
   if (!odo) return;
-  cudaDeviceSynchronize();  // as gm_map_destroy: the steps in flight read the trajectory
+  MapDeviceScope scope(odo->map->device, true);  // as gm_map_destroy: the steps in flight read the trajectory
   delete odo;
 }
 

@@ -118,20 +118,27 @@ __device__ __forceinline__ void d_map_add(unsigned long long key, int c, const l
   atomicAdd(&st->n_points, (unsigned long long)c);
 }
 
-// Raw re-insertion of saved voxels (gm_map_load): key, count and fixed-point sums as stored.
-__global__ void k_map_restore(const unsigned long long* __restrict__ in_keys, const int* __restrict__ in_cnt,
-                              const long long* __restrict__ in_sums, int n, unsigned long long* __restrict__ keys,
-                              int* __restrict__ cnt, long long* __restrict__ sums, unsigned long long slot_mask, MapState* st) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
-    d_map_add(in_keys[i], in_cnt[i], in_sums + 3 * (size_t)i, keys, cnt, sums, slot_mask, st);
-}
-
 // ---- window eviction (gm_map_evict) and merge (gm_map_merge) ----------------------------------------------------------
 // Linear probing has no parallel delete, so an eviction rebuilds the table: k_map_evict_split adds the evicted voxels to
 // the archive and compacts the kept ones into the map's scratch arrays, k_map_evict_clear empties the table and
-// k_map_evict_restore re-adds the kept voxels.  The last two return at once when nothing was evicted.
+// k_map_restore re-adds the kept voxels.  The last two return at once when nothing was evicted.
 
 struct MapEvictState { int n_kept; int evicted; };  // zeroed before every eviction
+
+// Add n dense voxels (key, count and fixed-point sums as stored) to the table: the saved voxels of gm_map_load (es null),
+// or the kept voxels of an eviction (n = es->n_kept) if es->evicted, which re-adds them to the emptied table and so
+// recounts n_voxels and n_points.  Kept voxels are at most the voxels the table held, so they all fit.
+__global__ void k_map_restore(const unsigned long long* __restrict__ in_keys, const int* __restrict__ in_cnt,
+                              const long long* __restrict__ in_sums, int n, const MapEvictState* __restrict__ es,
+                              unsigned long long* __restrict__ keys, int* __restrict__ cnt, long long* __restrict__ sums,
+                              unsigned long long slot_mask, MapState* st) {
+  if (es) {
+    if (!es->evicted) return;
+    n = es->n_kept;
+  }
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+    d_map_add(in_keys[i], in_cnt[i], in_sums + 3 * (size_t)i, keys, cnt, sums, slot_mask, st);
+}
 
 // The window's centre cell, c[a] = (int)floorf(center[a] * inv_leaf) as d_map_insert computes a point's cell.  false for a
 // non-finite centre or a cell outside the key range.  Host and device evaluate the same float product and floorf.
@@ -201,17 +208,6 @@ __global__ void k_map_evict_clear(unsigned long long* __restrict__ keys, int* __
   }
   for (unsigned long long s = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; s < 3 * n_slots; s += (unsigned long long)gridDim.x * blockDim.x)
     sums[s] = 0;
-}
-
-// Re-add the kept voxels to the emptied table (and so recount n_voxels and n_points), if anything was evicted.  They are
-// at most the voxels the table held, so they all fit.
-__global__ void k_map_evict_restore(const unsigned long long* __restrict__ in_keys, const int* __restrict__ in_cnt,
-                                    const long long* __restrict__ in_sums, const MapEvictState* __restrict__ es, unsigned long long* __restrict__ keys,
-                                    int* __restrict__ cnt, long long* __restrict__ sums, unsigned long long slot_mask, MapState* st) {
-  if (!es->evicted) return;
-  const int n = es->n_kept;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
-    d_map_add(in_keys[i], in_cnt[i], in_sums + 3 * (size_t)i, keys, cnt, sums, slot_mask, st);
 }
 
 // dst += src: every occupied slot of src added to dst (gm_map_merge).
@@ -313,30 +309,21 @@ __global__ void k_map_planes(const unsigned long long* __restrict__ keys, const 
   }
 }
 
-// Gather the occupied slots' keys and plane normals (order = slot order; the host sorts by key), as k_map_export.
-__global__ void k_map_export_planes(const unsigned long long* __restrict__ keys, const float4* __restrict__ nrm, unsigned long long n_slots,
-                                    unsigned long long* __restrict__ out_keys, float4* __restrict__ out_nrm, int capacity, int* cursor) {
+// Gather the occupied slots into dense arrays (order = slot order; the host sorts by key): the key, and the count, the
+// sums and the plane normal of k_map_planes into those of out_cnt, out_sums and out_nrm that are not null.
+__global__ void k_map_export(const unsigned long long* __restrict__ keys, const int* __restrict__ cnt, const long long* __restrict__ sums,
+                             const float4* __restrict__ nrm, unsigned long long n_slots, unsigned long long* __restrict__ out_keys,
+                             int* __restrict__ out_cnt, long long* __restrict__ out_sums, float4* __restrict__ out_nrm, int capacity, int* cursor) {
   for (unsigned long long s = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; s < n_slots; s += (unsigned long long)gridDim.x * blockDim.x) {
     const unsigned long long k = keys[s];
     if (k == MAP_EMPTY) continue;
     const int o = atomicAdd(cursor, 1);
     if (o >= capacity) continue;
     out_keys[o] = k;
-    out_nrm[o] = nrm[s];
-  }
-}
-
-// Gather the occupied slots into dense arrays (order = slot order; the host sorts by key).
-__global__ void k_map_export(const unsigned long long* __restrict__ keys, const int* __restrict__ cnt, const long long* __restrict__ sums,
-                             unsigned long long n_slots, unsigned long long* __restrict__ out_keys, int* __restrict__ out_cnt,
-                             long long* __restrict__ out_sums, int capacity, int* cursor) {
-  for (unsigned long long s = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; s < n_slots; s += (unsigned long long)gridDim.x * blockDim.x) {
-    const unsigned long long k = keys[s];
-    if (k == MAP_EMPTY) continue;
-    const int o = atomicAdd(cursor, 1);
-    if (o >= capacity) continue;
-    out_keys[o] = k; out_cnt[o] = cnt[s];
-    out_sums[3 * (size_t)o] = sums[3 * s]; out_sums[3 * (size_t)o + 1] = sums[3 * s + 1]; out_sums[3 * (size_t)o + 2] = sums[3 * s + 2];
+    if (out_cnt) out_cnt[o] = cnt[s];
+    if (out_sums)
+      for (int a = 0; a < 3; ++a) out_sums[3 * (size_t)o + a] = sums[3 * s + a];
+    if (out_nrm) out_nrm[o] = nrm[s];
   }
 }
 

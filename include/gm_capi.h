@@ -515,7 +515,10 @@ GM_API gm_status gm_encode_marker_array(const gm_arrow* arrows, int32_t n, const
  * the ctx stream), optionally only the points with label == label_filter (after gm_label; -1 = all), after the
  * rigid transform pose34 = row-major [R|t] (NULL = identity; p' = R p + t as fmaf chains).  gm_map_download
  * returns the voxels sorted by (z, y, x) index: integer cell, count, centroid = sum / count.  gm_map_save / load:
- * little-endian file 'GMM1' | leaf f64 | V u64 | keys u64[V] | counts i32[V] | sums i64[3V] (exact state). */
+ * little-endian file 'GMM1' | leaf f64 | V u64 | keys u64[V] | counts i32[V] | sums i64[3V] (exact state).
+ * A map lives on the device current at gm_map_create / gm_map_load.  The gm_map_* and gm_odometry_* calls that take no
+ * context work on that device whichever device is current, and leave the caller's current device as it was; one that
+ * synchronises the device synchronises the caller's current device and then, if that is another one, the map's. */
 typedef struct gm_map gm_map;
 GM_API gm_status gm_map_create(double leaf, size_t capacity_voxels, gm_map** out);
 GM_API void gm_map_destroy(gm_map* map);

@@ -13,7 +13,7 @@ stream.  Run five ways, each from a new map:
                   it fills to a load of about 0.9 and every hash probe sequence grows.
 Reported per step index: the step's device time (CUDA events on the context's stream around gm_odometry_step: the
 launches of one step, scan processing excluded), and, from torch.profiler in a separate pass, the device time of
-k_map_planes and of the eviction kernels (k_map_evict_split, k_map_evict_clear, k_map_evict_restore).  Also whether each
+k_map_planes and of the eviction kernels (k_map_evict_split, k_map_evict_clear, k_map_restore).  Also whether each
 windowed trajectory is bit-identical to the unwindowed one, and the final voxel counts.  The card's name and power
 limit are read in the same run.
 
@@ -39,7 +39,7 @@ LEAF, DMAX, RATIO, BORE_RATIO = 0.1, 0.5, 0.1, 1e-2
 SCANS, STEP, ARC_R, N = 64, 0.8, 50.0, 240_000
 B, S = 5.0, 1.3
 RULE = math.floor((math.sqrt(3.0) * B + S + DMAX) / LEAF) + 2
-EVICT = ("k_map_evict_split", "k_map_evict_clear", "k_map_evict_restore")
+EVICT = ("k_map_evict_split", "k_map_evict_clear", "k_map_restore")
 KERNELS = ("k_map_planes",) + EVICT
 CONFIGS = {"none": (0, 1 << 18, False), "window": (RULE, 1 << 16, True), "window_drop": (RULE, 1 << 16, False),
            "window_big": (RULE, 1 << 18, True), "window_tight": (RULE, 1 << 15, True)}
