@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libgm_b200.so")
 SOURCES = ["gm_capi.cu"]
-HEADERS = ["gm_device.cuh", "gm_sort.cuh", "gm_stages.cuh", "gm_ransac.cuh", "gm_polyline.cuh", "gm_compress.cuh", "gm_primitives.cuh", "gm_map.cuh", "gm_comm.cuh", "gm_register.cuh", "gm_odometry.cuh", "../../include/gm_capi.h"]
+HEADERS = ["gm_device.cuh", "gm_sort.cuh", "gm_stages.cuh", "gm_ransac.cuh", "gm_polyline.cuh", "gm_compress.cuh", "gm_primitives.cuh", "gm_map.cuh", "gm_comm.cuh", "gm_register.cuh", "gm_odometry.cuh", "gm_deskew.cuh", "../../include/gm_capi.h"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

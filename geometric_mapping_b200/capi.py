@@ -172,6 +172,7 @@ SYMBOLS = [
     "gm_download_correspondences", "gm_register_map", "gm_download_map_correspondences", "gm_map_download_planes",
     "gm_odometry_params_default", "gm_odometry_create", "gm_odometry_destroy", "gm_odometry_step", "gm_odometry_steps", "gm_odometry_get",
     "gm_map_evict", "gm_map_merge", "gm_odometry_set_window",
+    "gm_upload_pointcloud2_timed", "gm_download_point_times", "gm_deskew", "gm_odometry_deskew",
     "gm_encode_marker_array", "gm_store_open", "gm_store_close", "gm_store_append", "gm_store_append_blob", "gm_store_count", "gm_store_info", "gm_store_read",
 ]
 
@@ -314,6 +315,10 @@ def _lib():
         "gm_map_evict": (i32, [vp, vp, vp, vp, i32]),
         "gm_map_merge": (i32, [vp, vp]),
         "gm_odometry_set_window": (i32, [vp, i32, vp]),
+        "gm_upload_pointcloud2_timed": (i32, [vp, vp, sz, sz, sz, sz, sz, sz]),
+        "gm_download_point_times": (i32, [vp, vp, sz]),
+        "gm_deskew": (i32, [vp, vp, C.c_double, C.c_double]),
+        "gm_odometry_deskew": (i32, [vp, vp, C.c_double, C.c_double]),
     }
     assert set(sig) == set(SYMBOLS)
     for name, (res, args) in sig.items():
@@ -520,6 +525,26 @@ class Context:
     def upload_pointcloud2_raw(self, host_ptr: int, n: int, point_step: int, offset_x: int, offset_y: int, offset_z: int):
         """Same from a raw host address (e.g. a pinned torch tensor); the caller keeps the buffer alive."""
         self._ck(_lib().gm_upload_pointcloud2(self._h, C.c_void_p(host_ptr), n, point_step, offset_x, offset_y, offset_z), "gm_upload_pointcloud2")
+
+    def upload_pointcloud2_timed(self, data: np.ndarray, n: int, point_step: int, offset_x: int, offset_y: int, offset_z: int,
+                                 offset_t: int):
+        """upload_pointcloud2 plus the float32 per-point time (seconds) at byte offset offset_t, e.g. PointXYZIRT::time."""
+        raw = np.ascontiguousarray(data, dtype=np.uint8)
+        self._keepalive = raw
+        self._ck(_lib().gm_upload_pointcloud2_timed(self._h, _ptr(raw), n, point_step, offset_x, offset_y, offset_z, offset_t),
+                 "gm_upload_pointcloud2_timed")
+
+    def point_times(self) -> np.ndarray:
+        """The n decoded times of the timed scan (float32)."""
+        out = np.empty(max(self.counts().n_input, 0), np.float32)
+        self._ck(_lib().gm_download_point_times(self._h, _ptr(out), out.shape[0]), "gm_download_point_times")
+        return out
+
+    def deskew(self, delta34, t_ref: float, period: float):
+        """Express every point of the timed scan in the sensor frame at t_ref, the sensor moving by delta34 (3x4 or 4x4, the
+        previous scan's frame to this one's) over `period` seconds (include/gm_capi.h, gm_deskew).  Before crop()."""
+        d = np.ascontiguousarray(np.asarray(delta34, np.float32)[:3, :4].reshape(12))
+        self._ck(_lib().gm_deskew(self._h, _ptr(d), C.c_double(t_ref), C.c_double(period)), "gm_deskew")
 
     def set_scan_device(self, device_ptr: int, n: int):
         self._ck(_lib().gm_set_scan_device(self._h, C.c_void_p(device_ptr), n), "gm_set_scan_device")
@@ -1014,6 +1039,11 @@ class Odometry:
         frame, None = constant velocity."""
         d = None if delta34 is None else np.ascontiguousarray(np.asarray(delta34, np.float32)[:3, :4].reshape(12))
         ctx._ck(_lib().gm_odometry_step(self._h, ctx._h, _ptr(d)), "gm_odometry_step")
+
+    def deskew(self, ctx: "Context", t_ref: float, period: float):
+        """Deskew ctx's timed scan, the one the next step() takes, with the trajectory's constant-velocity increment (the
+        identity before step 2).  Waits on ctx's stream for the previous step (include/gm_capi.h, gm_odometry_deskew)."""
+        ctx._ck(_lib().gm_odometry_deskew(self._h, ctx._h, C.c_double(t_ref), C.c_double(period)), "gm_odometry_deskew")
 
     def set_window(self, half_cells: int, archive: VoxelMap | None = None):
         """From the next step on, end each step by evicting the map's voxels outside half_cells cells of the step's pose

@@ -11,6 +11,7 @@
 #include "gm_comm.cuh"
 #include "gm_register.cuh"
 #include "gm_odometry.cuh"
+#include "gm_deskew.cuh"
 #include <new>
 
 #include <algorithm>
@@ -147,6 +148,11 @@ struct gm_ctx {
 
   // device buffers
   DevBuf<unsigned char> d_raw;  // PointCloud2 staging (grown on demand)
+  // per-point times of a timed PointCloud2 upload, and the delta gm_odometry_deskew hands k_deskew (12 floats); both
+  // allocated by the first timed upload
+  DevBuf<float> d_time, d_delta;
+  bool scan_timed = false;   // the scan came from gm_upload_pointcloud2_timed: d_time holds its times
+  bool deskew_open = false;  // gm_deskew may still run on it: timed, not deskewed, no gm_crop since the upload
   DevBuf<float4> d_in, d_crop, d_sorted, d_cloud_c;
   DevBuf<float4> d_sorted_valid, d_leaf_bounds;  // inputs of the tile-culled counting (written by k_normals)
   int count_mode = 0;  // 0 = tile-culled when the cell-sorted cloud exists, 1 = always brute force
@@ -743,6 +749,7 @@ static void new_scan(gm_ctx* ctx, size_t n) {
   invalidate_from(ctx, CROP);
   mark(ctx, SCAN);
   ctx->injected = false;
+  ctx->scan_timed = ctx->deskew_open = false;
 }
 
 static gm_status begin_scan(gm_ctx* ctx, size_t n) {
@@ -768,9 +775,18 @@ gm_status gm_upload_scan(gm_ctx* ctx, const float* xyz_host, size_t n, size_t st
   return begin_scan(ctx, n);
 }
 
-gm_status gm_upload_pointcloud2(gm_ctx* ctx, const void* data_host, size_t n, size_t point_step, size_t ox, size_t oy, size_t oz) {
-  if (!ctx || (n && !data_host) || point_step < 4 || ox + 4 > point_step || oy + 4 > point_step || oz + 4 > point_step) return GM_ERR_INVALID_ARG;
+// ot < 0: untimed (gm_upload_pointcloud2); else the float32 time at byte offset ot goes to d_time
+static gm_status upload_pointcloud2(gm_ctx* ctx, const void* data_host, size_t n, size_t point_step, size_t ox, size_t oy, size_t oz, long long ot) {
+  if (!ctx || (n && !data_host) || point_step < 4 || ox + 4 > point_step || oy + 4 > point_step || oz + 4 > point_step ||
+      (ot >= 0 && (size_t)ot + 4 > point_step))
+    return GM_ERR_INVALID_ARG;
   if (n > ctx->cap) { ctx->err = "scan larger than max_points"; return GM_ERR_CAPACITY; }
+  const bool timed = ot >= 0;
+  if (timed && !ctx->d_time) {  // not on the per-scan fast path: only the first timed upload
+    GM_CUDA(cudaStreamSynchronize(ctx->stream));
+    GM_CUDA(ctx->d_time.alloc(ctx->cap));
+    GM_CUDA(ctx->d_delta.alloc(12));
+  }
   if (n) {
     const size_t bytes = n * point_step;
     if (bytes > ctx->d_raw.count) {  // not on the per-scan fast path: only when a larger message arrives
@@ -778,10 +794,62 @@ gm_status gm_upload_pointcloud2(gm_ctx* ctx, const void* data_host, size_t n, si
       GM_CUDA(ctx->d_raw.alloc(ctx->cap * point_step));
     }
     GM_CUDA(cudaMemcpyAsync(ctx->d_raw, data_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    GM_LAUNCH(ctx, k_decode_pointcloud2, div_up((long long)n, 256), 256, ctx->d_raw, (int)n, (int)point_step, (int)ox, (int)oy, (int)oz, ctx->d_in);
+    if (timed)
+      GM_LAUNCH(ctx, k_decode_pointcloud2<true>, div_up((long long)n, 256), 256, ctx->d_raw, (int)n, (int)point_step, (int)ox, (int)oy, (int)oz, ctx->d_in,
+                (int)ot, ctx->d_time);
+    else
+      GM_LAUNCH(ctx, k_decode_pointcloud2<false>, div_up((long long)n, 256), 256, ctx->d_raw, (int)n, (int)point_step, (int)ox, (int)oy, (int)oz, ctx->d_in,
+                0, nullptr);
   }
   ctx->d_scan = ctx->d_in;
-  return begin_scan(ctx, n);
+  gm_status s = begin_scan(ctx, n);
+  if (s == GM_OK) ctx->scan_timed = ctx->deskew_open = timed;
+  return s;
+}
+
+gm_status gm_upload_pointcloud2(gm_ctx* ctx, const void* data_host, size_t n, size_t point_step, size_t ox, size_t oy, size_t oz) {
+  return upload_pointcloud2(ctx, data_host, n, point_step, ox, oy, oz, -1);
+}
+
+gm_status gm_upload_pointcloud2_timed(gm_ctx* ctx, const void* data_host, size_t n, size_t point_step, size_t ox, size_t oy, size_t oz, size_t ot) {
+  if (ot > (size_t)INT32_MAX) return GM_ERR_INVALID_ARG;
+  return upload_pointcloud2(ctx, data_host, n, point_step, ox, oy, oz, (long long)ot);
+}
+
+gm_status gm_download_point_times(gm_ctx* ctx, float* out, size_t capacity_points) {
+  if (!ctx || !out) return GM_ERR_INVALID_ARG;
+  if (!ctx->scan_timed) return GM_ERR_STAGE_ORDER;
+  if (ctx->n_input > capacity_points) return GM_ERR_CAPACITY;
+  if (ctx->n_input) GM_CUDA(cudaMemcpyAsync(out, ctx->d_time, ctx->n_input * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+  GM_CUDA(cudaStreamSynchronize(ctx->stream));
+  return GM_OK;
+}
+
+// gm_deskew's rules (the caller checks the delta): GM_ERR_INVALID_ARG for t_ref or period, GM_ERR_STAGE_ORDER unless
+// the scan may still be deskewed
+static gm_status deskew_check(gm_ctx* ctx, double t_ref, double period) {
+  if (!std::isfinite(t_ref) || !std::isfinite(period) || !(period > 0.0)) return GM_ERR_INVALID_ARG;
+  if (!has(ctx, SCAN) || !ctx->deskew_open) return GM_ERR_STAGE_ORDER;
+  return GM_OK;
+}
+
+// The one launch of k_deskew over the scan, with the delta from the host (delta_dev null) or from device memory.
+static gm_status deskew_launch(gm_ctx* ctx, const Pose34& delta, const float* delta_dev, double t_ref, double period) {
+  const int blocks = std::max(1, std::min(div_up((long long)ctx->n_input, DSK_BLOCK), ctx->num_sms * 16));
+  GM_LAUNCH(ctx, k_deskew, blocks, DSK_BLOCK, ctx->d_st, ctx->d_in, ctx->d_time, delta, delta_dev, t_ref, period);
+  GM_CHECK_LAUNCHES(ctx);
+  ctx->deskew_open = false;
+  return GM_OK;
+}
+
+gm_status gm_deskew(gm_ctx* ctx, const float* delta34, double t_ref, double period) {
+  if (!ctx || !delta34) return GM_ERR_INVALID_ARG;
+  for (int e = 0; e < 12; ++e)
+    if (!std::isfinite(delta34[e])) return GM_ERR_INVALID_ARG;
+  if (gm_status s = deskew_check(ctx, t_ref, period)) return s;
+  Pose34 delta;
+  std::memcpy(delta.r, delta34, sizeof(delta.r));
+  return deskew_launch(ctx, delta, nullptr, t_ref, period);
 }
 
 gm_status gm_set_scan_device(gm_ctx* ctx, const float* xyzw_device, size_t n) {
@@ -804,6 +872,7 @@ gm_status gm_crop(gm_ctx* ctx) {
     GM_CHECK_LAUNCHES(ctx);
   }
   mark(ctx, CROP);
+  ctx->deskew_open = false;
   return GM_OK;
 }
 
@@ -1361,6 +1430,7 @@ static gm_status process_scan_body(gm_ctx* ctx, const int32_t* plane_samples_hos
 static void mark_processed(gm_ctx* ctx, int Hp, int Hc) {
   mark(ctx, CROP, NORMALS, COMPACTED, VOXEL, FRAME, LABELS, POLY);
   ctx->injected = false;
+  ctx->deskew_open = false;
   size_t key_range = 0;  // the VoxelGrid path the replayed gm_voxel took
   voxel_key_bits(ctx, ctx->n_grid, &key_range);
   ctx->vox_assign_on_demand = dense_voxel_path(ctx, key_range);
@@ -3012,6 +3082,18 @@ gm_status gm_odometry_step(gm_odometry* odo, gm_ctx* ctx, const float* delta34) 
   if (archive) GM_CUDA(cudaEventRecord(archive->ev_last, ctx->stream));
   odo->steps = k + 1;
   return GM_OK;
+}
+
+gm_status gm_odometry_deskew(gm_odometry* odo, gm_ctx* ctx, double t_ref, double period) {
+  if (!odo || !ctx) return GM_ERR_INVALID_ARG;
+  gm_map* map = odo->map;
+  const int k = odo->steps;
+  if (k >= odo->p.max_steps) return GM_ERR_CAPACITY;
+  if (ctx->device != map->device) { ctx->err = "gm_odometry_deskew: context and map on different devices"; return GM_ERR_INVALID_ARG; }
+  if (gm_status s = deskew_check(ctx, t_ref, period)) return s;
+  GM_CUDA(cudaStreamWaitEvent(ctx->stream, map->ev_last, 0));  // step k - 1 has written the records k_odom_delta reads
+  GM_LAUNCH(ctx, k_odom_delta, 1, 32, odo->d_rec, k, ctx->d_delta);
+  return deskew_launch(ctx, Pose34{}, ctx->d_delta, t_ref, period);
 }
 
 gm_status gm_odometry_set_window(gm_odometry* odo, int32_t half_cells, gm_map* archive) {

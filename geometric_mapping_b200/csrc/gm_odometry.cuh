@@ -1,7 +1,8 @@
 // gm_odometry.cuh — map odometry on the device (builder-defined: the reference computes no pose).  One step predicts
 // the scan's pose from the trajectory (k_odom_begin), runs gm_register_map's ICP from it (gm_register.cuh), gates the
 // result and records it (k_odom_gate), and inserts the scan at the recorded pose (k_map_insert_gated, gm_map.cuh), all
-// on the context's stream: the pose never travels to the host.
+// on the context's stream: the pose never travels to the host.  k_odom_delta gives gm_odometry_deskew the
+// constant-velocity increment for k_deskew (gm_deskew.cuh).
 // Semantics: include/gm_capi.h (gm_odometry_*).
 #pragma once
 #include "gm_register.cuh"
@@ -68,6 +69,22 @@ __global__ void k_odom_begin(OdomRecord* __restrict__ rec, int k, int mode, Pose
   }
   for (int e = 0; e < 12; ++e) rec[k].guess34[e] = G[e];
   if (st) d_reg_start(st, G, n_source);
+}
+
+// gm_odometry_deskew for step k, one thread: the constant-velocity increment float(P_{k-2}^-1 o P_{k-1}) of
+// k_odom_begin's ODOM_VELOCITY guess, element by element (the identity for k < 2), into delta[12] for k_deskew.
+__global__ void k_odom_delta(const OdomRecord* __restrict__ rec, int k, float* __restrict__ delta) {
+  if (threadIdx.x != 0 || blockIdx.x != 0) return;
+  if (k < 2) {
+    for (int e = 0; e < 12; ++e) delta[e] = (e == 0 || e == 5 || e == 10) ? 1.0f : 0.0f;
+    return;
+  }
+  double P1[12], P2[12], P2i[12], D[12];
+  d_pose_load(rec[k - 1].pose34, P1);
+  d_pose_load(rec[k - 2].pose34, P2);
+  d_pose_inverse(P2, P2i);
+  d_pose_compose(P2i, P1, D);
+  for (int e = 0; e < 12; ++e) delta[e] = (float)D[e];
 }
 
 // Step k, one thread: the gate and record k, and the insert's pose and flag.  st = null: an unregistered step (always

@@ -142,25 +142,33 @@ __global__ void k_begin_scan(DevState* st, int n_input, const float4* scan) {
   }
 }
 
-// PointCloud2 decode: gather the float32 x,y,z fields (byte offsets, arbitrary point_step) into PointXYZ
+// PointCloud2 decode: gather the float32 x,y,z fields (byte offsets, arbitrary point_step) into PointXYZ; TIMED also
+// gathers the float32 field at byte offset ot (the point's time, gm_upload_pointcloud2_timed) into times.  The untimed
+// instantiation ignores the two trailing arguments.
+template <bool TIMED>
 __global__ void k_decode_pointcloud2(const unsigned char* __restrict__ raw, int n, int point_step, int ox, int oy, int oz,
-                                     float4* __restrict__ out) {
+                                     float4* __restrict__ out, int ot, float* __restrict__ times) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const unsigned char* p = raw + (size_t)i * point_step;
-  float v[3];
-  const int off[3] = {ox, oy, oz};
-  if (((point_step | ox | oy | oz) & 3) == 0) {  // aligned records (the usual case: x,y,z,(intensity,ring) float32 fields)
+  constexpr int F = TIMED ? 4 : 3;
+  float v[F];
+  int off[F] = {ox, oy, oz};
+  int align = point_step | ox | oy | oz;
+  if constexpr (TIMED) { off[3] = ot; align |= ot; }
+  if ((align & 3) == 0) {  // aligned records (the usual case: x,y,z,(intensity,ring) float32 fields)
     const float* f = reinterpret_cast<const float*>(p);
     out[i] = make_float4(f[ox >> 2], f[oy >> 2], f[oz >> 2], 1.0f);
+    if constexpr (TIMED) times[i] = f[ot >> 2];
     return;
   }
 #pragma unroll
-  for (int k = 0; k < 3; ++k) {  // byte-wise: fields need not be 4-byte aligned inside the record
+  for (int k = 0; k < F; ++k) {  // byte-wise: fields need not be 4-byte aligned inside the record
     unsigned u = (unsigned)p[off[k]] | ((unsigned)p[off[k] + 1] << 8) | ((unsigned)p[off[k] + 2] << 16) | ((unsigned)p[off[k] + 3] << 24);
     v[k] = __uint_as_float(u);
   }
   out[i] = make_float4(v[0], v[1], v[2], 1.0f);
+  if constexpr (TIMED) times[i] = v[3];
 }
 
 __global__ void k_set_w_one(float4* p, int n) {

@@ -174,6 +174,42 @@ def second_scan(generator, sensor_pose34, seed: int, n: int, **kw) -> np.ndarray
     return view_from(generator(n, seed=seed, **kw), sensor_pose34)
 
 
+def _sweep_motion(delta34, a):
+    """M(a) of gm_deskew (include/gm_capi.h) in float64 for every a: R(a) (n x 3 x 3), rotation along the geodesic, and
+    a * td (n x 3), translation linear."""
+    D = np.asarray(delta34, np.float64)[:3, :4]
+    v = np.array([D[2, 1] - D[1, 2], D[0, 2] - D[2, 0], D[1, 0] - D[0, 1]])
+    nv = float(np.sqrt(v @ v))
+    theta = np.arctan2(nv / 2.0, (np.trace(D[:, :3]) - 1.0) / 2.0) if nv > 0.0 else 0.0
+    u = v / nv if nv > 0.0 else np.zeros(3)
+    a = np.asarray(a, np.float64)
+    phi = a * theta
+    K = np.array([[0.0, -u[2], u[1]], [u[2], 0.0, -u[0]], [-u[1], u[0], 0.0]])
+    R = (np.cos(phi)[:, None, None] * np.eye(3) + np.sin(phi)[:, None, None] * K
+         + (1.0 - np.cos(phi))[:, None, None] * np.outer(u, u))
+    return R, a[:, None] * D[:, 3]
+
+
+def swept_view(points: np.ndarray, sensor_pose34, delta34, period: float, t_ref: float = 0.0):
+    """The scene points `points` (world frame) as a spinning sensor sees them during one sweep: point i is taken at time
+    t_i = period * (azimuth + pi) / (2 pi) (float32 seconds, azimuth of the point seen from sensor_pose34) from the pose
+    sensor_pose34 o M(a_i), a_i = (t_i - t_ref) / period, where M is gm_deskew's interpolation of delta34 (the motion over
+    one period).  -> (n x 3 float64 sensor coordinates, t).  t_ref is the time at which the sensor is at sensor_pose34;
+    at period -> 0 this is view_from."""
+    T = np.asarray(sensor_pose34, np.float64)
+    snap = (np.asarray(points, np.float64)[:, :3] - T[:, 3]) @ T[:, :3]
+    t = (period * (np.arctan2(snap[:, 1], snap[:, 0]) + np.pi) / (2.0 * np.pi)).astype(np.float32)
+    R, at = _sweep_motion(delta34, (t.astype(np.float64) - t_ref) / period)
+    return np.einsum("nji,nj->ni", R, snap - at), t      # M(a)^-1 applied to the snapshot point: R(a)^T (p - a td)
+
+
+def swept_scan(generator, sensor_pose34, delta34, period: float, seed: int, n: int, t_ref: float = 0.0, **kw):
+    """A new draw of the scene of `generator` (`seed`) seen by a spinning sensor at sensor_pose34 (at time t_ref) that
+    moves by delta34 per period (swept_view).  -> (n x 4 float32 points, n float32 times)."""
+    q, t = swept_view(generator(n, seed=seed, **kw), sensor_pose34, delta34, period, t_ref)
+    return _xyzw(q[:, 0], q[:, 1], q[:, 2]), t
+
+
 def sample_draws(K: int, H: int, per: int, seed: int = 7) -> np.ndarray:
     """K x H x per uint32 draws for gm_extract_primitives, Philox(seed): round r maps draw u to the sample index
     R_r[(u * n_r) >> 32] of the points still unclaimed."""

@@ -223,6 +223,40 @@ GM_API gm_status gm_upload_pointcloud2(gm_ctx* ctx, const void* data_host, size_
 /* Scan already resident in HBM as n x float4 (not copied; must outlive the processing calls). */
 GM_API gm_status gm_set_scan_device(gm_ctx* ctx, const float* xyzw_device, size_t n);
 
+/* ---- per-point times and deskew (builder-defined: the reference treats every scan as a snapshot) -------------------
+ * A spinning lidar takes a sweep over a scan period (typically 0.1 s) while it moves: at 1.5 m/s a point at the end of a
+ * 10 Hz sweep is 15 cm from where a snapshot would put it.
+ * gm_upload_pointcloud2_timed is gm_upload_pointcloud2 plus the float32 field at byte offset offset_t (offset_t + 4 <=
+ *   point_step): each point's time in seconds, as velodyne_pointcloud publishes it (PointXYZIRT::time).  The times are
+ *   decoded on the device from the same staged bytes; the first timed upload allocates their buffer (4 bytes a point).
+ *   Every other upload (gm_upload_scan, gm_upload_pointcloud2, gm_set_scan_device, gm_inject_compacted) gives an untimed
+ *   scan.  gm_download_point_times copies the n decoded times of a timed scan (GM_ERR_STAGE_ORDER for an untimed one) and
+ *   synchronises the ctx stream like the other downloads.
+ * gm_deskew rewrites the uploaded scan in place, before gm_crop: every point is expressed in the sensor frame at time t_ref,
+ *   the sensor moving by delta34 over period seconds at constant velocity.  delta34 (row-major [R | t]) is the motion from
+ *   the previous scan's frame to this scan's frame, in the previous scan's frame (gm_odometry_step's delta34).
+ *   Constants, in double from D = double(delta34):
+ *     v = (R21 - R12, R02 - R20, R10 - R01),  theta = atan2(|v| / 2, (R00 + R11 + R22 - 1) / 2),  u = v / |v|,
+ *     td = (D[3], D[7], D[11]);  |v| = 0 gives theta = 0 and u = 0 (the identity rotation).
+ *   Per point i, in double:
+ *     a = ((double)t_i - t_ref) / period,  phi = a * theta,
+ *     R(a) = cos(phi) I + sin(phi) [u]x + (1 - cos(phi)) u u^T,
+ *     p' = R(a) p + a td,  stored as float(p') with w = 1.
+ *   The rotation is interpolated along the geodesic and the translation linearly (the decoupled form); a = 1 gives delta34
+ *   itself.  A motion near 180 degrees within one period is not supported (theta is taken from the trace and |v|).
+ *   Exact cases: an identity delta34, or a point with t_i == t_ref, leaves the point's coordinates unchanged (a zero
+ *   coordinate may change its sign); a point with a non-finite coordinate or time becomes (NaN, NaN, NaN, 1), which the
+ *   stages then treat as any NaN input point (gm_crop's is_dense rule).
+ *   One launch (k_deskew), no host synchronisation: each block derives the constants, the point count is read on the
+ *   device.  gm_process_scan and its CUDA graphs read the deskewed scan as any uploaded one.
+ *   Rules: GM_ERR_INVALID_ARG, with nothing launched, for a NULL or non-finite delta34, a non-finite t_ref, or period <= 0
+ *   or non-finite; GM_ERR_STAGE_ORDER for an untimed scan, after gm_crop (or gm_process_scan) of this upload, and for a
+ *   second gm_deskew / gm_odometry_deskew of the same upload (deskewing twice is almost always a bug). */
+GM_API gm_status gm_upload_pointcloud2_timed(gm_ctx* ctx, const void* data_host, size_t n, size_t point_step,
+                                             size_t offset_x, size_t offset_y, size_t offset_z, size_t offset_t);
+GM_API gm_status gm_download_point_times(gm_ctx* ctx, float* out, size_t capacity_points);
+GM_API gm_status gm_deskew(gm_ctx* ctx, const float* delta34, double t_ref, double period);
+
 /* ---- stages ---------------------------------------------------------------------------- */
 /* chopCloud(bound, cloud): src/tunnel_processing.cpp:39-49, called src/geometric_mapping.cpp:57 */
 GM_API gm_status gm_crop(gm_ctx* ctx);
@@ -677,6 +711,20 @@ GM_API gm_status gm_odometry_create(gm_map* map, const gm_odometry_params* p, gm
 GM_API void gm_odometry_destroy(gm_odometry* odo);
 GM_API gm_status gm_odometry_step(gm_odometry* odo, gm_ctx* ctx, const float* delta34 /* NULL = constant velocity */);
 GM_API gm_status gm_odometry_set_window(gm_odometry* odo, int32_t half_cells /* 0 = off, the default */, gm_map* archive /* may be NULL */);
+/* gm_odometry_deskew: gm_deskew of ctx's timed scan, the one the next gm_odometry_step (step k = gm_odometry_steps()) will
+ * take, with the constant-velocity increment of the trajectory in device memory as the delta:
+ *     delta = float(P_{k-2}^-1 o P_{k-1}) element by element (the guess's composition and order, above); the identity
+ *     for k < 2, which leaves the points unchanged.
+ * Launches: k_odom_delta (one thread, writes the 12 floats to ctx's delta slot), then gm_deskew's k_deskew reading them:
+ *   gm_launch_count(ctx) grows by 2, with no host synchronisation.  The results are those of gm_deskew with that delta.
+ * Ordering: it waits on ctx's stream for the map's last operation, i.e. for step k - 1 from whichever context issued it
+ *   (the records it reads).  The cost: with two contexts taking turns, scan k's crop, normals and voxel stages can no
+ *   longer overlap step k - 1's registration.  A caller with an IMU or wheel odometry calls gm_deskew with that delta
+ *   instead and keeps the overlap.
+ * Rules: those of gm_deskew for ctx, t_ref and period; GM_ERR_INVALID_ARG for a context on another device than the map;
+ *   GM_ERR_CAPACITY when k >= max_steps.  Nothing is launched when a call is refused. */
+#define GM_ODOMETRY_DESKEW_LAUNCHES 2
+GM_API gm_status gm_odometry_deskew(gm_odometry* odo, gm_ctx* ctx, double t_ref, double period);
 GM_API int32_t gm_odometry_steps(const gm_odometry* odo);  /* steps issued so far (host counter, no synchronisation) */
 /* the records of every step issued so far, in step order; *n = their number.  Waits for the last of them.  out = NULL: *n only */
 GM_API gm_status gm_odometry_get(gm_odometry* odo, gm_odometry_record* out, int32_t capacity, int32_t* n);
